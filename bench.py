@@ -2,7 +2,7 @@
 """Benchmark of the B200 segment-graph construction path (BASELINE.json metric: read pairs/s through
 segment-graph build, with % of HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: BuildNode_STAR + BuildEdges + breakpoint coverage on
 synthetic sorted alignment records of the configs[1] shape (GRCh38 layout, ~0.5 % discordant, SURVEY App. C block mix K = 1.35).
@@ -65,6 +65,23 @@ def output_crcs(nodes, edges, chim_blocks, cov) -> dict:
     nd = np.stack([nodes.Chr, nodes.Position, nodes.Length, nodes.Support], axis=1).astype(np.int32)
     return {"nodes": c(nd), "avgdepth": c(np.asarray(nodes.AvgDepth, np.float64)), "edges": c(edges.table()), "chim_after_edges": c(np.asarray(chim_blocks, np.int32)),
             "coverage": c(np.asarray(cov, np.int32)), "n_nodes": int(nd.shape[0]), "n_edges": int(edges.Ind1.shape[0]), "n_bp": int(np.asarray(cov).shape[0])}
+
+
+DUMP_BYTES_PER_ARRAY = 12 << 20  # five arrays: at most 60 MB in all
+
+
+def dump_outputs(outdir: str, nodes, edges, chim_blocks, cov) -> None:
+    """Writes the outputs of one step as float64 .npy files (exact for their int32 values), in the layout of output_crcs().
+    An array larger than DUMP_BYTES_PER_ARRAY is replaced by a fixed sample of its rows (seed 0, original order), which
+    depends on the row count only, so two builds that agree on the count dump the same rows."""
+    os.makedirs(outdir, exist_ok=True)
+    arrays = {"nodes": np.stack([nodes.Chr, nodes.Position, nodes.Length, nodes.Support], axis=1), "avgdepth": np.asarray(nodes.AvgDepth),
+              "edges": edges.table(), "chim_after_edges": np.asarray(chim_blocks), "coverage": np.asarray(cov)}
+    for name, a in arrays.items():
+        a = np.asarray(a, np.float64)
+        if a.nbytes > DUMP_BYTES_PER_ARRAY:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_BYTES_PER_ARRAY // a[:1].nbytes, replace=False))]
+        np.save(os.path.join(outdir, name + ".npy"), a)
 
 
 def pinned_crcs(pairs: int, seed: int):
@@ -372,6 +389,7 @@ def main():
     ap.add_argument("--pairs", type=int, default=DEFAULT_PAIRS, help="read pairs per GPU")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (resident batch) as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0)); world = int(os.environ.get("WORLD_SIZE", 1)); local = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -541,6 +559,9 @@ def main():
 
     sec, phases, clocks, launches = timed("resident", args.steps, args.warmup)
     timeline = dict(state["timeline_ms"])
+    if args.dump_outputs and rank == 0:
+        nodes_l, edges_l, cov_l = state["last"]
+        dump_outputs(args.dump_outputs, nodes_l, edges_l, state["chim"].block_table(), cov_l)
     if world > 1:
         print("[rank %d] resident step %.1f ms; host timeline %s" % (rank, 1e3 * sec, {k: round(v, 1) for k, v in timeline.items()}), file=sys.stderr, flush=True)
     # end to end from host memory: the wire form (13 + 8 B, what a front end hands over; packed once, outside the timed region, its

@@ -91,7 +91,7 @@ def run_restate(conc_sqmb: str, chim_sqmb: str, outdir: str, bps=None, opts=None
     if bps is not None:
         bf = os.path.join(outdir, "bps_in.bin")
         np.ascontiguousarray(bps, dtype=np.int32).reshape(-1, 2).tofile(bf)
-    o = (C.c_int * 6)(*(opts if opts is not None else (1, 10, 4, -1, 50000, 20)))
+    o = (C.c_int * 6)(*(opts if opts is not None else restate_opts()))
     rc = lib.sqo_run(conc_sqmb.encode(), chim_sqmb.encode(), outdir.encode(), o, bf.encode() if bf else None, stop_after)
     if rc != 0:
         raise RuntimeError("sqo_run failed rc=%d" % rc)
@@ -99,6 +99,60 @@ def run_restate(conc_sqmb: str, chim_sqmb: str, outdir: str, bps=None, opts=None
     cp = os.path.join(outdir, "cov_i32.bin")
     d["cov"] = np.fromfile(cp, dtype=np.int32) if os.path.exists(cp) else None
     return d
+
+
+_RESTATE_FLAGS = {"-pt": 0, "-pl": 1, "-pm": 2, "-mq": 3, "-dp": 4, "-di": 5}  # the reference's options (Config.cpp:18-25) -> sqo_run opts
+
+
+def restate_opts(extra_args=()) -> list:
+    o = [1, 10, 4, -1, 50000, 20]
+    args = list(extra_args)
+    if len(args) % 2 or any(f not in _RESTATE_FLAGS for f in args[::2]):
+        raise ValueError("the restatement takes only %s, each with a value: %s" % (sorted(_RESTATE_FLAGS), args))
+    for f, v in zip(args[::2], args[1::2]):
+        o[_RESTATE_FLAGS[f]] = int(v)
+    return o
+
+
+def components(n: int, a, b) -> np.ndarray:
+    """Connected-component label per node, components numbered in the order of their smallest node (SegmentGraph.cpp:2986-3003)."""
+    parent = list(range(n))
+
+    def root(x):
+        while parent[x] != x:
+            parent[x] = parent[parent[x]]
+            x = parent[x]
+        return x
+    for x, y in zip(np.asarray(a).tolist(), np.asarray(b).tolist()):
+        rx, ry = root(x), root(y)
+        if rx != ry:
+            parent[max(rx, ry)] = min(rx, ry)
+    label, out = {}, np.empty(n, np.int32)
+    for x in range(n):
+        out[x] = label.setdefault(root(x), len(label))
+    return out
+
+
+def run_restated(conc_sqmb: str, chim_sqmb: str, outdir: str, extra_args=(), timeout: float = None) -> dict:
+    """run() where the reference build is absent: the same dumps from the CPU restatement, which the committed golden dumps
+    pin to the reference.  The host stages between BuildEdges and ExactBPConcordantSupport (filters, CompressNode,
+    ExactBreakpoint) are not restated, so the final graph is every segment and every edge, without exact breakpoints: each
+    edge is covered at its two segment ends.  Writes labels_i32.bin of that graph like the reference harness."""
+    opts = restate_opts(extra_args)
+    d = run_restate(conc_sqmb, chim_sqmb, outdir, opts=opts, stop_after=3)
+    d["final_nodes"], d["final_edges"], d["exactbp"] = d["nodes"], d["edges"], np.zeros((0, 6), np.int32)
+    bps = breakpoints_of(d)
+    cov = run_restate(conc_sqmb, chim_sqmb, outdir, bps=bps, opts=opts)["cov"]
+    sup = support_from_cov(d, bps, cov)
+    d["support"] = np.array([k + c for k, v in sup.items() for c in v], np.int32).reshape(-1, 6)
+    components(d["nodes"].shape[0], d["edges"][:, 0], d["edges"][:, 1]).tofile(os.path.join(outdir, "labels_i32.bin"))
+    return d
+
+
+class Restated:
+    """The oracle interface of this module (run, load_dumps) backed by the CPU restatement."""
+    run = staticmethod(run_restated)
+    load_dumps = staticmethod(load_dumps)
 
 
 def breakpoints_of(d: dict) -> np.ndarray:

@@ -15,9 +15,9 @@ CASES = ["bwa_chr17_3k", "bwa_fourchr_6k"]
 
 
 @pytest.mark.parametrize("case", CASES)
-def test_reference_build_reproduces_bwa_golden(case, ref_oracle, tmp_path):
-    got = ref_oracle.run(os.path.join(GOLD, case, "all.sqmb"), "-", str(tmp_path), extra_args=("--bwa",))
-    want = ref_oracle.load_dumps(os.path.join(GOLD, case, "ref"))
+def test_reference_build_reproduces_bwa_golden(case, reference_build, tmp_path):
+    got = reference_build.run(os.path.join(GOLD, case, "all.sqmb"), "-", str(tmp_path), extra_args=("--bwa",))
+    want = reference_build.load_dumps(os.path.join(GOLD, case, "ref"))
     for k in ("nodes", "avgdepth", "edges", "chim_after_edges", "final_nodes", "final_edges", "exactbp", "support"):
         assert want[k].shape == got[k].shape and np.array_equal(want[k], got[k]), k
     assert got["read_len"] == want["read_len"] == 100

@@ -36,19 +36,19 @@ def test_restatement_decoder_kat(tmp_path):
 
 
 @pytest.mark.parametrize("case", CASES)
-def test_reference_build_reproduces_golden(case, tmp_path, ref_oracle):
+def test_reference_build_reproduces_golden(case, tmp_path, reference_build):
     """The goldens are what oracle/_ref produces today (guards against stale fixtures)."""
     g = _gold(case)
-    r = ref_oracle.run(os.path.join(GOLD, case, "conc.sqmb"), os.path.join(GOLD, case, "chim.sqmb"), str(tmp_path))
+    r = reference_build.run(os.path.join(GOLD, case, "conc.sqmb"), os.path.join(GOLD, case, "chim.sqmb"), str(tmp_path))
     common.assert_same(g, r, ("chim_loaded", "nodes", "avgdepth", "edges", "chim_after_edges", "final_nodes", "final_edges", "exactbp", "support"))
 
 
 @pytest.mark.parametrize("seed,n,disc,ref_len", [(101, 4000, 0.05, None), (202, 20000, 0.01, [3000000, 2000000, 500000, 16569]), (303, 30000, 0.02, "grch38")])
-def test_restatement_matches_reference_on_fuzz(seed, n, disc, ref_len, tmp_path, ref_oracle):
+def test_restatement_matches_reference_on_fuzz(seed, n, disc, ref_len, tmp_path, reference_build):
     from squid_b200 import synth
     rl = synth.GRCH38_LEN if ref_len == "grch38" else ref_len
     cp, hp, *_ = common.write_case(str(tmp_path), n, seed, disc, rl)
-    r = ref_oracle.run(cp, hp, str(tmp_path / "ref"))
+    r = reference_build.run(cp, hp, str(tmp_path / "ref"))
     bps = pyref.breakpoints_of(r)
     me = pyref.run_restate(cp, hp, str(tmp_path / "me"), bps=bps)
     common.assert_same(r, me, ("chim_loaded", "nodes", "avgdepth", "edges", "chim_after_edges"))
@@ -62,11 +62,11 @@ def test_restatement_matches_reference_on_fuzz(seed, n, disc, ref_len, tmp_path,
     # is 'J', above every synthetic quality, so every read has a low-phred run -- with offset 33 it would be '+'
     ((0, 10, 10, -1, 50000, 20), ["-pt", "0", "-pm", "10"]),
 ])
-def test_restatement_matches_reference_with_options(opts, args, tmp_path, ref_oracle):
+def test_restatement_matches_reference_with_options(opts, args, tmp_path, reference_build):
     """The -mq / -pl / -pm / -dp / -di rules (Config.cpp:18-25) on both sides; the options must change the outputs."""
     cp, hp, *_ = common.write_case(str(tmp_path), 20000, 47, 0.03)
-    base = ref_oracle.run(cp, hp, str(tmp_path / "ref0"))
-    r = ref_oracle.run(cp, hp, str(tmp_path / "ref"), extra_args=args)
+    base = reference_build.run(cp, hp, str(tmp_path / "ref0"))
+    r = reference_build.run(cp, hp, str(tmp_path / "ref"), extra_args=args)
     assert not (np.array_equal(r["edges"], base["edges"]) and pyref.support_map(r) == pyref.support_map(base))
     bps = pyref.breakpoints_of(r)
     me = pyref.run_restate(cp, hp, str(tmp_path / "me"), bps=bps, opts=opts)
@@ -78,10 +78,10 @@ def test_restatement_matches_reference_with_options(opts, args, tmp_path, ref_or
     (30000, 37, 0.2, dict(n_genes=100, fusion_support=20)),
     (20000, 36, 0.05, dict(n_genes=20, fusion_support=20, exon_len=(20, 170), intron_len=(60, 400))),
 ])
-def test_restatement_matches_reference_with_short_blocks(n, seed, disc, kw, tmp_path, ref_oracle):
+def test_restatement_matches_reference_with_short_blocks(n, seed, disc, kw, tmp_path, reference_build):
     """min_block=1: aligned blocks of 1-3 bp are left in (the generators' default drops them)."""
     cp, hp, *_ = common.write_case(str(tmp_path), n, seed, disc, None, min_block=1, **kw)
-    r = ref_oracle.run(cp, hp, str(tmp_path / "ref"))
+    r = reference_build.run(cp, hp, str(tmp_path / "ref"))
     bps = pyref.breakpoints_of(r)
     me = pyref.run_restate(cp, hp, str(tmp_path / "me"), bps=bps)
     common.assert_same(r, me, ("chim_loaded", "nodes", "avgdepth", "edges", "chim_after_edges"))

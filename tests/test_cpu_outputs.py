@@ -73,12 +73,12 @@ def test_twins_match_golden_outputs(case, n_ref, built_lib, tmp_path):
     (40000, 61, 0.05, dict(n_genes=40, fusion_support=30)),
     (25000, 62, 0.1, dict(n_genes=12, fusion_support=60)),
 ])
-def test_twins_match_reference_on_fresh_cases(n, seed, disc, kw, built_lib, ref_oracle, tmp_path):
+def test_twins_match_reference_on_fresh_cases(n, seed, disc, kw, built_lib, reference_build, tmp_path):
     """Denser graphs than the goldens: several breakpoint pairs per edge (CountTop's top-5 and its extreme-position fallback),
     ties in the weight sort of WriteBEDPE, tens of BEDPE lines."""
     from squid_b200 import synth
     ref_len = [30000000, 20000000, 5000000, 16569]
     cp, hp, *_ = common.write_case(str(tmp_path), n, seed, disc, ref_len, **kw)
-    ref_oracle.run(cp, hp, str(tmp_path / "ref"), extra_args=("--write-outputs",))
+    reference_build.run(cp, hp, str(tmp_path / "ref"), extra_args=("--write-outputs",))
     lines = _check_dir(str(tmp_path / "ref"), tmp_path, len(ref_len), min_sv_lines=3)
     print("sv lines", lines)

@@ -33,9 +33,9 @@ def dropin_bin(built_lib):
     (60000, 71, 0.04, [30000000, 20000000, 5000000, 16569], dict(n_genes=60, fusion_support=25), []),
     (40000, 72, 0.08, None, dict(n_genes=25, fusion_support=40), ["-mq", "3", "-pl", "25", "-dp", "3000", "-di", "2"]),
 ])
-def test_dropin_writes_the_reference_files(n, seed, disc, ref_len, kw, extra, dropin_bin, ref_oracle, tmp_path):
+def test_dropin_writes_the_reference_files(n, seed, disc, ref_len, kw, extra, reference_build, dropin_bin, tmp_path):
     cp, hp, *_ = common.write_case(str(tmp_path), n, seed, disc, ref_len, **kw)
-    ref_oracle.run(cp, hp, str(tmp_path / "ref"), extra_args=["--write-outputs"] + extra)
+    reference_build.run(cp, hp, str(tmp_path / "ref"), extra_args=["--write-outputs"] + extra)
     out = str(tmp_path / "ours")
     os.makedirs(out)
     r = subprocess.run([dropin_bin, cp, hp, out, "--quiet", "--write-outputs"] + extra, capture_output=True, text=True, timeout=600)
