@@ -81,7 +81,8 @@ def build_restate() -> None:
 
 
 def run_restate(conc_sqmb: str, chim_sqmb: str, outdir: str, bps=None, opts=None, stop_after: int = 0) -> dict:
-    """Runs the CPU restatement; `bps` = sorted (chr,pos) int array for the coverage pass.  Same dump layout as run()."""
+    """Runs the CPU restatement; `bps` = sorted (chr,pos) int array for the coverage pass.  Same dump layout as run().
+    stop_after: 0 = everything, 1/2/3 = stop after the chimeric loader / nodes / edges, -1 = the coverage pass alone."""
     import ctypes as C
     build_restate()
     lib = C.CDLL(RESTATE_LIB)

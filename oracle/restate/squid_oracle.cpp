@@ -697,7 +697,8 @@ static std::vector<int32_t> chim_rows(const std::vector<Rd> &c) {
 }  // namespace
 
 // opts: {phred33, max_lowphred_len, min_phred, min_mapq, concord_dist_pos, concord_dist_idx}; bps_file may be NULL.
-// stop_after: 0 = everything, 1 = chimeric loader only, 2 = nodes, 3 = edges.  Returns 0, or <0 on I/O error.
+// stop_after: 0 = everything, 1 = chimeric loader only, 2 = nodes, 3 = edges, -1 = the coverage pass alone (it reads neither
+// segments nor edges; a stream too short to trigger a segment group can still be covered).  Returns 0, or <0 on I/O error.
 extern "C" int sqo_run(const char *conc_path, const char *chim_path, const char *outdir, const int *opts, const char *bps_file, int stop_after) {
     SqmbView conc, chim;
     if (!conc.open(conc_path) || !chim.open(chim_path)) return -1;
@@ -714,23 +715,25 @@ extern "C" int sqo_run(const char *conc_path, const char *chim_path, const char 
     }
     dump(d + "/readlen.bin", std::vector<int32_t>{g.o.read_len});
     if (stop_after == 1) return 0;
-    g.build_nodes(conc, cr);
-    {
-        std::vector<int32_t> a;
-        std::vector<double> dep;
-        for (const Node &n : g.nodes) { a.push_back(n.chr); a.push_back(n.pos); a.push_back(n.len); a.push_back(n.support); dep.push_back(n.depth); }
-        dump(d + "/nodes_i32.bin", a);
-        FILE *f = fopen((d + "/nodes_f64.bin").c_str(), "wb");
-        if (f) { if (!dep.empty()) fwrite(dep.data(), 8, dep.size(), f); fclose(f); }
+    if (stop_after >= 0) {
+        g.build_nodes(conc, cr);
+        {
+            std::vector<int32_t> a;
+            std::vector<double> dep;
+            for (const Node &n : g.nodes) { a.push_back(n.chr); a.push_back(n.pos); a.push_back(n.len); a.push_back(n.support); dep.push_back(n.depth); }
+            dump(d + "/nodes_i32.bin", a);
+            FILE *f = fopen((d + "/nodes_f64.bin").c_str(), "wb");
+            if (f) { if (!dep.empty()) fwrite(dep.data(), 8, dep.size(), f); fclose(f); }
+        }
+        if (stop_after == 2) return 0;
+        g.build_edges(conc, cr);
+        {
+            std::vector<int32_t> a;
+            for (const Edge &e : g.edges) { a.push_back(e.a); a.push_back(e.b); a.push_back(e.ha); a.push_back(e.hb); a.push_back(e.w); }
+            dump(d + "/edges_i32.bin", a);
+        }
+        dump(d + "/chim_after_edges.bin", chim_rows(cr));
     }
-    if (stop_after == 2) return 0;
-    g.build_edges(conc, cr);
-    {
-        std::vector<int32_t> a;
-        for (const Edge &e : g.edges) { a.push_back(e.a); a.push_back(e.b); a.push_back(e.ha); a.push_back(e.hb); a.push_back(e.w); }
-        dump(d + "/edges_i32.bin", a);
-    }
-    dump(d + "/chim_after_edges.bin", chim_rows(cr));
     if (stop_after == 3 || !bps_file) return 0;
     std::vector<std::pair<int, int>> bps;
     FILE *f = fopen(bps_file, "rb");

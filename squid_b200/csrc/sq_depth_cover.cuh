@@ -105,6 +105,14 @@ SQ_HD int32_t cover_start(uint16_t f, int32_t rid, int32_t pos, int32_t mrid, in
     return (flag_mate_mapped(f) && mrid == rid) ? mpos : pos;
 }
 SQ_HD uint64_t chrpos_key(int32_t chr, int32_t pos) { return ((uint64_t)(uint32_t)(chr + 1) << 32) | (uint32_t)pos; }
+// indBP threshold (:3157): a qualifying record passes breakpoint (chr, pos) when its start key exceeds this key.  The reference
+// compares `start > pos + Concord_Dist_Pos` as ints, so with a negative -dp near a chromosome start every record of that
+// chromosome passes; the key then sits just below the chromosome's position 0 (cast to uint32, the negative sum would lie above
+// every record of the chromosome and stall indBP).  Sums above INT32_MAX overflow in the reference itself and are not handled.
+SQ_HD uint64_t cover_pass_key(int32_t chr, int32_t pos, int32_t dist) {
+    const int64_t s = (int64_t)pos + dist;
+    return s < 0 ? chrpos_key(chr, 0) - 1 : chrpos_key(chr, (int32_t)s);
+}
 
 // first index in [lo,hi) with a[i] >= v (uint64 keys)
 SQ_HD int64_t lower_bound_u64(const uint64_t *a, int64_t lo, int64_t hi, uint64_t v) {

@@ -48,7 +48,7 @@ __global__ void k_cov_r0_tiles(const uint64_t *qkey, const CovTile *tiles, int32
     const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (k >= K) return;
     bpkey[k] = chrpos_key(bp_chr[k], bp_pos[k]);
-    const uint64_t T = chrpos_key(bp_chr[k], bp_pos[k] + dist);
+    const uint64_t T = cover_pass_key(bp_chr[k], bp_pos[k], dist);
     int32_t lo = 0, hi = n_tiles;  // first tile whose inclusive maximum exceeds T
     while (lo < hi) { const int32_t m = (lo + hi) >> 1; if (tiles[m].incmax <= T) lo = m + 1; else hi = m; }
     int64_t v = nq;

@@ -583,7 +583,7 @@ __global__ void k_cov_r0(const uint64_t *M, int64_t nq, const int32_t *bp_chr, c
     const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (k >= K) return;
     bpkey[k] = chrpos_key(bp_chr[k], bp_pos[k]);
-    const uint64_t T = chrpos_key(bp_chr[k], bp_pos[k] + dist);
+    const uint64_t T = cover_pass_key(bp_chr[k], bp_pos[k], dist);
     const int64_t v = upper_bound_u64(M, 0, nq, T);  // first qualifying rank whose running-max key exceeds T
     r0[k] = v;
     t[k] = v - k;  // max-plus form of t[k] = max(r0[k], t[k-1]+1)
@@ -599,7 +599,7 @@ __global__ void k_cov_verify(const uint64_t *qkey, int64_t nq, const int32_t *bp
     const int64_t c = t[k] + k;  // candidate rank
     t[k] = c;
     if (c != r0[k] && c < nq) {  // lag mode: the qualifying record right after t[k-1] must itself pass breakpoint k
-        const uint64_t T = chrpos_key(bp_chr[k], bp_pos[k] + dist);
+        const uint64_t T = cover_pass_key(bp_chr[k], bp_pos[k], dist);
         if (!(qkey[c] > T)) *fail = 1;
     }
 }
@@ -652,7 +652,7 @@ __global__ void k_cov_chain(const uint64_t *qkey, int64_t nq, const int32_t *bp_
     for (int64_t kb = k_begin; kb < K; kb += 32) {
         const int64_t k = kb + lane;
         const int64_t my_r0 = k < K ? r0[k] : nq;
-        const uint64_t my_T = k < K ? chrpos_key(bp_chr[k], bp_pos[k] + dist) : ~0ull;
+        const uint64_t my_T = k < K ? cover_pass_key(bp_chr[k], bp_pos[k], dist) : ~0ull;
         int64_t my_t = 0;
         const int cnt = (int)((K - kb) < 32 ? (K - kb) : 32);
         for (int j = 0; j < cnt; j++) {

@@ -40,6 +40,7 @@ int main(int argc, char **argv) {
     if (argc < 4) { fprintf(stderr, "usage: %s conc.sqmb chim.sqmb outdir [bps.bin]\n", argv[0]); return 2; }
     outdir = argv[3];
     sqh::HostConfig cfg;
+    if (getenv("SQ_EMUL_DP")) cfg.concord_dist_pos = atoi(getenv("SQ_EMUL_DP"));  // -dp (Concord_Dist_Pos)
     SqmbView conc, chim;
     if (!conc.open(argv[1]) || !chim.open(argv[2])) { fprintf(stderr, "cannot open inputs\n"); return 2; }
     std::vector<sqh::Read> reads;
@@ -462,7 +463,7 @@ int main(int argc, char **argv) {
         std::vector<int64_t> t(K);
         int64_t tp = -1;
         for (int64_t k = 0; k < K; k++) {
-            const uint64_t T = chrpos_key(bp[2 * k], bp[2 * k + 1] + p.concord_dist_pos);
+            const uint64_t T = cover_pass_key(bp[2 * k], bp[2 * k + 1], p.concord_dist_pos);
             int64_t r0 = upper_bound_u64(M.data(), 0, n, T);
             int64_t c = r0 > tp ? r0 : tp + 1;
             while (c < n && !(q[c] && key[c] > T)) c++;

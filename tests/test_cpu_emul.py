@@ -15,14 +15,8 @@ GOLD = os.path.join(ROOT, "tests", "golden")
 
 
 @pytest.fixture(scope="module")
-def emul_bin():
-    out = os.path.join(ROOT, "tests", "emul", "_build", "emul")
-    os.makedirs(os.path.dirname(out), exist_ok=True)
-    srcs = ["tests/emul/emul_main.cpp", "squid_b200/csrc/host/readrec.cpp", "squid_b200/csrc/host/chimeric.cpp", "squid_b200/csrc/host/prepass.cpp"]
-    cmd = ["g++", "-std=c++17", "-O2", "-fopenmp", "-I", "include", "-I", "squid_b200/csrc", "-o", out] + srcs + ["-lpthread"]
-    r = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-3000:]
-    return out
+def emul_bin(tmp_path_factory):
+    return common.build_emul(tmp_path_factory.mktemp("emul"))
 
 
 @pytest.mark.parametrize("case", ["chr17_3k", "fourchr_6k"])
@@ -72,3 +66,43 @@ def test_stepped_rules_with_short_blocks(n, seed, disc, ref_len, kw, dense, emul
     common.assert_same(g, me, ("nodes", "avgdepth", "edges", "chim_after_edges"))
     cov = np.fromfile(str(tmp_path / "emu" / "cov_i32.bin"), dtype=np.int32)
     assert pyref.support_from_cov(g, bps, cov) == pyref.support_map(g)
+
+
+@pytest.fixture(scope="module")
+def cov_case(tmp_path_factory):
+    """Four chromosomes (one of 16569 bp), 30 k pairs, and the breakpoint list families of common.bp_families on its restated graph."""
+    d = str(tmp_path_factory.mktemp("cov_case"))
+    ref_len = [3000000, 2000000, 500000, 16569]
+    cp, hp, conc, _, _ = common.write_case(d, 30000, 29, 0.05, ref_len, n_genes=20)
+    g = pyref.run_restate(cp, hp, os.path.join(d, "graph"), stop_after=3)
+    g["final_nodes"], g["final_edges"], g["exactbp"] = g["nodes"], g["edges"], np.zeros((0, 6), np.int32)
+    fam = common.bp_families(ref_len, g["nodes"], conc, 29)
+    fam["segment_ends"] = pyref.breakpoints_of(g)
+    return cp, hp, ref_len, fam
+
+
+@pytest.mark.parametrize("dp", [50000, 0, 3000, 100000000, -100, -5000])
+@pytest.mark.parametrize("family", ["segment_ends", "uniform", "dups", "dense", "before", "after", "one", "empty"])
+def test_coverage_chain_matches_restatement(cov_case, family, dp, emul_bin, tmp_path):
+    """The stepped coverage rules (r0 over running maxima, the literal indBP chain, the count) against the literal BAM pass of the
+    restatement (SegmentGraph.cpp:3124-3166) on the same list, at several -dp.  Every list also holds breakpoints at 0, 1, 99 and
+    4999 of every chromosome (except the lists whose shape that would change): with a negative -dp, pos + dist < 0 there and every
+    record of the chromosome passes the breakpoint."""
+    cp, hp, ref_len, fam = cov_case
+    bps = fam[family]
+    if family not in ("before", "after", "one", "empty"):
+        bps = common.bp_array(np.concatenate([bps, common.chr_start_bps(ref_len)]))
+    if family == "before":
+        assert bps.shape[0] > 0
+    want = pyref.run_restate(cp, hp, str(tmp_path / "ref"), bps=bps, opts=pyref.restate_opts(["-dp", str(dp)]))
+    bps.tofile(str(tmp_path / "bps.bin"))
+    os.makedirs(str(tmp_path / "emu"))
+    r = subprocess.run([emul_bin, cp, hp, str(tmp_path / "emu"), str(tmp_path / "bps.bin")], capture_output=True, text=True,
+                       env=dict(os.environ, SQ_EMUL_DP=str(dp)))
+    assert r.returncode == 0, r.stderr[-2000:]
+    common.assert_same(want, pyref.load_dumps(str(tmp_path / "emu")), ("nodes", "edges"))  # -dp also gates edges (sq_locate.cuh)
+    got = np.fromfile(str(tmp_path / "emu" / "cov_i32.bin"), dtype=np.int32)
+    assert got.shape == want["cov"].shape
+    bad = np.flatnonzero(got != want["cov"])
+    assert bad.size == 0, "%d of %d breakpoints differ, first %s: restatement %s emul %s" % (
+        bad.size, got.size, bps[bad[:3]].tolist(), want["cov"][bad[:3]].tolist(), got[bad[:3]].tolist())

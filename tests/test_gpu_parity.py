@@ -162,15 +162,9 @@ def test_dense_breakpoints_lagging_chain(tmp_path, built_lib):
     """Tens of thousands of breakpoints packed into expressed regions: indBP lags far behind the stream (one breakpoint per
     qualifying record, SegmentGraph.cpp:3157-3158), so the max-plus shortcut fails and the chunked literal chain has to repair
     chunks that run into each other.  Checked against the literal chain of the CPU stepping harness."""
-    import os
     import subprocess
     from squid_b200 import api
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    emul = os.path.join(root, "tests", "emul", "_build", "emul_gpu_test")
-    os.makedirs(os.path.dirname(emul), exist_ok=True)
-    srcs = ["tests/emul/emul_main.cpp", "squid_b200/csrc/host/readrec.cpp", "squid_b200/csrc/host/chimeric.cpp", "squid_b200/csrc/host/prepass.cpp"]
-    r = subprocess.run(["g++", "-std=c++17", "-O2", "-fopenmp", "-I", "include", "-I", "squid_b200/csrc", "-o", emul] + srcs + ["-lpthread"], cwd=root, capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-2000:]
+    emul = common.build_emul(tmp_path / "bin")
     cp, hp, *_ = common.write_case(str(tmp_path), 60000, 23, 0.02, [3000000, 2000000, 500000, 16569], n_genes=40)
     case = api.HostCase(cp, hp)
     a = case.batch.a
