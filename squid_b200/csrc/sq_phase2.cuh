@@ -109,23 +109,6 @@ __device__ __noinline__ int32_t conc_edges_generic(const BatchDesc *desc, const 
     return conc_edges_sized<kMaxBlocks>(b, p, nt, r, edges);
 }
 
-// The same for a record of a staged tile: blocks and record fields come from shared memory (`tb` lives there too).
-__device__ __noinline__ int32_t conc_edges_tile(const TileBatch *tbp, const BatchDesc *desc, const NodeTable *ntp, int64_t r, TileEdgeTable *edges) {
-    const TileBatch &tb = *tbp;
-    const Params &p = desc->p;
-    const NodeTable nt = *ntp;
-    if (!conc_builds_edges(tb, p, r)) return -2;
-    const uint32_t nb = tb.blk_off[r + 1] - tb.blk_off[r];
-    Blk F[4], S[4];
-    int32_t node[8];
-    if (nb > 3) return -5;  // (rare: left to the out-of-tile kernel, whose frame holds 16 blocks per mate)
-    ReadView rv; rv.F = F; rv.S = S;
-    bool is_first;
-    conc_load_read(tb, r, rv, is_first);
-    if (rv.nF + rv.nS == 0) return -2;
-    return read_edges(nt, p, rv, MODE_OTHER, is_first, false, 0, node, *edges) ? node[0] : -3;
-}
-
 // ReadsOther, the two rare cases (sq_depth_cover.cuh): an entry that starts d <= 2 bp right of the start of its segment m2 goes
 // into that segment's start mask; a block of <= 3 bp is not counted here but deferred to the second pass.  Out of line.
 __device__ __noinline__ bool depth_other_rare(uint32_t *omask, int4 *shorts, int32_t *n_short, int32_t short_cap, int32_t rid, int32_t st, int32_t l, int32_t m2, int32_t d, bool on) {
@@ -140,9 +123,8 @@ __device__ __noinline__ bool depth_other_rare(uint32_t *omask, int4 *shorts, int
     return false;
 }
 
-template <bool DO_DEPTH, bool DO_EDGES, bool SLOW_IN_TILE>
+template <bool DO_DEPTH, bool DO_EDGES>
 __global__ void __launch_bounds__(kTileThreads, 7) k_assign_tiles(DevBatch b, P2Args a, int bulk_ok) {
-    __shared__ TileBatch s_tb;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     TileStage &s = *reinterpret_cast<TileStage *>(smem_raw);
     __shared__ TileEdgeTable s_edges;
@@ -165,7 +147,6 @@ __global__ void __launch_bounds__(kTileThreads, 7) k_assign_tiles(DevBatch b, P2
     stage_wait<kP2Fields>(s, b, a.cls, tk);
     const bool staged = ti.nb >= 0;
     const TileBatch tb = tile_view(s, ti, b);
-    if (SLOW_IN_TILE && tid == 0) s_tb = tb;
     if (tid == 0) {
         // The segment that holds the tile's first block: sorted input keeps most of the tile (usually all of it) inside this
         // one segment, so it is looked up once and every block of the tile is first tested against it.  The window of
@@ -311,42 +292,19 @@ __global__ void __launch_bounds__(kTileThreads, 7) k_assign_tiles(DevBatch b, P2
         }
     }
     // ---- the multi-block records that left the tile's segment ----------------------------------------------------------------
-    // They go to k_edges_generic's list.  (SLOW_IN_TILE, an experiment kept for measurements: processed right here with the generic
-    // rules, from the staged tile -- slower, see sqg_api.cu.  Also measured and dropped: a register-only rule set for the plain
-    // ones among them -- every block well inside one segment, nine in ten -- run here as a "pass B2": 43 M of the 53 M records of
-    // the benchmark leave the list, k_edges_generic 5.4 -> 1.5 ms, this kernel 5.5 -> 9.3 ms: the same cost per record either way.)
+    // They go to k_edges_generic's list.  (Measured and dropped: processing them right here with the generic rules, from the
+    // staged tile -- slower, see sqg_api.cu.  Also measured and dropped: a register-only rule set for the plain ones among them --
+    // every block well inside one segment, nine in ten -- run here as a "pass B2": 43 M of the 53 M records of the benchmark leave
+    // the list, k_edges_generic 5.4 -> 1.5 ms, this kernel 5.5 -> 9.3 ms: the same cost per record either way.)
     if (DO_EDGES) {
-        __shared__ int32_t s_slow_base, s_nleft;
-        int ns = s_nslow;
-        if (SLOW_IN_TILE && staged) {
-            if (tid == 0) s_nleft = 0;
-            __syncthreads();
-#pragma unroll 1
-            for (int q = tid; q < ns; q += kTileThreads) {
-                const int i = s_slow[q];
-                const int64_t r = rec0 + i;
-                const int32_t out = conc_edges_tile(&s_tb, a.desc, a.nt_dev, r, &s_edges);
-                if (out == -5) { s_mid[atomicAdd(&s_nleft, 1)] = (uint16_t)i; continue; }  // (s_mid is free again after pass B1)
-                a.res0[r] = out;
-                if (out == -3) { const int32_t k = atomicAdd(a.n_sens, 1); if (k < a.sens_cap) a.sens[k] = (int32_t)r; }
-            }
-            __syncthreads();
-            ns = s_nleft;
-            if (tid == 0 && ns > 0) s_slow_base = atomicAdd(a.n_slow, ns);
-            __syncthreads();
-            if (ns > 0) {
-                const int32_t base_q = s_slow_base;
-                for (int q = tid; q < ns; q += kTileThreads)
-                    if (base_q + q < a.slow_cap) a.slow_list[base_q + q] = (int32_t)(rec0 + s_mid[q]);
-            }
-        } else {
-            if (tid == 0 && ns > 0) s_slow_base = atomicAdd(a.n_slow, ns);
-            __syncthreads();
-            if (ns > 0) {
-                const int32_t base_q = s_slow_base;
-                for (int q = tid; q < ns; q += kTileThreads)
-                    if (base_q + q < a.slow_cap) a.slow_list[base_q + q] = (int32_t)(rec0 + s_slow[q]);
-            }
+        __shared__ int32_t s_slow_base;
+        const int ns = s_nslow;
+        if (tid == 0 && ns > 0) s_slow_base = atomicAdd(a.n_slow, ns);
+        __syncthreads();
+        if (ns > 0) {
+            const int32_t base_q = s_slow_base;
+            for (int q = tid; q < ns; q += kTileThreads)
+                if (base_q + q < a.slow_cap) a.slow_list[base_q + q] = (int32_t)(rec0 + s_slow[q]);
         }
     }
     // ---- ReadsMain with the tile-local cursor -----------------------------------------------------------------------

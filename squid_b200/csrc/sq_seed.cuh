@@ -64,7 +64,6 @@ struct SeedInputs {
     const RestBlock *rest; const uint32_t *rest_g; int32_t n_rest;  // ConcordRest candidates binned by the group they can matter to (rest_g ascending)
     int32_t read_len;
     int64_t first_kept;
-    long long *prof_out = nullptr;  // SQ_SEED_PROF builds: 12 int64 per island
     unsigned long long *win_count = nullptr;  // (device) total number of window records the groups looked at: the machine's algorithmic input
     // range shard of one genome: groups before g_lo belong to earlier shards; when a later shard follows, the record right
     // after this batch is a 0-coverage record for the pending group (the shard planner guarantees it, sqg_plan_shards)
@@ -74,7 +73,6 @@ struct SeedInputs {
     uint64_t end_other = 0;         // otherChr/otherrightmost after the last record of the batch
     const int32_t *ccmax = nullptr; int32_t cc_tile = 0;  // per tile of cc_tile records: maximum end of its ConcordantCluster entries (sq_classify.cuh)
     int32_t dense_max_r = 0;        // > 0: sub-clusters whose margins span at most this many positions use position-indexed tables
-    bool dense_all = false;         // ... on every island (tests); default: only islands whose windows span > kHeavySpan records
 };
 
 struct SeedState {
@@ -227,17 +225,8 @@ struct CoopBlock {  // every thread of the block (blockDim.x a multiple of 32): 
 };
 #endif
 
-#if defined(SQ_SEED_PROF) && defined(__CUDA_ARCH__)
-#define SQ_PROF_T0() long long prof_t_ = clock64()
-#define SQ_PROF_ADD(k) do { const long long n_ = clock64(); prof[k] += n_ - prof_t_; prof_t_ = n_; } while (0)
-#else
-#define SQ_PROF_T0() do {} while (0)
-#define SQ_PROF_ADD(k) do {} while (0)
-#endif
-
 template <class W>
 struct SeedMachineT {
-    long long prof[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     SeedInputs in;
     SeedState st;
     SeedOp *out; int32_t out_cap;
@@ -302,7 +291,7 @@ struct SeedMachineT {
     }
     SQ_HD int32_t mcap() const { return (margin_cap - 8) / 6; }     // six regions + 8 reserved cells at the end of the scratch
     SQ_HD int32_t *cell(int k) const { return margin + (margin_cap - 8) + k; }
-    bool use_dense = false;   // set per island by the caller (heavy islands; tests force it everywhere)
+    bool use_dense = false;   // set by the caller: every island on the device; the CPU stepping harness chooses
     int32_t n_dense = 0, n_sparse = 0;  // sub-clusters tabulated by position / through the sorted margins (statistics)
     // first index i in [lo,hi) with pred(i), else hi; the lanes split the range, the result is uniform
     template <class F> SQ_HD int32_t find_first(int32_t lo, int32_t hi, F pred) const {
@@ -687,7 +676,6 @@ struct SeedMachineT {
         const int32_t thresh = kSeedThresh, RL = in.read_len;
         int32_t *H = margin + mcap(), *PL = H + (R + 2), *PR = PL + (R + 2), *COV = PR + (R + 2), *REST = COV + (R + 2);
         const DiscBlock *D = in.D;
-        SQ_PROF_T0();  // (profile builds: [0] tables + margins + discordant blocks, [1] ConcordantCluster window, [3] other windows, [5] scans + candidates)
         W::sync();
         for (int32_t i = W::lane(); i < 5 * (R + 2); i += W::size()) H[i] = 0;
         W::sync();
@@ -710,7 +698,6 @@ struct SeedMachineT {
             for (int32_t i = W::lane(); i < (RESTw != REST ? 2 : 1) * (R + 2); i += W::size()) msearch[i] = 0;
             W::sync();
         }
-        SQ_PROF_ADD(0);
         if (st.offCC < rg) {  // ConcordantCluster window (:457-461); every record of [lo,hi) lies on chrG (sorted stream, rg is the group's trigger)
             const int64_t lo = lb_pos(st.offCC, rg, chrG, pmin), hi = lb_pos(lo, rg, chrG, pmax);
             constexpr int U = 8;
@@ -731,7 +718,6 @@ struct SeedMachineT {
                 }
             }
         }
-        SQ_PROF_ADD(1);
         if (st.offPC < szPC) {  // PartialAlignCluster window (:465-469)
             const int32_t lo = lb_pc_pos(st.offPC, szPC, chrG, pmin), hi = lb_pc_pos(lo, szPC, chrG, pmax);
             for (int32_t base = lo; base < hi; base += W::size()) {
@@ -778,7 +764,6 @@ struct SeedMachineT {
             for (int32_t i = W::lane(); i <= R; i += W::size()) { COV[i] += COVw[i]; if (RESTw != REST) REST[i] += RESTw[i]; }
             W::sync();
         }
-        SQ_PROF_ADD(3);
         scan_inplace(PL, R); scan_inplace(PR, R); scan_inplace(COV, R); scan_inplace(REST, R);
         // candidate breaks, in increasing position
         int32_t nC = 0;
@@ -804,7 +789,6 @@ struct SeedMachineT {
             nC += tot;
         }
         W::sync();
-        SQ_PROF_ADD(5);
         return nC;
     }
 
@@ -1049,7 +1033,6 @@ struct SeedMachineT {
     // Lines :353-612 for group g, reached at trigger record rg.
     SQ_HD void process_group(int32_t g, int64_t rg) {
         const int32_t thresh = kSeedThresh, RL = in.read_len;
-        SQ_PROF_T0();
         const Group grp = in.G[g];
         int32_t ds = grp.ds; const int32_t de = grp.de, chrG = grp.chr, nextright = grp.right;
         const DiscBlock *D = in.D;
@@ -1103,7 +1086,6 @@ struct SeedMachineT {
             while (lo < hi) { int32_t m = (lo + hi) >> 1; if (in.Pchr[m] == chrG && in.Ppos[m] < nextright + RL) lo = m + 1; else hi = m; }
             pe = lo;
         }
-        SQ_PROF_ADD(1);
         while (ds != de) {
             if (ds != 0 && D[ds].chr != D[ds - 1].chr && st.offCC >= rg && st.offPC >= szPC) curStartPos = D[ds].pos;
             isClusternSplit = false;
@@ -1140,7 +1122,6 @@ struct SeedMachineT {
             }
             if (error) return;
             W::sync();
-            SQ_PROF_ADD(2);
             BreakCtx bc;
             bc.lastCurser = -1; bc.lastSupport = 0; bc.curStartPos = curStartPos; bc.curEndPos = curEndPos; bc.isClusternSplit = false;
             bool dense = false;
@@ -1157,7 +1138,6 @@ struct SeedMachineT {
             if (dense) {
                 int32_t *CAND = margin + mcap() + 5 * (R + 2);
                 const int32_t nC = tabulate_dense(g, nM, P_lo, R, ds, de, chrG, in.D[grp.ds].pos, rg, szPC, CAND);
-                SQ_PROF_ADD(4);
                 for (int32_t ic = 0; ic < nC; ic++) {
                     const int32_t brk = CAND[2 * ic];
                     if (st.have_back && st.backChr == chrG && brk - st.backEnd < thresh * 20) continue;
@@ -1172,9 +1152,7 @@ struct SeedMachineT {
                     W::sync();
                     ms = msearch;
                 }
-                SQ_PROF_ADD(3);
                 tabulate_breaks(g, nM, ds, de, chrG, in.D[grp.ds].pos, rg, szPC);
-                SQ_PROF_ADD(4);
                 const int32_t *t_sr = margin + mcap(), *t_pl = margin + 2 * mcap(), *t_pr = margin + 3 * mcap(), *t_cov = margin + 4 * mcap(), *t_rest = margin + 5 * mcap();
                 for (int32_t ib = 0; ib < nM;) {
                     const int32_t brk = ms[ib];
@@ -1215,7 +1193,6 @@ struct SeedMachineT {
                 curStartPos = disEndPos; curEndPos = disEndPos;
                 st.markedStart = disEndPos; st.markedChr = chrG;
             }
-            SQ_PROF_ADD(5);
             // :529-532
             while (st.offCC < rg && e_chr(st.offCC) < chrG) st.offCC = nextCC(st.offCC + 1, rg);
             while (st.offPC < szPC && e_chr(in.pc_rec[st.offPC]) < chrG) st.offPC++;
@@ -1229,10 +1206,8 @@ struct SeedMachineT {
                 if (a > concord0pos) concord0pos = a;
                 if (bq > concord0pos) concord0pos = bq;
             }
-            SQ_PROF_ADD(6);
             // :570-601 extend the last segment to the next 0-coverage position if the stream already shows one
             extend_to_zero_coverage(rg, szPC, dc, recChr, recPos, concord0pos, curStartPos);
-            SQ_PROF_ADD(7);
             ds = dc;
             if (error) return;
         }
@@ -1250,7 +1225,7 @@ struct SeedMachineT {
             const int64_t rg = in.trigger[g];
             const Group grp = in.G[g];
             if (rg >= in.n_rec) break;
-            { SQ_PROF_T0(); replay_between(r_prev, rg, dChr, dRight, grp.chr, in.D[grp.ds].pos, true); SQ_PROF_ADD(0); }
+            replay_between(r_prev, rg, dChr, dRight, grp.chr, in.D[grp.ds].pos, true);
             process_group(g, rg);
             if (error) return g;
             dChr = grp.chr; dRight = grp.right;

@@ -2,8 +2,9 @@
 //   * a tile of kTile consecutive records and the contiguous run of aligned blocks they own is staged in shared memory
 //     with TMA bulk copies (cp.async.bulk, completion on an mbarrier) -- one elected thread issues ~14 copies instead of
 //     every thread issuing dependent blk_off -> block loads;
-//   * cross-tile prefix state (running maxima, compaction offsets) is carried with a decoupled look-back over per-tile
-//     descriptors, so every phase reads the batch exactly once;
+//   * cross-tile prefix state (running maxima, compaction offsets) comes from scans of per-tile aggregates; the one
+//     dependency a tile may have to resolve while it runs (the previous gate-passing record of the classification pass)
+//     is carried with a decoupled look-back over one word per tile;
 //   * tiles are handed out through an atomic ticket, which makes "tile t-1 is resident or done" hold for every running
 //     tile t (forward progress of the look-back).
 // sm_100a only (device code); nothing here runs on the host.
@@ -46,56 +47,10 @@ __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t by
 }
 
 // ---- decoupled look-back ----------------------------------------------------------------------------------------------
-// One chain = per tile a status word (0 nothing, 1 aggregate of the tile, 2 inclusive prefix) and two 64-bit payloads:
-// `a` combined with max, `b` combined with +.  Called by warp 0 of the tile (all 32 lanes).
-struct Chain {
-    uint32_t *status;
-    uint64_t *agg_a, *agg_b, *inc_a, *inc_b;
-};
-__device__ __forceinline__ uint32_t ld_acquire_u32(const uint32_t *p) { uint32_t v; asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory"); return v; }
-__device__ __forceinline__ void st_release_u32(uint32_t *p, uint32_t v) { asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-__device__ __forceinline__ uint64_t ld_relaxed_u64(const uint64_t *p) { uint64_t v; asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory"); return v; }
-__device__ __forceinline__ void st_relaxed_u64(uint64_t *p, uint64_t v) { asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory"); }
 __device__ __forceinline__ uint64_t warp_max_u64(uint64_t v) {
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) { const uint64_t o = __shfl_xor_sync(0xffffffffu, v, d); if (o > v) v = o; }
     return v;
-}
-__device__ __forceinline__ uint64_t warp_sum_u64(uint64_t v) {
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
-    return v;
-}
-// Publishes (agg_a, agg_b) of `tile`, waits for the exclusive prefix over tiles [0, tile), publishes the inclusive prefix,
-// returns the exclusive one in (*ex_a, *ex_b) on every lane.
-__device__ __forceinline__ void chain_scan(const Chain &c, int tile, uint64_t agg_a, uint64_t agg_b, uint64_t *ex_a, uint64_t *ex_b) {
-    const int lane = threadIdx.x & 31;
-    if (lane == 0) {
-        st_relaxed_u64(c.agg_a + tile, agg_a); st_relaxed_u64(c.agg_b + tile, agg_b);
-        st_release_u32(c.status + tile, 1u);
-    }
-    uint64_t xa = 0, xb = 0;
-    for (int base = tile - 1; base >= 0; base -= 32) {
-        const int p = base - lane;
-        uint32_t s = 2u;
-        uint64_t a = 0, b = 0;
-        if (p >= 0) {
-            do { s = ld_acquire_u32(c.status + p); } while (s == 0u);
-            a = ld_relaxed_u64((s == 2u ? c.inc_a : c.agg_a) + p); b = ld_relaxed_u64((s == 2u ? c.inc_b : c.agg_b) + p);
-        }
-        const unsigned pm = __ballot_sync(0xffffffffu, s == 2u);
-        const int stop = pm ? __ffs(pm) - 1 : 31;  // nearest predecessor that already knows its inclusive prefix
-        if (lane > stop) { a = 0; b = 0; }
-        const uint64_t ra = warp_max_u64(a), rb = warp_sum_u64(b);
-        if (ra > xa) xa = ra;
-        xb += rb;
-        if (pm) break;
-    }
-    if (lane == 0) {
-        st_relaxed_u64(c.inc_a + tile, xa > agg_a ? xa : agg_a); st_relaxed_u64(c.inc_b + tile, xb + agg_b);
-        st_release_u32(c.status + tile, 2u);
-    }
-    *ex_a = xa; *ex_b = xb;
 }
 
 // One-word chain: per tile a 64-bit word, status in the top two bits (0 nothing, 1 aggregate, 2 inclusive prefix), payload

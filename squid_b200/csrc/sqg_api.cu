@@ -8,7 +8,6 @@
 //   depth_edges: per-segment depth + read-to-segment assignment + raw edges        (phase-2 stream pass)
 //   edge_sort : radix sort by packed key + run-length reduce
 //   coverage  : breakpoint coverage with the reference's indBP lag                 (phase-3 stream pass)
-#include <cooperative_groups.h>
 #include <cub/cub.cuh>
 
 #include <algorithm>
@@ -90,7 +89,6 @@ static int cov_join(sqg_ctx *ctx) {
 struct MaxI32 { __device__ int32_t operator()(int32_t a, int32_t b) const { return a > b ? a : b; } };
 struct MaxU64 { __device__ uint64_t operator()(uint64_t a, uint64_t b) const { return a > b ? a : b; } };
 struct MaxI64 { __device__ int64_t operator()(int64_t a, int64_t b) const { return a > b ? a : b; } };
-struct MinI64 { __device__ int64_t operator()(int64_t a, int64_t b) const { return a < b ? a : b; } };
 
 // ------------------------------------------------------------------------------------------------
 // kernels: node building
@@ -252,7 +250,7 @@ __global__ void k_island_caps(SeedInputs in, const int32_t *isl_start, int32_t n
     // scratch: six regions of mcap ints (margin list + the five per-break tables) + 8 cells; islands that use position-indexed
     // tables need 5 (R + 2) + 2 min(nM, R) ints behind the list
     int64_t mc = pw;
-    if (in.dense_max_r > 0 && (in.dense_all || span[i] > kHeavySpanDev)) {
+    if (in.dense_max_r > 0) {
         const int64_t r = rmax < 16 * (int64_t)mmax + 4096 ? rmax : 16 * (int64_t)mmax + 4096;
         const int64_t need = (5 * (r + 2) + 2 * (r < mmax + 2 ? r : (int64_t)mmax + 2) + 2 + 4) / 5 + 1;
         if (need > mc) mc = need;
@@ -265,12 +263,10 @@ __global__ void k_gather_i32(const int32_t *src, const int32_t *idx, int32_t n, 
 }
 constexpr int kSeedBlock = 512;        // threads per block of the seed kernels
 constexpr int kHeavySpan = kHeavySpanDev;
-// Islands spanning more records than this would get a thread-block cluster (k_seed_giants).  Measured on the benchmark the
-// cluster policy is correct (GPU tests force it with SQG_GIANT_SPAN) but not yet faster than one 512-thread block: 11 islands of
-// 0.4-0.9 M records took 16 ms in clusters of 8 against 11 ms in single blocks (cluster barriers inside the chunked window
-// walks, 8x redundant scalar control).  Off by default until the walks are restructured around fewer barriers.
-constexpr int kGiantSpan = 0x7fffffff;
-constexpr int32_t kSeedMarginSmem = 11264;  // ints of shared memory per block: the sorted margins / the window accumulators of the position-indexed tables (44 KB)    // islands spanning more records than this get a whole block instead of a warp
+// Position-indexed break tables (sq_seed.cuh: tabulate_dense) on every island, for sub-clusters whose margins span at most this
+// many positions; wider ones keep the sorted margin lists.
+constexpr int32_t kSeedDenseRange = 1 << 16;
+constexpr int32_t kSeedMarginSmem = 11264;  // ints of shared memory per block: the sorted margins / the window accumulators of the position-indexed tables (44 KB)
 struct IsHeavyOp {
     const int32_t *span; const int32_t *n_prefix; bool want_heavy;
     __device__ bool operator()(int32_t i) const { return i >= *n_prefix && ((span[i] > kHeavySpan) == want_heavy); }
@@ -284,19 +280,8 @@ __device__ __forceinline__ void seed_one_island(const SeedInputs &in, int32_t i,
     sm.out = ops + off_ops[i]; sm.out_cap = (int32_t)(off_ops[i + 1] - off_ops[i]);
     sm.margin = margin + off_mar[i]; sm.margin_cap = (int32_t)(off_mar[i + 1] - off_mar[i]);
     sm.msearch = fast; sm.msearch_cap = fast_cap;
-    sm.use_dense = in.dense_max_r > 0 && (in.dense_all || W::size() > 32);  // block- and cluster-sized islands
-#ifdef SQ_SEED_PROF
-    long long t0_; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t0_));
-#endif
+    sm.use_dense = in.dense_max_r > 0;
     const int32_t gd = sm.run_island(ga, gb, inherited);
-#ifdef SQ_SEED_PROF
-    if (W::lane() == 0 && in.prof_out) {
-        long long t1_; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t1_));
-        long long *q = in.prof_out + (int64_t)i * 12;
-        q[0] = t0_; q[1] = t1_; q[2] = gb - ga; q[3] = W::size();
-        for (int k = 0; k < 8; k++) q[4 + k] = sm.prof[k];
-    }
-#endif
     if (W::lane() == 0) { g_done[i] = gd; n_out[i] = sm.st.n_out; if (sm.error) atomicMax(err, sm.error); }
     if (n_out_ret) *n_out_ret = sm.st.n_out;
 }
@@ -327,55 +312,6 @@ __global__ void __launch_bounds__(BLOCK, 1024 / BLOCK) k_seed_islands(SeedInputs
     if (k >= n_light) return;
     constexpr int32_t per_warp = kSeedMarginSmem / (BLOCK / 32);
     seed_one_island<CoopWarp>(in, light[k], true, isl_start, n_isl, off_ops, off_mar, ops, margin, n_out, g_done, err, nullptr, s_margins + (threadIdx.x >> 5) * per_warp, per_warp);
-}
-
-// A thread-block cluster stepping ONE island together: the few islands that span hundreds of thousands of records (highly
-// expressed genes) are bound by what a single SM can issue, so their window scans are spread over kGiantCluster SMs.  Same
-// contract as CoopBlock: every thread keeps identical scalar state; partial results cross CTAs through distributed shared
-// memory, and W::sync() is a cluster barrier (release/acquire at cluster scope, which also orders the scratch in HBM).
-namespace cg = cooperative_groups;
-constexpr int kGiantCluster = 8;
-struct CoopCluster {
-    template <int OP> static __device__ __forceinline__ int combine(int a, int b) { return OP == 0 ? a + b : (OP == 1 ? (a > b ? a : b) : (a < b ? a : b)); }
-    // value of every CTA -> all CTAs; `upto_self`: combine only the CTAs ranked before this one
-    template <int OP> static __device__ __forceinline__ int exchange(int block_value, int identity, bool before_self) {
-        __shared__ int slot;
-        cg::cluster_group cl = cg::this_cluster();
-        if (threadIdx.x == 0) slot = block_value;
-        cl.sync();
-        int r = identity;
-        const int n = before_self ? (int)cl.block_rank() : (int)cl.num_blocks();
-        for (int k = 0; k < n; k++) r = combine<OP>(r, *cl.map_shared_rank(&slot, k));
-        cl.sync();
-        return r;
-    }
-    static __device__ __forceinline__ int lane() { return (int)cg::this_cluster().block_rank() * blockDim.x + threadIdx.x; }
-    static __device__ __forceinline__ int size() { return (int)cg::this_cluster().num_blocks() * blockDim.x; }
-    static __device__ __forceinline__ int sum(int v) { return exchange<0>(CoopBlock::sum(v), 0, false); }
-    static __device__ __forceinline__ int max(int v) { return exchange<1>(CoopBlock::max(v), -2147483647 - 1, false); }
-    static __device__ __forceinline__ int min(int v) { return exchange<2>(CoopBlock::min(v), 2147483647, false); }
-    static __device__ __forceinline__ int excl_prefix_max(int v, int identity) {
-        const int e = CoopBlock::excl_prefix_max(v, identity), t = CoopBlock::max(v);
-        const int base = exchange<1>(t, identity, true);
-        return e > base ? e : base;
-    }
-    static __device__ __forceinline__ int excl_prefix_sum(int v) {
-        const int e = CoopBlock::excl_prefix_sum(v), t = CoopBlock::sum(v);
-        return exchange<0>(t, 0, true) + e;
-    }
-    static __device__ __forceinline__ void add(int32_t *p, int32_t v) { atomicAdd(p, v); }
-    static __device__ __forceinline__ void add_range(int32_t *diff, int32_t ja, int32_t jb, bool on) { CoopBlock::add_range(diff, ja, jb, on); }
-    static __device__ __forceinline__ void sync() { cg::this_cluster().sync(); }
-    static __device__ __forceinline__ void begin_append(int32_t *cell, int32_t n) { sync(); if (lane() == 0) *cell = n; sync(); }
-    static __device__ __forceinline__ int32_t reserve(bool has, int32_t &n, int32_t *cell) { return CoopBlock::reserve(has, n, cell); }
-    static __device__ __forceinline__ void end_append(int32_t *cell, int32_t &n) { sync(); n = *(volatile int32_t *)cell; sync(); }
-};
-__global__ void __cluster_dims__(kGiantCluster, 1, 1) __launch_bounds__(kSeedBlock, 2)
-k_seed_giants(SeedInputs in, const int32_t *isl_start, int32_t n_isl, const int64_t *off_ops, const int64_t *off_mar, SeedOp *ops, int32_t *margin, int32_t *n_out,
-              int32_t *g_done, int32_t *err, const int32_t *giant, int32_t n_giant) {
-    const int32_t gi = (int32_t)blockIdx.x / kGiantCluster;
-    if (gi >= n_giant) return;
-    seed_one_island<CoopCluster>(in, giant[gi], true, isl_start, n_isl, off_ops, off_mar, ops, margin, n_out, g_done, err, nullptr, nullptr, 0);
 }
 
 // The op lists of the islands, concatenated in island order WITHOUT their unused capacity (the scratch of an island is sized for
@@ -558,40 +494,6 @@ __global__ void k_unpack_edges(const uint64_t *keys, const int32_t *counts, int6
 // ------------------------------------------------------------------------------------------------
 // kernels: breakpoint coverage
 // ------------------------------------------------------------------------------------------------
-struct CoverKeyOp {
-    DevBatch b; const uint8_t *cls;
-    __device__ uint64_t operator()(int32_t r) const {
-        const uint16_t f = b.flag[r];
-        const int32_t rid = b.ref_id[r], pos = b.pos[r], mrid = b.mate_ref_id[r], mpos = b.mate_pos[r];
-        if (!cover_qualifies(cls[r], f, rid, pos, mrid, mpos)) return 0;
-        return chrpos_key(rid, cover_start(f, rid, pos, mrid, mpos));
-    }
-};
-struct CoverQualOp {
-    DevBatch b; const uint8_t *cls;
-    __device__ bool operator()(int32_t r) const { return cover_qualifies(cls[r], b.flag[r], b.ref_id[r], b.pos[r], b.mate_ref_id[r], b.mate_pos[r]); }
-};
-// key of the i-th QUALIFYING record (rank space): the reference's indBP advances at most once per qualifying record
-struct CoverRankKeyOp {
-    DevBatch b; const int32_t *qidx;
-    __device__ uint64_t operator()(int32_t i) const {
-        const int32_t r = qidx[i];
-        return chrpos_key(b.ref_id[r], cover_start(b.flag[r], b.ref_id[r], b.pos[r], b.mate_ref_id[r], b.mate_pos[r]));
-    }
-};
-__global__ void k_cov_r0(const uint64_t *M, int64_t nq, const int32_t *bp_chr, const int32_t *bp_pos, int64_t K, int32_t dist, uint64_t *bpkey, int64_t *r0, int64_t *t) {
-    const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (k >= K) return;
-    bpkey[k] = chrpos_key(bp_chr[k], bp_pos[k]);
-    const uint64_t T = cover_pass_key(bp_chr[k], bp_pos[k], dist);
-    const int64_t v = upper_bound_u64(M, 0, nq, T);  // first qualifying rank whose running-max key exceeds T
-    r0[k] = v;
-    t[k] = v - k;  // max-plus form of t[k] = max(r0[k], t[k-1]+1)
-}
-__global__ void k_cov_keys(CoverRankKeyOp key, int64_t nq, uint64_t *qkey) {
-    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i < nq) qkey[i] = key((int32_t)i);
-}
 __global__ void k_cov_verify(const uint64_t *qkey, int64_t nq, const int32_t *bp_chr, const int32_t *bp_pos, int64_t K, int32_t dist,
                              const int64_t *r0, int64_t *t, int32_t *fail) {
     const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -684,25 +586,6 @@ __global__ void k_cov_chain(const uint64_t *qkey, int64_t nq, const int32_t *bp_
         if (k < K) t[k] = my_t;
     }
 }
-__global__ void k_cov_count(DevBatch b, const int32_t *qidx, const uint64_t *qkey, int64_t nq, const uint64_t *bpkey, const int64_t *t, int64_t K, int32_t *cov) {
-    int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    const bool valid = i < nq;
-    if (!valid) i = nq - 1;  // keep the whole warp in the aggregation loop
-    const int32_t r = qidx[i];
-    const int32_t rid = b.ref_id[r];
-    const uint64_t ks = qkey[i];
-    const uint64_t ke = chrpos_key(rid, b.end_pos[r]);
-    // sorted input: neighbouring fragments cover the same breakpoints, so aggregate per warp before the atomic
-    int64_t k = lower_bound_u64(bpkey, 0, K, ks);
-    bool live = valid && k < K && bpkey[k] < ke;
-    const unsigned full = __activemask();
-    while (__any_sync(full, live)) {
-        const int32_t key = (live && i < t[k]) ? (int32_t)k : -1;
-        const unsigned m = __match_any_sync(full, key);
-        if (key >= 0 && (int)(threadIdx.x & 31) == __ffs(m) - 1) atomicAdd(&cov[key], __popc(m));
-        if (live) { k++; live = k < K && bpkey[k] < ke; }
-    }
-}
 
 // ------------------------------------------------------------------------------------------------
 // API
@@ -721,8 +604,7 @@ int sqg_create(sqg_ctx **out, const sqg_config *cfg, const int32_t *ref_len, int
     int prio_lo = 0, prio_hi = 0;
     cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);  // (numerically lower = more urgent)
     if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) { delete ctx; return SQG_ECUDA; }
-    if (cudaStreamCreateWithPriority(&ctx->stream2, cudaStreamNonBlocking, prio_hi) != cudaSuccess || cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming) != cudaSuccess ||
+    if (cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaStreamCreateWithFlags(&ctx->stream_cov, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&ctx->ev_cov_fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&ctx->ev_cov_done, cudaEventDisableTiming) != cudaSuccess ||
         cudaStreamCreateWithPriority(&ctx->stream3, cudaStreamNonBlocking, prio_hi) != cudaSuccess || cudaEventCreateWithFlags(&ctx->ev_chim, cudaEventDisableTiming) != cudaSuccess ||
@@ -757,16 +639,15 @@ void sqg_destroy(sqg_ctx *ctx) {
     ctx->d_trigger.release(); ctx->d_rest.release(); ctx->d_rest2.release(); ctx->d_restkey.release(); ctx->d_restkey2.release();
     ctx->d_omask.release(); ctx->d_shorts.release(); ctx->d_other_off.release(); ctx->d_other_key.release(); ctx->d_other_idx.release(); ctx->d_other_len.release(); ctx->d_other_own.release(); ctx->d_chimdiff.release(); ctx->h_chimdiff.release(); ctx->d_restbits.release(); ctx->d_restoff.release(); ctx->d_reflen.release(); ctx->d_ops.release(); ctx->d_ops_dense.release(); ctx->h_ops.release(); ctx->d_cutflag.release(); ctx->d_isl.release(); ctx->d_cap_ops.release(); ctx->d_cap_mar.release();
     ctx->d_isl_nout.release(); ctx->d_isl_gdone.release(); ctx->d_span.release(); ctx->d_heavy.release(); ctx->d_light.release(); ctx->d_off_ops.release(); ctx->d_off_mar.release(); ctx->d_dp.release();
-    ctx->d_margin.release(); ctx->d_seedstate.release();
-    ctx->d_bin_off.release(); ctx->d_bin_seg.release(); ctx->d_flen.release(); ctx->d_tileagg.release(); ctx->d_ccmax.release(); ctx->d_cov_nq.release(); ctx->d_cov_qmax.release(); ctx->d_cov_rank0.release(); ctx->d_cov_incmax.release(); ctx->d_temp_cov.release(); ctx->d_desc.release(); ctx->d_cand_key.release(); ctx->d_chain64.release(); ctx->d_chain32.release(); ctx->d_nchr.release(); ctx->d_npos.release(); ctx->d_nend.release(); ctx->d_chr_first.release(); ctx->d_cnt3.release(); ctx->d_sum3.release();
+    ctx->d_margin.release();
+    ctx->d_bin_off.release(); ctx->d_bin_seg.release(); ctx->d_flen.release(); ctx->d_tileagg.release(); ctx->d_ccmax.release(); ctx->d_cov_nq.release(); ctx->d_cov_qmax.release(); ctx->d_cov_rank0.release(); ctx->d_cov_incmax.release(); ctx->d_temp_cov.release(); ctx->d_desc.release(); ctx->d_cand_key.release(); ctx->d_chain64.release(); ctx->d_nchr.release(); ctx->d_npos.release(); ctx->d_nend.release(); ctx->d_chr_first.release(); ctx->d_cnt3.release(); ctx->d_sum3.release();
     ctx->d_chain_used.release(); ctx->d_qend.release(); ctx->d_covtile.release(); ctx->d_slow.release(); ctx->d_head.release(); ctx->d_ew.release(); ctx->d_dtile.release(); ctx->d_ekeys.release(); ctx->d_ekeys2.release(); ctx->d_ukeys.release(); ctx->d_ecount.release(); ctx->d_sens.release();
     ctx->d_e_ind1.release(); ctx->d_e_ind2.release(); ctx->d_e_w.release(); ctx->d_e_heads.release();
     ctx->d_bpkey.release(); ctx->d_covM.release(); ctx->d_qkey.release(); ctx->d_chunks.release(); ctx->d_r0.release(); ctx->d_t.release(); ctx->d_cov.release(); ctx->d_bpchr.release(); ctx->d_bppos.release();
     ctx->h_chr.release(); ctx->h_pos.release(); ctx->h_len.release(); ctx->h_cnt3.release(); ctx->h_sum3.release(); ctx->h_ind1.release(); ctx->h_ind2.release();
-    ctx->h_w.release(); ctx->h_chimblk.release(); ctx->h_heads.release(); ctx->h_seeds.release();
+    ctx->h_w.release(); ctx->h_heads.release();
     for (auto &kv : ctx->timers) { if (kv.second.a) cudaEventDestroy(kv.second.a); if (kv.second.b) cudaEventDestroy(kv.second.b); }
     cudaStreamDestroy(ctx->stream);
-    if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
     ctx->d_gs_keys.release(); ctx->d_gs_idx.release(); ctx->d_gs_scratch.release(); ctx->h_gs_keys.release(); ctx->h_gs_idx.release(); ctx->h_t.release();
     if (ctx->stream3) cudaStreamDestroy(ctx->stream3);
     if (ctx->ev_chim) cudaEventDestroy(ctx->ev_chim);
@@ -778,7 +659,6 @@ void sqg_destroy(sqg_ctx *ctx) {
     if (ctx->ev_cov_fork) cudaEventDestroy(ctx->ev_cov_fork);
     if (ctx->ev_cov_done) cudaEventDestroy(ctx->ev_cov_done);
     if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
-    if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
     delete ctx;
 }
 
@@ -800,7 +680,7 @@ int64_t sqg_stat(const sqg_ctx *ctx, const char *name) {
     if (n == "islands") return ctx->n_islands;
     if (n == "device_sort_status") return ctx->gs_last_status;  // 0: the pre-pass sort ran on the device; -100: on the cores
     if (n == "heavy_islands") return ctx->n_heavy;
-    if (n == "giant_islands") return ctx->n_giant;
+    if (n == "giant_islands") return 0;  // every island runs in one block or one warp
     if (n == "cov_chain_fallback") return ctx->cov_chain_fallback;
     if (n == "cov_chain_chunks") return ctx->cov_chain_chunks;
     if (n == "gap_records") return ctx->n_gap;
@@ -1340,19 +1220,6 @@ static int finish_prepass(sqg_ctx *ctx) {
 static int ensure_temp(sqg_ctx *ctx, size_t bytes) { CK(ctx->d_temp.ensure(bytes + 256)); return SQG_OK; }
 #define ENSURE_TEMP(bytes) do { int rc_ = ensure_temp(ctx, bytes); if (rc_) return rc_; } while (0)
 
-// look-back chains of a stream kernel: `n_chains` chains over `n_tiles` tiles; status words zeroed, ticket reset
-static int prepare_chains(sqg_ctx *ctx, int n_chains, int64_t n_tiles, Chain *out, int32_t **ticket, cudaStream_t st) {
-    CK(ctx->d_chain64.ensure((size_t)n_chains * 4 * n_tiles + 8));
-    CK(ctx->d_chain32.ensure((size_t)n_chains * n_tiles + 8));
-    CK(cudaMemsetAsync(ctx->d_chain32.p, 0, ((size_t)n_chains * n_tiles + 8) * 4, st));
-    for (int c = 0; c < n_chains; c++) {
-        out[c].status = ctx->d_chain32.p + (size_t)c * n_tiles;
-        uint64_t *q = ctx->d_chain64.p + (size_t)c * 4 * n_tiles;
-        out[c].agg_a = q; out[c].agg_b = q + n_tiles; out[c].inc_a = q + 2 * n_tiles; out[c].inc_b = q + 3 * n_tiles;
-    }
-    *ticket = (int32_t *)(ctx->d_chain32.p + (size_t)n_chains * n_tiles);
-    return SQG_OK;
-}
 static bool batch_bulk_ok(const DevBatch &b) {  // TMA bulk copies need 16-byte aligned sources
     const void *ptrs[] = {b.ref_id, b.pos, b.mate_ref_id, b.mate_pos, b.end_pos, b.flag, b.total_len, b.lowphred_run, b.mapq, b.aux, b.blk_off,
                           b.blk_ref_pos, b.blk_match_ref, b.blk_read_pos, b.blk_match_read};
@@ -1736,46 +1603,32 @@ static int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges) {
             }
             // two launches of the same tile kernel, one per job: each half is small enough for the instruction cache, and
             // reading the batch twice is cheap next to that
-            CK(cudaFuncSetAttribute(k_assign_tiles<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes));
-            CK(cudaFuncSetAttribute(k_assign_tiles<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes));
-            CK(cudaFuncSetAttribute(k_assign_tiles<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes));
-            // multi-block records that leave their tile's segment: all of them in k_edges_generic (default), or in the tile kernel from
-            // shared memory (SQG_SLOW_IN_TILE=1).  Measured at the App. C block mix, 100 M pairs: 4.6 + 8.3 ms against 21.3 ms -- inside
+            CK(cudaFuncSetAttribute(k_assign_tiles<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes));
+            CK(cudaFuncSetAttribute(k_assign_tiles<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes));
+            // multi-block records that leave their tile's segment all go to k_edges_generic.  Processing them in the tile kernel from
+            // shared memory was measured and dropped: at the App. C block mix, 100 M pairs, 4.6 + 8.3 ms against 21.3 ms -- inside
             // the tile kernel the generic rules stall on instruction fetch (ncu: no_instruction is the top stall) and the tile's warps
             // wait at the barrier behind the one that drew the longest records (profiles/r2_ncu_summary.txt).
-            static const bool slow_in_tile = getenv("SQG_SLOW_IN_TILE") && atoi(getenv("SQG_SLOW_IN_TILE")) == 1;
-            // The depth pass and the edge pass are independent: SQG_DEPTH_OVERLAP=1 runs the depth tile kernel on the second stream
-            // beside k_edges_generic instead of in front of it.  Measured (100 M pairs): no gain, 21.6 ms against 20.2 ms for the two
-            // passes together -- the two kernels compete for the same issue slots and L2 -- so the default keeps them in sequence.
-            static const bool overlap_env = getenv("SQG_DEPTH_OVERLAP") && atoi(getenv("SQG_DEPTH_OVERLAP")) == 1;
-            const bool overlap = do_depth && do_edges && overlap_env;
-            auto depth_pass = [&](cudaStream_t st) -> int {
-                { const int rc_ = phase_begin(ctx, "k_assign_depth", st); if (rc_) return rc_; }
-                k_assign_tiles<true, false, false><<<(unsigned)n_tiles, kTileThreads, kTileSmemBytes, st>>>(b, a, batch_bulk_ok(b) ? 1 : 0);
+            // The depth pass and the edge pass are independent, but running the depth tile kernel on a second stream beside
+            // k_edges_generic was measured and dropped (100 M pairs): no gain, 21.6 ms against 20.2 ms for the two passes together --
+            // the two kernels compete for the same issue slots and L2 -- so they run in sequence.
+            PHASE_BEGIN("k_assign");
+            if (do_depth) {
+                PHASE_BEGIN("k_assign_depth");
+                k_assign_tiles<true, false><<<(unsigned)n_tiles, kTileThreads, kTileSmemBytes, ctx->stream>>>(b, a, batch_bulk_ok(b) ? 1 : 0);
                 ctx->launches++;
                 CK(cudaGetLastError());
-                { const int rc_ = phase_end(ctx, "k_assign_depth", st); if (rc_) return rc_; }
-                LAUNCH_ON(st, k_depth_scan, 1, 1024, ctx->d_dtile.p, (int32_t)n_tiles);
-                LAUNCH_ON(st, k_depth_fix, blocks_for(n_tiles), kThreads, b, ctx->d_cls.p, ctx->nt, ctx->r_break, ctx->d_dtile.p, (int32_t)n_tiles, a.cnt_main, a.sum_main);
-                LAUNCH_ON(st, k_depth_short_nodes, 64, 128, ctx->nt, ctx->d_omask.p, ctx->d_shorts.p, a.n_short, a.short_cap, a.n_short + 1);
-                return SQG_OK;
-            };
-            PHASE_BEGIN("k_assign");
-            if (do_depth && !overlap) { const int rc_ = depth_pass(ctx->stream); if (rc_) return rc_; }
+                PHASE_END("k_assign_depth");
+                LAUNCH(k_depth_scan, 1, 1024, ctx->d_dtile.p, (int32_t)n_tiles);
+                LAUNCH(k_depth_fix, blocks_for(n_tiles), kThreads, b, ctx->d_cls.p, ctx->nt, ctx->r_break, ctx->d_dtile.p, (int32_t)n_tiles, a.cnt_main, a.sum_main);
+                LAUNCH(k_depth_short_nodes, 64, 128, ctx->nt, ctx->d_omask.p, ctx->d_shorts.p, a.n_short, a.short_cap, a.n_short + 1);
+            }
             if (do_edges) {
                 PHASE_BEGIN("k_assign_edges");
-                if (slow_in_tile) k_assign_tiles<false, true, true><<<(unsigned)n_tiles, kTileThreads, kTileSmemBytes, ctx->stream>>>(b, a, batch_bulk_ok(b) ? 1 : 0);
-                else k_assign_tiles<false, true, false><<<(unsigned)n_tiles, kTileThreads, kTileSmemBytes, ctx->stream>>>(b, a, batch_bulk_ok(b) ? 1 : 0);
+                k_assign_tiles<false, true><<<(unsigned)n_tiles, kTileThreads, kTileSmemBytes, ctx->stream>>>(b, a, batch_bulk_ok(b) ? 1 : 0);
                 ctx->launches++;
                 CK(cudaGetLastError());
                 PHASE_END("k_assign_edges");
-                if (overlap) {
-                    CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
-                    CK(cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork, 0));
-                    const int rc_ = depth_pass(ctx->stream2);
-                    if (rc_) return rc_;
-                    CK(cudaEventRecord(ctx->ev_join, ctx->stream2));
-                }
                 PHASE_BEGIN("k_edges_generic");
                 // the generic kernel is compiled for 8 resident blocks per SM (64 registers): it is bound by the latency of dependent
                 // loads, and more warps with fewer registers each beat fewer warps without local-memory traffic -- measured at 100 M
@@ -1785,7 +1638,6 @@ static int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges) {
                 LAUNCH(k_fix_heads, 256, 128, ctx->d_scratch32.p, ctx->d_sens.p, d_nsens, conc_sens_cap, ctx->d_head.p, ctx->shard_init_hint, (int32_t *)(ctx->d_counters.p + 22));
                 LAUNCH(k_fix_chains<false>, 256, 128, b, cd, ctx->params, ctx->nt, ctx->d_scratch32.p, n, ctx->d_sens.p, d_nsens, conc_sens_cap, ctx->d_head.p, sink);
                 if (ctx->shard_count > 1) LAUNCH(k_last_located, 1, 1, ctx->d_scratch32.p, n, (int32_t *)(ctx->d_counters.p + 23));
-                if (overlap) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
             }
             PHASE_END("k_assign");
         }
@@ -1920,11 +1772,7 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
     if (g_hi < g_lo) g_hi = g_lo;
     in.g_hi = g_hi;
     in.g_lo = g_lo; in.has_next = ctx->shard_index + 1 < ctx->shard_count; in.end_other = ctx->end_other;
-    {   // position-indexed break tables (sq_seed.cuh: tabulate_dense): SQG_SEED_DENSE = 0 off, 1 block-sized islands only, 2 every island (default)
-        static const int dense_mode = getenv("SQG_SEED_DENSE") ? atoi(getenv("SQG_SEED_DENSE")) : 2;
-        static const int dense_r = getenv("SQG_SEED_DENSE_R") ? atoi(getenv("SQG_SEED_DENSE_R")) : (1 << 16);
-        in.dense_max_r = dense_mode > 0 ? dense_r : 0; in.dense_all = dense_mode > 1;
-    }
+    in.dense_max_r = kSeedDenseRange;
     CK(ctx->d_cutflag.ensure(nG + 1)); CK(ctx->d_isl.ensure(nG + 2));
     LAUNCH(k_island_cuts, blocks_for(nG, 64), 64, in, ctx->d_cutflag.p);
     CK(cudaMemsetAsync(ctx->d_counters.p + 5, 0, sizeof(int64_t), ctx->stream));
@@ -1997,10 +1845,6 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
         CK(cudaMemcpyAsync(ctx->d_heavy.p, ctx->d_light.p + n_light, n_heavy * 4, cudaMemcpyDeviceToDevice, ctx->stream));
         ctx->launches += 2;
     }
-#ifdef SQ_SEED_PROF
-    long long *d_prof = nullptr;
-    if (getenv("SQG_SEED_PROF_OUT")) { cudaMalloc(&d_prof, (size_t)n_isl * 12 * 8); cudaMemset(d_prof, 0, (size_t)n_isl * 12 * 8); cudaDeviceSynchronize(); in.prof_out = d_prof; }
-#endif
     // Phase 3's compaction pass only needs the class bytes.  It is forked HERE, behind the short kernels of this stage and beside the
     // island machine: enqueued right after the classification, its 10^5 blocks sat in front of the ConcordRest collection, which is
     // on the critical path (5.7 ms instead of 1.4 ms).  (The two share the SMs without gaining from it: alone the island kernel
@@ -2008,51 +1852,18 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
     // same 2 ms there.  The step is bound by the sum of the work, not by a critical path.)
     rc = run_cov_compact(ctx);
     if (rc) return rc;
-    // the longest islands (sorted first) go to thread-block clusters on a second stream, concurrently with the rest
-    int32_t n_giant = 0;
-    if (n_heavy > 0) {
-        int32_t hs[64];
-        const int32_t m = std::min(n_heavy, 64);
-        if (n_heavy > 1) {  // (a single block-sized island stays with the block kernel)
-            CK(cudaMemcpyAsync(hs, ctx->d_cap_ops.p + n_heavy, m * 4, cudaMemcpyDeviceToHost, ctx->stream));  // spans, longest first
-            CK(cudaStreamSynchronize(ctx->stream));
-            const int64_t giant_span = getenv("SQG_GIANT_SPAN") ? atoll(getenv("SQG_GIANT_SPAN")) : (int64_t)kGiantSpan;  // env: test hook
-            while (n_giant < m && hs[n_giant] > giant_span) n_giant++;
-        }
-    }
-    ctx->n_giant = n_giant;
-    if (n_giant > 0) {
-        CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
-        CK(cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork, 0));
-        k_seed_giants<<<(unsigned)(n_giant * kGiantCluster), kSeedBlock, 0, ctx->stream2>>>(in, ctx->d_isl.p, n_isl, ctx->d_off_ops.p, ctx->d_off_mar.p, ctx->d_ops.p, ctx->d_margin.p,
-                                                                                         ctx->d_isl_nout.p, ctx->d_isl_gdone.p, d_err, ctx->d_heavy.p, n_giant);
-        ctx->launches++;
-        CK(cudaGetLastError());
-        CK(cudaEventRecord(ctx->ev_join, ctx->stream2));
-    }
-    if (n_heavy - n_giant + n_light > 0) {
+    if (n_heavy + n_light > 0) {
         PHASE_BEGIN("k_seed_islands");
         // (block size measured at 100 M pairs: 256 threads 9.6 ms, 512 threads 7.5 ms, 1024 threads 8.9 ms -- the kernel needs both
         // many islands in flight and many lanes on the few long ones)
-        k_seed_islands<kSeedBlock><<<(unsigned)(n_heavy - n_giant + (n_light + kSeedBlock / 32 - 1) / (kSeedBlock / 32)), kSeedBlock, 0, ctx->stream>>>(in, ctx->d_isl.p, n_isl, ctx->d_off_ops.p, ctx->d_off_mar.p,
-               ctx->d_ops.p, ctx->d_margin.p, ctx->d_isl_nout.p, ctx->d_isl_gdone.p, d_err, ctx->d_heavy.p + n_giant, n_heavy - n_giant, ctx->d_light.p, n_light);
+        k_seed_islands<kSeedBlock><<<(unsigned)(n_heavy + (n_light + kSeedBlock / 32 - 1) / (kSeedBlock / 32)), kSeedBlock, 0, ctx->stream>>>(in, ctx->d_isl.p, n_isl, ctx->d_off_ops.p, ctx->d_off_mar.p,
+               ctx->d_ops.p, ctx->d_margin.p, ctx->d_isl_nout.p, ctx->d_isl_gdone.p, d_err, ctx->d_heavy.p, n_heavy, ctx->d_light.p, n_light);
         ctx->launches++;
         CK(cudaGetLastError());
         PHASE_END("k_seed_islands");
     }
-    if (n_giant > 0) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
     PHASE_END("seed");
     lap("seed: enqueue");
-#ifdef SQ_SEED_PROF
-    if (d_prof) {
-        cudaStreamSynchronize(ctx->stream);
-        std::vector<long long> hp((size_t)n_isl * 12); std::vector<int32_t> hs(n_isl);
-        cudaMemcpy(hp.data(), d_prof, hp.size() * 8, cudaMemcpyDeviceToHost); cudaMemcpy(hs.data(), ctx->d_span.p, n_isl * 4, cudaMemcpyDeviceToHost);
-        FILE *f = fopen(getenv("SQG_SEED_PROF_OUT"), "wb");
-        if (f) { fwrite(&n_isl, 4, 1, f); fwrite(hs.data(), 4, n_isl, f); fwrite(hp.data(), 8, hp.size(), f); fclose(f); }
-        cudaFree(d_prof);
-    }
-#endif
     // this batch's op lists in island order: compacted on the device (the islands' scratch is sized for the worst case, two ops
     // per margin -- copying that capacity cost more than the whole tiling stage), then one small copy
     CK(ctx->d_ops_dense.ensure((size_t)(tot[0] > 0 ? tot[0] : 1)));

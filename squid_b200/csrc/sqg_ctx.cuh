@@ -95,8 +95,8 @@ struct PhaseTimer {
 
 struct sqg_ctx {
     int device = 0;
-    cudaStream_t stream = nullptr, stream2 = nullptr;  // stream2: the cluster kernel of the seed machine, forked / joined with events
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t ev_fork = nullptr;
     // the coverage compaction (phase 3, first pass) runs beside the seed machine on its own stream
     cudaStream_t stream_cov = nullptr;
     cudaEvent_t ev_cov_fork = nullptr, ev_cov_done = nullptr;
@@ -134,8 +134,7 @@ struct sqg_ctx {
     sq::DBuf<uint8_t> d_cls;
     sq::DBuf<uint16_t> d_flen;      // first-block length of every CLS_CONC record (seed machine windows)
     sq::DBuf<uint64_t> d_other;     // running otherChr/otherrightmost key at each coverage-gap record
-    sq::DBuf<uint64_t> d_chain64;   // look-back chains of the stream kernels
-    sq::DBuf<uint32_t> d_chain32;
+    sq::DBuf<uint64_t> d_chain64;   // look-back words of the classification tiles (P1Out::gate_word)
     sq::DBuf<sq::TileAgg> d_tileagg;  // per-tile aggregates / exclusive prefixes of phase 1
     sq::DBuf<uint32_t> d_cov_nq; sq::DBuf<uint64_t> d_cov_qmax, d_cov_incmax; sq::DBuf<int64_t> d_cov_rank0; sq::DBuf<uint8_t> d_temp_cov;  // phase 3: per classification tile
     sq::DBuf<uint64_t> d_qstage_key; sq::DBuf<int32_t> d_qstage_end;  // phase 3's pairs as the classification kernel leaves them (per tile)
@@ -156,9 +155,6 @@ struct sqg_ctx {
     sqh::ChimPrepass pre;
     sqg_chimeric chim_view{};
     sq::Worker prepass_worker;  // persistent host thread of the chimeric pre-pass (keeps its OpenMP team alive between runs)
-    std::vector<uint32_t> c_read_off;
-    std::vector<uint16_t> c_n_first;
-    std::vector<int32_t> c_first_total, c_second_total;
     int64_t c_n_reads = 0, c_n_blk = 0;
     sq::DBuf<sq::DiscBlock> d_disc;
     sq::DBuf<sq::Group> d_groups;
@@ -210,12 +206,11 @@ struct sqg_ctx {
     sq::HBuf<sq::SeedOp> h_ops;
     sq::DBuf<uint8_t> d_cutflag;
     sq::DBuf<int32_t> d_isl, d_cap_ops, d_cap_mar, d_isl_nout, d_isl_gdone, d_span, d_heavy, d_light;
-    int32_t n_heavy = 0, n_giant = 0;
+    int32_t n_heavy = 0;
     bool cov_chain_fallback = false;
     int64_t n_sensitive = 0, n_raw_edges = 0;
     sq::DBuf<int64_t> d_off_ops, d_off_mar;
     sq::DBuf<int32_t> d_margin;
-    sq::DBuf<sq::SeedState> d_seedstate;
     int64_t r_break = 0;
 
     // range shard of one genome (sqg_set_shard, SURVEY.md 8e): index 0 owns the chimeric edges and the discordant depth
@@ -258,8 +253,7 @@ struct sqg_ctx {
     sq::DBuf<sq::CovTile> d_covtile;
 
     // pinned outputs
-    sq::HBuf<int32_t> h_chr, h_pos, h_len, h_cnt3, h_sum3, h_ind1, h_ind2, h_w, h_chimblk;
+    sq::HBuf<int32_t> h_chr, h_pos, h_len, h_cnt3, h_sum3, h_ind1, h_ind2, h_w;
     sq::HBuf<uint8_t> h_heads;
-    sq::HBuf<sq::SeedNode> h_seeds;
 };
 #endif
