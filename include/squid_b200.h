@@ -163,7 +163,9 @@ int sqg_build_nodes(sqg_ctx *ctx, int32_t **chr, int32_t **pos, int32_t **len, i
                     int32_t **count3, int32_t **sumlen3, int32_t *reads_other_nonempty);
 
 /* Replaces SegmentGraph_t(string graphfile)'s node reload (SegmentGraph.cpp:126-157): installs a node
- * table (must tile the genome) so that edges/coverage can run on a stored graph. */
+ * table so that edges/coverage can run on a stored graph.  The table must tile the genome: sorted by chromosome, every
+ * chromosome covered from 0 to its length by contiguous segments of positive length.  Anything else is refused with
+ * SQG_EINVAL (sqg_last_error says which rule broke) and leaves the context as it was. */
 int sqg_set_nodes(sqg_ctx *ctx, const int32_t *chr, const int32_t *pos, const int32_t *len, int64_t n_nodes);
 
 /*

@@ -102,6 +102,27 @@ def run_restate(conc_sqmb: str, chim_sqmb: str, outdir: str, bps=None, opts=None
     return d
 
 
+def run_restate_on_nodes(conc_sqmb: str, chim_sqmb: str, outdir: str, nodes, opts=None, dump_raw: bool = False) -> dict:
+    """BuildEdges of the CPU restatement on a given segment table `nodes` (rows chr, pos, len[, ...]): the graph reload of
+    SegmentGraph_t(string).  Returns {"edges", "chim_after_edges"}; with dump_raw also "raw_edges", int64 rows (concordant
+    record index, packed edge key) for every edge RawEdgesOther emits, in emission order."""
+    import ctypes as C
+    build_restate()
+    lib = C.CDLL(RESTATE_LIB)
+    lib.sqo_edges_on_nodes.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.POINTER(C.c_int), C.c_char_p, C.c_int]
+    os.makedirs(outdir, exist_ok=True)
+    nf = os.path.join(outdir, "nodes_in.bin")
+    np.ascontiguousarray(np.asarray(nodes)[:, :3], dtype=np.int32).tofile(nf)
+    o = (C.c_int * 6)(*(opts if opts is not None else restate_opts()))
+    rc = lib.sqo_edges_on_nodes(conc_sqmb.encode(), chim_sqmb.encode(), outdir.encode(), o, nf.encode(), int(dump_raw))
+    if rc != 0:
+        raise RuntimeError("sqo_edges_on_nodes failed rc=%d" % rc)
+    d = {"edges": _i32(os.path.join(outdir, "edges_i32.bin"), 5), "chim_after_edges": _i32(os.path.join(outdir, "chim_after_edges.bin"), 8)}
+    if dump_raw:
+        d["raw_edges"] = np.fromfile(os.path.join(outdir, "raw_edges.bin"), dtype=np.int64).reshape(-1, 2)
+    return d
+
+
 _RESTATE_FLAGS = {"-pt": 0, "-pl": 1, "-pm": 2, "-mq": 3, "-dp": 4, "-di": 5}  # the reference's options (Config.cpp:18-25) -> sqo_run opts
 
 

@@ -14,7 +14,8 @@
 //
 // Entry point: sqo_run() reads two SQMB files (include/sqmb_format.h) and writes the same dump files as
 // oracle/ref_harness.cpp (nodes_i32.bin, nodes_f64.bin, edges_i32.bin, chim_loaded.bin, chim_after_edges.bin,
-// readlen.bin) plus cov_i32.bin for a supplied sorted breakpoint list.
+// readlen.bin) plus cov_i32.bin for a supplied sorted breakpoint list.  sqo_edges_on_nodes() runs the same BuildEdges on
+// a segment table the caller supplies.
 #include <algorithm>
 #include <cstdint>
 #include <cstdio>
@@ -632,7 +633,8 @@ struct Graph {
         }
     }
     // BuildEdges, SegmentGraph.cpp:1932-1959
-    void build_edges(const SqmbView &conc, std::vector<Rd> &chim) {
+    // raw: when non-null, one (record index, edge_key packing) pair per edge RawEdgesOther emits, in emission order
+    void build_edges(const SqmbView &conc, std::vector<Rd> &chim, std::vector<int64_t> *raw = nullptr) {
         int ffi = 0;
         for (Rd &r : chim) { if (r.F.empty() && r.S.empty()) continue; read_edges(r, ffi, true, true); }  // RawEdgesChim (weights = counts)
         const std::vector<std::string> names = names_of(chim);
@@ -648,7 +650,15 @@ struct Graph {
             last = rd;
             bool build = rd.F.empty() || rd.S.empty();
             if (!build) build = (rd.F.front().rpos <= 15 || (a.first() && rd.fl)) && (rd.S.front().rpos <= 15 || (!a.first() && rd.sl));
-            if (build) read_edges(rd, ffi, false, a.first());
+            if (!build) continue;
+            const size_t e0 = edges.size();
+            read_edges(rd, ffi, false, a.first());
+            if (raw)
+                for (size_t k = e0; k < edges.size(); k++) {
+                    const Edge &e = edges[k];
+                    raw->push_back((int64_t)ri);
+                    raw->push_back((int64_t)(((uint64_t)(uint32_t)e.a << 33) | ((uint64_t)(uint32_t)e.b << 2) | ((uint64_t)e.ha << 1) | (uint64_t)e.hb));
+                }
         }
         std::sort(edges.begin(), edges.end(), edge_lt);
         std::vector<Edge> u;
@@ -694,6 +704,14 @@ static std::vector<int32_t> chim_rows(const std::vector<Rd> &c) {
             for (const Blk &b : (m ? c[i].S : c[i].F)) { a.push_back((int32_t)i); a.push_back(m); a.push_back(b.chr); a.push_back(b.pos); a.push_back(b.rpos); a.push_back(b.mref); a.push_back(b.mread); a.push_back(b.rev); }
     return a;
 }
+static void set_opts(Opt &o, const int *opts) {
+    if (opts) { o.phred33 = opts[0]; o.max_lowphred = opts[1]; o.min_phred = opts[2]; o.min_mapq = opts[3] < 0 ? 255 : opts[3]; o.dist_pos = opts[4]; o.dist_idx = opts[5]; }
+}
+static void dump_edges(const std::string &path, const std::vector<Edge> &edges) {
+    std::vector<int32_t> a;
+    for (const Edge &e : edges) { a.push_back(e.a); a.push_back(e.b); a.push_back(e.ha); a.push_back(e.hb); a.push_back(e.w); }
+    dump(path, a);
+}
 }  // namespace
 
 // opts: {phred33, max_lowphred_len, min_phred, min_mapq, concord_dist_pos, concord_dist_idx}; bps_file may be NULL.
@@ -703,7 +721,7 @@ extern "C" int sqo_run(const char *conc_path, const char *chim_path, const char 
     SqmbView conc, chim;
     if (!conc.open(conc_path) || !chim.open(chim_path)) return -1;
     Graph g;
-    if (opts) { g.o.phred33 = opts[0]; g.o.max_lowphred = opts[1]; g.o.min_phred = opts[2]; g.o.min_mapq = opts[3] < 0 ? 255 : opts[3]; g.o.dist_pos = opts[4]; g.o.dist_idx = opts[5]; }
+    set_opts(g.o, opts);
     g.ref_len.assign(conc.ref_len, conc.ref_len + conc.n_ref);
     std::vector<Rd> cr = load_chim(chim, g.o);
     const std::string d = outdir;
@@ -727,11 +745,7 @@ extern "C" int sqo_run(const char *conc_path, const char *chim_path, const char 
         }
         if (stop_after == 2) return 0;
         g.build_edges(conc, cr);
-        {
-            std::vector<int32_t> a;
-            for (const Edge &e : g.edges) { a.push_back(e.a); a.push_back(e.b); a.push_back(e.ha); a.push_back(e.hb); a.push_back(e.w); }
-            dump(d + "/edges_i32.bin", a);
-        }
+        dump_edges(d + "/edges_i32.bin", g.edges);
         dump(d + "/chim_after_edges.bin", chim_rows(cr));
     }
     if (stop_after == 3 || !bps_file) return 0;
@@ -743,5 +757,35 @@ extern "C" int sqo_run(const char *conc_path, const char *chim_path, const char 
     fclose(f);
     const std::vector<int> cov = g.bp_coverage(conc, cr, bps);
     dump(d + "/cov_i32.bin", std::vector<int32_t>(cov.begin(), cov.end()));
+    return 0;
+}
+
+// BuildEdges on a segment table the caller supplies (the graph reload of SegmentGraph_t(string), SegmentGraph.cpp:126-157):
+// loads the chimeric reads, installs the (chr, pos, len) int32 rows of nodes_path as the segments and writes edges_i32.bin and
+// chim_after_edges.bin.  dump_raw != 0 also writes raw_edges.bin: int64 (record index, packed key) rows, one per edge that
+// RawEdgesOther emits, the key packed as sq_locate.cuh's edge_key packs it.  Returns 0, or <0 on I/O error.
+extern "C" int sqo_edges_on_nodes(const char *conc_path, const char *chim_path, const char *outdir, const int *opts, const char *nodes_path, int dump_raw) {
+    SqmbView conc, chim;
+    if (!conc.open(conc_path) || !chim.open(chim_path)) return -1;
+    Graph g;
+    set_opts(g.o, opts);
+    g.ref_len.assign(conc.ref_len, conc.ref_len + conc.n_ref);
+    std::vector<Rd> cr = load_chim(chim, g.o);
+    FILE *f = fopen(nodes_path, "rb");
+    if (!f) return -2;
+    int32_t row[3];
+    while (fread(row, 4, 3, f) == 3) g.nodes.push_back(Node{row[0], row[1], row[2], 0, 0});
+    fclose(f);
+    std::vector<int64_t> raw;
+    g.build_edges(conc, cr, dump_raw ? &raw : nullptr);
+    const std::string d = outdir;
+    dump_edges(d + "/edges_i32.bin", g.edges);
+    dump(d + "/chim_after_edges.bin", chim_rows(cr));
+    if (dump_raw) {
+        FILE *r = fopen((d + "/raw_edges.bin").c_str(), "wb");
+        if (!r) return -3;
+        if (!raw.empty()) fwrite(raw.data(), 8, raw.size(), r);
+        fclose(r);
+    }
     return 0;
 }

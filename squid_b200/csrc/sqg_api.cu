@@ -691,6 +691,7 @@ int64_t sqg_stat(const sqg_ctx *ctx, const char *name) {
     if (n == "disc_blocks") return ctx->pre_nD;
     if (n == "sensitive_reads") return ctx->n_sensitive;
     if (n == "raw_edges") return ctx->n_raw_edges;
+    if (n == "edge_pass_attempts") return ctx->edge_pass_attempts;  // > 1: a list of the last edge pass overflowed and the pass ran again
     if (n == "r_break") return ctx->r_break;
     if (n == "seed_window_records") return ctx->h_counters.p ? ctx->h_counters.p[29] : -1;  // concordant-cluster window sizes summed over the groups
     if (n == "n_rec") return ctx->have_batch ? ctx->batch.n_rec : -1;
@@ -1378,6 +1379,29 @@ static int install_nodes(sqg_ctx *ctx) {  // from h_nchr/h_npos/h_nend
 
 extern "C" int sqg_set_nodes(sqg_ctx *ctx, const int32_t *chr, const int32_t *pos, const int32_t *len, int64_t n_nodes) {
     if (!ctx || !chr || !pos || !len || n_nodes <= 0 || n_nodes > 0x7ffffff0ll) return SQG_EINVAL;
+    // the table must tile every chromosome from 0 to its length with segments of positive length: the position index (seg_at)
+    // and the closed-form LocateRead index a chromosome's segments as [chr_first[c], chr_first[c+1]) and take a position below
+    // the last segment's end to lie inside the chromosome's bins.  (Sortedness and contiguity are checked in install_nodes.)
+    {
+        const int32_t n_ref = ctx->params.n_ref;
+        int32_t prev = -1;
+        for (int64_t i = 0; i < n_nodes; i++) {
+            const int32_t c = chr[i];
+            if (c < 0 || c >= n_ref) FAIL(SQG_EINVAL, "set_nodes: segment " + std::to_string(i) + " has a chromosome outside [0, n_ref)");
+            if (len[i] <= 0) FAIL(SQG_EINVAL, "set_nodes: segment " + std::to_string(i) + " has length <= 0");
+            if (c != prev) {
+                if (c < prev) FAIL(SQG_EINVAL, "set_nodes: segments must be sorted by chromosome");
+                if (c > prev + 1) FAIL(SQG_EINVAL, "set_nodes: chromosome " + std::to_string(prev + 1) + " has no segment");
+                if (pos[i] != 0) FAIL(SQG_EINVAL, "set_nodes: the first segment of chromosome " + std::to_string(c) + " does not start at 0");
+                prev = c;
+            }
+            if (i + 1 == n_nodes || chr[i + 1] != c) {
+                if ((int64_t)pos[i] + len[i] != (int64_t)ctx->ref_len[c])
+                    FAIL(SQG_EINVAL, "set_nodes: the last segment of chromosome " + std::to_string(c) + " does not end at its length " + std::to_string(ctx->ref_len[c]));
+            }
+        }
+        if (prev != n_ref - 1) FAIL(SQG_EINVAL, "set_nodes: chromosome " + std::to_string(prev + 1) + " has no segment");
+    }
     CK(cudaSetDevice(ctx->device));
     ctx->h_nchr.assign(chr, chr + n_nodes); ctx->h_npos.assign(pos, pos + n_nodes); ctx->h_nend.resize(n_nodes);
     for (int64_t i = 0; i < n_nodes; i++) ctx->h_nend[i] = pos[i] + len[i];
@@ -1547,7 +1571,15 @@ static int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges) {
         ctx->chim_upload_pending = false;
     }
     PHASE_BEGIN(do_depth ? "depth_edges" : "edges_only");
-    for (int attempt = 0; attempt < 2; attempt++) {
+    // Capacity retries.  A list that overflows makes the pass run again with room for what it counted, but an attempt whose slow
+    // list overflowed never ran the records past its capacity, and one whose sensitive list overflowed never replayed the
+    // chains past it: their raw pairs (and, for deferred records, their sensitive reads) are missing from the counts, so the
+    // next attempt can overflow again.  The counts firm up one list at a time -- the slow-list count is always complete, so
+    // the second attempt runs every record; its sensitive count is then complete, so the third replays every chain; the raw
+    // count of the third is complete -- and the fourth attempt always fits.
+    constexpr int kEdgeAttempts = 4;
+    for (int attempt = 0; attempt < kEdgeAttempts; attempt++) {
+        if (do_edges) ctx->edge_pass_attempts = attempt + 1;
         if (do_edges) { CK(ctx->d_ekeys.ensure(cap)); CK(ctx->d_ew.ensure(cap)); CK(ctx->d_sens.ensure(sens_cap)); CK(ctx->d_head.ensure(sens_cap)); }
         cap = do_edges ? (int64_t)std::min(ctx->d_ekeys.cap, ctx->d_ew.cap) : 0;
         sens_cap = do_edges ? (int64_t)std::min(ctx->d_sens.cap, ctx->d_head.cap) : 0;
@@ -1657,7 +1689,7 @@ static int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges) {
         if (n_short <= short_cap && (!do_edges || (n_raw <= cap && ns_conc <= conc_sens_cap && n_slow <= slow_cap))) break;
         slow_cap = std::max(slow_cap, n_slow + 4096);
         short_cap = std::max(short_cap, n_short + 4096);
-        if (attempt == 1) FAIL(SQG_ENOMEM, "raw edge / sensitive read / short block buffer overflow");
+        if (attempt + 1 == kEdgeAttempts) FAIL(SQG_ENOMEM, "raw edge / sensitive read / short block buffer overflow");
         cap = std::max(cap, n_raw + 4096);  // rerun with room for everything (counters are reset, the chimeric blocks restored from their pristine copies)
         sens_cap = std::max<int64_t>(sens_cap, (int64_t)ns_conc + ctx->c_n_reads + 4096);
     }

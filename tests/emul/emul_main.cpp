@@ -41,6 +41,7 @@ int main(int argc, char **argv) {
     outdir = argv[3];
     sqh::HostConfig cfg;
     if (getenv("SQ_EMUL_DP")) cfg.concord_dist_pos = atoi(getenv("SQ_EMUL_DP"));  // -dp (Concord_Dist_Pos)
+    if (getenv("SQ_EMUL_DI")) cfg.concord_dist_idx = atoi(getenv("SQ_EMUL_DI"));  // -di (Concord_Dist_Idx)
     SqmbView conc, chim;
     if (!conc.open(argv[1]) || !chim.open(argv[2])) { fprintf(stderr, "cannot open inputs\n"); return 2; }
     std::vector<sqh::Read> reads;
@@ -204,7 +205,13 @@ int main(int argc, char **argv) {
         else norm.back().len = std::max(norm.back().pos + norm.back().len, s.pos + s.len) - norm.back().pos;
     }
     std::vector<int32_t> nchr, npos, nend;
-    {
+    if (const char *nf = getenv("SQ_EMUL_NODES")) {  // an injected table (the graph-reload seam): int32 rows chr, pos, len
+        FILE *f = fopen(nf, "rb");
+        if (!f) { fprintf(stderr, "cannot open %s\n", nf); return 2; }
+        int32_t row[3];
+        while (fread(row, 4, 3, f) == 3) { nchr.push_back(row[0]); npos.push_back(row[1]); nend.push_back(row[1] + row[2]); }
+        fclose(f);
+    } else {
         size_t k = 0;
         for (int32_t c = 0; c < n_ref; c++) {
             int32_t cur = 0;

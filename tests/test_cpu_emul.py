@@ -106,3 +106,41 @@ def test_coverage_chain_matches_restatement(cov_case, family, dp, emul_bin, tmp_
     bad = np.flatnonzero(got != want["cov"])
     assert bad.size == 0, "%d of %d breakpoints differ, first %s: restatement %s emul %s" % (
         bad.size, got.size, bps[bad[:3]].tolist(), want["cov"][bad[:3]].tolist(), got[bad[:3]].tolist())
+
+
+@pytest.fixture(scope="module")
+def family_cases(tmp_path_factory):
+    cache = {}
+
+    def get(name):
+        if name not in cache:
+            cache[name] = common.family_case(tmp_path_factory.mktemp(name), name)
+        return cache[name]
+    return get
+
+
+FAMILIES = ["built", "block_edges", "near_edges", "micro", "bins", "coarse", "random"]
+
+
+@pytest.mark.parametrize("case,family,opts", [(c, f, []) for c in ("chr17_s17", "short_s37") for f in FAMILIES] +
+                         [("chr17_s17", f, common.FAMILY_OPTS) for f in ("near_edges", "micro")])
+@pytest.mark.parametrize("bin_shift", [0, 4, 9, 12])
+@pytest.mark.parametrize("fast", [True, False])
+def test_edges_on_injected_tables(family_cases, case, family, opts, bin_shift, fast, emul_bin, tmp_path):
+    """BuildEdges on a segment table the caller installs (the graph-reload seam): the closed-form LocateRead, the hint replay and
+    the position index stepped on the CPU against the restatement's literal LocateRead, on tables with segments on and beside
+    block ends, runs of 1-6 bp segments, segments of one bin's size and one segment per chromosome.  Depth is not compared: the
+    reload seam keeps the stored values."""
+    cp, hp, ref_len, fam = family_cases(case)
+    nodes = fam[family]
+    want = pyref.run_restate_on_nodes(cp, hp, str(tmp_path / "ref"), nodes, opts=pyref.restate_opts(opts))
+    nodes.tofile(str(tmp_path / "nodes.bin"))
+    env = dict(os.environ, SQ_EMUL_NODES=str(tmp_path / "nodes.bin"), SQ_EMUL_BIN_SHIFT=str(bin_shift))
+    if not fast:
+        env["SQ_EMUL_NO_FAST_EDGES"] = "1"
+    if opts:
+        env["SQ_EMUL_DP"], env["SQ_EMUL_DI"] = opts[1], opts[3]
+    os.makedirs(str(tmp_path / "emu"))
+    r = subprocess.run([emul_bin, cp, hp, str(tmp_path / "emu")], capture_output=True, text=True, env=env)
+    assert r.returncode == 0, r.stderr[-2000:]
+    common.assert_same(want, pyref.load_dumps(str(tmp_path / "emu")), ("edges", "chim_after_edges"))

@@ -28,6 +28,23 @@ def test_restatement_reproduces_golden(case, tmp_path):
     assert pyref.support_from_cov(g, bps, me["cov"]) == pyref.support_map(g)
 
 
+@pytest.mark.parametrize("case", CASES)
+def test_restatement_edges_on_given_nodes(case, tmp_path):
+    """BuildEdges of the restatement on an injected table (sqo_edges_on_nodes): on the reference's own segments it must give the
+    reference's edges and trimmed chimeric blocks, so the reload entry shares the pinned path."""
+    g = _gold(case)
+    me = pyref.run_restate_on_nodes(os.path.join(GOLD, case, "conc.sqmb"), os.path.join(GOLD, case, "chim.sqmb"), str(tmp_path), g["nodes"], dump_raw=True)
+    common.assert_same(g, me, ("edges", "chim_after_edges"))
+    # every RawEdgesOther emission is one weight-1 row: their keys are a sub-multiset of the reduced table
+    raw = me["raw_edges"]
+    assert raw.shape[0] > 0 and np.all(np.diff(raw[:, 0]) >= 0)
+    e = g["edges"].astype(np.int64)
+    keys = (e[:, 0] << 33) | (e[:, 1] << 2) | (e[:, 2] << 1) | e[:, 3]
+    k, c = np.unique(raw[:, 1], return_counts=True)
+    at = np.searchsorted(keys, k)
+    assert np.all(keys[at] == k) and np.all(c <= e[at, 4])
+
+
 def test_restatement_decoder_kat(tmp_path):
     g = pyref.load_dumps(os.path.join(GOLD, "kat_decode", "ref"))
     me = pyref.run_restate(os.path.join(GOLD, "kat_decode", "conc.sqmb"), os.path.join(GOLD, "kat_decode", "chim.sqmb"), str(tmp_path), stop_after=1)
