@@ -250,8 +250,15 @@ float sqg_phase_ms(const sqg_ctx *ctx, const char *name);
 int64_t sqg_launch_count(const sqg_ctx *ctx);
 /* Counters of the most recent calls ("islands", "heavy_islands", "groups", "disc_blocks", "gap_records", "partial_records",
  * "displaced_records", "lmax", "sensitive_reads", "raw_edges" (= (key, count) pairs before the reduce), "cov_chain_fallback",
- * "r_break", "edges_single_path", "edges_generic_path"); -1 if unknown. */
+ * "r_break", "edges_single_path", "edges_generic_path", "first_kept", "end_other", "classify_attempts"); -1 if unknown. */
 int64_t sqg_stat(const sqg_ctx *ctx, const char *name);
+/* Test seam of the classification pass: copies the named phase-1 array of the resident batch to `out` (classifying it first if
+ * needed) and sets *n to its element count; nothing is copied when out is NULL or cap (in elements) < *n.  Names and element
+ * types: "cls" (uint8, per record), "first_len" (uint16, per record), "gap_rec" (int32) and "gap_key" (uint64) for the
+ * coverage-gap records, "pc_rec" and "dp_rec" (int32: partial, displaced records), per 512-record tile "okmax_excl" (uint64),
+ * "ccmax" (int32), "cov_nq" (uint32), "cov_qmax" (uint64), and per record "qstage_key" (uint64), "qstage_end" (int32), compacted
+ * inside each tile.  sqg_build_nodes reuses some of these buffers: call this before it. */
+int sqg_classify_dump(sqg_ctx *ctx, const char *name, void *out, int64_t cap, int64_t *n);
 
 #ifdef __cplusplus
 }

@@ -123,6 +123,28 @@ def run_restate_on_nodes(conc_sqmb: str, chim_sqmb: str, outdir: str, nodes, opt
     return d
 
 
+CLASSIFY_COLS = ("cls", "first_len", "cc_end", "other_end", "ex_chr", "ex_right", "cover_q", "frag_start", "frag_end")
+
+
+def run_restate_classify(conc_sqmb: str, chim_sqmb: str, outdir: str, opts=None) -> dict:
+    """The per-record preamble of BuildNode_STAR over the whole concordant stream (sqo_classify): one int32 array per column of
+    CLASSIFY_COLS (class bits as sq_common.cuh's CLS_* values; cc_end INT32_MIN and other_end -1 where the record has none;
+    (ex_chr, ex_right) = otherChr/otherRight in front of the record), plus "read_len"."""
+    import ctypes as C
+    build_restate()
+    lib = C.CDLL(RESTATE_LIB)
+    lib.sqo_classify.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.POINTER(C.c_int)]
+    os.makedirs(outdir, exist_ok=True)
+    o = (C.c_int * 6)(*(opts if opts is not None else restate_opts()))
+    rc = lib.sqo_classify(conc_sqmb.encode(), chim_sqmb.encode(), outdir.encode(), o)
+    if rc != 0:
+        raise RuntimeError("sqo_classify failed rc=%d" % rc)
+    a = _i32(os.path.join(outdir, "classify_i32.bin"), len(CLASSIFY_COLS))
+    d = {k: np.ascontiguousarray(a[:, i]) for i, k in enumerate(CLASSIFY_COLS)}
+    d["read_len"] = int(np.fromfile(os.path.join(outdir, "readlen.bin"), dtype=np.int32)[0])
+    return d
+
+
 _RESTATE_FLAGS = {"-pt": 0, "-pl": 1, "-pm": 2, "-mq": 3, "-dp": 4, "-di": 5}  # the reference's options (Config.cpp:18-25) -> sqo_run opts
 
 

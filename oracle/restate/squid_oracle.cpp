@@ -17,6 +17,7 @@
 // readlen.bin) plus cov_i32.bin for a supplied sorted breakpoint list.  sqo_edges_on_nodes() runs the same BuildEdges on
 // a segment table the caller supplies.
 #include <algorithm>
+#include <climits>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -265,6 +266,41 @@ struct Graph {
         Blk m{a.mchr, a.mpos, 0, 15, 15, 60, a.mate_rev(), false};
         (a.first() ? r.S : r.F).push_back(m);
     }
+    // The per-record preamble of BuildNode_STAR for one concordant record (:297-333 gate, Equal against the previous
+    // gate-passing record `last`, own blocks; :649-689 concordance and partial alignment).  Shared by build_nodes and sqo_classify.
+    struct RecClass {
+        Aln a;
+        Rd rd, tmp;  // rd: the record's own blocks in CIGAR order; tmp: sorted by read position, with the mate block (:305-314)
+        bool gate = false, keep = false, conc = false, part_f = false, part_s = false;
+        const std::vector<Blk> &own() const { return (a.first() && !rd.F.empty()) ? rd.F : rd.S; }  // :320-333
+        bool has_blk() const { return (a.first() && !rd.F.empty()) || !rd.S.empty(); }
+        const std::vector<Blk> *other_own() const { return a.first() ? &rd.F : (a.second() ? &rd.S : nullptr); }  // :657-663
+    };
+    void classify(const SqmbView &conc, uint64_t ri, const std::vector<std::string> &names, Rd &last, RecClass &c) const {
+        c = RecClass();
+        c.a = fetch(conc, ri);
+        const Aln &a = c.a;
+        c.gate = gate(a, names, true);
+        if (!c.gate) return;
+        c.rd = decode(a, o);
+        c.tmp = c.rd;
+        sort_rpos(c.tmp);
+        add_mate_block(a, c.tmp);
+        if (rd_equal(last, c.tmp)) return;
+        last = c.tmp;
+        c.keep = true;
+        bool concordant = false;  // :651-654
+        if (a.mapped() && a.mate_mapped() && a.mchr != -1 && a.chr == a.mchr && a.proper()) {
+            if (a.rev() && !a.mate_rev() && a.pos >= a.mpos && a.pos - a.mpos <= 750000) concordant = true;
+            else if (!a.rev() && a.mate_rev() && a.mpos >= a.pos && a.mpos - a.pos <= 750000) concordant = true;
+        }
+        c.conc = concordant && c.rd.F.size() + c.rd.S.size() > 0;
+        if (!c.conc) return;
+        const Rd &t = c.tmp;  // :668-683
+        c.part_f = a.first() && !t.fl && (t.F.front().rpos > 15 || t.ft - t.F.back().rpos - t.F.back().mread > 15);
+        c.part_s = a.second() && !t.sl && (t.S.front().rpos > 15 || t.st - t.S.back().rpos - t.S.back().mread > 15);
+    }
+
     bool edge_disc(const Edge &e) const {  // IsDiscordant(Edge_t), :181-190
         if (nodes[e.a].chr != nodes[e.b].chr) return true;
         if (nodes[e.b].pos - nodes[e.a].pos - nodes[e.a].len > o.dist_pos && e.b - e.a > o.dist_idx) return true;
@@ -326,16 +362,14 @@ struct Graph {
                 nextChr = dis[de].chr;
             }
         };
+        RecClass rc;
         for (uint64_t ri = 0; ri < conc.n_rec; ri++) {
-            const Aln a = fetch(conc, ri);
-            if (!gate(a, names, true)) continue;
-            Rd rd = decode(a, o), tmp = rd;
-            sort_rpos(tmp);
-            add_mate_block(a, tmp);
-            if (rd_equal(last, tmp)) continue;
-            last = tmp;
-            const std::vector<Blk> &own = (a.first() && !rd.F.empty()) ? rd.F : rd.S;  // :320-333
-            if ((a.first() && !rd.F.empty()) || !rd.S.empty()) {
+            classify(conc, ri, names, last, rc);
+            if (!rc.keep) continue;
+            const Aln &a = rc.a;
+            const Rd &rd = rc.rd;
+            const std::vector<Blk> &own = rc.own();
+            if (rc.has_blk()) {
                 main_.push_back({own[0].chr, {own[0].pos, own[0].mref}});
                 for (size_t k = 1; k < own.size(); k++) other_.push_back({own[k].chr, {own[k].pos, own[k].mref}});
             }
@@ -491,21 +525,15 @@ struct Graph {
                 }
             }
             // :649-700
-            bool concordant = false;
-            if (a.mapped() && a.mate_mapped() && a.mchr != -1 && a.chr == a.mchr && a.proper()) {
-                if (a.rev() && !a.mate_rev() && a.pos >= a.mpos && a.pos - a.mpos <= 750000) concordant = true;
-                else if (!a.rev() && a.mate_rev() && a.mpos >= a.pos && a.mpos - a.pos <= 750000) concordant = true;
-            }
-            if (concordant && rd.F.size() + rd.S.size() > 0) {
-                const std::vector<Blk> *ownp = a.first() ? &rd.F : (a.second() ? &rd.S : nullptr);
+            if (rc.conc) {
+                const std::vector<Blk> *ownp = rc.other_own();
                 if (ownp) {
                     const int e = ownp->front().pos + ownp->front().mref;
                     if (otherChr == a.chr) otherRight = std::max(otherRight, e); else { otherRight = e; otherChr = a.chr; }
                 }
-                bool partial = false;
-                if (a.first() && !tmp.fl && (tmp.F.front().rpos > 15 || tmp.ft - tmp.F.back().rpos - tmp.F.back().mread > 15)) { pc.push_back(rd.F.front()); partial = true; }
-                if (a.second() && !tmp.sl && (tmp.S.front().rpos > 15 || tmp.st - tmp.S.back().rpos - tmp.S.back().mread > 15)) { pc.push_back(rd.S.front()); partial = true; }
-                if (!partial) cc.push_back(a.first() ? rd.F.front() : rd.S.front());
+                if (rc.part_f) pc.push_back(rd.F.front());
+                if (rc.part_s) pc.push_back(rd.S.front());
+                if (!rc.part_f && !rc.part_s) cc.push_back(a.first() ? rd.F.front() : rd.S.front());
                 if (ownp && ownp->size() > 1)
                     for (size_t i = 1; i < ownp->size(); i++)
                         if (ds != nD && (*ownp)[i].pos >= dis[ds].pos - RL) { rest.push_back((*ownp)[i]); std::push_heap(rest.begin(), rest.end(), heap_cmp); }
@@ -757,6 +785,59 @@ extern "C" int sqo_run(const char *conc_path, const char *chim_path, const char 
     fclose(f);
     const std::vector<int> cov = g.bp_coverage(conc, cr, bps);
     dump(d + "/cov_i32.bin", std::vector<int32_t>(cov.begin(), cov.end()));
+    return 0;
+}
+
+// The per-record preamble of BuildNode_STAR over the WHOLE concordant stream (no stop at the last discordant group: that
+// truncation belongs to the seed machine, not to the filter).  Writes classify_i32.bin, one row of 9 int32 per record:
+//   class bits (sq_common.cuh's CLS_* values, defined from the reference's lines: GATE :302; KEEP = GATE and not Equal
+//   :315-318; HASBLK = KEEP and own blocks :320-333; DISPL = HASBLK and own[0].pos != pos; CONC :651-655; PART :668-683;
+//   REST = CONC, a mate flag and more than one own block),
+//   first-block length of a CONC record (else 0), ConcordantCluster end (else INT32_MIN), otherrightmost contribution (else -1),
+//   (otherChr, otherRight) in front of the record, coverage-pass qualification (:3136-3142), fragment start and end.
+// Also writes readlen.bin.  Returns 0, or <0 on I/O error.
+extern "C" int sqo_classify(const char *conc_path, const char *chim_path, const char *outdir, const int *opts) {
+    SqmbView conc, chim;
+    if (!conc.open(conc_path) || !chim.open(chim_path)) return -1;
+    Graph g;
+    set_opts(g.o, opts);
+    g.ref_len.assign(conc.ref_len, conc.ref_len + conc.n_ref);
+    const std::vector<Rd> cr = load_chim(chim, g.o);
+    const std::vector<std::string> names = Graph::names_of(cr);
+    std::vector<int32_t> rows;
+    rows.reserve((size_t)conc.n_rec * 9);
+    Rd last;
+    Graph::RecClass rc;
+    int otherChr = 0, otherRight = 0;
+    for (uint64_t ri = 0; ri < conc.n_rec; ri++) {
+        g.classify(conc, ri, names, last, rc);
+        const Aln &a = rc.a;
+        int cls = 0, flen = 0, cc_end = INT32_MIN, other_end = -1;
+        if (rc.gate) cls |= 1;
+        if (rc.keep) cls |= 2;
+        if (rc.keep && rc.has_blk()) { cls |= 16; if (rc.own()[0].pos != a.pos) cls |= 32; }
+        if (rc.conc) {
+            cls |= 4;
+            if (rc.part_f || rc.part_s) cls |= 8;
+            else cc_end = (a.first() ? rc.rd.F.front() : rc.rd.S.front()).pos + (a.first() ? rc.rd.F.front() : rc.rd.S.front()).mref;
+            flen = rc.own()[0].mref;
+            const std::vector<Blk> *ownp = rc.other_own();
+            if (ownp) {
+                if (ownp->size() > 1) cls |= 64;
+                other_end = ownp->front().pos + ownp->front().mref;
+            }
+        }
+        const bool same = a.mate_mapped() && a.mchr == a.chr;
+        const bool q = rc.gate && !(same && a.mpos > a.pos) && !(same && a.mpos == a.pos && a.second());
+        const int32_t row[9] = {cls, flen, cc_end, other_end, otherChr, otherRight, q, same ? a.mpos : a.pos, a.end()};
+        rows.insert(rows.end(), row, row + 9);
+        if (other_end >= 0) {
+            if (otherChr == a.chr) otherRight = std::max(otherRight, other_end); else { otherRight = other_end; otherChr = a.chr; }
+        }
+    }
+    const std::string d = outdir;
+    dump(d + "/classify_i32.bin", rows);
+    dump(d + "/readlen.bin", std::vector<int32_t>{g.o.read_len});
     return 0;
 }
 

@@ -73,7 +73,7 @@ CHIM_DTYPES = {
 EXPORTS = [
     "sqg_create", "sqg_destroy", "sqg_last_error", "sqg_load_concordant", "sqg_load_concordant_wire", "sqg_download_concordant", "sqg_connected_components", "sqg_attach_concordant_device", "sqg_load_chimeric",
     "sqg_build_nodes", "sqg_set_nodes", "sqg_build_edges", "sqg_bp_coverage", "sqg_edges_device_table", "sqg_merge_edge_tables",
-    "sqg_phase_ms", "sqg_launch_count", "sqg_stat", "sqg_selftest_gpu_sort",
+    "sqg_phase_ms", "sqg_launch_count", "sqg_stat", "sqg_classify_dump", "sqg_selftest_gpu_sort",
     "sqg_plan_shards", "sqg_set_shard", "sqg_shard_seeds", "sqg_shard_build", "sqg_shard_hint_state", "sqg_shard_redo_edges",
     "sqg_shard_cov_begin", "sqg_shard_cov_chain", "sqg_shard_cov_owned_t", "sqg_shard_cov_count",
     "sqh_default_options", "sqh_open_case", "sqh_open_concordant", "sqh_open_bam_case", "sqh_probe_bam", "sqh_close_case", "sqh_case_batch", "sqh_case_chimeric", "sqh_case_config",
@@ -117,6 +117,7 @@ def lib() -> C.CDLL:
     L.sqg_phase_ms.argtypes = [_P, C.c_char_p]; L.sqg_phase_ms.restype = C.c_float
     L.sqg_launch_count.argtypes = [_P]; L.sqg_launch_count.restype = C.c_int64
     L.sqg_stat.argtypes = [_P, C.c_char_p]; L.sqg_stat.restype = C.c_int64
+    L.sqg_classify_dump.argtypes = [_P, C.c_char_p, _P, C.c_int64, pp(C.c_int64)]
     L.sqg_plan_shards.argtypes = [pp(sqg_batch), pp(sqg_chimeric), pp(sqg_config), C.c_int32, C.c_int32, _P, pp(C.c_int32)]
     L.sqg_set_shard.argtypes = [_P, C.c_int32, C.c_int32]
     L.sqg_shard_seeds.argtypes = [_P, C.c_int32, pp(_P), pp(C.c_int64)]
@@ -564,6 +565,18 @@ class SegmentGraph:
 
     def stat(self, name: str) -> int:
         return int(self.L.sqg_stat(self._h, name.encode()))
+
+    CLASSIFY_DTYPES = {"cls": np.uint8, "first_len": np.uint16, "gap_rec": np.int32, "gap_key": np.uint64, "pc_rec": np.int32,
+                       "dp_rec": np.int32, "okmax_excl": np.uint64, "ccmax": np.int32, "cov_nq": np.uint32, "cov_qmax": np.uint64,
+                       "qstage_key": np.uint64, "qstage_end": np.int32}
+
+    def classify_dump(self, name: str) -> np.ndarray:
+        """One phase-1 array of the resident batch (sqg_classify_dump); call before BuildNode_STAR, which reuses the buffers."""
+        n = C.c_int64()
+        self._ck(self.L.sqg_classify_dump(self._h, name.encode(), None, 0, C.byref(n)))
+        out = np.zeros(n.value, self.CLASSIFY_DTYPES[name])
+        self._ck(self.L.sqg_classify_dump(self._h, name.encode(), out.ctypes.data, out.shape[0], C.byref(n)))
+        return out
 
 
 def ExactBreakpoint(final_nodes: np.ndarray, Chimrecord: "ChimericReads", Concord_Dist_Pos: int = 50000, Concord_Dist_Idx: int = 20) -> np.ndarray:

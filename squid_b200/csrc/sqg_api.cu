@@ -691,6 +691,9 @@ int64_t sqg_stat(const sqg_ctx *ctx, const char *name) {
     if (n == "disc_blocks") return ctx->pre_nD;
     if (n == "sensitive_reads") return ctx->n_sensitive;
     if (n == "raw_edges") return ctx->n_raw_edges;
+    if (n == "first_kept") return ctx->first_kept;                  // first record that is gate-passing and not a duplicate (n_rec: none)
+    if (n == "end_other") return (int64_t)ctx->end_other;            // otherChr/otherrightmost key after the last record
+    if (n == "classify_attempts") return ctx->classify_attempts;    // 2: the coverage-gap candidate buffer overflowed and phase 1 ran again
     if (n == "edge_pass_attempts") return ctx->edge_pass_attempts;  // > 1: a list of the last edge pass overflowed and the pass ran again
     if (n == "r_break") return ctx->r_break;
     if (n == "seed_window_records") return ctx->h_counters.p ? ctx->h_counters.p[29] : -1;  // concordant-cluster window sizes summed over the groups
@@ -1275,7 +1278,7 @@ static int run_classify(sqg_ctx *ctx) {
     const int64_t n = b.n_rec;
     PHASE_BEGIN("classify");
     CK(ctx->d_counters.ensure(32)); CK(ctx->h_counters.ensure(32));
-    ctx->n_gap = 0; ctx->n_pc = 0; ctx->n_dp = 0; ctx->lmax = 0; ctx->first_kept = n; ctx->end_other = 0;
+    ctx->n_gap = 0; ctx->n_pc = 0; ctx->n_dp = 0; ctx->lmax = 0; ctx->first_kept = n; ctx->end_other = 0; ctx->classify_attempts = 0;
     if (n > 0) {
         const int64_t n_tiles = (n + kTile - 1) / kTile;
         int64_t cand_cap = std::max<int64_t>({(int64_t)ctx->d_cand_key.cap, n / 16, (int64_t)1 << 20});
@@ -1306,6 +1309,7 @@ static int run_classify(sqg_ctx *ctx) {
             if (flags & 4) FAIL(SQG_EUNSUPPORTED, "record with more than 16 aligned blocks or a decreasing blk_off");
             if (flags & 8) FAIL(SQG_EINVAL, "batch is not sorted by (ref_id, pos)");
             n_cand = *(int32_t *)(ctx->h_counters.p + 4);
+            ctx->classify_attempts = attempt + 1;
             if (!(flags & 16)) break;
             if (attempt == 1) FAIL(SQG_ENOMEM, "coverage-gap candidate buffer overflow");
             cand_cap = n + 1;  // every record can be a candidate at worst
@@ -1334,6 +1338,45 @@ static int run_classify(sqg_ctx *ctx) {
         CK(ctx->d_gap.ensure(1)); CK(ctx->d_other.ensure(1)); CK(ctx->d_pc.ensure(1)); CK(ctx->d_dp.ensure(1));
     }
     ctx->classified = true;
+    return SQG_OK;
+}
+
+// Test seam of phase 1: one named output of the classification (run first if it has not run on the resident batch) copied to
+// host memory.  Valid before sqg_build_nodes, which reuses some of these buffers.
+extern "C" int sqg_classify_dump(sqg_ctx *ctx, const char *name, void *out, int64_t cap, int64_t *n_out) {
+    if (!ctx || !name || !n_out || cap < 0) return SQG_EINVAL;
+    if (!ctx->have_batch) FAIL(SQG_ESTATE, "no concordant batch");
+    CK(cudaSetDevice(ctx->device));
+    { const int rc = run_classify(ctx); if (rc) return rc; }
+    const std::string k(name);
+    const int64_t n = ctx->batch.n_rec, n_tiles = (n + kTile - 1) / kTile;
+    const void *src = nullptr;
+    int64_t cnt = 0;
+    size_t elem = 0;
+    if (k == "cls") { src = ctx->d_cls.p; cnt = n; elem = 1; }
+    else if (k == "first_len") { src = ctx->d_flen.p; cnt = n; elem = 2; }
+    else if (k == "gap_rec") { src = ctx->d_gap.p; cnt = ctx->n_gap; elem = 4; }
+    else if (k == "gap_key") { src = ctx->d_other.p; cnt = ctx->n_gap; elem = 8; }
+    else if (k == "pc_rec") { src = ctx->d_pc.p; cnt = ctx->n_pc; elem = 4; }
+    else if (k == "dp_rec") { src = ctx->d_dp.p; cnt = ctx->n_dp; elem = 4; }
+    else if (k == "okmax_excl") { cnt = n_tiles; elem = 8; }
+    else if (k == "ccmax") { src = ctx->d_ccmax.p; cnt = n_tiles; elem = 4; }
+    else if (k == "cov_nq") { src = ctx->d_cov_nq.p; cnt = n_tiles; elem = 4; }
+    else if (k == "cov_qmax") { src = ctx->d_cov_qmax.p; cnt = n_tiles; elem = 8; }
+    else if (k == "qstage_key") { src = ctx->d_qstage_key.p; cnt = n; elem = 8; }
+    else if (k == "qstage_end") { src = ctx->d_qstage_end.p; cnt = n; elem = 4; }
+    else FAIL(SQG_EINVAL, "sqg_classify_dump: unknown array " + k);
+    *n_out = cnt;
+    if (!out || cap < cnt || cnt == 0) return SQG_OK;
+    if (k == "okmax_excl") {  // the okmax member of the tile aggregates (exclusive maxima after k_tile_scan)
+        std::vector<TileAgg> agg((size_t)cnt);
+        CK(cudaMemcpyAsync(agg.data(), ctx->d_tileagg.p, (size_t)cnt * sizeof(TileAgg), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        for (int64_t t = 0; t < cnt; t++) ((uint64_t *)out)[t] = agg[(size_t)t].okmax;
+        return SQG_OK;
+    }
+    CK(cudaMemcpyAsync(out, src, (size_t)cnt * elem, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     return SQG_OK;
 }
 

@@ -209,6 +209,7 @@ struct sqg_ctx {
     int32_t n_heavy = 0;
     bool cov_chain_fallback = false;
     int64_t n_sensitive = 0, n_raw_edges = 0;
+    int32_t classify_attempts = 0;   // passes the last run_classify needed (2: the coverage-gap candidate buffer overflowed)
     int32_t edge_pass_attempts = 0;  // passes the last run_assign needed (1 unless a list overflowed; at most 4)
     sq::DBuf<int64_t> d_off_ops, d_off_mar;
     sq::DBuf<int32_t> d_margin;

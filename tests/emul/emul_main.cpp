@@ -106,6 +106,19 @@ int main(int argc, char **argv) {
         if ((cls[r] & CLS_CONC) && (cls[r] & CLS_DISPL)) dprec.push_back((int32_t)r);
         if (cls[r] & CLS_CONC) lmax = std::max(lmax, b.blk_match_ref[b.blk_off[r]]);
     }
+    if (getenv("SQ_EMUL_CLASSIFY")) {  // phase 1's outputs, in the layouts of sqg_classify_dump; then stop
+        outdir = getenv("SQ_EMUL_CLASSIFY");
+        dump_i32("cls_i32.bin", std::vector<int32_t>(cls.begin(), cls.end()));
+        dump_i32("first_len_i32.bin", std::vector<int32_t>(first_len.begin(), first_len.end()));
+        dump_i32("gap_rec_i32.bin", gap);
+        std::vector<int32_t> go;
+        for (uint64_t k : gap_other) { go.push_back((int32_t)(k >> 32)); go.push_back((int32_t)(uint32_t)k); }
+        dump_i32("gap_key_2xi32.bin", go);
+        dump_i32("pc_rec_i32.bin", pcrec);
+        dump_i32("dp_rec_i32.bin", dprec);
+        dump_i32("lmax_first_kept_i32.bin", std::vector<int32_t>{lmax, (int32_t)first_kept});
+        return 0;
+    }
     const int32_t nD = (int32_t)pre.disc.size() - 1, nG = (int32_t)pre.groups.size();
     std::vector<int64_t> trig(nG);
     for (int32_t g = 0; g < nG; g++) {

@@ -144,3 +144,52 @@ def test_edges_on_injected_tables(family_cases, case, family, opts, bin_shift, f
     r = subprocess.run([emul_bin, cp, hp, str(tmp_path / "emu")], capture_output=True, text=True, env=env)
     assert r.returncode == 0, r.stderr[-2000:]
     common.assert_same(want, pyref.load_dumps(str(tmp_path / "emu")), ("edges", "chim_after_edges"))
+
+
+@pytest.fixture(scope="module")
+def stream_families(tmp_path_factory):
+    return common.write_stream_families(tmp_path_factory.mktemp("streams"))
+
+
+def _emul_phase1(emul_bin, cp, hp, d):
+    os.makedirs(d)
+    r = subprocess.run([emul_bin, cp, hp, d], capture_output=True, text=True, env=dict(os.environ, SQ_EMUL_CLASSIFY=d))
+    assert r.returncode == 0, r.stderr[-2000:]
+    rd = lambda f: np.fromfile(os.path.join(d, f), np.int32)
+    gk = rd("gap_key_2xi32.bin").reshape(-1, 2).astype(np.int64)
+    lm = rd("lmax_first_kept_i32.bin")
+    return {"cls": rd("cls_i32.bin"), "first_len": rd("first_len_i32.bin"), "gap_rec": rd("gap_rec_i32.bin"),
+            "gap_key": ((gk[:, 0] << 32) | (gk[:, 1] & 0xFFFFFFFF)).astype(np.uint64), "pc_rec": rd("pc_rec_i32.bin"),
+            "dp_rec": rd("dp_rec_i32.bin"), "lmax": int(lm[0]), "first_kept": int(lm[1])}
+
+
+@pytest.mark.parametrize("family", common.FAMILY_STREAMS)
+def test_classify_rules_match_restatement(stream_families, family, emul_bin, tmp_path):
+    """The classification rules (sq_classify.cuh) stepped record by record against the restatement's own per-record preamble of
+    BuildNode_STAR (sqo_classify) on every stream family: class bytes, first-block lengths, the coverage-gap list and its
+    otherrightmost keys, the partial and displaced lists, lmax and the first kept record.  A difference here is a wrong rule; a
+    difference only on the device (tests/test_gpu_classify.py) is a wrong decomposition."""
+    cp, hp, tab = stream_families[family]
+    want = common.expected_phase1(pyref.run_restate_classify(cp, hp, str(tmp_path / "ref")), tab.ref_id, tab.pos)
+    got = _emul_phase1(emul_bin, cp, hp, str(tmp_path / "emu"))
+    for k in ("cls", "first_len", "gap_rec", "gap_key", "pc_rec", "dp_rec"):
+        a, b = want[k].astype(np.int64), got[k].astype(np.int64)
+        assert a.shape == b.shape, (k, a.shape, b.shape)
+        bad = np.flatnonzero(a != b)
+        assert bad.size == 0, "%s differs at %s: restatement %s emul %s" % (k, bad[:5], a[bad[:5]], b[bad[:5]])
+    assert (got["lmax"], got["first_kept"]) == (want["lmax"], want["first_kept"])
+    if family == "long_first_block":
+        assert want["lmax"] == 70100 and (want["first_len"] == 65535).sum() > 0
+    if family == "dup_shapes":
+        assert want["first_kept"] == 1  # the leading empty record equals the default-constructed ReadRec_t
+
+
+@pytest.mark.parametrize("family", common.FAMILY_STREAMS)
+def test_stream_families_end_to_end(stream_families, family, emul_bin, tmp_path):
+    """Segments, AvgDepth, edges and trimmed chimeric blocks of the stepped rules against sqo_run on every stream family."""
+    cp, hp, _ = stream_families[family]
+    want = pyref.run_restate(cp, hp, str(tmp_path / "ref"), stop_after=3)
+    os.makedirs(str(tmp_path / "emu"))
+    r = subprocess.run([emul_bin, cp, hp, str(tmp_path / "emu")], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-2000:]
+    common.assert_same(want, pyref.load_dumps(str(tmp_path / "emu")))
