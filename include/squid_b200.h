@@ -140,6 +140,28 @@ typedef struct sqg_wire {
  * resident sqg_batch layout by k_wire_decode -- and classified -- while the next ones are still in flight.  Page-locked arrays make the copies
  * asynchronous.  An inconsistent wire batch is reported (SQG_EINVAL) by the next sqg_build_nodes/sqg_build_edges/sqg_bp_coverage. */
 int sqg_load_concordant_wire(sqg_ctx *ctx, const sqg_wire *wire, int64_t first_record_index);
+/*
+ * sqg_load_concordant() straight from the concordant BAM file (BGZF, or an uncompressed BAM stream): the compressed bytes go to
+ * HBM and are inflated, cut into records and decoded there, into the same resident batch that sqh_open_bam_case packs from the
+ * same file (bit-identical), so every phase after the load runs unchanged.  The inflated stream is processed in windows of whole
+ * BGZF members (about 1 GiB; SQG_BAM_WINDOW_MB), so it never has to be resident as a whole.  `opt` carries the decode inputs of the
+ * host packer: the quality offset and -pm threshold of the low-quality run, and ChimName (the suffix-stripped Qnames of the
+ * chimeric reads and the empty name: sqh_case_chim_names of a case opened with sqh_open_bam_chimeric) as n_names names, name i =
+ * names[name_off[i], name_off[i+1]); n_names = 0 probes no names.  Refusals, with the host front end's wording:
+ *   SQG_EINVAL        not BGZF, no BC subfield, truncated member, member > 64 KiB, corrupt deflate stream (ISIZE mismatch
+ *                     included), CRC32 mismatch, malformed header or record;
+ *   SQG_EUNSUPPORTED  more than 16 blocks or TotalLen > 65535 in a record, >= 2^31 records, >= 2^32 blocks.
+ * A refused load leaves no batch; the context stays usable.  Phases "bam_h2d", "bam_inflate", "bam_records", "bam_decode" (summed
+ * over the windows); stats "bam_members", "bam_windows", "bam_repair_rounds".
+ */
+typedef struct sqg_bam_decode {
+    int32_t phred33;     /* 1: qualities offset 33 (Phred_Type) */
+    int32_t min_phred;   /* -pm */
+    int64_t n_names;
+    const char *names;
+    const int64_t *name_off;  /* n_names + 1 */
+} sqg_bam_decode;
+int sqg_load_concordant_bam(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, int64_t first_record_index);
 /* Copies the resident batch back into caller-allocated host arrays of `out` (n_rec / n_blk must match): the check that a wire
  * upload reproduces the sqg_batch it was packed from. */
 int sqg_download_concordant(sqg_ctx *ctx, sqg_batch *out);

@@ -29,6 +29,13 @@ int sqh_open_case(const char *concordant_sqmb, const char *chimeric_sqmb, const 
  * GetNextAlignment on the path (src/ReadRec.cpp:271-279, 340-343; src/SegmentGraph.cpp:293-296, 1570-1577, 3126-3129).
  * The file is inflated on all cores and decoded once for all three phases (SURVEY.md 8f row 1). */
 int sqh_open_bam_case(const char *concordant_bam, const char *chimeric_bam, const sqh_options *opt, sqh_case **out, char *errbuf, int errlen);
+/* The chimeric BAM decoded as sqh_open_bam_case does, and only the header of the concordant BAM (ref_len, reference names): the
+ * case's concordant batch is empty, because sqg_load_concordant_bam (squid_b200.h) decodes that file on the device.  config.read_len
+ * and the chimeric reads come from the chimeric file. */
+int sqh_open_bam_chimeric(const char *concordant_bam, const char *chimeric_bam, const sqh_options *opt, sqh_case **out, char *errbuf, int errlen);
+/* The ChimName list the concordant packer probes (the suffix-stripped Qnames of the chimeric reads plus the empty name,
+ * src/SegmentGraph.cpp:196-201): *n names, name i = blob[off[i], off[i+1]).  Owned by the case. */
+int sqh_case_chim_names(const sqh_case *c, const char **blob, const int64_t **off, int64_t *n);
 /* The concordant file alone (SQMB), for a caller that already holds Chimrecord -- the binding of INTEGRATION.md
  * (integration/binding.cpp): chim_qnames[n_names] = the Qnames of Chimrecord, from which ChimName is built
  * (src/SegmentGraph.cpp:196-201).  The chimeric side of the case stays empty and config.read_len 0. */

@@ -54,6 +54,10 @@ WIRE_REC_EXC = np.dtype([("idx", "<u4"), ("ref_id", "<i4"), ("pos", "<i4"), ("ma
 WIRE_BLK_EXC = np.dtype([("idx", "<u4"), ("ref_pos", "<i4"), ("match_ref", "<i4")])
 
 
+class sqg_bam_decode(C.Structure):  # include/squid_b200.h
+    _fields_ = [("phred33", C.c_int32), ("min_phred", C.c_int32), ("n_names", C.c_int64), ("names", C.c_void_p), ("name_off", C.c_void_p)]
+
+
 class sqh_options(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("phred33", "max_lowphred_len", "min_phred", "min_mapq", "concord_dist_pos", "concord_dist_idx")]
 
@@ -71,12 +75,12 @@ CHIM_DTYPES = {
 }
 
 EXPORTS = [
-    "sqg_create", "sqg_destroy", "sqg_last_error", "sqg_load_concordant", "sqg_load_concordant_wire", "sqg_download_concordant", "sqg_connected_components", "sqg_attach_concordant_device", "sqg_load_chimeric",
+    "sqg_create", "sqg_destroy", "sqg_last_error", "sqg_load_concordant", "sqg_load_concordant_wire", "sqg_load_concordant_bam", "sqg_download_concordant", "sqg_connected_components", "sqg_attach_concordant_device", "sqg_load_chimeric",
     "sqg_build_nodes", "sqg_set_nodes", "sqg_build_edges", "sqg_bp_coverage", "sqg_edges_device_table", "sqg_merge_edge_tables",
     "sqg_phase_ms", "sqg_launch_count", "sqg_stat", "sqg_classify_dump", "sqg_selftest_gpu_sort",
     "sqg_plan_shards", "sqg_set_shard", "sqg_shard_seeds", "sqg_shard_build", "sqg_shard_hint_state", "sqg_shard_redo_edges",
     "sqg_shard_cov_begin", "sqg_shard_cov_chain", "sqg_shard_cov_owned_t", "sqg_shard_cov_count",
-    "sqh_default_options", "sqh_open_case", "sqh_open_concordant", "sqh_open_bam_case", "sqh_probe_bam", "sqh_close_case", "sqh_case_batch", "sqh_case_chimeric", "sqh_case_config",
+    "sqh_default_options", "sqh_open_case", "sqh_open_concordant", "sqh_open_bam_case", "sqh_open_bam_chimeric", "sqh_case_chim_names", "sqh_probe_bam", "sqh_close_case", "sqh_case_batch", "sqh_case_chimeric", "sqh_case_config",
     "sqh_case_n_ref", "sqh_case_ref_len", "sqh_case_blocks",
     "sqh_exact_breakpoint", "sqh_free", "sqh_write_graph", "sqh_write_bedpe", "sqh_pack_wire", "sqh_free_wire", "sqh_wire_bytes",
 ]
@@ -102,6 +106,7 @@ def lib() -> C.CDLL:
     L.sqg_load_concordant.argtypes = [_P, pp(sqg_batch), C.c_int64]
     L.sqg_attach_concordant_device.argtypes = [_P, pp(sqg_batch), C.c_int64]
     L.sqg_load_concordant_wire.argtypes = [_P, pp(sqg_wire), C.c_int64]
+    L.sqg_load_concordant_bam.argtypes = [_P, C.c_char_p, pp(sqg_bam_decode), C.c_int64]
     L.sqg_download_concordant.argtypes = [_P, pp(sqg_batch)]
     L.sqg_connected_components.argtypes = [C.c_int32, C.c_int64, _P, _P, C.c_int64, _P, pp(C.c_int32)]
     L.sqh_pack_wire.argtypes = [pp(sqg_batch), C.c_int32, pp(pp(sqg_wire))]
@@ -131,6 +136,8 @@ def lib() -> C.CDLL:
     L.sqh_default_options.argtypes = [pp(sqh_options)]; L.sqh_default_options.restype = None
     L.sqh_open_case.argtypes = [C.c_char_p, C.c_char_p, pp(sqh_options), pp(_P), C.c_char_p, C.c_int]
     L.sqh_open_bam_case.argtypes = [C.c_char_p, C.c_char_p, pp(sqh_options), pp(_P), C.c_char_p, C.c_int]
+    L.sqh_open_bam_chimeric.argtypes = [C.c_char_p, C.c_char_p, pp(sqh_options), pp(_P), C.c_char_p, C.c_int]
+    L.sqh_case_chim_names.argtypes = [_P, pp(_P), pp(_P), pp(C.c_int64)]
     L.sqh_close_case.argtypes = [_P]; L.sqh_close_case.restype = None
     L.sqh_case_batch.argtypes = [_P]; L.sqh_case_batch.restype = pp(sqg_batch)
     L.sqh_case_chimeric.argtypes = [_P]; L.sqh_case_chimeric.restype = pp(sqg_chimeric)
@@ -294,8 +301,12 @@ class ChimericReads:
 class HostCase:
     """Host twin front end: SQMB files -> Chimrecord + packed concordant batch (sqh_open_case)."""
 
-    def __init__(self, concordant_sqmb: str, chimeric_sqmb: str, bam: bool = False, **opts):
-        """bam=True: the two paths are coordinate-sorted BAM files (sqh_open_bam_case), else SQMB tables."""
+    def __init__(self, concordant_sqmb: str, chimeric_sqmb: str, bam: bool = False, header_only: bool = False, **opts):
+        """bam=True: the two paths are coordinate-sorted BAM files (sqh_open_bam_case), else SQMB tables.  header_only=True (BAM
+        only): the concordant file's header alone is read and the batch stays empty (sqh_open_bam_chimeric), for
+        SegmentGraph.load_concordant_bam, which decodes that file on the device."""
+        if header_only and not bam:
+            raise ValueError("header_only needs bam=True")
         L = lib()
         o = sqh_options()
         L.sqh_default_options(C.byref(o))
@@ -303,7 +314,8 @@ class HostCase:
             setattr(o, k, v)
         h = _P()
         err = C.create_string_buffer(512)
-        rc = (L.sqh_open_bam_case if bam else L.sqh_open_case)(concordant_sqmb.encode(), chimeric_sqmb.encode(), C.byref(o), C.byref(h), err, 512)
+        opener = L.sqh_open_bam_chimeric if header_only else L.sqh_open_bam_case if bam else L.sqh_open_case
+        rc = opener(concordant_sqmb.encode(), chimeric_sqmb.encode(), C.byref(o), C.byref(h), err, 512)
         if rc != 0:
             raise SquidB200Error(rc, err.value.decode())
         self._h = h
@@ -313,6 +325,16 @@ class HostCase:
         self.config = Config(True, o.phred33, g.max_lowphred_len, o.min_phred, g.min_mapq, g.concord_dist_pos, g.concord_dist_idx, g.read_len)
         n_ref = L.sqh_case_n_ref(h)
         self.ref_len = _np_from(C.cast(L.sqh_case_ref_len(h), _P), n_ref, np.int32)
+        self.options = o
+
+    def chim_names(self):
+        """The ChimName list the concordant packer probes, as (blob bytes, int64 offsets[n + 1])."""
+        blob, off, n = _P(), _P(), C.c_int64()
+        rc = lib().sqh_case_chim_names(self._h, C.byref(blob), C.byref(off), C.byref(n))
+        if rc != 0:
+            raise SquidB200Error(rc, "sqh_case_chim_names failed")
+        offs = _np_from(off, n.value + 1, np.int64)
+        return (C.string_at(blob.value, int(offs[-1])) if offs[-1] else b""), offs
 
     def blocks(self, r: int):
         L = lib()
@@ -407,6 +429,17 @@ class SegmentGraph:
     def load_concordant_wire(self, wire: "WireBatch", first_record_index: int = 0):
         self._wire = wire
         self._ck(self.L.sqg_load_concordant_wire(self._h, wire._h, int(first_record_index)))
+
+    def load_concordant_bam(self, path: str, case: "HostCase", first_record_index: int = 0):
+        """sqg_load_concordant_bam: the concordant BAM file inflated and decoded on the device into the resident batch -- the
+        batch sqh_open_bam_case would pack from it.  `case` (HostCase(conc, chim, bam=True, header_only=True)) gives the decode
+        options and ChimName."""
+        blob, off = case.chim_names()
+        self._names = (C.create_string_buffer(blob, max(1, len(blob))), np.ascontiguousarray(off, np.int64))
+        opt = sqg_bam_decode(int(case.options.phred33), int(case.options.min_phred), int(off.shape[0] - 1), C.cast(self._names[0], C.c_void_p).value,
+                             self._names[1].ctypes.data)
+        self._batch = None
+        self._ck(self.L.sqg_load_concordant_bam(self._h, path.encode(), C.byref(opt), int(first_record_index)))
 
     def download_concordant(self) -> "RecordBatch":
         """The resident batch copied back (check of the wire upload)."""

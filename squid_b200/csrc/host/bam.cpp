@@ -20,8 +20,6 @@ inline uint16_t rd16(const uint8_t *p) { uint16_t v; memcpy(&v, p, 2); return v;
 inline uint32_t rd32(const uint8_t *p) { uint32_t v; memcpy(&v, p, 4); return v; }
 inline int32_t rdi32(const uint8_t *p) { int32_t v; memcpy(&v, p, 4); return v; }
 
-struct Member { size_t cdata, clen, off; uint32_t isize; };  // deflate payload [cdata, cdata+clen) -> out[off, off+isize)
-
 // size in bytes of one aux value of type `t` starting at p (p points behind the type byte); 0 on malformed input
 size_t aux_size(char t, const uint8_t *p, const uint8_t *end) {
     switch (t) {
@@ -41,8 +39,8 @@ size_t aux_size(char t, const uint8_t *p, const uint8_t *end) {
 }
 }  // namespace
 
-bool bgzf_inflate_all(const uint8_t *d, size_t len, RawBuf<uint8_t> &out, std::string &err, int threads, std::vector<size_t> *member_off) {
-    std::vector<Member> mem;
+bool bgzf_parse_members(const uint8_t *d, size_t len, std::vector<BgzfMember> &mem, std::string &err) {
+    mem.clear();
     size_t o = 0, total = 0;
     while (o < len) {
         if (o + 18 > len || d[o] != 0x1f || d[o + 1] != 0x8b || d[o + 2] != 8 || !(d[o + 3] & 4)) { err = "not a BGZF member at offset " + std::to_string(o); return false; }
@@ -58,24 +56,31 @@ bool bgzf_inflate_all(const uint8_t *d, size_t len, RawBuf<uint8_t> &out, std::s
         if (bsize < 0) { err = "gzip member without a BC subfield (plain gzip is not BGZF)"; return false; }
         const size_t msize = (size_t)bsize + 1;
         if (o + msize > len || msize < (size_t)xlen + 20) { err = "truncated BGZF block"; return false; }
-        Member m;
-        m.cdata = o + 12 + xlen; m.clen = msize - xlen - 20; m.isize = rd32(d + o + msize - 4); m.off = total;
+        BgzfMember m;
+        m.cdata = o + 12 + xlen; m.clen = msize - xlen - 20; m.isize = rd32(d + o + msize - 4); m.crc = rd32(d + o + msize - 8); m.off = total;
         if (m.isize > 65536) { err = "BGZF block larger than 64 KiB"; return false; }
         total += m.isize;
         mem.push_back(m);
         o += msize;
     }
+    return true;
+}
+
+bool bgzf_inflate_all(const uint8_t *d, size_t len, RawBuf<uint8_t> &out, std::string &err, int threads, std::vector<size_t> *member_off) {
+    std::vector<BgzfMember> mem;
+    if (!bgzf_parse_members(d, len, mem, err)) return false;
+    const size_t total = mem.empty() ? 0 : mem.back().off + mem.back().isize;
     if (!out.resize(total)) { err = "out of memory"; return false; }
     if (member_off) {
         member_off->clear();
-        for (const Member &m : mem) if (m.isize) member_off->push_back(m.off);
+        for (const BgzfMember &m : mem) if (m.isize) member_off->push_back(m.off);
         member_off->push_back(total);
     }
     const int T = threads > 0 ? threads : omp_get_num_procs();
     int bad = 0;  // bit 0: corrupt deflate stream, bit 1: CRC mismatch
 #pragma omp parallel for num_threads(T) schedule(dynamic, 16) reduction(| : bad)
     for (long long i = 0; i < (long long)mem.size(); i++) {
-        const Member &m = mem[(size_t)i];
+        const BgzfMember &m = mem[(size_t)i];
         if (m.isize == 0) continue;  // the EOF marker
         z_stream z;
         memset(&z, 0, sizeof(z));
@@ -84,11 +89,80 @@ bool bgzf_inflate_all(const uint8_t *d, size_t len, RawBuf<uint8_t> &out, std::s
         z.next_out = out.data() + m.off; z.avail_out = m.isize;
         const int rc = inflate(&z, Z_FINISH);
         if (rc != Z_STREAM_END || z.avail_out != 0) bad |= 1;
-        else if (crc32(crc32(0L, Z_NULL, 0), out.data() + m.off, m.isize) != rd32(d + m.cdata + m.clen)) bad |= 2;
+        else if (crc32(crc32(0L, Z_NULL, 0), out.data() + m.off, m.isize) != m.crc) bad |= 2;
         inflateEnd(&z);
     }
     if (bad) { err = !(bad & 1) ? "BGZF block fails its CRC32" : "corrupt deflate stream in a BGZF block"; return false; }
     return true;
+}
+
+int bam_parse_header(const uint8_t *b, size_t n, std::vector<std::string> &ref_name, std::vector<int32_t> &ref_len, size_t &end, std::string &err) {
+    ref_name.clear(); ref_len.clear();
+    if (n < 12 || memcmp(b, "BAM\1", 4) != 0) { err = "not a BAM file (magic)"; return n < 12 && (n < 4 || memcmp(b, "BAM\1", 4) == 0) ? 0 : -1; }
+    size_t o = 4;
+    const int32_t l_text = rdi32(b + o); o += 4;
+    if (l_text < 0) { err = "truncated BAM header"; return -1; }
+    if (o + (size_t)l_text + 4 > n) { err = "truncated BAM header"; return 0; }
+    o += (size_t)l_text;
+    const int32_t n_ref = rdi32(b + o); o += 4;
+    if (n_ref < 0) { err = "truncated BAM reference list"; return -1; }
+    for (int32_t i = 0; i < n_ref; i++) {
+        if (o + 4 > n) { err = "truncated BAM reference list"; return 0; }
+        const int32_t l_name = rdi32(b + o); o += 4;
+        if (l_name < 1) { err = "truncated BAM reference list"; return -1; }
+        if (o + (size_t)l_name + 4 > n) { err = "truncated BAM reference list"; return 0; }
+        ref_name.emplace_back((const char *)b + o, (size_t)l_name - 1); o += (size_t)l_name;
+        ref_len.push_back(rdi32(b + o)); o += 4;
+    }
+    end = o;
+    return 1;
+}
+
+bool bam_read_header(const uint8_t *f, size_t flen, const std::vector<BgzfMember> *mem, std::vector<std::string> &ref_name, std::vector<int32_t> &ref_len,
+                     size_t &end, std::string &err) {
+    if (!mem) return bam_parse_header(f, flen, ref_name, ref_len, end, err) == 1;
+    std::vector<uint8_t> buf;
+    int rc = 0;
+    for (const BgzfMember &m : *mem) {
+        if (m.isize == 0) continue;
+        const size_t at = buf.size();
+        buf.resize(at + m.isize);
+        z_stream z;
+        memset(&z, 0, sizeof(z));
+        if (inflateInit2(&z, -15) != Z_OK) { err = "corrupt deflate stream in a BGZF block"; return false; }
+        z.next_in = const_cast<Bytef *>(f + m.cdata); z.avail_in = (uInt)m.clen;
+        z.next_out = buf.data() + at; z.avail_out = m.isize;
+        const int zr = inflate(&z, Z_FINISH);
+        const bool ok = zr == Z_STREAM_END && z.avail_out == 0;
+        inflateEnd(&z);
+        if (!ok) { err = "corrupt deflate stream in a BGZF block"; return false; }
+        if (crc32(crc32(0L, Z_NULL, 0), buf.data() + at, m.isize) != m.crc) { err = "BGZF block fails its CRC32"; return false; }
+        rc = bam_parse_header(buf.data(), buf.size(), ref_name, ref_len, end, err);
+        if (rc != 0) break;
+    }
+    if (rc == 0 && err.empty()) err = "not a BAM file (magic)";
+    return rc == 1;
+}
+
+bool bam_read_header_file(const std::string &path, std::vector<std::string> &ref_name, std::vector<int32_t> &ref_len, std::string &err) {
+    int fd = ::open(path.c_str(), O_RDONLY);
+    if (fd < 0) { err = "cannot open " + path; return false; }
+    struct stat st;
+    if (fstat(fd, &st) != 0 || st.st_size < 4) { ::close(fd); err = path + " is empty"; return false; }
+    const size_t flen = (size_t)st.st_size;
+    void *map = mmap(nullptr, flen, PROT_READ, MAP_PRIVATE, fd, 0);
+    ::close(fd);
+    if (map == MAP_FAILED) { err = "cannot map " + path; return false; }
+    const uint8_t *f = (const uint8_t *)map;
+    size_t end = 0;
+    bool ok;
+    if (memcmp(f, "BAM\1", 4) == 0) ok = bam_read_header(f, flen, nullptr, ref_name, ref_len, end, err);
+    else {
+        std::vector<BgzfMember> mem;
+        ok = bgzf_parse_members(f, flen, mem, err) && bam_read_header(f, flen, &mem, ref_name, ref_len, end, err);
+    }
+    munmap(map, flen);
+    return ok;
 }
 
 bool BamTable::open(const std::string &path, std::string &err, int threads) {
@@ -116,21 +190,8 @@ bool BamTable::open(const std::string &path, std::string &err, int threads) {
     lap("inflate");
     bool ok = false;
     do {
-        if (n < 12 || memcmp(b, "BAM\1", 4) != 0) { err = "not a BAM file (magic)"; break; }
-        size_t o = 4;
-        const int32_t l_text = rdi32(b + o); o += 4;
-        if (l_text < 0 || o + (size_t)l_text + 4 > n) { err = "truncated BAM header"; break; }
-        o += (size_t)l_text;
-        const int32_t n_ref = rdi32(b + o); o += 4;
-        bool hdr_ok = n_ref >= 0;
-        for (int32_t i = 0; hdr_ok && i < n_ref; i++) {
-            if (o + 4 > n) { hdr_ok = false; break; }
-            const int32_t l_name = rdi32(b + o); o += 4;
-            if (l_name < 1 || o + (size_t)l_name + 4 > n) { hdr_ok = false; break; }
-            ref_name.emplace_back((const char *)b + o, (size_t)l_name - 1); o += (size_t)l_name;
-            ref_len.push_back(rdi32(b + o)); o += 4;
-        }
-        if (!hdr_ok) { err = "truncated BAM reference list"; break; }
+        size_t o = 0;
+        if (bam_parse_header(b, n, ref_name, ref_len, o, err) != 1) break;
         // Record boundaries.  htslib never lets a record straddle two BGZF members (bgzf_flush_try before every record), so in
         // the files aligners and samtools write every member starts at a record boundary and the members can be walked
         // independently.  That is an assumption about the writer, so it is PROVEN before it is used: the walk of member k

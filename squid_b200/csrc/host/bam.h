@@ -48,6 +48,18 @@ struct BamTable {
     AlnSource source() const;
 };
 
+// One BGZF member: deflate payload [cdata, cdata + clen) of the file inflates to `isize` bytes at offset `off` of the stream.
+struct BgzfMember { size_t cdata, clen, off; uint32_t isize, crc; };
+// Locates every member of a BGZF file by its BC subfield (shared by the host inflater and the device loader, sqg_load_concordant_bam).
+bool bgzf_parse_members(const uint8_t *data, size_t len, std::vector<BgzfMember> &mem, std::string &err);
+// BAM header of an inflated stream prefix: 1 = parsed (`end` = offset of the first record), 0 = the prefix is too short, -1 = malformed.
+int bam_parse_header(const uint8_t *b, size_t n, std::vector<std::string> &ref_name, std::vector<int32_t> &ref_len, size_t &end, std::string &err);
+// The header of a mapped file: members inflated with zlib one by one until it is complete (mem = nullptr: an uncompressed stream).
+bool bam_read_header(const uint8_t *f, size_t flen, const std::vector<BgzfMember> *mem, std::vector<std::string> &ref_name, std::vector<int32_t> &ref_len,
+                     size_t &end, std::string &err);
+// bam_read_header() of a file on disk (BGZF or uncompressed)
+bool bam_read_header_file(const std::string &path, std::vector<std::string> &ref_name, std::vector<int32_t> &ref_len, std::string &err);
+
 // inflate a whole BGZF file (concatenated gzip members with BSIZE) on `threads` threads
 // (`member_off`, optional: offset of every member's data in `out`, plus the total as the last entry)
 bool bgzf_inflate_all(const uint8_t *data, size_t len, RawBuf<uint8_t> &out, std::string &err, int threads, std::vector<size_t> *member_off = nullptr);

@@ -23,6 +23,12 @@ struct sqh_case {
     sqg_chimeric cview;
     sqg_config gcfg;
     std::vector<int32_t> ref_len;
+    std::string chim_blob;               // the ChimName list the packer probes, as a blob with offsets (sqh_case_chim_names)
+    std::vector<int64_t> chim_off;
+    void set_chim_names(const std::unordered_set<std::string> &names) {
+        chim_blob.clear(); chim_off.assign(1, 0);
+        for (const std::string &s : names) { chim_blob += s; chim_off.push_back((int64_t)chim_blob.size()); }
+    }
 };
 
 extern "C" {
@@ -43,7 +49,7 @@ struct HostLaps {  // SQH_TIMING=1: wall-clock laps of the host front end, to st
     }
 };
 }  // namespace
-static int open_case(bool bam, const char *conc_path, const char *chim_path, const sqh_options *opt, sqh_case **out, char *errbuf, int errlen) {
+static int open_case(bool bam, bool conc_header_only, const char *conc_path, const char *chim_path, const sqh_options *opt, sqh_case **out, char *errbuf, int errlen) {
     auto fail = [&](int code, const std::string &m) { if (errbuf && errlen > 0) snprintf(errbuf, errlen, "%s", m.c_str()); return code; };
     if (!conc_path || !chim_path || !out) return fail(SQG_EINVAL, "null argument");
     *out = nullptr;
@@ -56,10 +62,13 @@ static int open_case(bool bam, const char *conc_path, const char *chim_path, con
     sqh::AlnSource sconc, schim;
     if (bam) {  // BGZF/BAM front end (host/bam.h): BamReader::Open + GetHeader + GetNextAlignment of the reference
         std::string e;
-        if (!c->bconc.open(conc_path, e)) { delete c; return fail(SQG_EINVAL, e); }
+        if (conc_header_only) {  // the records are decoded on the device (sqg_load_concordant_bam): an empty concordant source
+            std::vector<std::string> names;
+            if (!sqh::bam_read_header_file(conc_path, names, c->ref_len, e)) { delete c; return fail(SQG_EINVAL, e); }
+        } else if (!c->bconc.open(conc_path, e)) { delete c; return fail(SQG_EINVAL, e); }
         if (!c->bchim.open(chim_path, e)) { delete c; return fail(SQG_EINVAL, e); }
-        c->ref_len = c->bconc.ref_len;  // BuildRefName reads the header of the concordant BAM (ReadRec.cpp:267-283)
-        sconc = c->bconc.source(); schim = c->bchim.source();
+        if (!conc_header_only) { c->ref_len = c->bconc.ref_len; sconc = c->bconc.source(); }  // BuildRefName reads the header of the concordant BAM (ReadRec.cpp:267-283)
+        schim = c->bchim.source();
     } else {
         if (!c->conc.open(conc_path)) { delete c; return fail(SQG_EINVAL, std::string("cannot open ") + conc_path); }
         if (!c->chim.open(chim_path)) { delete c; return fail(SQG_EINVAL, std::string("cannot open ") + chim_path); }
@@ -73,6 +82,7 @@ static int open_case(bool bam, const char *conc_path, const char *chim_path, con
     std::unordered_set<std::string> names;
     names.insert("");  // ChimName is pre-sized with empty strings before the names are appended (SegmentGraph.cpp:196-198)
     for (const sqh::Read &r : c->reads) names.insert(r.qname);
+    c->set_chim_names(names);
     lap("ChimName set");
     std::string err;
     int rc = sqh::pack_concordant(sconc, c->cfg, names, c->batch, err);
@@ -88,10 +98,13 @@ static int open_case(bool bam, const char *conc_path, const char *chim_path, con
     return SQG_OK;
 }
 int sqh_open_case(const char *conc_path, const char *chim_path, const sqh_options *opt, sqh_case **out, char *errbuf, int errlen) {
-    return open_case(false, conc_path, chim_path, opt, out, errbuf, errlen);
+    return open_case(false, false, conc_path, chim_path, opt, out, errbuf, errlen);
 }
 int sqh_open_bam_case(const char *conc_bam, const char *chim_bam, const sqh_options *opt, sqh_case **out, char *errbuf, int errlen) {
-    return open_case(true, conc_bam, chim_bam, opt, out, errbuf, errlen);
+    return open_case(true, false, conc_bam, chim_bam, opt, out, errbuf, errlen);
+}
+int sqh_open_bam_chimeric(const char *conc_bam, const char *chim_bam, const sqh_options *opt, sqh_case **out, char *errbuf, int errlen) {
+    return open_case(true, true, conc_bam, chim_bam, opt, out, errbuf, errlen);
 }
 // The concordant BAM alone, for a caller that already holds Chimrecord (the binding of INTEGRATION.md): ChimName is built from
 // the Qnames it passes (SegmentGraph.cpp:196-201), the chimeric side of the case stays empty.
@@ -110,6 +123,7 @@ int sqh_open_concordant(const char *conc_path, const char *const *chim_qnames, i
     std::unordered_set<std::string> names;
     names.insert("");  // ChimName is pre-sized with empty strings before the names are appended (SegmentGraph.cpp:196-198)
     for (int64_t i = 0; i < n_names; i++) names.insert(chim_qnames[i] ? chim_qnames[i] : "");
+    c->set_chim_names(names);
     std::string err;
     const int rc = sqh::pack_concordant(sqh::source_of(c->conc), c->cfg, names, c->batch, err);
     if (rc) { delete c; return fail(rc, err); }
@@ -125,6 +139,11 @@ void sqh_close_case(sqh_case *c) { delete c; }
 const sqg_batch *sqh_case_batch(const sqh_case *c) { return c ? &c->bview : nullptr; }
 sqg_chimeric *sqh_case_chimeric(sqh_case *c) { return c ? &c->cview : nullptr; }
 const sqg_config *sqh_case_config(const sqh_case *c) { return c ? &c->gcfg : nullptr; }
+int sqh_case_chim_names(const sqh_case *c, const char **blob, const int64_t **off, int64_t *n) {
+    if (!c || !blob || !off || !n) return SQG_EINVAL;
+    *blob = c->chim_blob.data(); *off = c->chim_off.data(); *n = (int64_t)c->chim_off.size() - 1;
+    return SQG_OK;
+}
 int32_t sqh_case_n_ref(const sqh_case *c) { return c ? (int32_t)c->ref_len.size() : 0; }
 const int32_t *sqh_case_ref_len(const sqh_case *c) { return c ? c->ref_len.data() : nullptr; }
 int32_t sqh_case_blocks(const sqh_case *c, int64_t r, int32_t *out4, int32_t max_blocks, int32_t *total_len, int32_t *lowphred_run) {

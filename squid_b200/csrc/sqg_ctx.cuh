@@ -13,6 +13,7 @@
 #include <vector>
 
 #include "host/prepass.h"
+#include "sq_bam.cuh"
 #include "sq_common.cuh"
 #include "sq_seed.cuh"
 #include "sq_phase1.cuh"
@@ -35,6 +36,19 @@ template <class T> struct DBuf {
         return e;
     }
     void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+    // capacity for n elements keeping the first `used` (geometric growth: a batch whose size is only known window by window)
+    cudaError_t grow(size_t n, size_t used, cudaStream_t st) {
+        if (n <= cap) return cudaSuccess;
+        const size_t want = n + n / 8 + 64 > 2 * cap ? n + n / 8 + 64 : 2 * cap;
+        T *q = nullptr;
+        cudaError_t e = cudaMalloc((void **)&q, want * sizeof(T));
+        if (e != cudaSuccess) return e;
+        if (used && p) e = cudaMemcpyAsync(q, p, used * sizeof(T), cudaMemcpyDeviceToDevice, st);
+        if (e != cudaSuccess) { cudaFree(q); return e; }
+        if (p) cudaFree(p);  // (waits for the device, so the copy is complete)
+        p = q; cap = want;
+        return cudaSuccess;
+    }
 };
 template <class T> struct HBuf {  // pinned host
     T *p = nullptr;
@@ -129,6 +143,23 @@ struct sqg_ctx {
     // classification launched chunk by chunk behind the widening kernels of a wire upload (run_classify then only finishes it)
     bool classify_prelaunched = false;
     int64_t pre_cand_cap = 0;
+
+    // device BAM decode (sqg_load_concordant_bam): compressed window, two inflated windows (the tail of one is the head of the
+    // next), segment walks, record offsets, per-record block counts, the ChimName hash set, pinned staging of the file
+    sq::DBuf<uint8_t> bam_comp, bam_win[2], bam_nblob;
+    sq::DBuf<sq::BamMember> bam_mem;
+    sq::DBuf<int64_t> bam_seg, bam_start, bam_exit, bam_newstart, bam_recoff, bam_small, bam_noff;
+    sq::DBuf<uint32_t> bam_cnt, bam_base, bam_nblk;
+    sq::DBuf<uint64_t> bam_incl, bam_nhash;
+    sq::DBuf<int32_t> bam_nlen;
+    sq::DBuf<uint8_t> bam_bad, bam_redo;
+    sq::DBuf<uint16_t> bam_lseq;           // read length from the CIGAR, kept only for the synthesised-quality rule (see sqg_api.cu)
+    sq::HBuf<uint8_t> bam_stage[2];
+    sq::HBuf<int64_t> bam_hsmall;
+    std::vector<cudaEvent_t> bam_ev;       // [0..1]: staging buffer free again
+    std::map<std::string, float> acc_ms;   // phases summed over the windows of the last BAM load
+    int64_t bam_members = -1, bam_windows = -1, bam_repair_rounds = -1;
+    int64_t bam_win_len = 0;               // bytes of the previous window (its unconsumed tail is copied to the front of the next)
 
     // classify products
     sq::DBuf<uint8_t> d_cls;
