@@ -14,29 +14,14 @@
 #include <cstdlib>
 #include <cstring>
 
+#include "sq_bam.cuh"
+
 namespace sqh {
 namespace {
 inline uint16_t rd16(const uint8_t *p) { uint16_t v; memcpy(&v, p, 2); return v; }
 inline uint32_t rd32(const uint8_t *p) { uint32_t v; memcpy(&v, p, 4); return v; }
 inline int32_t rdi32(const uint8_t *p) { int32_t v; memcpy(&v, p, 4); return v; }
 
-// size in bytes of one aux value of type `t` starting at p (p points behind the type byte); 0 on malformed input
-size_t aux_size(char t, const uint8_t *p, const uint8_t *end) {
-    switch (t) {
-        case 'A': case 'c': case 'C': return 1;
-        case 's': case 'S': return 2;
-        case 'i': case 'I': case 'f': return 4;
-        case 'Z': case 'H': { const uint8_t *q = p; while (q < end && *q) q++; return q < end ? (size_t)(q - p) + 1 : 0; }
-        case 'B': {
-            if (p + 5 > end) return 0;
-            const char st = (char)p[0];
-            const uint32_t cnt = rd32(p + 1);
-            const size_t es = (st == 'c' || st == 'C') ? 1 : (st == 's' || st == 'S') ? 2 : (st == 'i' || st == 'I' || st == 'f') ? 4 : 0;
-            return es ? 5 + (size_t)cnt * es : 0;
-        }
-        default: return 0;
-    }
-}
 }  // namespace
 
 bool bgzf_parse_members(const uint8_t *d, size_t len, std::vector<BgzfMember> &mem, std::string &err) {
@@ -209,16 +194,14 @@ bool BamTable::open(const std::string &path, std::string &err, int threads) {
         auto walk = [&](size_t a, size_t e, Tot &t, size_t *rec_out, uint64_t *no, uint64_t *co, uint64_t *so) -> bool {
             size_t p = a;
             while (p < e) {
-                if (p + 4 > e) return false;
-                const int32_t bs = rdi32(b + p);
-                if (bs < 32 || p + 4 + (size_t)bs > e) return false;
+                // the variable-length fields have to fit the record before their sizes enter the totals that size the allocations
+                int64_t next = 0;
+                if (sq::bam_rec_check(b, (int64_t)p, (int64_t)e, (int64_t)e, &next) != 1) return false;
                 const uint8_t *q = b + p + 4;
                 const uint32_t l_name = q[8], n_cig = rd16(q + 12), l_seq = rd32(q + 16);
-                // the variable-length fields have to fit the record before their sizes enter the totals that size the allocations
-                if (32ull + l_name + 4ull * n_cig + ((uint64_t)l_seq + 1) / 2 + l_seq > (uint64_t)bs) return false;
                 if (rec_out) { rec_out[t.rec] = p + 4; no[t.rec] = t.name; co[t.rec] = t.cig; so[t.rec] = t.seq; }
                 t.rec++; t.name += l_name ? l_name - 1 : 0; t.cig += n_cig; t.seq += l_seq;
-                p += 4 + (size_t)bs;
+                p = (size_t)next;
             }
             return true;
         };
@@ -268,7 +251,6 @@ bool BamTable::open(const std::string &path, std::string &err, int threads) {
             const uint32_t l_seq = rd32(p + 16);
             mate_ref_id[r] = rdi32(p + 20); mate_pos[r] = rdi32(p + 24);
             const uint8_t *q = p + 32;
-            if (q + l_name + 4ull * n_cig + (l_seq + 1) / 2 + l_seq > end) { bad |= 1; continue; }
             if (l_name) memcpy(names.data() + name_off[r], q, l_name - 1);
             q += l_name;
             memcpy(cigar.data() + cigar_off[r], q, 4ull * n_cig);
@@ -279,31 +261,16 @@ bool BamTable::open(const std::string &path, std::string &err, int threads) {
                 for (int v = 0; v < 256; v++) t[(size_t)v] = (uint16_t)((uint8_t)code[v >> 4] | ((uint16_t)(uint8_t)code[v & 15] << 8));
                 return t;
             }();
-            char *sq = seq.data() + seq_off[r], *ql = qual.data() + seq_off[r];
-            for (uint32_t k = 0; k + 1 < l_seq; k += 2) { const uint16_t w = pair[q[k >> 1]]; memcpy(sq + k, &w, 2); }
-            if (l_seq & 1) sq[l_seq - 1] = code[q[l_seq >> 1] >> 4];
+            char *sb = seq.data() + seq_off[r], *ql = qual.data() + seq_off[r];
+            for (uint32_t k = 0; k + 1 < l_seq; k += 2) { const uint16_t w = pair[q[k >> 1]]; memcpy(sb + k, &w, 2); }
+            if (l_seq & 1) sb[l_seq - 1] = code[q[l_seq >> 1] >> 4];
             q += (l_seq + 1) / 2;
             for (uint32_t k = 0; k < l_seq; k++) ql[k] = (char)(uint8_t)(q[k] + 33);
             q += l_seq;
-            while (q + 3 <= end) {  // aux: tag[2] type value
-                const char t0 = (char)q[0], t1 = (char)q[1], ty = (char)q[2];
-                const size_t sz = aux_size(ty, q + 3, end);
-                if (sz == 0 || q + 3 + sz > end) { bad |= 1; break; }
-                if (t0 == 'X' && t1 == 'A') tags[r] |= 1;
-                else if (t0 == 'I' && t1 == 'H') {
-                    tags[r] |= 2;
-                    const uint8_t *v = q + 3;
-                    // BamTools' GetTag<int>: the destination is zeroed and the 1, 2 or 4 value bytes are copied over its low end --
-                    // no sign extension of the narrow signed types; 'A' (one character) converts as well
-                    switch (ty) {
-                        case 'A': case 'c': case 'C': ih[r] = v[0]; break;
-                        case 's': case 'S': ih[r] = rd16(v); break;
-                        case 'i': case 'I': ih[r] = (int32_t)rd32(v); break;
-                        default: break;  // GetTag<int> fails on any other type: the value stays 0
-                    }
-                }
-                q += 3 + sz;
-            }
+            sq::BamAux a;
+            if (!sq::bam_aux_scan(q, end, a)) bad |= 1;
+            tags[r] = (uint8_t)(a.xa | a.ih << 1);
+            ih[r] = a.ih_value;
         }
         if (bad) { err = "malformed BAM alignment record"; break; }
         lap("fields");
@@ -312,6 +279,52 @@ bool BamTable::open(const std::string &path, std::string &err, int threads) {
     munmap(map, flen);
     if (!ok) *this = BamTable();
     return ok;
+}
+
+bool bam_loader_members(const uint8_t *f, size_t len, bool raw, std::vector<BgzfMember> &mem, std::string &err) {
+    mem.clear();
+    if (raw) {
+        for (size_t o = 0; o < len; o += 65536) mem.push_back(BgzfMember{o, std::min<size_t>(65536, len - o), o, (uint32_t)std::min<size_t>(65536, len - o), kRawMember});
+        return true;
+    }
+    if (!bgzf_parse_members(f, len, mem, err)) return false;
+    mem.erase(std::remove_if(mem.begin(), mem.end(), [](const BgzfMember &m) { return m.isize == 0; }), mem.end());
+    return true;
+}
+
+std::vector<size_t> bam_window_cuts(const std::vector<BgzfMember> &mem, int64_t win_bytes, size_t hdr_end) {
+    std::vector<size_t> cut{0};
+    for (size_t i = 0; i < mem.size();) {
+        size_t j = i;
+        int64_t bytes = 0;
+        while (j < mem.size() && (j == i || bytes + mem[j].isize <= win_bytes || (cut.size() == 1 && mem[j].off <= hdr_end))) { bytes += mem[j].isize; j++; }
+        cut.push_back(j);
+        i = j;
+    }
+    return cut;
+}
+
+std::vector<int64_t> bam_window_segments(const std::vector<BgzfMember> &mem, const std::vector<size_t> &cut, size_t w, int64_t carry, size_t hdr_end) {
+    std::vector<int64_t> seg{w == 0 ? (int64_t)hdr_end : 0};
+    const int64_t wstream = (int64_t)mem[cut[w]].off;
+    for (size_t i = cut[w]; i < cut[w + 1]; i++) { const int64_t s = carry + ((int64_t)mem[i].off - wstream); if (s > seg[0]) seg.push_back(s); }
+    return seg;
+}
+
+NameTable bam_name_table(const char *blob, const int64_t *name_off, int64_t n) {
+    size_t cap = 2;
+    while (cap < 2 * (size_t)n) cap <<= 1;
+    NameTable t{std::vector<uint64_t>(cap, 0), std::vector<int32_t>(cap, -1), std::vector<int64_t>(cap, 0)};
+    for (int64_t i = 0; i < n; i++) {
+        const uint8_t *p = (const uint8_t *)blob + name_off[i];
+        const uint32_t len = (uint32_t)(name_off[i + 1] - name_off[i]);
+        const uint64_t h = sq::name_hash(p, len);
+        size_t k = h & (cap - 1);
+        for (; t.len[k] >= 0; k = (k + 1) & (cap - 1))
+            if (t.hash[k] == h && (uint32_t)t.len[k] == len && memcmp(blob + t.off[k], p, len) == 0) break;
+        t.hash[k] = h; t.len[k] = (int32_t)len; t.off[k] = name_off[i];
+    }
+    return t;
 }
 
 }  // namespace sqh

@@ -60,6 +60,22 @@ bool bam_read_header(const uint8_t *f, size_t flen, const std::vector<BgzfMember
 // bam_read_header() of a file on disk (BGZF or uncompressed)
 bool bam_read_header_file(const std::string &path, std::vector<std::string> &ref_name, std::vector<int32_t> &ref_len, std::string &err);
 
+// The plan of the device loader (sqg_load_concordant_bam), which its CPU stepping (tests/emul/emul_bam.cpp) runs as well.
+constexpr uint32_t kRawMember = 0xFFFFFFFFu;  // crc of a pseudo-member of an uncompressed stream: copied, not inflated
+// The members a mapped file is uploaded in: its BGZF members with data (EOF markers dropped), or for an uncompressed stream (raw)
+// 64 KiB pieces that stand in for members (segment starts of the record walk).
+bool bam_loader_members(const uint8_t *f, size_t len, bool raw, std::vector<BgzfMember> &mem, std::string &err);
+// Windows of whole members, about win_bytes inflated bytes each, the first one holding the whole header: window w is the members
+// [cut[w], cut[w + 1]).
+std::vector<size_t> bam_window_cuts(const std::vector<BgzfMember> &mem, int64_t win_bytes, size_t hdr_end);
+// Walk segments of window w in its buffer, behind the `carry` bytes of the previous window's tail: the first record start (the
+// end of the header in window 0) and every member start past it.
+std::vector<int64_t> bam_window_segments(const std::vector<BgzfMember> &mem, const std::vector<size_t> &cut, size_t w, int64_t carry, size_t hdr_end);
+// ChimName as the loader probes it (sq_bam.cuh NameSet): open addressing over the names' hashes, duplicates dropped, each slot with
+// its name's length (-1: empty) and offset into the blob for the exact compare.
+struct NameTable { std::vector<uint64_t> hash; std::vector<int32_t> len; std::vector<int64_t> off; };
+NameTable bam_name_table(const char *blob, const int64_t *name_off, int64_t n);
+
 // inflate a whole BGZF file (concatenated gzip members with BSIZE) on `threads` threads
 // (`member_off`, optional: offset of every member's data in `out`, plus the total as the last entry)
 bool bgzf_inflate_all(const uint8_t *data, size_t len, RawBuf<uint8_t> &out, std::string &err, int threads, std::vector<size_t> *member_off = nullptr);

@@ -7,6 +7,8 @@
 #include <cstdlib>
 #include <thread>
 
+#include "sq_cigar.cuh"
+
 namespace sqh {
 
 Alignment alignment_at(const SqmbView &v, uint64_t r) {
@@ -127,6 +129,12 @@ sqg_batch PackedBatch::view() const {
     return b;
 }
 
+std::string packer_refusal(uint64_t r, int limit, int64_t total_len) {
+    if (limit == 1) return "record " + std::to_string(r) + " has more than 16 aligned blocks";
+    // the batch keeps read coordinates in 16 bits (include/squid_b200.h): a longer read is refused, never wrapped
+    return "record " + std::to_string(r) + " is longer than 65535 bases (TotalLen " + std::to_string(total_len) + ")";
+}
+
 int pack_concordant(const AlnSource &conc, const HostConfig &cfg, const std::unordered_set<std::string> &chim_names, PackedBatch &out, std::string &err) {
     const uint64_t n = conc.n_rec;
     const bool timing = getenv("SQH_TIMING") != nullptr;
@@ -163,10 +171,8 @@ int pack_concordant(const AlnSource &conc, const HostConfig &cfg, const std::uno
             out.ref_id[r] = a.ref_id; out.pos[r] = a.pos; out.mate_ref_id[r] = a.mate_ref_id; out.mate_pos[r] = a.mate_pos;
             out.flag[r] = a.flag; out.mapq[r] = a.mapq;
             decode_alignment(a, cfg, d);
-            if (d.blocks.size() > 16) { terr[t] = "record " + std::to_string(r) + " has more than 16 aligned blocks"; return; }
+            if (const int lim = sq::packer_limit((uint32_t)d.blocks.size(), d.total_len)) { terr[t] = packer_refusal(r, lim, d.total_len); return; }
             out.end_pos[r] = d.end_pos;
-            // the batch keeps read coordinates in 16 bits (include/squid_b200.h): a longer read is refused, never wrapped
-            if (d.total_len > 65535) { terr[t] = "record " + std::to_string(r) + " is longer than 65535 bases (TotalLen " + std::to_string(d.total_len) + ")"; return; }
             out.total_len[r] = (uint16_t)d.total_len;
             out.lowphred_run[r] = (uint16_t)std::min(d.lowphred_run, 65535);  // <= total_len
             uint8_t aux = 0;

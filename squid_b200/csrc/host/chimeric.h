@@ -45,6 +45,8 @@ struct PackedBatch {
 // (ReadRec_t ctor + tag/ChimName probes, SegmentGraph.cpp:297-304).  `chim_names` holds the
 // suffix-stripped Qnames of Chimrecord; the gate compares the RAW record name against them
 // (SURVEY.md App. A-3), so a "/1" or "/2" suffixed name never matches.
+// Why the packer refuses record r (sq::packer_limit `limit`, 1 or 2), in the words every front end reports.
+std::string packer_refusal(uint64_t r, int limit, int64_t total_len);
 int pack_concordant(const SqmbView &conc, const HostConfig &cfg, const std::unordered_set<std::string> &chim_names, PackedBatch &out, std::string &err);
 int pack_concordant(const AlnSource &conc, const HostConfig &cfg, const std::unordered_set<std::string> &chim_names, PackedBatch &out, std::string &err);
 

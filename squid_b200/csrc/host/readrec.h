@@ -47,7 +47,6 @@ struct Alignment {
     bool is_second() const { return flag & 0x80; }
     bool is_dup() const { return flag & 0x400; }
     bool is_proper() const { return flag & 0x2; }
-    int32_t end_pos() const;  // BamTools GetEndPosition(): pos + sum(M,D,N,=,X)
 };
 
 struct Block {  // SingleBamRec_t (src/SingleBamRec.h:25-61)
@@ -65,7 +64,7 @@ struct Block {  // SingleBamRec_t (src/SingleBamRec.h:25-61)
 // What ReadRec_t::ReadRec_t derives from one alignment (src/ReadRec.cpp:10-88).
 struct Decoded {
     int total_len = 0;        // ReadRec.cpp:16-18
-    int32_t end_pos = 0;      // BamTools GetEndPosition(): pos + sum(M,D,N,=,X), from the same walk over the CIGAR
+    int32_t end_pos = 0;      // BamTools GetEndPosition()
     int lowphred_run = 0;     // ReadRec.cpp:19-38 (longest run below threshold)
     std::vector<Block> blocks;  // CIGAR order, poly-A/T blocks removed, read_pos strand-flipped
 };

@@ -1,18 +1,20 @@
-// BAM records in an inflated window, as `SQ_HD` rules (device: sqg_load_concordant_bam in sqg_api.cu; CPU: tests/emul/emul_bam.cpp).
+// The BAM record rules, as `SQ_HD` code: the one definition the host BAM front end (host/bam.cpp), the device decoder
+// (sqg_load_concordant_bam in sqg_api.cu) and its CPU stepping (tests/emul/emul_bam.cpp) all run.
+//   * Record well-formedness (bam_rec_check), aux value sizes and the XA / IH scan with BamTools' GetTag<int> semantics.
 //   * Record boundaries, whatever the writer.  A window is cut into segments at its BGZF member starts.  Per segment a
 //     speculative first record start is searched (the first offset from which a chain of plausible records reaches the
 //     segment's end or kSpecDepth records), and the segment is walked from it to its exit (the first record start at or past
 //     its end).  Segment k is proven when the exit of segment k-1 equals its start: by induction from segment 0, which starts at
 //     a true boundary (end of the header or of the previous window's last whole record), every proven start is a true one.
 //     Segments that are not proven are walked again from their true entry, in rounds, until nothing changes; correctness never
-//     depends on the search, only the number of rounds does.  The walk itself checks exactly what host/bam.cpp checks.
-//   * The per-record decode of host/bam.cpp + pack_concordant + decode_alignment (host/readrec.cpp): fields, TotalLen,
-//     GetEndPosition, the low-quality run, XA / IH with BamTools' GetTag<int> semantics, the ChimName probe, and the aligned
-//     blocks (poly-A/T test on the 4-bit bases, strand flip).
+//     depends on the search, only the number of rounds does.
+//   * The per-record decode of the device: fields, the CIGAR rules of sq_cigar.cuh (TotalLen, GetEndPosition, the low-quality
+//     run, the aligned blocks with the poly-A/T test on the 4-bit bases), XA / IH and the ChimName probe.
 #ifndef SQ_BAM_CUH
 #define SQ_BAM_CUH
 #include <stdint.h>
 
+#include "sq_cigar.cuh"
 #include "sq_common.cuh"
 #include "squid_b200.h"
 
@@ -27,8 +29,9 @@ struct BamMember { uint64_t cdata, out; uint32_t clen, isize, crc, pad; };
 SQ_HD uint32_t bam_u16(const uint8_t *p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }
 SQ_HD uint32_t bam_u32(const uint8_t *p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
 
-// The record whose block_size sits at b[p]: 1 = well formed as host/bam.cpp requires (*next = the following record), 0 = it
-// does not end before L but could end before the stream does (Lstream: end of the stream in the same coordinates), -1 = malformed.
+// The record whose block_size sits at b[p]: 1 = well formed (block_size >= 32 and the variable-length fields fit inside it; *next =
+// the following record), 0 = it does not end before L but could end before the stream does (Lstream: end of the stream in the
+// same coordinates), -1 = malformed.
 SQ_HD int bam_rec_check(const uint8_t *b, int64_t p, int64_t L, int64_t Lstream, int64_t *next) {
     if (p + 4 > L) return p + 4 > Lstream ? -1 : 0;
     const int32_t bs = (int32_t)bam_u32(b + p);
@@ -86,7 +89,7 @@ SQ_HD int64_t bam_spec_start(const uint8_t *b, int64_t s, int64_t e, int64_t L, 
     return e;
 }
 
-// size of one aux value of type t at p (behind the type byte), 0 when malformed (host/bam.cpp aux_size)
+// size of one aux value of type t at p (behind the type byte), 0 when malformed
 SQ_HD uint64_t bam_aux_size(char t, const uint8_t *p, const uint8_t *end) {
     switch (t) {
         case 'A': case 'c': case 'C': return 1;
@@ -102,6 +105,32 @@ SQ_HD uint64_t bam_aux_size(char t, const uint8_t *p, const uint8_t *end) {
         }
         default: return 0;
     }
+}
+
+// The aux fields [q, end) of a record: XA present, IH present and its value as BamTools' GetTag<int> reads it (the destination is
+// zeroed and the 1, 2 or 4 value bytes are copied over its low end: no sign extension of the narrow signed types; 'A' converts as
+// well; any other type leaves the value as it was; the last IH wins).  false when a field is malformed.
+struct BamAux { bool xa, ih; int32_t ih_value; };
+SQ_HD bool bam_aux_scan(const uint8_t *q, const uint8_t *end, BamAux &a) {
+    a = BamAux{false, false, 0};
+    while (q + 3 <= end) {
+        const char t0 = (char)q[0], t1 = (char)q[1], ty = (char)q[2];
+        const uint64_t sz = bam_aux_size(ty, q + 3, end);
+        if (sz == 0 || sz > (uint64_t)(end - (q + 3))) return false;
+        if (t0 == 'X' && t1 == 'A') a.xa = true;
+        else if (t0 == 'I' && t1 == 'H') {
+            a.ih = true;
+            const uint8_t *v = q + 3;
+            switch (ty) {
+                case 'A': case 'c': case 'C': a.ih_value = v[0]; break;
+                case 's': case 'S': a.ih_value = (int32_t)bam_u16(v); break;
+                case 'i': case 'I': a.ih_value = (int32_t)bam_u32(v); break;
+                default: break;
+            }
+        }
+        q += 3 + sz;
+    }
+    return true;
 }
 
 // ChimName as an open-addressing set of 64-bit FNV-1a hashes (the packer's hash), each with its name for the exact compare.
@@ -127,60 +156,35 @@ SQ_HD bool nameset_has(const NameSet &s, const uint8_t *p, uint32_t n) {
     }
 }
 
-struct BamDecodeParams { int32_t thr; };  // (signed char)(phred offset + min_phred), as decode_alignment compares
+struct BamDecodeParams { int32_t thr; };  // phred_threshold(-pt, -pm)
 
-// The aligned blocks of a record (decode_alignment): block k goes to sink(k, ref_pos, match_ref, read_pos, match_read); returns
-// their number.  rec: the record's block_size field.
+// CIGAR element i of a record whose CIGAR starts at cig (unaligned little-endian bytes)
+struct BamCigar {
+    const uint8_t *cig;
+    SQ_HD uint32_t operator()(uint32_t i) const { return bam_u32(cig + 4 * i); }
+};
+
+// The aligned blocks of a record (cigar_blocks, the poly-A/T test on the 4-bit bases): block k goes to sink(k, ref_pos, match_ref,
+// read_pos, match_read); returns their number.  rec: the record's block_size field.
 template <class Sink>
 SQ_HD uint32_t bam_blocks(const uint8_t *rec, Sink &&sink) {
     const uint8_t *p = rec + 4;
     const int32_t pos = (int32_t)bam_u32(p + 4);
     const uint32_t l_name = p[8], n_cig = bam_u16(p + 12), l_seq = bam_u32(p + 16);
     const uint16_t flag = (uint16_t)bam_u16(p + 14);
-    const uint8_t *cig = p + 32 + l_name, *seq = cig + 4 * n_cig;
-    int total = 0;
-    for (uint32_t i = 0; i < n_cig; i++) {
-        const uint32_t op = bam_u32(cig + 4 * i) & 15;
-        if (op == 0 || op == 4 || op == 5 || op == 1 || op == 7 || op == 8) total += (int)(bam_u32(cig + 4 * i) >> 4);
-    }
-    const bool rev = (flag & 0x10) != 0;
-    int read_pos = 0, ref_pos = pos, hard = 0;
-    uint32_t nb = 0;
-    for (uint32_t i = 0; i < n_cig; i++) {
-        const uint32_t c = bam_u32(cig + 4 * i), op = c & 15;
-        const int l = (int)(c >> 4);
-        if (op == 4 || op == 5) {
-            read_pos += l;
-            if (op == 5) hard += l;
-        } else if (op == 0 || op == 7) {  // a block opens at M or = and runs up to the next S, H or N
-            int span_read = 0, span_ref = 0;
-            uint32_t j = i;
-            for (; j < n_cig; j++) {
-                const uint32_t cj = bam_u32(cig + 4 * j), oj = cj & 15;
-                if (oj == 4 || oj == 5 || oj == 3) break;
-                if (oj != 2) span_read += (int)(cj >> 4);
-                if (oj != 1) span_ref += (int)(cj >> 4);
-            }
-            int n_a = 0, n_t = 0;
-            int k0 = read_pos - hard, k1 = read_pos + span_read - hard;
-            if (k0 < 0) k0 = 0;
-            if (k1 > (int)l_seq) k1 = (int)l_seq;
-            for (int k = k0; k < k1; k++) {  // 4-bit codes: 1 = A, 8 = T
-                const uint32_t v = (seq[k >> 1] >> ((k & 1) ? 0 : 4)) & 15;
-                n_a += v == 1; n_t += v == 8;
-            }
-            if (4 * n_a < 3 * span_read && 4 * n_t < 3 * span_read) {  // poly-A/T blocks (>= 75 %) are dropped
-                sink(nb, ref_pos, span_ref, rev ? total - read_pos - span_read : read_pos, span_read);
-                nb++;
-            }
-            read_pos += span_read;
-            ref_pos += span_ref;
-            i = j - 1;
-        } else if (op == 3) {
-            ref_pos += l;
+    const BamCigar op{p + 32 + l_name};
+    const uint8_t *seq = op.cig + 4 * n_cig;
+    uint32_t k = 0;
+    return cigar_blocks(op, n_cig, pos, cigar_summary(op, n_cig, pos).total_len, flag_rev(flag), [&](uint32_t, int32_t lo, int32_t hi) {
+        ATCount n{0, 0};
+        if (lo < 0) lo = 0;
+        if (hi > (int32_t)l_seq) hi = (int32_t)l_seq;
+        for (int32_t i = lo; i < hi; i++) {  // 4-bit codes: 1 = A, 8 = T
+            const uint32_t v = (seq[i >> 1] >> ((i & 1) ? 0 : 4)) & 15;
+            n.a += v == 1; n.t += v == 8;
         }
-    }
-    return nb;
+        return n;
+    }, [&](int32_t ref_pos, int32_t match_ref, int32_t read_pos, int32_t match_read) { sink(k++, ref_pos, match_ref, read_pos, match_read); });
 }
 
 // One decoded record: the per-record fields of sqg_batch and the block count.
@@ -203,50 +207,18 @@ SQ_HD void bam_decode(const uint8_t *rec, const BamDecodeParams &prm, const Name
     const uint32_t l_seq = bam_u32(p + 16);
     o.l_seq = l_seq;
     o.mate_ref_id = (int32_t)bam_u32(p + 20); o.mate_pos = (int32_t)bam_u32(p + 24);
-    const uint8_t *name = p + 32, *cig = name + l_name, *seq = cig + 4 * n_cig, *qual = seq + (l_seq + 1) / 2;
-    // TotalLen, GetEndPosition and the read length the synthesised qualities would have (decode_alignment)
-    int total = 0, lseq = 0;
-    uint32_t endp = (uint32_t)o.pos;
-    for (uint32_t i = 0; i < n_cig; i++) {
-        const uint32_t c = bam_u32(cig + 4 * i), op = c & 15;
-        const int l = (int)(c >> 4);
-        if (op == 0 || op == 4 || op == 5 || op == 1 || op == 7 || op == 8) total += l;
-        if (op == 0 || op == 2 || op == 3 || op == 7 || op == 8) endp += (uint32_t)l;
-        if (op == 0 || op == 1 || op == 4 || op == 7 || op == 8) lseq += l;
-    }
-    o.total_len = total; o.end_pos = (int32_t)endp; o.lseq_cigar = lseq;
-    // longest run of qualities below the threshold, compared as the host compares (signed char)(q + 33)
-    int best = 0, run = 0;
-    for (uint32_t i = 0; i < l_seq; i++) {
-        run = ((int)(signed char)(uint8_t)(qual[i] + 33) < prm.thr) ? run + 1 : 0;
-        if (run > best) best = run;
-    }
-    o.lowphred = best;
-    // aux: XA present, IH as GetTag<int> reads it (the last IH tag wins; non-integer types leave the value as it was)
-    bool xa = false, ih = false;
-    int32_t ihv = 0;
-    o.aux_bad = false;
-    const uint8_t *q = qual + l_seq;
-    while (q + 3 <= end) {
-        const char t0 = (char)q[0], t1 = (char)q[1], ty = (char)q[2];
-        const uint64_t sz = bam_aux_size(ty, q + 3, end);
-        if (sz == 0 || sz > (uint64_t)(end - (q + 3))) { o.aux_bad = true; break; }
-        if (t0 == 'X' && t1 == 'A') xa = true;
-        else if (t0 == 'I' && t1 == 'H') {
-            ih = true;
-            const uint8_t *v = q + 3;
-            switch (ty) {
-                case 'A': case 'c': case 'C': ihv = v[0]; break;
-                case 's': case 'S': ihv = (int32_t)bam_u16(v); break;
-                case 'i': case 'I': ihv = (int32_t)bam_u32(v); break;
-                default: break;
-            }
-        }
-        q += 3 + sz;
-    }
+    const uint8_t *name = p + 32;
+    const BamCigar op{name + l_name};
+    const uint8_t *qual = op.cig + 4 * n_cig + (l_seq + 1) / 2;
+    const CigarSummary s = cigar_summary(op, n_cig, o.pos);
+    o.total_len = s.total_len; o.end_pos = s.end_pos; o.lseq_cigar = s.lseq;
+    // qualities compared as the host front end spells them: (signed char)(q + 33)
+    o.lowphred = low_quality_run([qual](uint32_t i) { return (int32_t)(signed char)(uint8_t)(qual[i] + 33); }, l_seq, prm.thr);
+    BamAux a;
+    o.aux_bad = !bam_aux_scan(qual + l_seq, end, a);
     uint8_t aux = 0;
-    if (xa) aux |= SQG_AUX_XA;
-    if (ih && ihv > 1) aux |= SQG_AUX_IH_GT1;
+    if (a.xa) aux |= SQG_AUX_XA;
+    if (a.ih && a.ih_value > 1) aux |= SQG_AUX_IH_GT1;
     if (names.active && nameset_has(names, name, l_name ? l_name - 1 : 0)) aux |= SQG_AUX_CHIMNAME;
     o.aux = aux;
     o.n_blk = bam_blocks(rec, [](uint32_t, int32_t, int32_t, int32_t, int32_t) {});

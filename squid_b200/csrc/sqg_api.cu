@@ -2392,7 +2392,6 @@ extern "C" int sqg_shard_cov_count(sqg_ctx *ctx, int64_t rank_offset, const int6
 // ------------------------------------------------------------------------------------------------
 constexpr int kInflWarps = 8;
 constexpr size_t kBamStage = 32u << 20;  // bytes per pinned staging buffer
-constexpr uint32_t kRawMember = 0xFFFFFFFFu;  // crc of a pseudo-member of an uncompressed stream: copied, not inflated
 enum { BS_CHANGED = 0, BS_BAD, BS_AUXBAD, BS_ERRKEY, BS_SEQ, BS_INFL, BS_N };
 
 __global__ void __launch_bounds__(kInflWarps * 32) k_bam_inflate(const BamMember *mem, int64_t n, const uint8_t *comp, uint8_t *win, int64_t *small) {
@@ -2492,9 +2491,9 @@ __global__ void k_bam_decode(const uint8_t *b, const int64_t *rec_off, int64_t n
     nblk[i] = x.n_blk;
     if (x.aux_bad) atomicOr((unsigned long long *)&small[BS_AUXBAD], 1ull);
     if (x.l_seq) small[BS_SEQ] = 1;
-    // pack_concordant's refusals, the first record in file order wins (more than 16 blocks is tested before TotalLen)
-    if (x.n_blk > 16) atomicMin((unsigned long long *)&small[BS_ERRKEY], (unsigned long long)r << 33);
-    else if (x.total_len > 65535) atomicMin((unsigned long long *)&small[BS_ERRKEY], ((unsigned long long)r << 33) | (1ull << 32) | (uint32_t)x.total_len);
+    // pack_concordant's refusals, the first record in file order wins: key = record << 33 | (limit - 1) << 32 | TotalLen
+    if (const int lim = packer_limit(x.n_blk, x.total_len))
+        atomicMin((unsigned long long *)&small[BS_ERRKEY], ((unsigned long long)r << 33) | ((unsigned long long)(lim - 1) << 32) | (uint32_t)x.total_len);
 }
 __global__ void k_bam_blocks(const uint8_t *b, const int64_t *rec_off, int64_t n, int64_t r0, uint64_t b0, const uint64_t *incl, const uint32_t *nblk, BamOut o) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -2535,12 +2534,7 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
     const bool raw = memcmp(f, "BAM\1", 4) == 0;
     std::vector<sqh::BgzfMember> mem;
     std::string e;
-    if (raw) {  // an uncompressed stream: 64 KiB pieces stand in for members (segment starts of the walk), uploaded as they are
-        for (size_t o = 0; o < mf.n; o += 65536) mem.push_back(sqh::BgzfMember{o, std::min<size_t>(65536, mf.n - o), o, (uint32_t)std::min<size_t>(65536, mf.n - o), kRawMember});
-    } else {
-        if (!sqh::bgzf_parse_members(f, mf.n, mem, e)) FAIL(SQG_EINVAL, e);
-        mem.erase(std::remove_if(mem.begin(), mem.end(), [](const sqh::BgzfMember &m) { return m.isize == 0; }), mem.end());  // EOF markers
-    }
+    if (!sqh::bam_loader_members(f, mf.n, raw, mem, e)) FAIL(SQG_EINVAL, e);
     std::vector<std::string> ref_names;
     std::vector<int32_t> ref_lens;
     size_t hdr_end = 0;
@@ -2549,46 +2543,26 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
     if (raw && !hdr_ok) FAIL(SQG_EINVAL, hdr_err);
     lap("bam: index + header");
     const int64_t T = mem.empty() ? 0 : (int64_t)(mem.back().off + mem.back().isize);
-    // windows of whole members, about SQG_BAM_WINDOW_MB of inflated bytes; the first one holds the whole header
+    // windows of whole members, about SQG_BAM_WINDOW_MB of inflated bytes
     const int64_t win_bytes = (int64_t)std::max(1, getenv("SQG_BAM_WINDOW_MB") ? atoi(getenv("SQG_BAM_WINDOW_MB")) : 1024) << 20;
-    std::vector<size_t> wcut{0};
-    for (size_t i = 0; i < mem.size();) {
-        size_t j = i;
-        int64_t bytes = 0;
-        while (j < mem.size() && (j == i || bytes + mem[j].isize <= win_bytes || (wcut.size() == 1 && (int64_t)mem[j].off <= (int64_t)hdr_end))) { bytes += mem[j].isize; j++; }
-        wcut.push_back(j);
-        i = j;
-    }
+    const std::vector<size_t> wcut = sqh::bam_window_cuts(mem, win_bytes, hdr_end);
     const size_t W = wcut.size() - 1;
     if (W == 0) FAIL(SQG_EINVAL, hdr_err);  // no data at all
     ctx->bam_members = (int64_t)mem.size(); ctx->bam_windows = (int64_t)W; ctx->bam_repair_rounds = 0;
-    // ChimName: open addressing over the names' hashes (duplicates dropped), with the names for the exact compare
     const int64_t nn = opt->n_names;
-    size_t cap = 2;
-    while (cap < 2 * (size_t)nn) cap <<= 1;
-    std::vector<uint64_t> nh(cap, 0);
-    std::vector<int32_t> nl(cap, -1);
-    std::vector<int64_t> no(cap, 0);
-    for (int64_t i = 0; i < nn; i++) {
-        const uint8_t *p = (const uint8_t *)opt->names + opt->name_off[i];
-        const uint32_t len = (uint32_t)(opt->name_off[i + 1] - opt->name_off[i]);
-        const uint64_t h = name_hash(p, len);
-        size_t k = h & (cap - 1);
-        for (; nl[k] >= 0; k = (k + 1) & (cap - 1))
-            if (nh[k] == h && (uint32_t)nl[k] == len && memcmp(opt->names + no[k], p, len) == 0) break;
-        nh[k] = h; nl[k] = (int32_t)len; no[k] = opt->name_off[i];
-    }
+    const sqh::NameTable nt = sqh::bam_name_table(opt->names, opt->name_off, nn);
+    const size_t cap = nt.hash.size();
     const int64_t blob_len = nn > 0 ? opt->name_off[nn] : 0;
     cudaStream_t st = ctx->stream;
     if (!ctx->stream_up) CK(cudaStreamCreateWithFlags(&ctx->stream_up, cudaStreamNonBlocking));
     cudaStream_t up = ctx->stream_up;
     while (ctx->bam_ev.size() < 3) { cudaEvent_t ev; CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)); ctx->bam_ev.push_back(ev); }
     CK(ctx->bam_nhash.ensure(cap)); CK(ctx->bam_nlen.ensure(cap)); CK(ctx->bam_noff.ensure(cap)); CK(ctx->bam_nblob.ensure((size_t)blob_len + 1));
-    CK(cudaMemcpyAsync(ctx->bam_nhash.p, nh.data(), cap * 8, cudaMemcpyHostToDevice, st)); CK(cudaMemcpyAsync(ctx->bam_nlen.p, nl.data(), cap * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->bam_noff.p, no.data(), cap * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->bam_nhash.p, nt.hash.data(), cap * 8, cudaMemcpyHostToDevice, st)); CK(cudaMemcpyAsync(ctx->bam_nlen.p, nt.len.data(), cap * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->bam_noff.p, nt.off.data(), cap * 8, cudaMemcpyHostToDevice, st));
     if (blob_len) CK(cudaMemcpyAsync(ctx->bam_nblob.p, opt->names, (size_t)blob_len, cudaMemcpyHostToDevice, st));
     NameSet ns{ctx->bam_nhash.p, ctx->bam_nlen.p, ctx->bam_noff.p, ctx->bam_nblob.p, cap - 1, nn > 0};
-    const int thr = (int)(signed char)(char)((opt->phred33 ? 33 : 64) + opt->min_phred);
+    const int thr = phred_threshold(opt->phred33, opt->min_phred);
     const BamDecodeParams prm{thr};
     // with no qualities anywhere in the file the host decoder synthesises them ('I' everywhere, decode_alignment), which only
     // matters when the threshold lies above 'I': then the run is the read length of the CIGAR
@@ -2653,8 +2627,7 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
         if (infl_bits || fatal) { CK(cudaStreamSynchronize(st)); elapsed("bam_h2d"); elapsed("bam_inflate"); carry = 0; continue; }
         // -- record boundaries
         CK(cudaEventRecord(ctx->timers["bam_records"].a, st));
-        std::vector<int64_t> seg{w == 0 ? (int64_t)hdr_end : 0};
-        for (size_t i = wcut[w]; i < wcut[w + 1]; i++) { const int64_t s = carry + ((int64_t)mem[i].off - wstream); if (s > seg[0]) seg.push_back(s); }
+        const std::vector<int64_t> seg = sqh::bam_window_segments(mem, wcut, w, carry, hdr_end);
         const int64_t S = (int64_t)seg.size();
         CK(ctx->bam_seg.ensure((size_t)S)); CK(ctx->bam_start.ensure((size_t)S)); CK(ctx->bam_exit.ensure((size_t)S)); CK(ctx->bam_newstart.ensure((size_t)S));
         CK(ctx->bam_cnt.ensure((size_t)S + 1)); CK(ctx->bam_base.ensure((size_t)S + 1)); CK(ctx->bam_bad.ensure((size_t)S)); CK(ctx->bam_redo.ensure((size_t)S));
@@ -2741,9 +2714,7 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
     if (aux_bad) FAIL(SQG_EINVAL, "malformed BAM alignment record");
     const uint64_t key = (uint64_t)ctx->bam_hsmall.p[BS_ERRKEY];
     if (key != ~0ull) {
-        const int64_t r = (int64_t)(key >> 33);
-        if (key & (1ull << 32)) FAIL(SQG_EUNSUPPORTED, "record " + std::to_string(r) + " is longer than 65535 bases (TotalLen " + std::to_string((uint32_t)key) + ")");
-        FAIL(SQG_EUNSUPPORTED, "record " + std::to_string(r) + " has more than 16 aligned blocks");
+        FAIL(SQG_EUNSUPPORTED, sqh::packer_refusal(key >> 33, (int)(key >> 32 & 1) + 1, (uint32_t)key));
     }
     if (fatal) FAIL(fatal, fatal_msg);
     if (R == 0) {  // an empty batch still has its blk_off[0]

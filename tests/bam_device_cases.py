@@ -78,6 +78,91 @@ def known_answer_tables():
     return t, ch
 
 
+def random_cigar_table(seed: int, n_reads: int = 1500):
+    """Records with random CIGARs over all nine ops: leading / trailing I, D, X, P and clips, H and S between blocks, blocks opened
+    by M or =, N runs, A/T fractions of blocks at and around 3/4, both strands and mates, explicit bases and qualities (runs of
+    qualities in narrow random bands, so that every threshold cuts them somewhere) and synthesised ones.  Within the packer's
+    limits: at most 16 blocks and TotalLen <= 65535.  Read i sits alone in its own 200 kb stretch, so no two reads share a front
+    position."""
+    import random
+    F = sqmb
+    rng = random.Random(seed)
+    ln = lambda lo, hi: rng.randint(lo, hi)
+
+    def cigar(p):  # p: P may follow the first M / =, where it can fall inside a block
+        ops = []
+        for _ in range(rng.choice([0, 0, 1, 2])):  # leading clips and ops outside any block
+            ops.append((rng.choice("HSIDXP"), ln(1, 12)))
+        for b in range(ln(1, rng.choice([3, 8, 16]))):
+            if b:
+                for _ in range(ln(1, 3)):  # separators, with strays that fall outside the blocks
+                    o = rng.choice("SHNNNIDX" + p)
+                    ops.append((o, ln(1, 400) if o == "N" else ln(1, 15)))
+            ops.append((rng.choice("MM="), ln(1, 60)))
+            for _ in range(rng.choice([0, 0, 1, 2, 3])):
+                ops.append((rng.choice("MID=X" + p), ln(1, 20)))
+        for _ in range(rng.choice([0, 0, 1, 2])):
+            ops.append((rng.choice("HSIDX" + p), ln(1, 12)))
+        return "".join("%d%s" % (l, o) for o, l in ops), ops
+
+    def windows(ops):  # the read windows the poly-A/T test reads, as decode_alignment walks the CIGAR
+        out, rp, hard, i = [], 0, 0, 0
+        while i < len(ops):
+            o, l = ops[i]
+            if o in "SH":
+                rp += l
+                hard += l if o == "H" else 0
+            elif o in "M=":
+                j, span = i, 0
+                while j < len(ops) and ops[j][0] not in "SHN":
+                    span += ops[j][1] if ops[j][0] != "D" else 0
+                    j += 1
+                out.append((rp - hard, span))
+                rp += span
+                i = j - 1
+            i += 1
+        return out
+
+    recs = []
+    for i in range(n_reads):
+        mates = [F.FLAG_FIRST, F.FLAG_SECOND] if rng.random() < 0.8 else [rng.choice([F.FLAG_FIRST, F.FLAG_SECOND])]
+        for m, mate in enumerate(mates):
+            # the first block of a read's first record always stays: a read left without blocks has no place in the loader's sort
+            synth = rng.random() < 0.3
+            # A P inside a block widens its read span past the bases the block covers, so a synthesised poly-A/T block would
+            # be all A/T for the packer but not for a reader of the materialised bases: synthesised records keep P outside blocks.
+            cig, ops = cigar("" if synth else "P")
+            lseq = sum(l for o, l in ops if o in "MIS=X")
+            flag = F.FLAG_PAIRED | mate | (F.FLAG_REVERSE if rng.random() < 0.5 else 0) | (F.FLAG_MATE_REVERSE if rng.random() < 0.5 else 0)
+            r = dict(ref_id=i % 2, pos=1000 + (i // 2) * 200000 + (0 if mate == F.FLAG_FIRST else 20000) + ln(0, 999), cigar=cig, flag=flag,
+                     mate_ref_id=i % 2, mate_pos=1000 + (i // 2) * 200000, mapq=rng.choice([0, 3, 60, 255]), name_id=i,
+                     name_suffix=rng.random() < 0.2, xa=rng.random() < 0.1)
+            if rng.random() < 0.3:
+                r["ih"] = rng.choice([0, 1, 2, 200])
+            if synth:
+                r["lowrun"] = rng.choice([0, ln(0, lseq), lseq, lseq + 5])
+                r["polya"] = rng.getrandbits(8) & (0xEE if m == 0 else 0xFF)
+            else:
+                seq = [rng.choice("CGNCGT") for _ in range(lseq)]
+                for b, (a, span) in enumerate(windows(ops)):
+                    if m == 0 and b == 0:
+                        seq[a:a + span] = [rng.choice("CG") for _ in seq[a:a + span]]
+                        continue
+                    base = rng.choice("AaTt")
+                    k = max(0, (3 * span + 3) // 4 + rng.choice([-2, -1, -1, 0, 0, 0, 1, 1]) if rng.random() < 0.7 else rng.choice([0, span]))
+                    for p in rng.sample(range(span), min(k, span)):
+                        if 0 <= a + p < lseq:
+                            seq[a + p] = base
+                qual = []
+                while len(qual) < lseq:
+                    lo = ln(33, 120)
+                    qual += [chr(ln(lo, lo + 4)) for _ in range(ln(1, 30))]
+                r["seq"], r["qual"] = "".join(seq), "".join(qual[:lseq])
+            recs.append(r)
+    recs.sort(key=lambda r: (r["ref_id"], r["pos"]))
+    return F.from_records([1 << 30, 1 << 30], recs)
+
+
 def build_emul_bam(out_dir) -> str:
     """Compiles tests/emul/emul_bam.cpp into `out_dir` (not into the repository tree, which may be read-only)."""
     out = os.path.join(str(out_dir), "emul_bam")

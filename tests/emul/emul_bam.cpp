@@ -1,6 +1,6 @@
-// CPU stepping of the device BAM decode (squid_b200/csrc/sq_inflate.cuh, sq_bam.cuh): the same SQ_HD rules, run serially in the
-// order the kernels of sqg_load_concordant_bam run them, so that tests/test_cpu_bam_device.py can compare them with zlib and with
-// the host front end without a GPU.
+// CPU stepping of the device BAM decode (squid_b200/csrc/sq_inflate.cuh, sq_bam.cuh): the loader's own plan (host/bam.h) and the
+// same SQ_HD rules, run serially in the order the kernels of sqg_load_concordant_bam run them, so that tests/test_cpu_bam_device.py
+// can compare them with zlib and with the host front end without a GPU.
 //   emul_bam inflate <bgzf file> <out>
 //       every member inflated as k_bam_inflate does it (matches of kInflWarpCopyMin bytes or more copied by the "warp", the CRC
 //       summed over 32 slices and combined); writes the stream to <out>, prints "status <bits>" (1: a corrupt member, 2: a CRC mismatch)
@@ -96,53 +96,32 @@ int main(int argc, char **argv) {
     std::vector<int64_t> name_off(offb.size() / 8);
     if (!offb.empty()) memcpy(name_off.data(), offb.data(), offb.size());
     const int64_t nn = name_off.empty() ? 0 : (int64_t)name_off.size() - 1;
-    const int thr = (int)(signed char)(char)((atoi(argv[5]) ? 33 : 64) + atoi(argv[6]));
+    const int thr = phred_threshold(atoi(argv[5]) != 0, atoi(argv[6]));
     const int64_t win_bytes = atoll(argv[7]);
     const std::string outdir = argv[8];
     const bool raw = memcmp(f.data(), "BAM\1", 4) == 0;
     std::vector<sqh::BgzfMember> mem;
     std::string e;
-    if (raw) { for (size_t o = 0; o < f.size(); o += 65536) mem.push_back(sqh::BgzfMember{o, std::min<size_t>(65536, f.size() - o), o, (uint32_t)std::min<size_t>(65536, f.size() - o), 0}); }
-    else {
-        if (!sqh::bgzf_parse_members(f.data(), f.size(), mem, e)) return fail(-1, e);
-        mem.erase(std::remove_if(mem.begin(), mem.end(), [](const sqh::BgzfMember &m) { return m.isize == 0; }), mem.end());
-    }
+    if (!sqh::bam_loader_members(f.data(), f.size(), raw, mem, e)) return fail(-1, e);
     std::vector<std::string> rn; std::vector<int32_t> rl;
     size_t hdr_end = 0;
     std::string herr;
     const bool hdr_ok = sqh::bam_read_header(f.data(), f.size(), raw ? nullptr : &mem, rn, rl, hdr_end, herr);
     if (raw && !hdr_ok) return fail(-1, herr);
     const int64_t T = mem.empty() ? 0 : (int64_t)(mem.back().off + mem.back().isize);
-    std::vector<size_t> wcut{0};
-    for (size_t i = 0; i < mem.size();) {
-        size_t j = i; int64_t bytes = 0;
-        while (j < mem.size() && (j == i || bytes + mem[j].isize <= win_bytes || (wcut.size() == 1 && (int64_t)mem[j].off <= (int64_t)hdr_end))) { bytes += mem[j].isize; j++; }
-        wcut.push_back(j); i = j;
-    }
+    const std::vector<size_t> wcut = sqh::bam_window_cuts(mem, win_bytes, hdr_end);
     const size_t W = wcut.size() - 1;
     if (W == 0) return fail(-1, herr);
-    // ChimName set as the loader builds it
-    size_t cap = 2;
-    while (cap < 2 * (size_t)nn) cap <<= 1;
-    std::vector<uint64_t> nh(cap, 0); std::vector<int32_t> nl(cap, -1); std::vector<int64_t> no(cap, 0);
-    for (int64_t i = 0; i < nn; i++) {
-        const uint8_t *p = blob.data() + name_off[i];
-        const uint32_t len = (uint32_t)(name_off[i + 1] - name_off[i]);
-        const uint64_t h = name_hash(p, len);
-        size_t k = h & (cap - 1);
-        for (; nl[k] >= 0; k = (k + 1) & (cap - 1)) if (nh[k] == h && (uint32_t)nl[k] == len && memcmp(blob.data() + no[k], p, len) == 0) break;
-        nh[k] = h; nl[k] = (int32_t)len; no[k] = name_off[i];
-    }
-    const NameSet ns{nh.data(), nl.data(), no.data(), blob.data(), cap - 1, nn > 0};
+    const sqh::NameTable nt = sqh::bam_name_table((const char *)blob.data(), name_off.data(), nn);
+    const NameSet ns{nt.hash.data(), nt.len.data(), nt.off.data(), blob.data(), nt.hash.size() - 1, nn > 0};
     const BamDecodeParams prm{thr};
     std::vector<int32_t> ref_id, pos, mref, mpos, endp, bref, bmref; std::vector<uint16_t> flag, tlen, low, brpos, bmread, lseq; std::vector<uint8_t> mapq, aux;
     std::vector<uint32_t> blk_off{0};
     std::vector<uint8_t> prev, cur;
     int64_t carry = 0, rounds = 0;
     int infl = 0, fatal = 0;
-    std::string fmsg;
+    std::string fmsg, refusal;
     bool aux_bad = false, any_seq = false;
-    uint64_t errkey = ~0ull;
     for (size_t w = 0; w < W; w++) {
         const sqh::BgzfMember &m0 = mem[wcut[w]], &m1 = mem[wcut[w + 1] - 1];
         const int64_t wstream = (int64_t)m0.off, wis = (int64_t)(m1.off + m1.isize) - wstream, L = carry + wis, Ls = carry + (T - wstream);
@@ -156,8 +135,7 @@ int main(int argc, char **argv) {
         }
         if (w == 0 && !hdr_ok && !fatal) { fatal = -1; fmsg = herr; }
         if (infl || fatal) { carry = 0; continue; }
-        std::vector<int64_t> seg{w == 0 ? (int64_t)hdr_end : 0};
-        for (size_t i = wcut[w]; i < wcut[w + 1]; i++) { const int64_t s = carry + ((int64_t)mem[i].off - wstream); if (s > seg[0]) seg.push_back(s); }
+        const std::vector<int64_t> seg = sqh::bam_window_segments(mem, wcut, w, carry, hdr_end);
         const int64_t S = (int64_t)seg.size();
         auto send = [&](int64_t k) { return k + 1 < S ? seg[k + 1] : L; };
         std::vector<int64_t> start(S), ex(S), ns2(S); std::vector<uint32_t> cnt(S); std::vector<uint8_t> bad(S), redo(S);
@@ -196,8 +174,8 @@ int main(int argc, char **argv) {
             flag.push_back(x.flag); mapq.push_back(x.mapq); aux.push_back(x.aux); tlen.push_back((uint16_t)x.total_len);
             low.push_back((uint16_t)std::min(x.lowphred, 65535)); lseq.push_back((uint16_t)std::min<uint32_t>((uint32_t)x.lseq_cigar, 65535u));
             aux_bad |= x.aux_bad; any_seq |= x.l_seq > 0;
-            if (x.n_blk > 16) errkey = std::min<uint64_t>(errkey, r << 33);
-            else if (x.total_len > 65535) errkey = std::min<uint64_t>(errkey, (r << 33) | (1ull << 32) | (uint32_t)x.total_len);
+            const int lim = packer_limit(x.n_blk, x.total_len);
+            if (lim && refusal.empty()) refusal = sqh::packer_refusal(r, lim, x.total_len);
             bam_blocks(b + rec[i], [&](uint32_t, int32_t rp, int32_t mr, int32_t qp, int32_t mq) {
                 bref.push_back(rp); bmref.push_back(mr); brpos.push_back((uint16_t)qp); bmread.push_back((uint16_t)mq);
             });
@@ -209,11 +187,7 @@ int main(int argc, char **argv) {
     if (infl) return fail(-1, (infl & 1) ? "corrupt deflate stream in a BGZF block" : "BGZF block fails its CRC32");
     if (fatal) return fail(fatal, fmsg);
     if (aux_bad) return fail(-1, "malformed BAM alignment record");
-    if (errkey != ~0ull) {
-        const uint64_t r = errkey >> 33;
-        if (errkey & (1ull << 32)) return fail(-5, "record " + std::to_string(r) + " is longer than 65535 bases (TotalLen " + std::to_string((uint32_t)errkey) + ")");
-        return fail(-5, "record " + std::to_string(r) + " has more than 16 aligned blocks");
-    }
+    if (!refusal.empty()) return fail(-5, refusal);
     if (thr > 'I' && !any_seq) low = lseq;
     dump(outdir, "ref_id", ref_id); dump(outdir, "pos", pos); dump(outdir, "mate_ref_id", mref); dump(outdir, "mate_pos", mpos); dump(outdir, "end_pos", endp);
     dump(outdir, "flag", flag); dump(outdir, "total_len", tlen); dump(outdir, "lowphred_run", low); dump(outdir, "mapq", mapq); dump(outdir, "aux", aux);

@@ -92,6 +92,16 @@ def test_known_answers(tmp_path, built_lib, opts):
     assert (got.a["aux"] & 8).any() and (got.a["aux"] & 2).any()
 
 
+@pytest.mark.parametrize("opts", [{}, dict(phred33=0, min_phred=70)])
+def test_random_cigars(tmp_path, built_lib, opts):
+    """Random CIGARs over all nine ops (bam_device_cases.random_cigar_table), records straddling members, 1 MB windows."""
+    t = cases.random_cigar_table(2024)
+    cb = str(tmp_path / "c.bam")
+    open(cb, "wb").write(cases.layouts(t)["straddle_997"])
+    g, got = _device_batch(cb, cb, window_mb=1, **opts)
+    _assert_same(api.HostCase(cb, cb, bam=True, **opts).batch, got)
+
+
 def test_adversarial_member_start(case6k, tmp_path, built_lib):
     """A member that starts inside a B-array tag whose bytes form a chain of valid-looking records."""
     d, conc, hb = case6k
