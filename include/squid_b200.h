@@ -223,12 +223,16 @@ int sqg_merge_edge_tables(sqg_ctx *ctx, const uint64_t *d_keys, const int32_t *d
  * cuts the stream with sqg_plan_shards(), gives every context its record range (sqg_load_concordant) and ALL chimeric reads
  * (sqg_load_chimeric), and runs the stages below, exchanging the small per-shard results between them (NCCL / torch.distributed
  * all_gather when the contexts live in different processes; squid_b200/sharded.py is that driver).  The combined outputs are
- * bit-identical to the single-context calls above.
+ * bit-identical to the single-context calls above.  A stream decoded on the device needs no host batch: every context loads
+ * the whole stream (sqg_load_concordant_bam) and all chimeric reads, plans the same cuts on it (sqg_plan_shards_resident) and
+ * keeps its own range (sqg_keep_records) -- ShardedSegmentGraph.load_bam.
  *
  *   sqg_plan_shards   cuts[0..n_planned] (cuts[0] = 0, cuts[n_planned] = n_rec); shard i owns records [cuts[i], cuts[i+1]).
  *                     Cuts are placed at coverage gaps clear of every discordant group, where BuildNode_STAR's windows are
  *                     empty and its pending segment closed (:616-636); n_planned < n_shards when the stream has too few.
  *                     All arrays of `batch` are HOST pointers.
+ *   sqg_plan_shards_resident / sqg_keep_records
+ *                     the same cuts from the resident batch, and one shard's range of it (see below).
  *   sqg_set_shard     declares the context shard `index` of `count` (before the stages).  Shard 0 owns the edges of the chimeric
  *                     reads and the discordant-block depth.
  *   sqg_shard_seeds   stage 1 = BuildNode_STAR up to the seed segments (:296-701) on this shard: *ops = n_ops x 4 int32
@@ -253,6 +257,23 @@ int sqg_merge_edge_tables(sqg_ctx *ctx, const uint64_t *d_keys, const int32_t *d
  */
 int sqg_plan_shards(const sqg_batch *batch, const sqg_chimeric *chim, const sqg_config *cfg, int32_t n_ref, int32_t n_shards,
                     int64_t *cuts, int32_t *n_planned);
+/*
+ * sqg_plan_shards() on the context's resident batch (any loader) and the chimeric reads of sqg_load_chimeric: cuts[0..n_planned]
+ * (n_shards + 1 entries) equal to what sqg_plan_shards returns for the same stream.  The per-record part of the planner's rules
+ * runs on the device on the class bytes of the classification pass (run first when the batch is not classified yet: an unsorted
+ * or malformed batch is refused as there) and the discordant groups of the chimeric pre-pass; the candidates come back to the host
+ * for the greedy choice of the cuts.  May be called on a context that sqg_set_shard has declared a shard.  Phase "plan".
+ *   SQG_EINVAL  n_shards < 1;   SQG_ESTATE  no batch, no chimeric reads, or after sqg_keep_records.
+ */
+int sqg_plan_shards_resident(sqg_ctx *ctx, int32_t n_shards, int64_t *cuts, int32_t *n_planned);
+/*
+ * Restricts the resident batch to records [lo, hi): they become the batch (blk_off rebased to 0, block arrays from blk_off[lo]),
+ * moved to the front of the context's own arrays on the device, and every product computed from the whole batch (class bytes,
+ * coverage pairs, edge table) is dropped -- the context is then as if [lo, hi) had been loaded with sqg_load_concordant (with
+ * first_record_index advanced by lo).  SQG_EINVAL unless 0 <= lo <= hi <= n_rec; SQG_ESTATE without a batch or when the batch is
+ * attached (sqg_attach_concordant_device: caller-owned arrays).
+ */
+int sqg_keep_records(sqg_ctx *ctx, int64_t lo, int64_t hi);
 int sqg_set_shard(sqg_ctx *ctx, int32_t index, int32_t count);
 int sqg_shard_seeds(sqg_ctx *ctx, int32_t prior_emission, const int32_t **ops, int64_t *n_ops);
 int sqg_shard_build(sqg_ctx *ctx, const int32_t *ops_all, int64_t n_ops_all, int32_t **chr, int32_t **pos, int32_t **len, int64_t *n_nodes,
@@ -265,7 +286,7 @@ int sqg_shard_cov_owned_t(sqg_ctx *ctx, int64_t rank_offset, int64_t k_in, int64
 int sqg_shard_cov_count(sqg_ctx *ctx, int64_t rank_offset, const int64_t *t_global, int32_t *cov_partial);
 
 /* Device time in ms of the named phase/kernel of the most recent call ("classify", "seed", "tile", "depth_edges",
- * "edge_sort", "coverage"; kernels: "k_classify", "k_cov_compact", "k_assign_depth", "k_assign_edges", "k_edges_generic",
+ * "edge_sort", "coverage", "plan"; kernels: "k_classify", "k_cov_compact", "k_assign_depth", "k_assign_edges", "k_edges_generic",
  * "k_cov_count"), measured with CUDA events on the context's stream; <0 if unknown. */
 float sqg_phase_ms(const sqg_ctx *ctx, const char *name);
 /* Number of kernel launches issued by this context so far. */

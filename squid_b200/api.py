@@ -78,7 +78,7 @@ EXPORTS = [
     "sqg_create", "sqg_destroy", "sqg_last_error", "sqg_load_concordant", "sqg_load_concordant_wire", "sqg_load_concordant_bam", "sqg_download_concordant", "sqg_connected_components", "sqg_attach_concordant_device", "sqg_load_chimeric",
     "sqg_build_nodes", "sqg_set_nodes", "sqg_build_edges", "sqg_bp_coverage", "sqg_edges_device_table", "sqg_merge_edge_tables",
     "sqg_phase_ms", "sqg_launch_count", "sqg_stat", "sqg_classify_dump", "sqg_selftest_gpu_sort",
-    "sqg_plan_shards", "sqg_set_shard", "sqg_shard_seeds", "sqg_shard_build", "sqg_shard_hint_state", "sqg_shard_redo_edges",
+    "sqg_plan_shards", "sqg_plan_shards_resident", "sqg_keep_records", "sqg_set_shard", "sqg_shard_seeds", "sqg_shard_build", "sqg_shard_hint_state", "sqg_shard_redo_edges",
     "sqg_shard_cov_begin", "sqg_shard_cov_chain", "sqg_shard_cov_owned_t", "sqg_shard_cov_count",
     "sqh_default_options", "sqh_open_case", "sqh_open_concordant", "sqh_open_bam_case", "sqh_open_bam_chimeric", "sqh_case_chim_names", "sqh_probe_bam", "sqh_close_case", "sqh_case_batch", "sqh_case_chimeric", "sqh_case_config",
     "sqh_case_n_ref", "sqh_case_ref_len", "sqh_case_blocks",
@@ -124,6 +124,8 @@ def lib() -> C.CDLL:
     L.sqg_stat.argtypes = [_P, C.c_char_p]; L.sqg_stat.restype = C.c_int64
     L.sqg_classify_dump.argtypes = [_P, C.c_char_p, _P, C.c_int64, pp(C.c_int64)]
     L.sqg_plan_shards.argtypes = [pp(sqg_batch), pp(sqg_chimeric), pp(sqg_config), C.c_int32, C.c_int32, _P, pp(C.c_int32)]
+    L.sqg_plan_shards_resident.argtypes = [_P, C.c_int32, _P, pp(C.c_int32)]
+    L.sqg_keep_records.argtypes = [_P, C.c_int64, C.c_int64]
     L.sqg_set_shard.argtypes = [_P, C.c_int32, C.c_int32]
     L.sqg_shard_seeds.argtypes = [_P, C.c_int32, pp(_P), pp(C.c_int64)]
     L.sqg_shard_build.argtypes = [_P, _P, C.c_int64, pp(_P), pp(_P), pp(_P), pp(C.c_int64), pp(_P), pp(_P), pp(C.c_int32)]
@@ -486,6 +488,18 @@ class SegmentGraph:
         return self.vNodes
 
     # -- range shards of one stream (include/squid_b200.h "Exact range sharding"; driver: squid_b200/sharded.py) ---------
+    def plan_shards(self, n_shards: int):
+        """sqg_plan_shards_resident: the cuts of module-level plan_shards, planned on the resident batch and the loaded chimeric
+        reads.  Returns [c_0 = 0, ..., c_m = n_rec] with m <= n_shards."""
+        cuts = np.zeros(int(n_shards) + 1, np.int64)
+        m = C.c_int32()
+        self._ck(self.L.sqg_plan_shards_resident(self._h, int(n_shards), cuts.ctypes.data, C.byref(m)))
+        return [int(x) for x in cuts[: m.value + 1]]
+
+    def keep_records(self, lo: int, hi: int):
+        """sqg_keep_records: records [lo, hi) of the resident batch become the batch (one shard's range)."""
+        self._ck(self.L.sqg_keep_records(self._h, int(lo), int(hi)))
+
     def set_shard(self, index: int, count: int):
         self._ck(self.L.sqg_set_shard(self._h, index, count))
 

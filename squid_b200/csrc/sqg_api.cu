@@ -27,6 +27,7 @@
 #include "sq_phase1.cuh"
 #include "sq_phase2.cuh"
 #include "sq_phase3.cuh"
+#include "sq_plan.cuh"
 #include "sq_seed.cuh"
 #include "sq_gpusort.cuh"
 #include "sq_prepass.cuh"
@@ -647,6 +648,7 @@ void sqg_destroy(sqg_ctx *ctx) {
     ctx->d_omask.release(); ctx->d_shorts.release(); ctx->d_other_off.release(); ctx->d_other_key.release(); ctx->d_other_idx.release(); ctx->d_other_len.release(); ctx->d_other_own.release(); ctx->d_chimdiff.release(); ctx->h_chimdiff.release(); ctx->d_restbits.release(); ctx->d_restoff.release(); ctx->d_reflen.release(); ctx->d_ops.release(); ctx->d_ops_dense.release(); ctx->h_ops.release(); ctx->d_cutflag.release(); ctx->d_isl.release(); ctx->d_cap_ops.release(); ctx->d_cap_mar.release();
     ctx->d_isl_nout.release(); ctx->d_isl_gdone.release(); ctx->d_span.release(); ctx->d_heavy.release(); ctx->d_light.release(); ctx->d_off_ops.release(); ctx->d_off_mar.release(); ctx->d_dp.release();
     ctx->d_margin.release();
+    ctx->d_plan_reach.release(); ctx->d_plan_keep.release(); ctx->d_plan_upd.release(); ctx->d_plan_cand.release(); ctx->d_plan_sel.release(); ctx->h_plan_sel.release();
     ctx->d_bin_off.release(); ctx->d_bin_seg.release(); ctx->d_flen.release(); ctx->d_tileagg.release(); ctx->d_ccmax.release(); ctx->d_cov_nq.release(); ctx->d_cov_qmax.release(); ctx->d_cov_rank0.release(); ctx->d_cov_incmax.release(); ctx->d_temp_cov.release(); ctx->d_desc.release(); ctx->d_cand_key.release(); ctx->d_chain64.release(); ctx->d_nchr.release(); ctx->d_npos.release(); ctx->d_nend.release(); ctx->d_chr_first.release(); ctx->d_cnt3.release(); ctx->d_sum3.release();
     ctx->d_chain_used.release(); ctx->d_qend.release(); ctx->d_covtile.release(); ctx->d_slow.release(); ctx->d_head.release(); ctx->d_ew.release(); ctx->d_dtile.release(); ctx->d_ekeys.release(); ctx->d_ekeys2.release(); ctx->d_ukeys.release(); ctx->d_ecount.release(); ctx->d_sens.release();
     ctx->d_e_ind1.release(); ctx->d_e_ind2.release(); ctx->d_e_w.release(); ctx->d_e_heads.release();
@@ -756,7 +758,7 @@ extern "C" int sqg_load_concordant(sqg_ctx *ctx, const sqg_batch *hb, int64_t fi
     b.blk_off = ctx->o_blk_off.p; b.blk_ref_pos = ctx->o_blk_ref_pos.p; b.blk_match_ref = ctx->o_blk_match_ref.p;
     b.blk_read_pos = ctx->o_blk_read_pos.p; b.blk_match_read = ctx->o_blk_match_read.p;
     PHASE_END("h2d");
-    ctx->have_batch = true; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
+    ctx->have_batch = true; ctx->batch_restricted = false; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
     ctx->wire_loaded = false; ctx->classify_prelaunched = false;
     return SQG_OK;
 }
@@ -864,7 +866,7 @@ extern "C" int sqg_load_concordant_wire(sqg_ctx *ctx, const sqg_wire *w, int64_t
 #undef UPW
     if (n == 0) CK(cudaMemsetAsync(ctx->o_blk_off.p, 0, sizeof(uint32_t), ctx->stream));
     PHASE_END("h2d");
-    ctx->have_batch = true; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
+    ctx->have_batch = true; ctx->batch_restricted = false; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
     ctx->wire_loaded = true;
     return SQG_OK;
 }
@@ -922,7 +924,7 @@ extern "C" int sqg_download_concordant(sqg_ctx *ctx, sqg_batch *out) {
     DN(ref_id, n); DN(pos, n); DN(mate_ref_id, n); DN(mate_pos, n); DN(end_pos, n); DN(flag, n); DN(total_len, n); DN(lowphred_run, n); DN(mapq, n); DN(aux, n);
     DN(blk_off, n + 1); DN(blk_ref_pos, nb); DN(blk_match_ref, nb); DN(blk_read_pos, nb); DN(blk_match_read, nb);
 #undef DN
-    CK(cudaMemcpyAsync(ctx->h_counters.p + 28, ctx->d_counters.p + 28, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    if (ctx->wire_loaded) CK(cudaMemcpyAsync(ctx->h_counters.p + 28, ctx->d_counters.p + 28, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     if (ctx->wire_loaded && *(int32_t *)(ctx->h_counters.p + 28)) FAIL(SQG_EINVAL, "wire batch is inconsistent (escape without an exception entry, or block counts that contradict the tile table)");
     return SQG_OK;
@@ -938,7 +940,7 @@ extern "C" int sqg_attach_concordant_device(sqg_ctx *ctx, const sqg_batch *db, i
     b.ref_id = db->ref_id; b.pos = db->pos; b.mate_ref_id = db->mate_ref_id; b.mate_pos = db->mate_pos; b.end_pos = db->end_pos;
     b.flag = db->flag; b.total_len = db->total_len; b.lowphred_run = db->lowphred_run; b.mapq = db->mapq; b.aux = db->aux;
     b.blk_off = db->blk_off; b.blk_ref_pos = db->blk_ref_pos; b.blk_match_ref = db->blk_match_ref; b.blk_read_pos = db->blk_read_pos; b.blk_match_read = db->blk_match_read;
-    ctx->have_batch = true; ctx->batch_owned = false; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
+    ctx->have_batch = true; ctx->batch_restricted = false; ctx->batch_owned = false; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
     ctx->wire_loaded = false; ctx->classify_prelaunched = false;
     return SQG_OK;
 }
@@ -2089,6 +2091,101 @@ extern "C" int sqg_shard_redo_edges(sqg_ctx *ctx, int32_t init_hint) {
     return run_assign(ctx, false, true);
 }
 
+// host/plan.cpp's cuts from the resident batch (sq_plan.cuh): class bytes of the classification pass, groups of the chimeric
+// pre-pass, three exclusive scans, one candidate per record, compacted and sent back; the greedy runs on the host.
+static int plan_resident(sqg_ctx *ctx, int32_t n_shards, int64_t *cuts, int32_t *n_planned) {
+    int rc = run_classify(ctx);
+    if (rc) return rc;
+    rc = finish_prepass(ctx);
+    if (rc) return rc;
+    const DevBatch &b = ctx->batch;
+    const int64_t n = b.n_rec;
+    int64_t n_cand = 0;
+    PHASE_BEGIN("plan");
+    if (n > 0) {
+        CK(ctx->d_plan_reach.ensure((size_t)n)); CK(ctx->d_plan_keep.ensure((size_t)n)); CK(ctx->d_plan_upd.ensure((size_t)n));
+        CK(ctx->d_plan_cand.ensure((size_t)n)); CK(ctx->d_plan_sel.ensure((size_t)n));
+        LAUNCH(k_plan_prep, blocks_for(n), kThreads, b, ctx->d_cls.p, ctx->d_plan_reach.p, ctx->d_plan_keep.p, ctx->d_plan_upd.p);
+        size_t tb1 = 0, tb2 = 0, tb3 = 0;
+        int32_t *d_nsel = (int32_t *)(ctx->d_counters.p + 5);
+        CK(cub::DeviceScan::ExclusiveScan(nullptr, tb1, ctx->d_plan_reach.p, ctx->d_plan_reach.p, MaxU64(), (uint64_t)0, (int)n, ctx->stream));
+        CK(cub::DeviceScan::ExclusiveScan(nullptr, tb2, ctx->d_plan_keep.p, ctx->d_plan_keep.p, MaxI32(), (int32_t)-1, (int)n, ctx->stream));
+        CK(cub::DeviceSelect::If(nullptr, tb3, ctx->d_plan_cand.p, ctx->d_plan_sel.p, d_nsel, (int)n, PlanIsCand(), ctx->stream));
+        ENSURE_TEMP(std::max({tb1, tb2, tb3}));
+        CK(cub::DeviceScan::ExclusiveScan(ctx->d_temp.p, tb1, ctx->d_plan_reach.p, ctx->d_plan_reach.p, MaxU64(), (uint64_t)0, (int)n, ctx->stream));
+        CK(cub::DeviceScan::ExclusiveScan(ctx->d_temp.p, tb2, ctx->d_plan_keep.p, ctx->d_plan_keep.p, MaxI32(), (int32_t)-1, (int)n, ctx->stream));
+        CK(cub::DeviceScan::ExclusiveScan(ctx->d_temp.p, tb2, ctx->d_plan_upd.p, ctx->d_plan_upd.p, MaxI32(), (int32_t)-1, (int)n, ctx->stream));
+        LAUNCH(k_plan_cands, blocks_for(n), kThreads, b, ctx->params, ctx->d_cls.p, ctx->d_plan_reach.p, ctx->d_plan_keep.p, ctx->d_plan_upd.p,
+               ctx->d_groups.p, ctx->d_disc.p, ctx->pre_nG, ctx->d_plan_cand.p);
+        CK(cub::DeviceSelect::If(ctx->d_temp.p, tb3, ctx->d_plan_cand.p, ctx->d_plan_sel.p, d_nsel, (int)n, PlanIsCand(), ctx->stream));
+        ctx->launches += 4;
+        CK(cudaMemcpyAsync(ctx->h_counters.p + 5, ctx->d_counters.p + 5, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        n_cand = *(const int32_t *)(ctx->h_counters.p + 5);
+        CK(ctx->h_plan_sel.ensure((size_t)n_cand + 1));
+        if (n_cand > 0) CK(cudaMemcpyAsync(ctx->h_plan_sel.p, ctx->d_plan_sel.p, (size_t)n_cand * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    PHASE_END("plan");
+    CK(cudaStreamSynchronize(ctx->stream));
+    *n_planned = plan_greedy(ctx->h_plan_sel.p, n_cand, n, n_shards, cuts);
+    return SQG_OK;
+}
+
+extern "C" int sqg_plan_shards_resident(sqg_ctx *ctx, int32_t n_shards, int64_t *cuts, int32_t *n_planned) {
+    if (!ctx || !cuts || !n_planned || n_shards < 1) return SQG_EINVAL;
+    if (!ctx->have_batch || !ctx->have_chim) FAIL(SQG_ESTATE, "load the concordant batch and the chimeric reads first");
+    if (ctx->batch_restricted) FAIL(SQG_ESTATE, "sqg_plan_shards_resident: the batch is one shard's range already (sqg_keep_records); plan on the whole stream");
+    CK(cudaSetDevice(ctx->device));
+    CK(ctx->d_counters.ensure(32)); CK(ctx->h_counters.ensure(32));
+    const int rc = plan_resident(ctx, n_shards, cuts, n_planned);
+    // the scratch is as large as the batch and only needed once per load
+    ctx->d_plan_reach.release(); ctx->d_plan_keep.release(); ctx->d_plan_upd.release(); ctx->d_plan_cand.release(); ctx->d_plan_sel.release();
+    return rc;
+}
+
+// Records [lo, hi) of the resident batch become the batch, moved to the front of the context's own arrays: the tile loads of
+// the classification pass (cp.async.bulk) need every array to start 16-byte aligned, which an offset pointer would not be.
+extern "C" int sqg_keep_records(sqg_ctx *ctx, int64_t lo, int64_t hi) {
+    if (!ctx) return SQG_EINVAL;
+    if (!ctx->have_batch) FAIL(SQG_ESTATE, "no concordant batch loaded");
+    if (!ctx->batch_owned) FAIL(SQG_ESTATE, "sqg_keep_records: the batch is attached (caller-owned device arrays)");
+    if (lo < 0 || lo > hi || hi > ctx->batch.n_rec) FAIL(SQG_EINVAL, "sqg_keep_records: need 0 <= lo <= hi <= n_rec");
+    CK(cudaSetDevice(ctx->device));
+    { const int rcj = cov_join(ctx); if (rcj) return rcj; }
+    cudaStream_t st = ctx->stream;
+    uint32_t ends[2];
+    CK(cudaMemcpyAsync(&ends[0], ctx->o_blk_off.p + lo, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&ends[1], ctx->o_blk_off.p + hi, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (ends[1] < ends[0] || (int64_t)ends[1] > ctx->batch.n_blk) FAIL(SQG_EINVAL, "sqg_keep_records: blk_off of the batch is not monotone");
+    const int64_t nr = hi - lo, b0 = ends[0], nb = (int64_t)ends[1] - b0;
+    DBuf<uint8_t> tmp;  // a range that overlaps its destination goes through here
+    struct Release { DBuf<uint8_t> &t; ~Release() { t.release(); } } release_tmp{tmp};
+    CK(tmp.ensure((size_t)std::max<int64_t>(4 * (nr + 1), 4 * nb)));
+    cudaError_t e = cudaSuccess;
+    auto move = [&](void *arr, size_t elem, int64_t first, int64_t count) {
+        char *p = (char *)arr;
+        const size_t bytes = (size_t)count * elem;
+        if (e != cudaSuccess || first == 0 || count == 0) return;
+        if (first >= count) { e = cudaMemcpyAsync(p, p + (size_t)first * elem, bytes, cudaMemcpyDeviceToDevice, st); return; }
+        e = cudaMemcpyAsync(tmp.p, p + (size_t)first * elem, bytes, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(p, tmp.p, bytes, cudaMemcpyDeviceToDevice, st);
+    };
+    move(ctx->o_ref_id.p, 4, lo, nr); move(ctx->o_pos.p, 4, lo, nr); move(ctx->o_mate_ref_id.p, 4, lo, nr); move(ctx->o_mate_pos.p, 4, lo, nr);
+    move(ctx->o_end_pos.p, 4, lo, nr); move(ctx->o_flag.p, 2, lo, nr); move(ctx->o_total_len.p, 2, lo, nr); move(ctx->o_lowphred_run.p, 2, lo, nr);
+    move(ctx->o_mapq.p, 1, lo, nr); move(ctx->o_aux.p, 1, lo, nr);
+    move(ctx->o_blk_ref_pos.p, 4, b0, nb); move(ctx->o_blk_match_ref.p, 4, b0, nb); move(ctx->o_blk_read_pos.p, 2, b0, nb); move(ctx->o_blk_match_read.p, 2, b0, nb);
+    CK(e);
+    CK(cudaMemcpyAsync(tmp.p, ctx->o_blk_off.p + lo, (size_t)(nr + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+    LAUNCH(k_keep_offsets, blocks_for(nr + 1), kThreads, ctx->o_blk_off.p, (const uint32_t *)tmp.p, nr + 1, (uint32_t)b0);
+    CK(cudaStreamSynchronize(st));
+    DevBatch &b = ctx->batch;
+    b.n_rec = nr; b.n_blk = nb;
+    ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->classify_prelaunched = false;
+    ctx->first_record_index += lo; ctx->batch_restricted = true;
+    return SQG_OK;
+}
+
 // sort raw keys, run-length reduce, unpack
 static int reduce_edges(sqg_ctx *ctx, int64_t n_raw, const int32_t *d_weights_in) {
     ctx->n_unique_edges = 0;
@@ -2731,7 +2828,7 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
     b.flag = ctx->o_flag.p; b.total_len = ctx->o_total_len.p; b.lowphred_run = ctx->o_lowphred_run.p; b.mapq = ctx->o_mapq.p; b.aux = ctx->o_aux.p;
     b.blk_off = ctx->o_blk_off.p; b.blk_ref_pos = ctx->o_blk_ref_pos.p; b.blk_match_ref = ctx->o_blk_match_ref.p;
     b.blk_read_pos = ctx->o_blk_read_pos.p; b.blk_match_read = ctx->o_blk_match_read.p;
-    ctx->have_batch = true; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
+    ctx->have_batch = true; ctx->batch_restricted = false; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
     ctx->wire_loaded = false; ctx->classify_prelaunched = false;
     return SQG_OK;
 }

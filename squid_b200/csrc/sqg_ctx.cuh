@@ -19,6 +19,7 @@
 #include "sq_phase1.cuh"
 #include "sq_phase2.cuh"
 #include "sq_phase3.cuh"
+#include "sq_plan.cuh"
 #include "squid_b200.h"
 
 namespace sq {
@@ -123,6 +124,7 @@ struct sqg_ctx {
 
     // concordant batch
     bool have_batch = false, batch_owned = false, classified = false, cov_compacted = false;
+    bool batch_restricted = false;   // sqg_keep_records has cut the batch down to one shard's range
     int64_t first_record_index = 0;
     sq::DevBatch batch;
     sq::DBuf<int32_t> o_ref_id, o_pos, o_mate_ref_id, o_mate_pos, o_end_pos, o_blk_ref_pos, o_blk_match_ref;
@@ -245,6 +247,12 @@ struct sqg_ctx {
     sq::DBuf<int64_t> d_off_ops, d_off_mar;
     sq::DBuf<int32_t> d_margin;
     int64_t r_break = 0;
+
+    // the shard planner on the resident batch (sqg_plan_shards_resident): scan inputs / outputs, candidates; released after each plan
+    sq::DBuf<uint64_t> d_plan_reach;
+    sq::DBuf<int32_t> d_plan_keep, d_plan_upd;
+    sq::DBuf<uint64_t> d_plan_cand, d_plan_sel;
+    sq::HBuf<uint64_t> h_plan_sel;
 
     // range shard of one genome (sqg_set_shard, SURVEY.md 8e): index 0 owns the chimeric edges and the discordant depth
     int32_t shard_index = 0, shard_count = 1;

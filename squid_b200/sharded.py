@@ -179,6 +179,27 @@ class ShardedSegmentGraph:
             g.load_concordant(b)
             g.load_chimeric(chim_factory())
 
+    def load_bam(self, path: str, case):
+        """Every local shard context decodes the whole concordant BAM on its device (load_concordant_bam), loads all chimeric
+        reads, plans the cuts on the resident batch (plan_shards) and keeps its own record range (keep_records).  No records
+        travel between the ranks: each plans the same cuts from the same file, and one all-gather checks that they did.
+        `case` = HostCase(conc, chim, bam=True, header_only=True).  Returns the cuts; raises ValueError when the stream has
+        fewer clean cuts than shards."""
+        mine = []
+        for g in self.g:
+            g.load_concordant_bam(path, case)
+            g.load_chimeric(ChimericReads(case.chimeric.a))
+            mine.append(g.plan_shards(self.n_shards))
+        every = self.comm.allgather(mine)
+        if any(c != every[0] for c in every):
+            raise RuntimeError("shard contexts planned different cuts: %s" % every)
+        cuts = every[0]
+        if len(cuts) - 1 < self.n_shards:
+            raise ValueError("the stream has %d clean shards, not %d: cuts %s" % (len(cuts) - 1, self.n_shards, cuts))
+        for g, sid in zip(self.g, self.ids):
+            g.keep_records(cuts[sid], cuts[sid + 1])
+        return cuts
+
     # -- BuildNode_STAR ------------------------------------------------------------------------------------------------
     def BuildNode_STAR(self) -> Nodes:
         N = self.n_shards
