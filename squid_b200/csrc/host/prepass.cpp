@@ -204,7 +204,7 @@ extern "C" double sqh_time_sort(int64_t n, uint64_t seed, uint64_t range, int th
     return 1e3 * std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
 }
 
-void chimeric_prepass(const sqg_chimeric &c, int32_t n_ref, int32_t read_len, ChimPrepass &out, const SortHook &sort_hook) {
+void chimeric_prepass(const sqg_chimeric &c, int32_t n_ref, int32_t read_len, ChimPrepass &out) {
     const bool timing = getenv("SQH_TIMING") != nullptr;
     auto T0 = std::chrono::steady_clock::now();
     auto lap = [&](const char *w) { if (timing) { auto t = std::chrono::steady_clock::now(); fprintf(stderr, "[prepass] %s %.1f ms\n", w, 1e3 * std::chrono::duration<double>(t - T0).count()); T0 = t; } };
@@ -314,18 +314,13 @@ void chimeric_prepass(const sqg_chimeric &c, int32_t n_ref, int32_t read_len, Ch
     // the order among equal (RefID,RefPos) which the sub-cluster walk observes (SURVEY.md App. A-11).  The packed key
     // compares exactly like operator< of SingleBamRec_t (RefID, RefPos are non-negative here).
     lap("part sort");
-    bool sorted = false;
-    if (sort_hook && dis.size() >= 2) {  // the device computes the same permutation and leaves the cores alone
-        sorted = sort_hook(dis.data(), dis.size());
-    }
-    if (!sorted) sort_like_std(dis.data(), dis.data() + dis.size(), std::min(cores, 16));
-    lap(sorted ? "disc sort (device)" : "disc sort");
+    sort_like_std(dis.data(), dis.data() + dis.size(), std::min(cores, 16));
+    lap("disc sort");
     out.part_chr.reserve(part.size()); out.part_pos.reserve(part.size());
     for (auto &p : part) { out.part_chr.push_back(p.first); out.part_pos.push_back(p.second); }
     if (out.disc.capacity() < dis.size() + 1) {
-        if (out.before_disc_realloc) out.before_disc_realloc();
         out.disc.clear();
-        out.disc.reserve(dis.size() + 1 + dis.size() / 8);  // head room: the storage (and its page-lock) survives slightly larger inputs
+        out.disc.reserve(dis.size() + 1 + dis.size() / 8);  // head room: the storage survives slightly larger inputs
     }
     if (out.disc.size() != dis.size() + 1) out.disc.resize(dis.size() + 1);
     {   // gather the sorted blocks (random access into the caller's arrays)

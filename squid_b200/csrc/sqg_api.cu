@@ -37,6 +37,7 @@
 #include "sq_bam.cuh"
 #include "sqg_ctx.cuh"
 #include "host/bam.h"
+#include "host/prepass.h"
 
 using namespace sq;
 
@@ -634,46 +635,19 @@ void sqg_destroy(sqg_ctx *ctx) {
     cudaStreamSynchronize(ctx->stream);
     if (ctx->stream_cov) cudaStreamSynchronize(ctx->stream_cov);
     if (ctx->stream3) cudaStreamSynchronize(ctx->stream3);
-    // DBuf/HBuf members are plain pointers: release explicitly
-    ctx->o_ref_id.release(); ctx->o_pos.release(); ctx->o_mate_ref_id.release(); ctx->o_mate_pos.release(); ctx->o_end_pos.release();
-    ctx->o_blk_ref_pos.release(); ctx->o_blk_match_ref.release(); ctx->o_flag.release(); ctx->o_total_len.release(); ctx->o_lowphred_run.release();
-    ctx->o_blk_read_pos.release(); ctx->o_blk_match_read.release(); ctx->o_mapq.release(); ctx->o_aux.release(); ctx->o_blk_off.release();
-    ctx->d_cls.release(); ctx->d_other.release(); ctx->d_scratch32.release(); ctx->d_gap.release(); ctx->d_pc.release(); ctx->d_temp.release();
-    ctx->d_counters.release(); ctx->h_counters.release();
-    ctx->d_disc.release(); ctx->d_groups.release(); ctx->d_pchr.release(); ctx->d_ppos.release(); ctx->dc_read_off.release(); ctx->dc_n_first.release();
-    ctx->dc_first_total.release(); ctx->dc_second_total.release(); ctx->dc_ref_id.release(); ctx->dc_ref_pos.release(); ctx->dc_read_pos.release();
-    ctx->dc_match_ref.release(); ctx->dc_match_read.release(); ctx->dc_res0.release(); ctx->dc_rev.release();
-    ctx->dc0_ref_pos.release(); ctx->dc0_read_pos.release(); ctx->dc0_match_ref.release(); ctx->dc0_match_read.release();
-    ctx->d_trigger.release(); ctx->d_rest.release(); ctx->d_rest2.release(); ctx->d_restkey.release(); ctx->d_restkey2.release();
-    ctx->d_omask.release(); ctx->d_shorts.release(); ctx->d_other_off.release(); ctx->d_other_key.release(); ctx->d_other_idx.release(); ctx->d_other_len.release(); ctx->d_other_own.release(); ctx->d_chimdiff.release(); ctx->h_chimdiff.release(); ctx->d_restbits.release(); ctx->d_restoff.release(); ctx->d_reflen.release(); ctx->d_ops.release(); ctx->d_ops_dense.release(); ctx->h_ops.release(); ctx->d_cutflag.release(); ctx->d_isl.release(); ctx->d_cap_ops.release(); ctx->d_cap_mar.release();
-    ctx->d_isl_nout.release(); ctx->d_isl_gdone.release(); ctx->d_span.release(); ctx->d_heavy.release(); ctx->d_light.release(); ctx->d_off_ops.release(); ctx->d_off_mar.release(); ctx->d_dp.release();
-    ctx->d_margin.release();
-    ctx->d_plan_reach.release(); ctx->d_plan_keep.release(); ctx->d_plan_upd.release(); ctx->d_plan_cand.release(); ctx->d_plan_sel.release(); ctx->h_plan_sel.release();
-    ctx->d_bin_off.release(); ctx->d_bin_seg.release(); ctx->d_flen.release(); ctx->d_tileagg.release(); ctx->d_ccmax.release(); ctx->d_cov_nq.release(); ctx->d_cov_qmax.release(); ctx->d_cov_rank0.release(); ctx->d_cov_incmax.release(); ctx->d_temp_cov.release(); ctx->d_desc.release(); ctx->d_cand_key.release(); ctx->d_chain64.release(); ctx->d_nchr.release(); ctx->d_npos.release(); ctx->d_nend.release(); ctx->d_chr_first.release(); ctx->d_cnt3.release(); ctx->d_sum3.release();
-    ctx->d_chain_used.release(); ctx->d_qend.release(); ctx->d_covtile.release(); ctx->d_slow.release(); ctx->d_head.release(); ctx->d_ew.release(); ctx->d_dtile.release(); ctx->d_ekeys.release(); ctx->d_ekeys2.release(); ctx->d_ukeys.release(); ctx->d_ecount.release(); ctx->d_sens.release();
-    ctx->d_e_ind1.release(); ctx->d_e_ind2.release(); ctx->d_e_w.release(); ctx->d_e_heads.release();
-    ctx->d_bpkey.release(); ctx->d_covM.release(); ctx->d_qkey.release(); ctx->d_chunks.release(); ctx->d_r0.release(); ctx->d_t.release(); ctx->d_cov.release(); ctx->d_bpchr.release(); ctx->d_bppos.release();
-    ctx->h_chr.release(); ctx->h_pos.release(); ctx->h_len.release(); ctx->h_cnt3.release(); ctx->h_sum3.release(); ctx->h_ind1.release(); ctx->h_ind2.release();
-    ctx->h_w.release(); ctx->h_heads.release();
-    ctx->bam_comp.release(); ctx->bam_win[0].release(); ctx->bam_win[1].release(); ctx->bam_nblob.release(); ctx->bam_mem.release(); ctx->bam_seg.release();
-    ctx->bam_start.release(); ctx->bam_exit.release(); ctx->bam_newstart.release(); ctx->bam_recoff.release(); ctx->bam_small.release(); ctx->bam_noff.release();
-    ctx->bam_cnt.release(); ctx->bam_base.release(); ctx->bam_nblk.release(); ctx->bam_incl.release(); ctx->bam_nhash.release(); ctx->bam_nlen.release();
-    ctx->bam_bad.release(); ctx->bam_redo.release(); ctx->bam_lseq.release(); ctx->bam_stage[0].release(); ctx->bam_stage[1].release(); ctx->bam_hsmall.release();
     for (cudaEvent_t e : ctx->bam_ev) cudaEventDestroy(e);
     for (auto &kv : ctx->timers) { if (kv.second.a) cudaEventDestroy(kv.second.a); if (kv.second.b) cudaEventDestroy(kv.second.b); }
     cudaStreamDestroy(ctx->stream);
-    ctx->d_gs_keys.release(); ctx->d_gs_idx.release(); ctx->d_gs_scratch.release(); ctx->h_gs_keys.release(); ctx->h_gs_idx.release(); ctx->h_t.release();
     if (ctx->stream3) cudaStreamDestroy(ctx->stream3);
     if (ctx->ev_chim) cudaEventDestroy(ctx->ev_chim);
     if (ctx->ev_pre) cudaEventDestroy(ctx->ev_pre);
-    for (auto &pp : ctx->pre_pinned) if (pp.p) cudaHostUnregister(const_cast<void *>(pp.p));
     if (ctx->stream_cov) cudaStreamDestroy(ctx->stream_cov);
     if (ctx->stream_up) cudaStreamDestroy(ctx->stream_up);
     for (cudaEvent_t e : ctx->ev_up) cudaEventDestroy(e);
     if (ctx->ev_cov_fork) cudaEventDestroy(ctx->ev_cov_fork);
     if (ctx->ev_cov_done) cudaEventDestroy(ctx->ev_cov_done);
     if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
-    delete ctx;
+    delete ctx;  // (the buffers free themselves, on this device)
 }
 
 const char *sqg_last_error(const sqg_ctx *ctx) { return ctx ? ctx->err.c_str() : "null context"; }
@@ -694,7 +668,7 @@ int64_t sqg_stat(const sqg_ctx *ctx, const char *name) {
     if (!ctx || !name) return -1;
     const std::string n(name);
     if (n == "islands") return ctx->n_islands;
-    if (n == "device_sort_status") return ctx->gs_last_status;  // 0: the pre-pass sort ran on the device; -100: on the cores
+    if (n == "device_sort_status") return ctx->gs_last_status;  // 0: the pre-pass sort ran on the device (also on no discordant blocks); 2/3: it declined, the cores sorted; -100: no pre-pass yet
     if (n == "heavy_islands") return ctx->n_heavy;
     if (n == "giant_islands") return 0;  // every island runs in one block or one warp
     if (n == "cov_chain_fallback") return ctx->cov_chain_fallback;
@@ -730,6 +704,24 @@ int64_t sqg_stat(const sqg_ctx *ctx, const char *name) {
 
 }  // extern "C"
 
+// ctx->batch = the context's own arrays (o_*) holding n_rec records and n_blk blocks
+static void point_batch_at_own_arrays(sqg_ctx *ctx, int64_t n_rec, int64_t n_blk) {
+    DevBatch &b = ctx->batch;
+    b.n_rec = n_rec; b.n_blk = n_blk;
+    b.ref_id = ctx->o_ref_id.p; b.pos = ctx->o_pos.p; b.mate_ref_id = ctx->o_mate_ref_id.p; b.mate_pos = ctx->o_mate_pos.p; b.end_pos = ctx->o_end_pos.p;
+    b.flag = ctx->o_flag.p; b.total_len = ctx->o_total_len.p; b.lowphred_run = ctx->o_lowphred_run.p; b.mapq = ctx->o_mapq.p; b.aux = ctx->o_aux.p;
+    b.blk_off = ctx->o_blk_off.p; b.blk_ref_pos = ctx->o_blk_ref_pos.p; b.blk_match_ref = ctx->o_blk_match_ref.p;
+    b.blk_read_pos = ctx->o_blk_read_pos.p; b.blk_match_read = ctx->o_blk_match_read.p;
+}
+// A new batch is resident: nothing computed on the previous one applies (the segment table, have_nodes, still does).  `wire`: its
+// arrays come from the wire decode, whose consistency flag run_classify checks and whose classification may already be running
+// (classify_prelaunched, set during that upload, stands); every other batch starts unclassified.
+static void reset_batch_state(sqg_ctx *ctx, bool owned, int64_t first_record_index, bool wire) {
+    ctx->have_batch = true; ctx->batch_owned = owned; ctx->batch_restricted = false; ctx->first_record_index = first_record_index;
+    ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->wire_loaded = wire;
+    if (!wire) ctx->classify_prelaunched = false;
+}
+
 extern "C" int sqg_load_concordant(sqg_ctx *ctx, const sqg_batch *hb, int64_t first_record_index) {
     if (!ctx || !hb || hb->n_rec < 0 || hb->n_blk < 0) return SQG_EINVAL;
     if (hb->n_rec >= 0x7fffff00ll) FAIL(SQG_EUNSUPPORTED, "more than 2^31 records per context: shard the stream");
@@ -751,15 +743,9 @@ extern "C" int sqg_load_concordant(sqg_ctx *ctx, const sqg_batch *hb, int64_t fi
     UP(o_blk_off, blk_off, n + 1);
     UP(o_blk_ref_pos, blk_ref_pos, nb); UP(o_blk_match_ref, blk_match_ref, nb); UP(o_blk_read_pos, blk_read_pos, nb); UP(o_blk_match_read, blk_match_read, nb);
 #undef UP
-    DevBatch &b = ctx->batch;
-    b.n_rec = hb->n_rec; b.n_blk = hb->n_blk;
-    b.ref_id = ctx->o_ref_id.p; b.pos = ctx->o_pos.p; b.mate_ref_id = ctx->o_mate_ref_id.p; b.mate_pos = ctx->o_mate_pos.p; b.end_pos = ctx->o_end_pos.p;
-    b.flag = ctx->o_flag.p; b.total_len = ctx->o_total_len.p; b.lowphred_run = ctx->o_lowphred_run.p; b.mapq = ctx->o_mapq.p; b.aux = ctx->o_aux.p;
-    b.blk_off = ctx->o_blk_off.p; b.blk_ref_pos = ctx->o_blk_ref_pos.p; b.blk_match_ref = ctx->o_blk_match_ref.p;
-    b.blk_read_pos = ctx->o_blk_read_pos.p; b.blk_match_read = ctx->o_blk_match_read.p;
+    point_batch_at_own_arrays(ctx, hb->n_rec, hb->n_blk);
     PHASE_END("h2d");
-    ctx->have_batch = true; ctx->batch_restricted = false; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
-    ctx->wire_loaded = false; ctx->classify_prelaunched = false;
+    reset_batch_state(ctx, true, first_record_index, false);
     return SQG_OK;
 }
 
@@ -820,12 +806,7 @@ extern "C" int sqg_load_concordant_wire(sqg_ctx *ctx, const sqg_wire *w, int64_t
     wo.lowphred_run = ctx->o_lowphred_run.p; wo.aux = ctx->o_aux.p; wo.blk_off = ctx->o_blk_off.p; wo.blk_ref_pos = ctx->o_blk_ref_pos.p; wo.blk_match_ref = ctx->o_blk_match_ref.p;
     wo.blk_read_pos = ctx->o_blk_read_pos.p; wo.blk_match_read = ctx->o_blk_match_read.p;
     wo.bad = (int32_t *)(ctx->d_counters.p + 28);
-    DevBatch &b = ctx->batch;
-    b.n_rec = n; b.n_blk = nb;
-    b.ref_id = ctx->o_ref_id.p; b.pos = ctx->o_pos.p; b.mate_ref_id = ctx->o_mate_ref_id.p; b.mate_pos = ctx->o_mate_pos.p; b.end_pos = ctx->o_end_pos.p;
-    b.flag = ctx->o_flag.p; b.total_len = ctx->o_total_len.p; b.lowphred_run = ctx->o_lowphred_run.p; b.mapq = ctx->o_mapq.p; b.aux = ctx->o_aux.p;
-    b.blk_off = ctx->o_blk_off.p; b.blk_ref_pos = ctx->o_blk_ref_pos.p; b.blk_match_ref = ctx->o_blk_match_ref.p;
-    b.blk_read_pos = ctx->o_blk_read_pos.p; b.blk_match_read = ctx->o_blk_match_read.p;
+    point_batch_at_own_arrays(ctx, n, nb);
     // The classification tile kernel needs nothing but the batch: it follows every chunk's widening kernel on the main stream, so
     // that it, too, runs while the later chunks are on the bus (run_classify then only finishes: scans, lists).  A tile looks at
     // the first record of the NEXT tile (sortedness), so the last tile of a chunk waits for the next chunk.
@@ -866,8 +847,7 @@ extern "C" int sqg_load_concordant_wire(sqg_ctx *ctx, const sqg_wire *w, int64_t
 #undef UPW
     if (n == 0) CK(cudaMemsetAsync(ctx->o_blk_off.p, 0, sizeof(uint32_t), ctx->stream));
     PHASE_END("h2d");
-    ctx->have_batch = true; ctx->batch_restricted = false; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
-    ctx->wire_loaded = true;
+    reset_batch_state(ctx, true, first_record_index, true);
     return SQG_OK;
 }
 
@@ -878,31 +858,32 @@ extern "C" int sqg_connected_components(int32_t device, int64_t n_nodes, const i
     if (n_nodes == 0) return n_edges == 0 ? SQG_OK : SQG_EINVAL;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev || cudaSetDevice(device) != cudaSuccess) return SQG_ENODEVICE;
-    DBuf<int32_t> parent, flag, rank, e1, e2, bad;
-    DBuf<uint8_t> temp;
     cudaStream_t st;
     if (cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) != cudaSuccess) return SQG_ECUDA;
+    DBuf<int32_t> mem;  // one allocation per call: parent, flag, rank, e1, e2, bad and the scan's scratch, each 256-byte aligned
     int rc = SQG_OK;
     do {
 #define CC_CK(x) if ((x) != cudaSuccess) { cudaGetLastError(); rc = SQG_ECUDA; break; }
-        CC_CK(parent.ensure((size_t)n_nodes)); CC_CK(flag.ensure((size_t)n_nodes)); CC_CK(rank.ensure((size_t)n_nodes)); CC_CK(bad.ensure(1));
-        CC_CK(e1.ensure((size_t)(n_edges ? n_edges : 1))); CC_CK(e2.ensure((size_t)(n_edges ? n_edges : 1)));
-        CC_CK(cudaMemsetAsync(bad.p, 0, 4, st));
-        if (n_edges) { CC_CK(cudaMemcpyAsync(e1.p, ind1, (size_t)n_edges * 4, cudaMemcpyHostToDevice, st)); CC_CK(cudaMemcpyAsync(e2.p, ind2, (size_t)n_edges * 4, cudaMemcpyHostToDevice, st)); }
-        k_cc_init<<<blocks_for(n_nodes), kThreads, 0, st>>>(parent.p, n_nodes);
-        if (n_edges) k_cc_hook<<<blocks_for(n_edges), kThreads, 0, st>>>(parent.p, e1.p, e2.p, n_edges, n_nodes, bad.p);
-        k_cc_flatten<<<blocks_for(n_nodes), kThreads, 0, st>>>(parent.p, n_nodes, flag.p);
         size_t tb = 0;
-        CC_CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, flag.p, rank.p, (int)n_nodes, st));
-        CC_CK(temp.ensure(tb ? tb : 1));
-        CC_CK(cub::DeviceScan::ExclusiveSum(temp.p, tb, flag.p, rank.p, (int)n_nodes, st));
-        k_cc_label<<<blocks_for(n_nodes), kThreads, 0, st>>>(parent.p, rank.p, n_nodes, flag.p);  // (flag is free again: the labels)
+        CC_CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, (int32_t *)nullptr, (int32_t *)nullptr, (int)n_nodes, st));
+        auto words = [](size_t k) { return (k + 63) & ~(size_t)63; };
+        const size_t wn = words((size_t)n_nodes), we = words((size_t)(n_edges ? n_edges : 1));
+        CC_CK(mem.ensure(3 * wn + 2 * we + 64 + words(tb / 4 + 1)));
+        int32_t *parent = mem.p, *flag = parent + wn, *rank = flag + wn, *e1 = rank + wn, *e2 = e1 + we, *bad = e2 + we;
+        void *temp = bad + 64;
+        CC_CK(cudaMemsetAsync(bad, 0, 4, st));
+        if (n_edges) { CC_CK(cudaMemcpyAsync(e1, ind1, (size_t)n_edges * 4, cudaMemcpyHostToDevice, st)); CC_CK(cudaMemcpyAsync(e2, ind2, (size_t)n_edges * 4, cudaMemcpyHostToDevice, st)); }
+        k_cc_init<<<blocks_for(n_nodes), kThreads, 0, st>>>(parent, n_nodes);
+        if (n_edges) k_cc_hook<<<blocks_for(n_edges), kThreads, 0, st>>>(parent, e1, e2, n_edges, n_nodes, bad);
+        k_cc_flatten<<<blocks_for(n_nodes), kThreads, 0, st>>>(parent, n_nodes, flag);
+        CC_CK(cub::DeviceScan::ExclusiveSum(temp, tb, flag, rank, (int)n_nodes, st));
+        k_cc_label<<<blocks_for(n_nodes), kThreads, 0, st>>>(parent, rank, n_nodes, flag);  // (flag is free again: the labels)
         CC_CK(cudaGetLastError());
         int32_t hbad = 0, last_rank = 0, last_root = 0;
-        CC_CK(cudaMemcpyAsync(label_out, flag.p, (size_t)n_nodes * 4, cudaMemcpyDeviceToHost, st));
-        CC_CK(cudaMemcpyAsync(&hbad, bad.p, 4, cudaMemcpyDeviceToHost, st));
-        CC_CK(cudaMemcpyAsync(&last_rank, rank.p + (n_nodes - 1), 4, cudaMemcpyDeviceToHost, st));
-        CC_CK(cudaMemcpyAsync(&last_root, parent.p + (n_nodes - 1), 4, cudaMemcpyDeviceToHost, st));
+        CC_CK(cudaMemcpyAsync(label_out, flag, (size_t)n_nodes * 4, cudaMemcpyDeviceToHost, st));
+        CC_CK(cudaMemcpyAsync(&hbad, bad, 4, cudaMemcpyDeviceToHost, st));
+        CC_CK(cudaMemcpyAsync(&last_rank, rank + (n_nodes - 1), 4, cudaMemcpyDeviceToHost, st));
+        CC_CK(cudaMemcpyAsync(&last_root, parent + (n_nodes - 1), 4, cudaMemcpyDeviceToHost, st));
         CC_CK(cudaStreamSynchronize(st));
 #undef CC_CK
         if (hbad) { rc = SQG_EINVAL; break; }
@@ -940,35 +921,8 @@ extern "C" int sqg_attach_concordant_device(sqg_ctx *ctx, const sqg_batch *db, i
     b.ref_id = db->ref_id; b.pos = db->pos; b.mate_ref_id = db->mate_ref_id; b.mate_pos = db->mate_pos; b.end_pos = db->end_pos;
     b.flag = db->flag; b.total_len = db->total_len; b.lowphred_run = db->lowphred_run; b.mapq = db->mapq; b.aux = db->aux;
     b.blk_off = db->blk_off; b.blk_ref_pos = db->blk_ref_pos; b.blk_match_ref = db->blk_match_ref; b.blk_read_pos = db->blk_read_pos; b.blk_match_read = db->blk_match_read;
-    ctx->have_batch = true; ctx->batch_restricted = false; ctx->batch_owned = false; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
-    ctx->wire_loaded = false; ctx->classify_prelaunched = false;
+    reset_batch_state(ctx, false, first_record_index, false);
     return SQG_OK;
-}
-
-// The discordant-block sort of the chimeric pre-pass on the device (sq_gpusort.cuh): called on the pre-pass thread, works on
-// its own stream next to the classification kernels.  Leaves `a` untouched unless it returns true.
-static bool device_sort_hook(sqg_ctx *ctx, sqh::SortKey *a, size_t n) {
-    const size_t min_n = getenv("SQG_GPU_SORT_MIN") ? (size_t)atoll(getenv("SQG_GPU_SORT_MIN")) : (size_t)(1 << 15);
-    ctx->gs_last_status = -100;
-    if (n < min_n || n >= 0x7fffff00ull) return false;  // small sorts are faster on the cores than a round trip
-    if (cudaSetDevice(ctx->device) != cudaSuccess) return false;
-    // (stream3 has the highest priority: its short kernels take the SM slots that the big stream kernels free, ahead of their own CTAs)
-    if (ctx->d_gs_keys.ensure(n) != cudaSuccess || ctx->d_gs_idx.ensure(n) != cudaSuccess || ctx->d_gs_scratch.ensure(gsort::bytes_needed(n)) != cudaSuccess ||
-        ctx->h_gs_keys.ensure(n) != cudaSuccess || ctx->h_gs_idx.ensure(n) != cudaSuccess) { cudaGetLastError(); return false; }
-    uint64_t *hk = ctx->h_gs_keys.p; uint32_t *hi = ctx->h_gs_idx.p;
-#pragma omp parallel for num_threads(4) schedule(static)
-    for (long long i = 0; i < (long long)n; i++) { hk[i] = a[i].key; hi[i] = a[i].k; }
-    if (cudaMemcpyAsync(ctx->d_gs_keys.p, hk, n * 8, cudaMemcpyHostToDevice, ctx->stream3) != cudaSuccess) return false;
-    if (cudaMemcpyAsync(ctx->d_gs_idx.p, hi, n * 4, cudaMemcpyHostToDevice, ctx->stream3) != cudaSuccess) return false;
-    const int rc = gsort::sort_like_std_device(ctx->d_gs_keys.p, ctx->d_gs_idx.p, n, ctx->d_gs_scratch.p, ctx->stream3, &ctx->gs_launches);
-    ctx->gs_last_status = rc;
-    if (rc != 0) { cudaGetLastError(); return false; }
-    // only the permutation comes back: the pre-pass reads nothing but the block indices after the sort
-    if (cudaMemcpyAsync(hi, ctx->d_gs_idx.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream3) != cudaSuccess) return false;
-    if (cudaStreamSynchronize(ctx->stream3) != cudaSuccess) return false;
-#pragma omp parallel for num_threads(4) schedule(static)
-    for (long long i = 0; i < (long long)n; i++) a[i].k = hi[i];
-    return true;
 }
 
 // test hook: does the device sort reproduce std::sort's permutation (payload included) on n keys drawn from [0,range)?
@@ -988,33 +942,34 @@ extern "C" int sqg_selftest_gpu_sort(int32_t device, int64_t n, uint64_t seed, u
     std::vector<uint64_t> hk((size_t)n); std::vector<uint32_t> hi((size_t)n);
     for (int64_t i = 0; i < n; i++) { hk[(size_t)i] = a[(size_t)i].key; hi[(size_t)i] = a[(size_t)i].k; }
     std::sort(a.begin(), a.end(), [](const sqh::SortKey &p, const sqh::SortKey &q) { return p.key < q.key; });
-    uint64_t *dk = nullptr; uint32_t *di = nullptr; unsigned char *ds = nullptr;
+    DBuf<uint64_t> dk; DBuf<uint32_t> di; DBuf<unsigned char> ds;
     cudaStream_t st;
     int verdict = -1;
     if (cudaStreamCreate(&st) != cudaSuccess) return -1;
-    if (cudaMalloc(&dk, (size_t)n * 8 + 8) == cudaSuccess && cudaMalloc(&di, (size_t)n * 4 + 4) == cudaSuccess && cudaMalloc(&ds, gsort::bytes_needed((size_t)n)) == cudaSuccess) {
-        cudaMemcpy(dk, hk.data(), (size_t)n * 8, cudaMemcpyHostToDevice); cudaMemcpy(di, hi.data(), (size_t)n * 4, cudaMemcpyHostToDevice);
+    if (dk.ensure((size_t)n + 1) == cudaSuccess && di.ensure((size_t)n + 1) == cudaSuccess && ds.ensure(gsort::bytes_needed((size_t)n)) == cudaSuccess) {
+        cudaMemcpy(dk.p, hk.data(), (size_t)n * 8, cudaMemcpyHostToDevice); cudaMemcpy(di.p, hi.data(), (size_t)n * 4, cudaMemcpyHostToDevice);
         cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
         cudaEventRecord(e0, st);
-        const int rc = gsort::sort_like_std_device(dk, di, (size_t)n, ds, st, nullptr);
+        const int rc = gsort::sort_like_std_device(dk.p, di.p, (size_t)n, ds.p, st, nullptr);
         cudaEventRecord(e1, st); cudaEventSynchronize(e1);
         if (ms_out) cudaEventElapsedTime(ms_out, e0, e1);
         cudaEventDestroy(e0); cudaEventDestroy(e1);
         if (rc != 0) verdict = rc;
         else {
-            cudaMemcpy(hk.data(), dk, (size_t)n * 8, cudaMemcpyDeviceToHost); cudaMemcpy(hi.data(), di, (size_t)n * 4, cudaMemcpyDeviceToHost);
+            cudaMemcpy(hk.data(), dk.p, (size_t)n * 8, cudaMemcpyDeviceToHost); cudaMemcpy(hi.data(), di.p, (size_t)n * 4, cudaMemcpyDeviceToHost);
             verdict = cudaGetLastError() == cudaSuccess ? 1 : -2;
             for (int64_t i = 0; verdict == 1 && i < n; i++) if (a[(size_t)i].key != hk[(size_t)i] || a[(size_t)i].k != hi[(size_t)i]) verdict = 0;
         }
     }
-    cudaFree(dk); cudaFree(di); cudaFree(ds); cudaStreamDestroy(st);
+    cudaStreamDestroy(st);
     return verdict;
 }
 
 // The chimeric pre-pass on the device (sq_prepass.cuh), run by the pre-pass thread on stream3 beside the classification: the
 // chimeric arrays are in HBM already (this thread uploaded them), the products never touch the host -- only their sizes do.
+// Reads without blocks, or no reads, push nothing: the zeroed sentinel alone, no groups, PartAlignPos = n_ref entries (0, 0).
 #define PCK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) return (int)e_; } while (0)
-static int device_prepass(sqg_ctx *ctx, size_t nr, size_t nb) {
+static int device_prepass(sqg_ctx *ctx, size_t nr) {
     cudaStream_t st = ctx->stream3;
     const int32_t n_ref = ctx->params.n_ref;
     PreChim c;
@@ -1106,8 +1061,8 @@ static int device_prepass(sqg_ctx *ctx, size_t nr, size_t nb) {
     ctx->pre_nD = (int32_t)nD; ctx->pre_nG = nG; ctx->pre_nP = (int32_t)nP;
     ctx->gs_launches += launches;
     if (ctx->shard_count > 1) {  // a range shard looks its first group up on the host (seed_stage: g_lo)
-        ctx->pre.groups.resize((size_t)nG);
-        if (nG) PCK(cudaMemcpyAsync(ctx->pre.groups.data(), ctx->d_groups.p, (size_t)nG * sizeof(Group), cudaMemcpyDeviceToHost, st));
+        ctx->h_groups.resize((size_t)nG);
+        if (nG) PCK(cudaMemcpyAsync(ctx->h_groups.data(), ctx->d_groups.p, (size_t)nG * sizeof(Group), cudaMemcpyDeviceToHost, st));
         PCK(cudaStreamSynchronize(st));
     }
     return 0;
@@ -1125,8 +1080,8 @@ extern "C" int sqg_load_chimeric(sqg_ctx *ctx, const sqg_chimeric *c) {
         const uint32_t nb = c->read_off[i + 1] - c->read_off[i], nf = c->n_first[i];
         if (nf > nb || nf > (uint32_t)kMaxBlocks || nb - nf > (uint32_t)kMaxBlocks) FAIL(SQG_EUNSUPPORTED, "chimeric read with more than 16 blocks in one mate");
     }
-    // The chimeric pre-pass (BuildNode_STAR part A, host std::sort for tie-order fidelity) runs on a host thread while the
-    // stream copies and classifies the concordant batch; it is joined in sqg_build_nodes / sqg_build_edges.
+    // The upload of the chimeric reads and their pre-pass (BuildNode_STAR part A) are driven by a host thread on stream3 while the
+    // caller's stream copies and classifies the concordant batch; they are joined in sqg_build_nodes / sqg_build_edges.
     ctx->prepass_worker.wait();
     ctx->chim_view = *c;
     ctx->chim_undo.clear();  // fresh arrays: nothing of an earlier patch applies
@@ -1143,7 +1098,6 @@ extern "C" int sqg_load_chimeric(sqg_ctx *ctx, const sqg_chimeric *c) {
     CK(cudaStreamWaitEvent(ctx->stream3, ctx->ev_fork, 0));
     ctx->chim_upload_err = 0;
     ctx->chim_upload_pending = true;
-    ctx->prepass_stage.store(0);
     {   // "prepass" phase timer: created here, on the caller's thread (the map is not touched by the pre-pass thread, only its events)
         PhaseTimer &t = ctx->timers["prepass"];
         if (!t.a) { CK(cudaEventCreate(&t.a)); CK(cudaEventCreate(&t.b)); }
@@ -1151,89 +1105,31 @@ extern "C" int sqg_load_chimeric(sqg_ctx *ctx, const sqg_chimeric *c) {
         ctx->prepass_timer = &t;
     }
     ctx->prepass_worker.submit([ctx, nr, nb]() {
-        sqh::SortHook hook;
-        static const bool gpu_sort = !(getenv("SQG_GPU_SORT") && atoi(getenv("SQG_GPU_SORT")) == 0);
-        if (gpu_sort) hook = [ctx](sqh::SortKey *a, size_t n) { return device_sort_hook(ctx, a, n); };
+        // the chimeric arrays first, then the pre-pass itself on the device (sq_prepass.cuh): nothing of it runs on the cores
         cudaSetDevice(ctx->device);
-        cudaStreamSynchronize(ctx->stream3);  // a previous job's DMA out of ctx->pre must be over before the vectors are rewritten
-        static const bool dev_pre = !(getenv("SQG_DEVICE_PREPASS") && atoi(getenv("SQG_DEVICE_PREPASS")) == 0);
-        if (dev_pre && nr > 0 && nb > 0) {
-            // the chimeric arrays first, then the pre-pass itself on the device (sq_prepass.cuh): nothing of it runs on the cores
-            const sqg_chimeric &c = ctx->chim_view;
-            cudaError_t e = cudaEventRecord(ctx->prepass_timer->a, ctx->stream3);
-#define UPW(buf, src, cnt) do { if (e == cudaSuccess && (cnt)) e = cudaMemcpyAsync(ctx->buf.p, (src), (cnt) * sizeof(*(src)), cudaMemcpyHostToDevice, ctx->stream3); } while (0)
-            UPW(dc_read_off, c.read_off, nr + 1); UPW(dc_n_first, c.n_first, nr);
-            UPW(dc_first_total, c.first_total_len, nr); UPW(dc_second_total, c.second_total_len, nr);
-            UPW(dc_first_low, c.first_lowphred, nr); UPW(dc_second_low, c.second_lowphred, nr); UPW(dc_multi, c.multi_filter, nr);
-            UPW(dc_ref_id, c.blk_ref_id, nb); UPW(dc0_ref_pos, c.blk_ref_pos, nb); UPW(dc0_read_pos, c.blk_read_pos, nb);
-            UPW(dc0_match_ref, c.blk_match_ref, nb); UPW(dc0_match_read, c.blk_match_read, nb); UPW(dc_rev, c.blk_is_reverse, nb);
-#undef UPW
-            if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_chim, ctx->stream3);
-            ctx->chim_upload_err = (int)e;
-            int rc = e == cudaSuccess ? device_prepass(ctx, nr, nb) : (int)e;
-            if (rc == 0) rc = (int)cudaEventRecord(ctx->ev_pre, ctx->stream3);
-            if (rc == 0) { rc = (int)cudaEventRecord(ctx->prepass_timer->b, ctx->stream3); ctx->prepass_timer->done = rc == 0; }
-            ctx->pre_upload_err = rc;
-            ctx->prepass_stage.store(1, std::memory_order_release);
-            ctx->prepass_stage.store(2, std::memory_order_release);
-            return;
-        }
-        ctx->pre.before_disc_realloc = [ctx]() {  // the page-lock must go before the storage does
-            sqg_ctx::Pinned &pp = ctx->pre_pinned[0];
-            if (pp.p) { cudaSetDevice(ctx->device); cudaStreamSynchronize(ctx->stream3); cudaHostUnregister(const_cast<void *>(pp.p)); pp.p = nullptr; pp.bytes = 0; }
-        };
-        sqh::chimeric_prepass(ctx->chim_view, ctx->params.n_ref, ctx->params.read_len, ctx->pre, hook);
-        {   // its products go to HBM from here (DMA from the registered vectors), the caller's stream waits for ev_pre only
-            cudaError_t e = cudaSetDevice(ctx->device);
-            const size_t nD1 = ctx->pre.disc.size(), nG = ctx->pre.groups.size(), nP = ctx->pre.part_chr.size();
-            if (e == cudaSuccess) e = ctx->d_disc.ensure(nD1 ? nD1 : 1);
-            if (e == cudaSuccess) e = ctx->d_groups.ensure(nG ? nG : 1);
-            if (e == cudaSuccess) e = ctx->d_pchr.ensure(nP ? nP : 1);
-            if (e == cudaSuccess) e = ctx->d_ppos.ensure(nP ? nP : 1);
-            const void *src[4] = {ctx->pre.disc.data(), ctx->pre.groups.data(), ctx->pre.part_chr.data(), ctx->pre.part_pos.data()};
-            const size_t cap[4] = {ctx->pre.disc.capacity() * sizeof(DiscBlock), ctx->pre.groups.capacity() * sizeof(Group), ctx->pre.part_chr.capacity() * 4, ctx->pre.part_pos.capacity() * 4};
-            const size_t len[4] = {nD1 * sizeof(DiscBlock), nG * sizeof(Group), nP * 4, nP * 4};
-            void *dst[4] = {ctx->d_disc.p, ctx->d_groups.p, ctx->d_pchr.p, ctx->d_ppos.p};
-            for (int k = 0; k < 4 && e == cudaSuccess; k++) {
-                sqg_ctx::Pinned &pp = ctx->pre_pinned[k];
-                if (k == 0 && cap[k] >= (1u << 16) && (pp.p != src[k] || pp.bytes != cap[k])) {  // the big one; (re)register when the vector moved or grew
-                    if (pp.p) cudaHostUnregister(const_cast<void *>(pp.p));
-                    pp.p = nullptr; pp.bytes = 0;
-                    if (cudaHostRegister(const_cast<void *>(src[k]), cap[k], cudaHostRegisterDefault) == cudaSuccess) { pp.p = src[k]; pp.bytes = cap[k]; }
-                    else cudaGetLastError();  // not fatal: the copy is staged instead
-                }
-                if (len[k]) e = cudaMemcpyAsync(dst[k], src[k], len[k], cudaMemcpyHostToDevice, ctx->stream3);
-            }
-            if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_pre, ctx->stream3);
-            ctx->pre_upload_err = (int)e;
-            ctx->pre_nD = (int32_t)nD1 - 1; ctx->pre_nG = (int32_t)nG; ctx->pre_nP = (int32_t)nP;
-        }
-        ctx->prepass_stage.store(1, std::memory_order_release);  // finish_prepass() may go on
-        // then the chimeric arrays themselves (needed by the edge pass only): from this thread, so that the caller's thread
-        // goes straight on to the classification
         const sqg_chimeric &c = ctx->chim_view;
-        cudaError_t e = cudaSetDevice(ctx->device);
+        cudaError_t e = cudaEventRecord(ctx->prepass_timer->a, ctx->stream3);
 #define UPW(buf, src, cnt) do { if (e == cudaSuccess && (cnt)) e = cudaMemcpyAsync(ctx->buf.p, (src), (cnt) * sizeof(*(src)), cudaMemcpyHostToDevice, ctx->stream3); } while (0)
         UPW(dc_read_off, c.read_off, nr + 1); UPW(dc_n_first, c.n_first, nr);
         UPW(dc_first_total, c.first_total_len, nr); UPW(dc_second_total, c.second_total_len, nr);
+        UPW(dc_first_low, c.first_lowphred, nr); UPW(dc_second_low, c.second_lowphred, nr); UPW(dc_multi, c.multi_filter, nr);
         UPW(dc_ref_id, c.blk_ref_id, nb); UPW(dc0_ref_pos, c.blk_ref_pos, nb); UPW(dc0_read_pos, c.blk_read_pos, nb);
         UPW(dc0_match_ref, c.blk_match_ref, nb); UPW(dc0_match_read, c.blk_match_read, nb); UPW(dc_rev, c.blk_is_reverse, nb);
 #undef UPW
         if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_chim, ctx->stream3);
         ctx->chim_upload_err = (int)e;
-        ctx->prepass_stage.store(2, std::memory_order_release);
+        int rc = e == cudaSuccess ? device_prepass(ctx, nr) : (int)e;
+        if (rc == 0) rc = (int)cudaEventRecord(ctx->ev_pre, ctx->stream3);
+        if (rc == 0) { rc = (int)cudaEventRecord(ctx->prepass_timer->b, ctx->stream3); ctx->prepass_timer->done = rc == 0; }
+        ctx->pre_upload_err = rc;
     });
     ctx->have_chim = true; ctx->have_edge_table = false;
     return SQG_OK;
 }
 
-// join the host pre-pass and put its products (discordant blocks, groups, PartAlignPos) into HBM
+// join the pre-pass thread: the caller's stream waits for the pre-pass products (discordant blocks, groups, PartAlignPos)
 static int finish_prepass(sqg_ctx *ctx) {
-    // the products (the thread may still be uploading the chimeric arrays): a short spin, then sleep -- a busy-waiting thread per
-    // process is exactly what several processes on one host cannot afford
-    for (int spins = 0; ctx->prepass_stage.load(std::memory_order_acquire) < 1; spins++) {
-        if (spins < 2000) std::this_thread::yield(); else std::this_thread::sleep_for(std::chrono::microseconds(20));
-    }
+    ctx->prepass_worker.wait();
     if (ctx->prepass_uploaded) return SQG_OK;
     if (ctx->pre_upload_err) { ctx->err = std::string("upload of the pre-pass products: ") + cudaGetErrorString((cudaError_t)ctx->pre_upload_err); return SQG_ECUDA; }
     CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_pre, 0));
@@ -1847,7 +1743,7 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
             CK(cudaStreamSynchronize(ctx->stream));
             g_lo = 0;
             while (g_lo < nG) {
-                const Group &gg = ctx->pre.groups[g_lo];
+                const Group &gg = ctx->h_groups[g_lo];
                 if (rp[0] < 0 || gg.chr < rp[0] || (gg.chr == rp[0] && gg.right < rp[1])) g_lo++; else break;
             }
         }
@@ -2160,7 +2056,6 @@ extern "C" int sqg_keep_records(sqg_ctx *ctx, int64_t lo, int64_t hi) {
     if (ends[1] < ends[0] || (int64_t)ends[1] > ctx->batch.n_blk) FAIL(SQG_EINVAL, "sqg_keep_records: blk_off of the batch is not monotone");
     const int64_t nr = hi - lo, b0 = ends[0], nb = (int64_t)ends[1] - b0;
     DBuf<uint8_t> tmp;  // a range that overlaps its destination goes through here
-    struct Release { DBuf<uint8_t> &t; ~Release() { t.release(); } } release_tmp{tmp};
     CK(tmp.ensure((size_t)std::max<int64_t>(4 * (nr + 1), 4 * nb)));
     cudaError_t e = cudaSuccess;
     auto move = [&](void *arr, size_t elem, int64_t first, int64_t count) {
@@ -2179,10 +2074,9 @@ extern "C" int sqg_keep_records(sqg_ctx *ctx, int64_t lo, int64_t hi) {
     CK(cudaMemcpyAsync(tmp.p, ctx->o_blk_off.p + lo, (size_t)(nr + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
     LAUNCH(k_keep_offsets, blocks_for(nr + 1), kThreads, ctx->o_blk_off.p, (const uint32_t *)tmp.p, nr + 1, (uint32_t)b0);
     CK(cudaStreamSynchronize(st));
-    DevBatch &b = ctx->batch;
-    b.n_rec = nr; b.n_blk = nb;
-    ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->classify_prelaunched = false;
-    ctx->first_record_index += lo; ctx->batch_restricted = true;
+    ctx->batch.n_rec = nr; ctx->batch.n_blk = nb;
+    reset_batch_state(ctx, true, ctx->first_record_index + lo, ctx->wire_loaded);
+    ctx->batch_restricted = true; ctx->classify_prelaunched = false;  // (a classification launched on the whole batch does not apply)
     return SQG_OK;
 }
 
@@ -2822,14 +2716,8 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
     for (auto *b : {&ctx->o_ref_id, &ctx->o_pos, &ctx->o_mate_ref_id, &ctx->o_mate_pos, &ctx->o_end_pos, &ctx->o_blk_ref_pos, &ctx->o_blk_match_ref}) CK(b->grow(1, 0, st));
     for (auto *b : {&ctx->o_flag, &ctx->o_total_len, &ctx->o_lowphred_run, &ctx->o_blk_read_pos, &ctx->o_blk_match_read}) CK(b->grow(1, 0, st));
     CK(ctx->o_mapq.grow(1, 0, st)); CK(ctx->o_aux.grow(1, 0, st));
-    DevBatch &b = ctx->batch;
-    b.n_rec = R; b.n_blk = (int64_t)B;
-    b.ref_id = ctx->o_ref_id.p; b.pos = ctx->o_pos.p; b.mate_ref_id = ctx->o_mate_ref_id.p; b.mate_pos = ctx->o_mate_pos.p; b.end_pos = ctx->o_end_pos.p;
-    b.flag = ctx->o_flag.p; b.total_len = ctx->o_total_len.p; b.lowphred_run = ctx->o_lowphred_run.p; b.mapq = ctx->o_mapq.p; b.aux = ctx->o_aux.p;
-    b.blk_off = ctx->o_blk_off.p; b.blk_ref_pos = ctx->o_blk_ref_pos.p; b.blk_match_ref = ctx->o_blk_match_ref.p;
-    b.blk_read_pos = ctx->o_blk_read_pos.p; b.blk_match_read = ctx->o_blk_match_read.p;
-    ctx->have_batch = true; ctx->batch_restricted = false; ctx->batch_owned = true; ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->first_record_index = first_record_index;
-    ctx->wire_loaded = false; ctx->classify_prelaunched = false;
+    point_batch_at_own_arrays(ctx, R, (int64_t)B);
+    reset_batch_state(ctx, true, first_record_index, false);
     return SQG_OK;
 }
 

@@ -12,7 +12,6 @@
 #include <string>
 #include <vector>
 
-#include "host/prepass.h"
 #include "sq_bam.cuh"
 #include "sq_common.cuh"
 #include "sq_seed.cuh"
@@ -24,9 +23,16 @@
 
 namespace sq {
 
+// Device / pinned host buffers own their storage: freed by the destructor, or earlier by release().  Moves hand it over.
 template <class T> struct DBuf {
     T *p = nullptr;
     size_t cap = 0;
+    DBuf() = default;
+    DBuf(const DBuf &) = delete;
+    DBuf &operator=(const DBuf &) = delete;
+    DBuf(DBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DBuf &operator=(DBuf &&o) noexcept { if (this != &o) { release(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; } return *this; }
+    ~DBuf() { release(); }
     cudaError_t ensure(size_t n) {
         if (n <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -54,6 +60,12 @@ template <class T> struct DBuf {
 template <class T> struct HBuf {  // pinned host
     T *p = nullptr;
     size_t cap = 0;
+    HBuf() = default;
+    HBuf(const HBuf &) = delete;
+    HBuf &operator=(const HBuf &) = delete;
+    HBuf(HBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    HBuf &operator=(HBuf &&o) noexcept { if (this != &o) { release(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; } return *this; }
+    ~HBuf() { release(); }
     cudaError_t ensure(size_t n) {
         if (n <= cap) return cudaSuccess;
         if (p) cudaFreeHost(p);
@@ -185,7 +197,7 @@ struct sqg_ctx {
 
     // chimeric side
     bool have_chim = false, prepass_uploaded = false;
-    sqh::ChimPrepass pre;
+    std::vector<sq::Group> h_groups;  // the pre-pass's groups on the host, for a range shard only (seed_stage looks up g_lo)
     sqg_chimeric chim_view{};
     sq::Worker prepass_worker;  // persistent host thread of the chimeric pre-pass (keeps its OpenMP team alive between runs)
     int64_t c_n_reads = 0, c_n_blk = 0;
@@ -202,19 +214,14 @@ struct sqg_ctx {
 
     // std::sort's permutation of the discordant blocks on the device (sq_gpusort.cuh), driven by the pre-pass thread
     cudaStream_t stream3 = nullptr;
-    cudaEvent_t ev_chim = nullptr;       // the chimeric arrays are in HBM (uploaded by the pre-pass thread behind its own work)
+    cudaEvent_t ev_chim = nullptr;       // the chimeric arrays are in HBM (uploaded by the pre-pass thread before its own work)
     bool chim_upload_pending = false;
     int chim_upload_err = 0;
     cudaEvent_t ev_pre = nullptr;        // the pre-pass products (discordant blocks, groups, PartAlignPos) are in HBM
     int pre_upload_err = 0;
-    struct Pinned { const void *p = nullptr; size_t bytes = 0; };
-    Pinned pre_pinned[4];                // host vectors of `pre` registered for DMA (they keep their storage from step to step)
-    std::atomic<int> prepass_stage{2};   // 0: pre-pass running, 1: its products are ready (uploads still going), 2: thread idle
     sq::DBuf<uint64_t> d_gs_keys;
     sq::DBuf<uint32_t> d_gs_idx;
     sq::DBuf<unsigned char> d_gs_scratch;
-    sq::HBuf<uint64_t> h_gs_keys;
-    sq::HBuf<uint32_t> h_gs_idx;
     int64_t gs_launches = 0;
     int gs_last_status = -100;   // status of the most recent device sort (-100: not run)
 
@@ -233,7 +240,7 @@ struct sqg_ctx {
     sq::DBuf<int32_t> d_pre_ndis, d_pre_pusher, d_pre_lastk, d_pre_open; sq::DBuf<int64_t> d_pre_off; sq::DBuf<uint64_t> d_pre_part, d_pre_part2, d_pre_endkey, d_pre_excl, d_pre_incl;
     sq::DBuf<uint8_t> d_pre_opens, dc_first_low, dc_second_low, dc_multi, d_temp3; sq::DBuf<int64_t> d_pre_cnt; sq::HBuf<int64_t> h_pre_cnt;
     sq::PhaseTimer *prepass_timer = nullptr;
-    int32_t pre_nD = 0, pre_nG = 0, pre_nP = 0;   // sizes of the pre-pass products (either path)
+    int32_t pre_nD = 0, pre_nG = 0, pre_nP = 0;   // sizes of the pre-pass products
     sq::DBuf<sq::SeedOp> d_ops;
     sq::DBuf<sq::SeedOp> d_ops_dense;  // the islands' op lists without their unused capacity, island order
     sq::HBuf<sq::SeedOp> h_ops;

@@ -23,11 +23,9 @@ CASES = [
 
 
 @pytest.mark.parametrize("n_pairs,seed,disc,ref_len,kw", CASES)
-def test_hot_path_matches_reference(tmp_path, built_lib, ref_oracle, monkeypatch, n_pairs, seed, disc, ref_len, kw):
+def test_hot_path_matches_reference(tmp_path, built_lib, ref_oracle, n_pairs, seed, disc, ref_len, kw):
     from oracle import pyref
     from squid_b200 import synth
-    if seed in (17, 1003):  # force the chunked (multi-threaded) read loop of the chimeric pre-pass on a small input
-        monkeypatch.setenv("SQH_PREPASS_CHUNKS", "13")
     rl = synth.GRCH38_LEN if ref_len == "grch38" else ref_len
     cp, hp, conc, chim, info = common.write_case(str(tmp_path), n_pairs, seed, disc, rl, **kw)
     ref = ref_oracle.run(cp, hp, str(tmp_path / "ref"))

@@ -31,13 +31,11 @@ def test_structured_inputs(built_lib, pattern):
         assert v == 1 or (pattern == 3 and v == 2), "pattern %d n=%d: verdict %d" % (pattern, n, v)
 
 
-def test_prepass_uses_the_device_sort(tmp_path, built_lib, ref_oracle, monkeypatch):
-    """End to end with the device sort forced on a small input: same segments / edges as the reference build."""
+def test_prepass_uses_the_device_sort(tmp_path, built_lib, ref_oracle):
+    """End to end on a small input: the pre-pass sort runs on the device, same segments / edges as the reference build."""
     from tests import common
-    monkeypatch.setenv("SQG_GPU_SORT_MIN", "64")
     cp, hp, *_ = common.write_case(str(tmp_path), 60000, 1031, 0.05, fusion_support=10)
     ref = ref_oracle.run(cp, hp, str(tmp_path / "ref"))
     got = common.run_cuda(cp, hp)
     assert got["graph"].stat("device_sort_status") == 0
     common.assert_same(ref, got)
-    monkeypatch.setenv("SQG_GPU_SORT", "0")  # read once per process: may already be latched; the CPU twin is covered elsewhere

@@ -20,7 +20,7 @@ ref = rnd.choice([synth.CHR17_LEN, [30000000, 20000000, 5000000, 16569], synth.G
 kw = {"n_genes": rnd.choice([None, 30, 300, 2000]), "fusion_support": rnd.choice([5, 10, 20, 100])}
 if rnd.random() < 0.25:
     kw.update(exon_len=(20, 170), intron_len=(60, 400))
-print("case", n, d, ref, kw, "GPU_SORT", os.environ.get("SQG_GPU_SORT"), "MIN", os.environ.get("SQG_GPU_SORT_MIN"))
+print("case", n, d, ref, kw)
 with tempfile.TemporaryDirectory() as td:
     cp, hp, *_ = common.write_case(td, n, seed, d, ref, **kw)
     refd = pyref.run(cp, hp, os.path.join(td, "ref"))
