@@ -66,17 +66,37 @@ struct Params {
     int32_t min_mapq, max_lowphred_len, concord_dist_pos, concord_dist_idx, read_len, n_ref;
 };
 
-// Segment table: segments tile every chromosome; chr_first[c]..chr_first[c+1] are the segments of c.
-// bin_seg is a coarse position index over the tiling: for chromosome c, bin k (positions [k<<bin_shift, (k+1)<<bin_shift))
-// starts inside segment bin_seg[bin_off[c] + k].  Every "which segment holds position x" question of the path (LocateRead's
-// scans, the depth cursor, the spanning-block fallback) is then one table read plus a step or two along the tiling instead
-// of a binary search over the whole table.  With bin_seg == nullptr the lookups fall back to binary searches.
+// Segment table: segments tile every chromosome; chr_head(nt, c).c0..c1 are the segments of c.
+// The position index answers "which segment holds position x" (LocateRead's scans, the depth cursor, the spanning-block
+// fallback) in two dependent loads: the chromosome's 16-byte header, then the 16-byte entry of the bin that holds x
+// (positions [k<<bin_shift, (k+1)<<bin_shift) of chromosome c are entry head[c].bin0 + k), which names the segment holding
+// the bin's start together with its Position and End.  Only a position past that segment walks on, bounded by the segment
+// that holds the next bin's start.  Without bins the lookups fall back to binary searches.
+// The index comes in two forms with the same content: packed (head, bins: what the device reads, built by install_nodes) and
+// plain (chr_first, bin_off, bin_seg: what a host-side caller such as the CPU stepping harness builds).  chr_head / bin_ent
+// read either; every lookup above them is written once.
+struct alignas(16) ChrHead {
+    int32_t c0, c1;  // segments of the chromosome: [c0, c1), c1 == c0 when it has none
+    int32_t bin0;    // its first bin entry
+    int32_t end1;    // End of its last segment
+};
+struct alignas(16) BinEnt {
+    int32_t j;         // segment holding the bin's start (the last segment of the chromosome when that is its end)
+    int32_t pos, end;  // Position and End of segment j
+    int32_t hi;        // segment holding the next bin's start (the last segment of the chromosome for its last bin)
+};
 struct NodeTable {
     int32_t n = 0, n_ref = 0;
     const int32_t *chr = nullptr, *pos = nullptr, *end = nullptr;  // end = Position + Length
-    const int32_t *chr_first = nullptr;                            // n_ref + 1
-    const int32_t *bin_seg = nullptr, *bin_off = nullptr;          // bin_off: n_ref + 1
+    const ChrHead *head = nullptr;                                 // packed: n_ref headers
+    const BinEnt *bins = nullptr;                                  //         and the bin entries
+    const int32_t *chr_first = nullptr;                            // plain:  n_ref + 1
+    const int32_t *bin_seg = nullptr, *bin_off = nullptr;          //         bin_seg[bin_off[c] + k] = BinEnt::j; bin_off: n_ref + 1
     int32_t bin_shift = 12;
+};
+// A segment with its Position and End, as a lookup returns it.
+struct SegHit {
+    int32_t s, pos, end;
 };
 
 // An aligned block in registers/local memory (SingleBamRec_t).
@@ -118,42 +138,83 @@ SQ_HD int32_t upper_bound_i32(const int32_t *a, int32_t lo, int32_t hi, int32_t 
     return lo;
 }
 
-// Segment of chromosome c (c0 = chr_first[c] <= result < c1 = chr_first[c+1], c1 > c0) that holds position x,
-// clamped to the first / last segment of the chromosome when x lies outside [0, chromosome length).
-SQ_HD int32_t seg_at(const NodeTable &nt, int32_t c, int32_t c0, int32_t c1, int32_t x) {
-    if (x < nt.pos[c0]) return c0;
-    if (x >= nt.end[c1 - 1]) return c1 - 1;
-    if (nt.bin_seg) {
-        const int32_t bo = nt.bin_off[c] + (x >> nt.bin_shift);
-        int32_t j = nt.bin_seg[bo];
-        if (nt.end[j] > x) return j;
-        int32_t hi = bo + 1 < nt.bin_off[c + 1] ? nt.bin_seg[bo + 1] : c1 - 1;  // segment holding the start of the next bin
-        if (hi - j <= 4) { do { j++; } while (nt.end[j] <= x); return j; }
-        return upper_bound_i32(nt.end, j + 1, hi + 1, x);
-    }
-    return upper_bound_i32(nt.end, c0, c1, x);
+// Header of chromosome c over a table whose chromosomes start at chr_first[c] (n_ref + 1 entries), with its bins starting at
+// bin_off[c].
+SQ_HD ChrHead chr_head_value(const int32_t *chr_first, const int32_t *end, const int32_t *bin_off, int32_t c) {
+    const int32_t c0 = chr_first[c], c1 = chr_first[c + 1];
+    return ChrHead{c0, c1, bin_off ? bin_off[c] : 0, c1 > c0 ? end[c1 - 1] : 0};
 }
+SQ_HD bool has_bins(const NodeTable &nt) { return nt.bins || nt.bin_seg; }
+#if defined(__CUDA_ARCH__)
+SQ_HD ChrHead chr_head(const NodeTable &nt, int32_t c) {
+    const int4 v = __ldg(reinterpret_cast<const int4 *>(nt.head) + c);
+    return ChrHead{v.x, v.y, v.z, v.w};
+}
+SQ_HD BinEnt bin_ent(const NodeTable &nt, const ChrHead &, int32_t k) {
+    const int4 v = __ldg(reinterpret_cast<const int4 *>(nt.bins) + k);
+    return BinEnt{v.x, v.y, v.z, v.w};
+}
+#else
+SQ_HD ChrHead chr_head(const NodeTable &nt, int32_t c) { return nt.head ? nt.head[c] : chr_head_value(nt.chr_first, nt.end, nt.bin_off, c); }
+// (the plain form names no next-bin segment: the chromosome's last segment bounds the walk instead, which changes how the
+// lookup steps, never what it returns)
+SQ_HD BinEnt bin_ent(const NodeTable &nt, const ChrHead &h, int32_t k) {
+    if (nt.bins) return nt.bins[k];
+    const int32_t j = nt.bin_seg[k];
+    return BinEnt{j, nt.pos[j], nt.end[j], h.c1 - 1};
+}
+#endif
+
 // value of bin k of chromosome c: the segment holding position k << bin_shift (the last segment of c at the chromosome end)
 SQ_HD int32_t bin_seg_value(const NodeTable &nt, int32_t c, int32_t k) {
-    const int32_t c0 = nt.chr_first[c], c1 = nt.chr_first[c + 1];
-    if (c1 <= c0) return c0;
-    const int32_t j = upper_bound_i32(nt.end, c0, c1, k << nt.bin_shift);
-    return j < c1 ? j : c1 - 1;
+    const ChrHead h = chr_head(nt, c);
+    if (h.c1 <= h.c0) return h.c0;
+    const int32_t j = upper_bound_i32(nt.end, h.c0, h.c1, k << nt.bin_shift);
+    return j < h.c1 ? j : h.c1 - 1;
 }
-// first segment of c with End > v   (== upper_bound_i32(nt.end, c0, c1, v))
-SQ_HD int32_t seg_first_end_gt(const NodeTable &nt, int32_t c, int32_t c0, int32_t c1, int32_t v) {
-    if (c1 <= c0) return c0;
-    if (v >= nt.end[c1 - 1]) return c1;
-    return seg_at(nt, c, c0, c1, v);
+// packed entry of bin k of chromosome c (nb bins); the headers must be in place
+SQ_HD BinEnt bin_ent_value(const NodeTable &nt, int32_t c, int32_t k, int32_t nb) {
+    const ChrHead h = chr_head(nt, c);
+    if (h.c1 <= h.c0) return BinEnt{h.c0, 0, 0, h.c0};
+    const int32_t j = bin_seg_value(nt, c, k);
+    return BinEnt{j, nt.pos[j], nt.end[j], k + 1 < nb ? bin_seg_value(nt, c, k + 1) : h.c1 - 1};
 }
-// first segment of c with End >= v  (== lower_bound_i32(nt.end, c0, c1, v))
-SQ_HD int32_t seg_first_end_ge(const NodeTable &nt, int32_t c, int32_t c0, int32_t c1, int32_t v) {
-    return seg_first_end_gt(nt, c, c0, c1, v - 1);
+
+// Segment of the chromosome of header h (h.c1 > h.c0) that holds position x, clamped to its first / last segment when x lies
+// outside [Position of the first, End of the last); == upper_bound_i32(nt.end, h.c0, h.c1, x), clamped to h.c1 - 1.
+SQ_HD SegHit seg_at(const NodeTable &nt, const ChrHead &h, int32_t x) {
+    int32_t j;
+    if (x >= h.end1) j = h.c1 - 1;
+    else if (has_bins(nt)) {
+        const BinEnt e = bin_ent(nt, h, h.bin0 + (x < 0 ? 0 : x >> nt.bin_shift));
+        if (e.end > x) return SegHit{e.j, e.pos, e.end};
+        if (e.hi - e.j <= 4) {  // the tiling: each step's Position is the End before it
+            int32_t q = e.end;
+            j = e.j;
+            for (;;) { j++; const int32_t t = nt.end[j]; if (t > x) return SegHit{j, q, t}; q = t; }
+        }
+        j = upper_bound_i32(nt.end, e.j + 1, e.hi + 1, x);
+    } else j = upper_bound_i32(nt.end, h.c0, h.c1, x);
+    return SegHit{j, nt.pos[j], nt.end[j]};
 }
-// last segment of c with Position <= v, c0-1 if none  (== upper_bound_i32(nt.pos, c0, c1, v) - 1)
+// first segment of the chromosome with End > v (== upper_bound_i32(nt.end, c0, c1, v)); s == c1 (Position, End unset) if none
+SQ_HD SegHit seg_first_end_gt(const NodeTable &nt, const ChrHead &h, int32_t v) {
+    if (h.c1 <= h.c0 || v >= h.end1) return SegHit{h.c1, 0, 0};
+    return seg_at(nt, h, v);
+}
+// first segment of the chromosome with End >= v  (== lower_bound_i32(nt.end, c0, c1, v))
+SQ_HD int32_t seg_first_end_ge(const NodeTable &nt, const ChrHead &h, int32_t v) {
+    return seg_first_end_gt(nt, h, v - 1).s;
+}
+// last segment of the chromosome with Position <= v, c0 - 1 if none  (== upper_bound_i32(nt.pos, c0, c1, v) - 1)
+SQ_HD int32_t seg_last_pos_le(const NodeTable &nt, const ChrHead &h, int32_t v) {
+    if (h.c1 <= h.c0) return h.c0 - 1;
+    const SegHit x = seg_at(nt, h, v);
+    return x.pos <= v ? x.s : x.s - 1;  // (Position > v only for the first segment: v lies left of the chromosome's table)
+}
+// the same with the chromosome's segments [c0, c1) at hand
 SQ_HD int32_t seg_last_pos_le(const NodeTable &nt, int32_t c, int32_t c0, int32_t c1, int32_t v) {
-    if (c1 <= c0 || v < nt.pos[c0]) return c0 - 1;
-    return seg_at(nt, c, c0, c1, v);
+    return c1 <= c0 ? c0 - 1 : seg_last_pos_le(nt, chr_head(nt, c), v);
 }
 
 // Own blocks of record r sorted by read position (SortbyReadPos: std::sort on <=16 elements is an

@@ -17,16 +17,23 @@ SQ_HD bool depth_contained(const NodeTable &nt, int32_t j, int32_t chr, int32_t 
 // segment max(cursor, n(start)) where n(start) is the first segment of its chromosome that ends
 // right of `start`; blocks of <= 3 bp can already be "contained" (+-3) in one of the <= 3
 // segments just left of n(start), which then is where the cursor stops.  This returns that
-// per-read target m; the cursor is the running maximum of m over the stream.
-SQ_HD int32_t depth_target(const NodeTable &nt, int32_t chr, int32_t start, int32_t len) {
-    if (chr < 0 || chr >= nt.n_ref) return kNoNode;
-    const int32_t c0 = nt.chr_first[chr], c1 = nt.chr_first[chr + 1];
-    const int32_t n = seg_first_end_gt(nt, chr, c0, c1, start);  // first segment with End > start
+// per-read target m; the cursor is the running maximum of m over the stream.  depth_target_hit gives the target with its
+// Position and End (s == kNoNode: none).
+SQ_HD SegHit depth_target_hit(const NodeTable &nt, int32_t chr, int32_t start, int32_t len) {
+    const SegHit none{kNoNode, 0, 0};
+    if (chr < 0 || chr >= nt.n_ref) return none;
+    const ChrHead h = chr_head(nt, chr);
+    const SegHit n = seg_first_end_gt(nt, h, start);  // first segment with End > start
     if (len <= kSeedThresh) {
-        for (int32_t j = (n - 3 > c0 ? n - 3 : c0); j < n; j++)
-            if (depth_contained(nt, j, chr, start, len)) return j;
+        for (int32_t j = (n.s - 3 > h.c0 ? n.s - 3 : h.c0); j < n.s; j++)
+            if (depth_contained(nt, j, chr, start, len)) return SegHit{j, nt.pos[j], nt.end[j]};
     }
-    return n < c1 ? n : kNoNode;  // a start at/after the chromosome end walks the cursor off the table
+    return n.s < h.c1 ? n : none;  // a start at/after the chromosome end walks the cursor off the table
+}
+SQ_HD int32_t depth_target(const NodeTable &nt, int32_t chr, int32_t start, int32_t len) { return depth_target_hit(nt, chr, start, len).s; }
+// depth_contained for a segment on chromosome chr, with its Position and End at hand
+SQ_HD bool depth_contained(const SegHit &j, int32_t start, int32_t len) {
+    return start >= j.pos - kSeedThresh && start + len <= j.end + kSeedThresh;
 }
 
 // ---- ReadsOther (:781, :806-825): blocks of <= 3 bp ----------------------------------------------------------------
@@ -50,10 +57,11 @@ SQ_HD int32_t depth_short_own(const NodeTable &nt, int32_t chr, int32_t c0, int3
 SQ_HD int32_t depth_other_mark(const NodeTable &nt, int32_t chr, int32_t start, int32_t len, uint32_t *bit) {
     *bit = 0;
     if (chr < 0 || chr >= nt.n_ref) return -1;
-    const int32_t c0 = nt.chr_first[chr], c1 = nt.chr_first[chr + 1];
-    const int32_t n = seg_first_end_gt(nt, chr, c0, c1, start);
-    if (n >= c1) return -1;
-    const int32_t d = start - nt.pos[n];
+    const ChrHead h = chr_head(nt, chr);
+    const SegHit x = seg_first_end_gt(nt, h, start);
+    const int32_t n = x.s;
+    if (n >= h.c1) return -1;
+    const int32_t d = start - x.pos;
     if (d < 0 || d > 2) return -1;
     if (len > kSeedThresh) *bit = 1u << d;
     else { const int32_t l = len < 1 ? 1 : len; *bit = 1u << (3 + 3 * d + (l - 1)); }
@@ -62,8 +70,9 @@ SQ_HD int32_t depth_other_mark(const NodeTable &nt, int32_t chr, int32_t start, 
 // segment in which the short entry (chr, start, len <= 3) of ReadsOther is counted, or kNoNode
 SQ_HD int32_t depth_short_node(const NodeTable &nt, const uint32_t *mask, int32_t chr, int32_t start, int32_t len, bool *unstable) {
     if (chr < 0 || chr >= nt.n_ref) return kNoNode;
-    const int32_t c0 = nt.chr_first[chr], c1 = nt.chr_first[chr + 1];
-    const int32_t n = seg_first_end_gt(nt, chr, c0, c1, start);
+    const ChrHead h = chr_head(nt, chr);
+    const int32_t c0 = h.c0, c1 = h.c1;
+    const int32_t n = seg_first_end_gt(nt, h, start).s;
     const int32_t i = depth_short_own(nt, chr, c0, n, start, len);
     if (i == n) return (n < c1 && depth_contained(nt, n, chr, start, len)) ? n : kNoNode;  // as a long entry: tested at n only
     int32_t at = i;

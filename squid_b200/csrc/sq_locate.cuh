@@ -42,63 +42,66 @@ struct Cursor {
     bool known;
 };
 
-// One iteration of LocateRead's per-block body.  Returns the segment (or -1); updates `cur`.
+// The segment j with its Position and End, read from the table.
+SQ_HD SegHit seg_hit(const NodeTable &nt, int32_t j) { return SegHit{j, nt.pos[j], nt.end[j]}; }
+
+// One iteration of LocateRead's per-block body.  Returns the segment with its Position and End (s == -1: none); updates `cur`.
 // Sets *sensitive when the outcome cannot be decided without the concrete hint.
-SQ_HD int32_t locate_block(const NodeTable &nt, const Blk &b, Cursor &cur, bool hint_known, int32_t hint, bool *sensitive) {
+SQ_HD SegHit locate_block(const NodeTable &nt, const Blk &b, Cursor &cur, bool hint_known, int32_t hint, bool *sensitive) {
+    const SegHit none{-1, 0, 0};
     // `if(i<0 || i>=vNodes.size()) i=initialguess;`
     if (cur.known && (cur.idx < 0 || cur.idx >= nt.n)) { cur.known = hint_known; cur.idx = hint; }
-    if (cur.known && block_fits(nt, cur.idx, b)) return cur.idx;
+    if (cur.known && block_fits(nt, cur.idx, b)) return seg_hit(nt, cur.idx);
     const int32_t c = b.ref_id;
     if (c < 0 || c >= nt.n_ref) {  // no segment can fit; the scan direction still moves the cursor
-        if (!cur.known) { return -1; }
+        if (!cur.known) { return none; }
         cur.idx = (nt.chr[cur.idx] < c) ? nt.n : -1;
-        return -1;
+        return none;
     }
-    const int32_t c0 = nt.chr_first[c], c1 = nt.chr_first[c + 1];
-    if (!cur.known && c1 > c0 && b.match_ref > kLocateTol) {
+    const ChrHead h = chr_head(nt, c);
+    if (!cur.known && h.c1 > h.c0 && b.match_ref > kLocateTol) {
         // the common case in closed form: the block lies inside the segment s that holds its start, clear of both ends
         // by more than the tolerance.  Then s is the only segment it fits (lo == hi == s below) and no scan can miss it.
-        const int32_t s = seg_at(nt, c, c0, c1, b.ref_pos);
-        const int32_t q = nt.pos[s], e = nt.end[s];
-        if (q <= b.ref_pos && b.ref_pos + kLocateTol < e && b.ref_pos + b.match_ref - kLocateTol <= e) { cur.known = true; cur.idx = s; return s; }
+        const SegHit s = seg_at(nt, h, b.ref_pos);
+        if (s.pos <= b.ref_pos && b.ref_pos + kLocateTol < s.end && b.ref_pos + b.match_ref - kLocateTol <= s.end) { cur.known = true; cur.idx = s.s; return s; }
     }
     // segments that fit: lo = first with End >= p+m-5, hi = last with Position <= p+5
-    const int32_t lo = seg_first_end_ge(nt, c, c0, c1, b.ref_pos + b.match_ref - kLocateTol);
-    const int32_t hi = seg_last_pos_le(nt, c, c0, c1, b.ref_pos + kLocateTol);
+    const int32_t lo = seg_first_end_ge(nt, h, b.ref_pos + b.match_ref - kLocateTol);
+    const int32_t hi = seg_last_pos_le(nt, h, b.ref_pos + kLocateTol);
     if (cur.known) {
         const int32_t i = cur.idx;
         const bool forward = nt.chr[i] < c || (nt.chr[i] == c && nt.pos[i] <= b.ref_pos);  // :1214
         if (forward) {
             const int32_t j = i > lo ? i : lo;
-            if (lo <= hi && j <= hi) { cur.idx = j; return j; }
-            cur.idx = c1;  // ran off the chromosome to the right
-            return -1;
+            if (lo <= hi && j <= hi) { cur.idx = j; return seg_hit(nt, j); }
+            cur.idx = h.c1;  // ran off the chromosome to the right
+            return none;
         }
         const int32_t j = i < hi ? i : hi;
-        if (lo <= hi && j >= lo) { cur.idx = j; return j; }
-        cur.idx = c0 - 1;
-        return -1;
+        if (lo <= hi && j >= lo) { cur.idx = j; return seg_hit(nt, j); }
+        cur.idx = h.c0 - 1;
+        return none;
     }
     // unknown start index (it equals the hint): decidable only if every possible start agrees
-    if (lo > hi) { cur.known = false; return -1; }  // nothing fits; cursor ends off-chromosome on a side we do not know
+    if (lo > hi) { cur.known = false; return none; }  // nothing fits; cursor ends off-chromosome on a side we do not know
     if (lo == hi) {
         // a start left of lo on the same chromosome whose Position is already > p scans backwards and misses
-        const bool trap = lo - 1 >= c0 && nt.pos[lo - 1] > b.ref_pos;
-        if (!trap) { cur.known = true; cur.idx = lo; return lo; }
+        const bool trap = lo - 1 >= h.c0 && nt.pos[lo - 1] > b.ref_pos;
+        if (!trap) { cur.known = true; cur.idx = lo; return seg_hit(nt, lo); }
     }
     *sensitive = true;
-    return -1;
+    return none;
 }
 
-// Clip a located block to its segment, strand-aware (:1229-1248).
-SQ_HD void trim_block(const NodeTable &nt, int32_t j, Blk &b) {
-    if (b.ref_pos < nt.pos[j]) {
-        const int32_t d = nt.pos[j] - b.ref_pos;
+// Clip a block located in segment j (Position, End as the lookup returned them) to it, strand-aware (:1229-1248).
+SQ_HD void trim_block(const SegHit &j, Blk &b) {
+    if (b.ref_pos < j.pos) {
+        const int32_t d = j.pos - b.ref_pos;
         if (!b.rev) b.read_pos += d;
-        b.match_ref -= d; b.match_read -= d; b.ref_pos = nt.pos[j];
+        b.match_ref -= d; b.match_read -= d; b.ref_pos = j.pos;
     }
-    if (b.ref_pos + b.match_ref > nt.end[j]) {
-        const int32_t d = b.ref_pos + b.match_ref - nt.end[j];
+    if (b.ref_pos + b.match_ref > j.end) {
+        const int32_t d = b.ref_pos + b.match_ref - j.end;
         if (b.rev) b.read_pos += d;
         b.match_ref -= d; b.match_read -= d;
     }
@@ -133,11 +136,10 @@ SQ_HD bool read_pair_discordant_nocheck(const ReadView &rv) {  // IsPairDiscorda
 // n0 = segment containing p.  The forward scan stops one segment early when p sits exactly on a
 // boundary and the scan started at or left of that segment.
 SQ_HD int32_t spanning_node(const NodeTable &nt, const Blk &b, bool ffi_known, int32_t ffi, bool *sensitive) {
-    const int32_t c = b.ref_id;
-    const int32_t c0 = nt.chr_first[c], c1 = nt.chr_first[c + 1];
-    int32_t n0 = seg_last_pos_le(nt, c, c0, c1, b.ref_pos);  // last segment with Position <= p
-    if (n0 < c0) n0 = c0;
-    if (nt.pos[n0] == b.ref_pos && n0 - 1 >= c0) {
+    const ChrHead h = chr_head(nt, b.ref_id);
+    const SegHit x = seg_at(nt, h, b.ref_pos);  // n0 = last segment with Position <= p, clamped to the first
+    const int32_t n0 = x.s;
+    if (x.pos == b.ref_pos && n0 - 1 >= h.c0) {
         if (!ffi_known) { *sensitive = true; return n0; }
         if (ffi <= n0 - 1) return n0 - 1;
     }
@@ -156,10 +158,10 @@ SQ_HD bool read_edges(const NodeTable &nt, const Params &p, ReadView &rv, int mo
     cur.idx = hint; cur.known = hint_known;
     for (int k = 0; k < n; k++) {
         Blk &b = k < rv.nF ? rv.F[k] : rv.S[k - rv.nF];
-        const int32_t j = locate_block(nt, b, cur, hint_known, hint, &sensitive);
+        const SegHit j = locate_block(nt, b, cur, hint_known, hint, &sensitive);
         if (sensitive) return false;
-        node_out[k] = j;
-        if (j >= 0) trim_block(nt, j, b);
+        node_out[k] = j.s;
+        if (j.s >= 0) trim_block(j, b);
     }
     // firstfrontindex after this read (:1402-1403, :1608-1609)
     bool ffi_known = hint_known;
@@ -249,14 +251,16 @@ SQ_HD int32_t read_edges_single(const NodeTable &nt, const Params &p, bool has_o
     bool sensitive = false;
     Cursor cur;
     cur.idx = 0; cur.known = false;
-    const int32_t jA = locate_block(nt, A, cur, false, 0, &sensitive);
+    const SegHit hA = locate_block(nt, A, cur, false, 0, &sensitive);
     if (sensitive) return -3;
-    if (jA >= 0) trim_block(nt, jA, A);
+    const int32_t jA = hA.s;
+    if (jA >= 0) trim_block(hA, A);
     int32_t jB = -1;
     if (two) {
-        jB = locate_block(nt, Bk, cur, false, 0, &sensitive);
+        const SegHit hB = locate_block(nt, Bk, cur, false, 0, &sensitive);
         if (sensitive) return -3;
-        if (jB >= 0) trim_block(nt, jB, Bk);
+        jB = hB.s;
+        if (jB >= 0) trim_block(hB, Bk);
     }
     const bool ffi_known = jA != -1;  // firstfrontindex after this read (:1608-1609); the incoming one is not known
     const int32_t ffi = jA;

@@ -1,7 +1,7 @@
 // Phase 2 of the path in ONE pass over the record batch, once the segment table exists: per-segment depth of the
 // concordant stream (BuildNode_STAR part D, SegmentGraph.cpp:784-825) and read-to-segment assignment + raw edges of the
 // stream (RawEdgesOther, :1557-1696).  Tiles are staged with TMA bulk copies (sq_stream.cuh) and are independent.
-//   * Segment lookups go through the position index of the segment table (seg_at): one table read and a step or two.
+//   * Segment lookups go through the position index of the segment table (seg_at): a chromosome header and a bin entry.
 //   * Records with at most one aligned block (nine in ten) take a register-only path (read_edges_single); the others
 //     are collected per tile and run the generic read_edges densely packed, so a warp never drags 31 idle lanes through it.
 //   * Edges are not written one by one: every tile counts them in a small shared-memory hash table (keys repeat massively
@@ -155,12 +155,13 @@ __global__ void __launch_bounds__(kTileThreads, 7) k_assign_tiles(DevBatch b, P2
         for (int i = 0; i < n; i++) {
             const uint32_t o0 = s.blk_off[i];
             if (s.blk_off[i + 1] > o0 && s.ref_id[i] >= 0 && s.ref_id[i] < a.nt.n_ref) {
-                const int32_t c = s.ref_id[i], c0 = a.nt.chr_first[c], c1 = a.nt.chr_first[c + 1];
+                const int32_t c = s.ref_id[i];
+                const ChrHead h = chr_head(a.nt, c);
                 const int32_t st = staged ? tb.blk_ref_pos[o0] : b.blk_ref_pos[o0];
-                if (c1 > c0) {
-                    const int32_t sg = seg_at(a.nt, c, c0, c1, st);
-                    s_base = sg - 1;
-                    s_seg[0] = c; s_seg[1] = sg; s_seg[2] = a.nt.pos[sg]; s_seg[3] = a.nt.end[sg];
+                if (h.c1 > h.c0) {
+                    const SegHit sg = seg_at(a.nt, h, st);
+                    s_base = sg.s - 1;
+                    s_seg[0] = c; s_seg[1] = sg.s; s_seg[2] = sg.pos; s_seg[3] = sg.end;
                 }
                 break;
             }
@@ -189,7 +190,7 @@ __global__ void __launch_bounds__(kTileThreads, 7) k_assign_tiles(DevBatch b, P2
             if (counted) {
                 st0 = staged ? tb.blk_ref_pos[o0] : b.blk_ref_pos[o0]; l0 = staged ? tb.blk_match_ref[o0] : b.blk_match_ref[o0];
                 if (rid == wc && wq <= st0 && st0 < we && l0 > kSeedThresh) { m = ws; cont = st0 + l0 <= we + kSeedThresh; }  // depth_target / depth_contained in the tile's segment
-                else { m = depth_target(nt, rid, st0, l0); cont = m != kNoNode && depth_contained(nt, m, rid, st0, l0); }
+                else { const SegHit t = depth_target_hit(nt, rid, st0, l0); m = t.s; cont = m != kNoNode && depth_contained(t, st0, l0); }
                 if (nb > 1) s_other = 1;
             }
             const uint32_t nb_max = __reduce_max_sync(full, counted ? nb : 0u);
@@ -202,9 +203,10 @@ __global__ void __launch_bounds__(kTileThreads, 7) k_assign_tiles(DevBatch b, P2
                     int32_t pj;
                     if (rid == wc && wq <= st && st < we) { m2 = ws; pj = wq; on = st + l <= we + kSeedThresh; }  // the tile's segment
                     else {
-                        m2 = depth_target(nt, rid, st, kSeedThresh + 1);  // first segment ending right of the start
+                        const SegHit t = depth_target_hit(nt, rid, st, kSeedThresh + 1);  // first segment ending right of the start
+                        m2 = t.s;
                         pj = st - 100;
-                        if (m2 != kNoNode) { pj = nt.pos[m2]; on = nt.chr[m2] == rid && st >= pj - kSeedThresh && st + l <= nt.end[m2] + kSeedThresh; }
+                        if (m2 != kNoNode) { pj = t.pos; on = depth_contained(t, st, l); }
                     }
                     // rare: a block of <= 3 bp (deferred), or one that starts within 2 bp of its segment's start (start mask)
                     if (l <= kSeedThresh || (uint32_t)(st - pj) <= 2u) on = depth_other_rare(a.omask, a.shorts, a.n_short, a.short_cap, rid, st, l, m2, st - pj, on);

@@ -365,14 +365,13 @@ __global__ void __launch_bounds__(1024) k_ops_dense(const int32_t *isl_start, in
 // ------------------------------------------------------------------------------------------------
 // kernels: segment table index
 // ------------------------------------------------------------------------------------------------
-// bin_seg[bin_off[c] + k] = segment of chromosome c holding position k << bin_shift (the last segment of c when that
-// position is the chromosome end itself)
-__global__ void k_build_bins(NodeTable nt, int32_t *bin_seg, int32_t n_bins) {
+// entry i of the position index (sq_common.cuh: seg_at); bin_off: n_ref + 1
+__global__ void k_build_bins(NodeTable nt, const int32_t *bin_off, BinEnt *bins, int32_t n_bins) {
     const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_bins) return;
     int32_t lo = 0, hi = nt.n_ref;  // chromosome of bin i: last c with bin_off[c] <= i
-    while (lo < hi) { const int32_t m = (lo + hi) >> 1; if (nt.bin_off[m + 1] <= i) lo = m + 1; else hi = m; }
-    bin_seg[i] = bin_seg_value(nt, lo, i - nt.bin_off[lo]);
+    while (lo < hi) { const int32_t m = (lo + hi) >> 1; if (bin_off[m + 1] <= i) lo = m + 1; else hi = m; }
+    bins[i] = bin_ent_value(nt, lo, i - bin_off[lo], bin_off[lo + 1] - bin_off[lo]);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -383,9 +382,10 @@ __global__ void k_depth_disc(NodeTable nt, const DiscBlock *D, int32_t nD, int32
     if (k >= nD) return;
     const DiscBlock d = D[k];
     if (d.chr < 0 || d.chr >= nt.n_ref) return;
-    const int32_t c0 = nt.chr_first[d.chr], c1 = nt.chr_first[d.chr + 1];
-    const int32_t j = seg_last_pos_le(nt, d.chr, c0, c1, d.pos);  // segment whose turn consumes this block (:774)
-    if (j >= c0 && d.pos >= nt.pos[j] && d.pos + d.len <= nt.end[j]) { atomicAdd(&cnt[j], 1); atomicAdd(&sum[j], d.len); }
+    const ChrHead h = chr_head(nt, d.chr);
+    if (h.c1 <= h.c0) return;
+    const SegHit j = seg_at(nt, h, d.pos);  // segment whose turn consumes this block (:774): the last with Position <= pos
+    if (d.pos >= j.pos && d.pos + d.len <= j.end) { atomicAdd(&cnt[j.s], 1); atomicAdd(&sum[j.s], d.len); }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1308,27 +1308,29 @@ static int install_nodes(sqg_ctx *ctx) {  // from h_nchr/h_npos/h_nend
         const bool same = ctx->h_nchr[i] == ctx->h_nchr[i + 1];
         if (ctx->h_nchr[i] > ctx->h_nchr[i + 1] || (same && ctx->h_nend[i] != ctx->h_npos[i + 1])) FAIL(SQG_EINVAL, "segments must be sorted and tile each chromosome");
     }
-    CK(ctx->d_nchr.ensure(N + 1)); CK(ctx->d_npos.ensure(N + 1)); CK(ctx->d_nend.ensure(N + 1)); CK(ctx->d_chr_first.ensure(n_ref + 2));
+    CK(ctx->d_nchr.ensure(N + 1)); CK(ctx->d_npos.ensure(N + 1)); CK(ctx->d_nend.ensure(N + 1)); CK(ctx->d_chr_head.ensure(n_ref + 1));
     if (N) {
         CK(cudaMemcpyAsync(ctx->d_nchr.p, ctx->h_nchr.data(), N * 4, cudaMemcpyHostToDevice, ctx->stream));
         CK(cudaMemcpyAsync(ctx->d_npos.p, ctx->h_npos.data(), N * 4, cudaMemcpyHostToDevice, ctx->stream));
         CK(cudaMemcpyAsync(ctx->d_nend.p, ctx->h_nend.data(), N * 4, cudaMemcpyHostToDevice, ctx->stream));
     }
-    CK(cudaMemcpyAsync(ctx->d_chr_first.p, ctx->h_chr_first.data(), (n_ref + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->nt.n = N; ctx->nt.n_ref = n_ref; ctx->nt.chr = ctx->d_nchr.p; ctx->nt.pos = ctx->d_npos.p; ctx->nt.end = ctx->d_nend.p; ctx->nt.chr_first = ctx->d_chr_first.p;
-    {   // coarse position index over the tiling (sq_common.cuh: seg_at)
+    ctx->nt.n = N; ctx->nt.n_ref = n_ref; ctx->nt.chr = ctx->d_nchr.p; ctx->nt.pos = ctx->d_npos.p; ctx->nt.end = ctx->d_nend.p;
+    {   // position index over the tiling (sq_common.cuh: seg_at): per-chromosome headers and 16-byte bin entries
         int64_t total = 0;
         for (int32_t c = 0; c < n_ref; c++) total += ctx->ref_len[c] > 0 ? ctx->ref_len[c] : 0;
         int32_t sh = 9;  // 512-bp bins: reads pile up exactly where segments are dense (fusion genes), so the bins must be fine
-        while ((total >> sh) > (16ll << 20)) sh++;  // at most ~16M bins (64 MB, L2-resident where it is hot)
+        while ((total >> sh) > (16ll << 20)) sh++;  // at most ~16M bins (256 MB; only the bins the reads touch are hot in L2)
         ctx->h_bin_off.assign(n_ref + 1, 0);
         for (int32_t c = 0; c < n_ref; c++) ctx->h_bin_off[c + 1] = ctx->h_bin_off[c] + ((ctx->ref_len[c] > 0 ? ctx->ref_len[c] : 0) >> sh) + 1;
         const int32_t n_bins = ctx->h_bin_off[n_ref];
-        CK(ctx->d_bin_off.ensure(n_ref + 2)); CK(ctx->d_bin_seg.ensure(n_bins + 1));
+        ctx->h_head.resize(n_ref);
+        for (int32_t c = 0; c < n_ref; c++) ctx->h_head[c] = chr_head_value(ctx->h_chr_first.data(), ctx->h_nend.data(), ctx->h_bin_off.data(), c);
+        CK(ctx->d_bin_off.ensure(n_ref + 2)); CK(ctx->d_bins.ensure(n_bins + 1));
         CK(cudaMemcpyAsync(ctx->d_bin_off.p, ctx->h_bin_off.data(), (n_ref + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
-        ctx->nt.bin_off = ctx->d_bin_off.p; ctx->nt.bin_shift = sh; ctx->nt.bin_seg = nullptr;
-        LAUNCH(k_build_bins, blocks_for(n_bins), kThreads, ctx->nt, ctx->d_bin_seg.p, n_bins);
-        ctx->nt.bin_seg = ctx->d_bin_seg.p;
+        if (n_ref) CK(cudaMemcpyAsync(ctx->d_chr_head.p, ctx->h_head.data(), n_ref * sizeof(ChrHead), cudaMemcpyHostToDevice, ctx->stream));
+        ctx->nt.head = ctx->d_chr_head.p; ctx->nt.bin_shift = sh; ctx->nt.bins = nullptr;
+        LAUNCH(k_build_bins, blocks_for(n_bins), kThreads, ctx->nt, ctx->d_bin_off.p, ctx->d_bins.p, n_bins);
+        ctx->nt.bins = ctx->d_bins.p;
     }
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->have_nodes = true; ctx->have_edge_table = false;
@@ -1338,7 +1340,7 @@ static int install_nodes(sqg_ctx *ctx) {  // from h_nchr/h_npos/h_nend
 extern "C" int sqg_set_nodes(sqg_ctx *ctx, const int32_t *chr, const int32_t *pos, const int32_t *len, int64_t n_nodes) {
     if (!ctx || !chr || !pos || !len || n_nodes <= 0 || n_nodes > 0x7ffffff0ll) return SQG_EINVAL;
     // the table must tile every chromosome from 0 to its length with segments of positive length: the position index (seg_at)
-    // and the closed-form LocateRead index a chromosome's segments as [chr_first[c], chr_first[c+1]) and take a position below
+    // and the closed-form LocateRead index a chromosome's segments as [head[c].c0, head[c].c1) and take a position below
     // the last segment's end to lie inside the chromosome's bins.  (Sortedness and contiguity are checked in install_nodes.)
     {
         const int32_t n_ref = ctx->params.n_ref;

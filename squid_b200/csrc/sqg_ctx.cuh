@@ -278,8 +278,11 @@ struct sqg_ctx {
     // segment table
     bool have_nodes = false;
     std::vector<int32_t> h_nchr, h_npos, h_nend, h_chr_first;
-    sq::DBuf<int32_t> d_nchr, d_npos, d_nend, d_chr_first, d_bin_off, d_bin_seg;
+    sq::DBuf<int32_t> d_nchr, d_npos, d_nend, d_bin_off;
+    sq::DBuf<sq::ChrHead> d_chr_head;
+    sq::DBuf<sq::BinEnt> d_bins;
     std::vector<int32_t> h_bin_off;
+    std::vector<sq::ChrHead> h_head;
     sq::NodeTable nt;
     sq::DBuf<int32_t> d_cnt3, d_sum3;
 
