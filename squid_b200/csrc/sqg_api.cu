@@ -91,6 +91,15 @@ static int cov_join(sqg_ctx *ctx) {
 }
 #define PHASE_BEGIN(name) do { int rc_ = phase_begin(ctx, name); if (rc_) return rc_; } while (0)
 #define PHASE_END(name) do { int rc_ = phase_end(ctx, name); if (rc_) return rc_; } while (0)
+// One CUB device-wide call: `call(temp, bytes)` with temp == nullptr for the size query, the scratch grown to fit, the call.
+// The scratch belongs to the stream of the call: d_temp (ctx->stream), d_temp3 (the pre-pass, stream3) and d_temp_cov
+// (stream_cov) are in use at the same time.
+template <class F> static cudaError_t cub_call(DBuf<unsigned char> &temp, F &&call) {
+    size_t bytes = 0;
+    cudaError_t e = call(nullptr, bytes);
+    if (e == cudaSuccess) e = temp.ensure(bytes + 256);
+    return e == cudaSuccess ? call(temp.p, bytes) : e;
+}
 
 // ------------------------------------------------------------------------------------------------
 // functors / kernels: classify
@@ -667,6 +676,7 @@ int64_t sqg_launch_count(const sqg_ctx *ctx) { return ctx ? ctx->launches + ctx-
 int64_t sqg_stat(const sqg_ctx *ctx, const char *name) {
     if (!ctx || !name) return -1;
     const std::string n(name);
+    const Counters *hc = ctx->cnt.h.p;  // (-1 for its fields until a stage has allocated it)
     if (n == "islands") return ctx->n_islands;
     if (n == "device_sort_status") return ctx->gs_last_status;  // 0: the pre-pass sort ran on the device (also on no discordant blocks); 2/3: it declined, the cores sorted; -100: no pre-pass yet
     if (n == "heavy_islands") return ctx->n_heavy;
@@ -686,19 +696,19 @@ int64_t sqg_stat(const sqg_ctx *ctx, const char *name) {
     if (n == "classify_attempts") return ctx->classify_attempts;    // 2: the coverage-gap candidate buffer overflowed and phase 1 ran again
     if (n == "edge_pass_attempts") return ctx->edge_pass_attempts;  // > 1: a list of the last edge pass overflowed and the pass ran again
     if (n == "r_break") return ctx->r_break;
-    if (n == "seed_window_records") return ctx->h_counters.p ? ctx->h_counters.p[29] : -1;  // concordant-cluster window sizes summed over the groups
+    if (n == "seed_window_records") return hc ? (int64_t)hc->win_count : -1;  // concordant-cluster window sizes summed over the groups
     if (n == "n_rec") return ctx->have_batch ? ctx->batch.n_rec : -1;
     if (n == "n_blk") return ctx->have_batch ? ctx->batch.n_blk : -1;
-    if (n == "slow_records") return ctx->h_counters.p ? (int64_t)*(int32_t *)(ctx->h_counters.p + 18) : -1;  // records handled by k_edges_generic
+    if (n == "slow_records") return hc ? hc->n_slow : -1;  // records handled by k_edges_generic
     if (n == "qualifying_records") return ctx->cov_nq;
     if (n == "short_other_blocks") return ctx->n_short_other;        // ReadsOther blocks of <= 3 bp in the last depth pass
     if (n == "unstable_depth_blocks") return ctx->n_unstable_other;  // ... whose segment depends on the tie order of sort(ReadsOther): resolved by replaying that sort
     if (n == "other_sort_status") return ctx->other_sort_status;
-    if (n == "edges_single_path") return ctx->h_counters.p ? ctx->h_counters.p[16] : -1;
+    if (n == "edges_single_path") return hc ? (int64_t)hc->path_counts[0] : -1;
     if (n == "bam_members") return ctx->bam_members;                // BGZF members (with data) of the last sqg_load_concordant_bam
     if (n == "bam_windows") return ctx->bam_windows;
     if (n == "bam_repair_rounds") return ctx->bam_repair_rounds;    // rounds of segments walked again from their true entry, summed over the windows
-    if (n == "edges_generic_path") return ctx->h_counters.p ? ctx->h_counters.p[17] : -1;
+    if (n == "edges_generic_path") return hc ? (int64_t)hc->path_counts[1] : -1;
     return -1;
 }
 
@@ -708,10 +718,9 @@ int64_t sqg_stat(const sqg_ctx *ctx, const char *name) {
 static void point_batch_at_own_arrays(sqg_ctx *ctx, int64_t n_rec, int64_t n_blk) {
     DevBatch &b = ctx->batch;
     b.n_rec = n_rec; b.n_blk = n_blk;
-    b.ref_id = ctx->o_ref_id.p; b.pos = ctx->o_pos.p; b.mate_ref_id = ctx->o_mate_ref_id.p; b.mate_pos = ctx->o_mate_pos.p; b.end_pos = ctx->o_end_pos.p;
-    b.flag = ctx->o_flag.p; b.total_len = ctx->o_total_len.p; b.lowphred_run = ctx->o_lowphred_run.p; b.mapq = ctx->o_mapq.p; b.aux = ctx->o_aux.p;
-    b.blk_off = ctx->o_blk_off.p; b.blk_ref_pos = ctx->o_blk_ref_pos.p; b.blk_match_ref = ctx->o_blk_match_ref.p;
-    b.blk_read_pos = ctx->o_blk_read_pos.p; b.blk_match_read = ctx->o_blk_match_read.p;
+#define X(T, name, ext) b.name = ctx->o_##name.p;
+    SQ_BATCH_ARRAYS(X)
+#undef X
 }
 // A new batch is resident: nothing computed on the previous one applies (the segment table, have_nodes, still does).  `wire`: its
 // arrays come from the wire decode, whose consistency flag run_classify checks and whose classification may already be running
@@ -720,6 +729,11 @@ static void reset_batch_state(sqg_ctx *ctx, bool owned, int64_t first_record_ind
     ctx->have_batch = true; ctx->batch_owned = owned; ctx->batch_restricted = false; ctx->first_record_index = first_record_index;
     ctx->classified = false; ctx->cov_compacted = false; ctx->have_edge_table = false; ctx->wire_loaded = wire;
     if (!wire) ctx->classify_prelaunched = false;
+}
+// A batch from the wire decode is refused when the decode flagged it; the caller has copied the flag to the mirror and synchronised.
+static int wire_check(sqg_ctx *ctx) {
+    if (ctx->wire_loaded && ctx->cnt.h.p->wire_bad) FAIL(SQG_EINVAL, "wire batch is inconsistent (escape without an exception entry, or block counts that contradict the tile table)");
+    return SQG_OK;
 }
 
 extern "C" int sqg_load_concordant(sqg_ctx *ctx, const sqg_batch *hb, int64_t first_record_index) {
@@ -733,16 +747,14 @@ extern "C" int sqg_load_concordant(sqg_ctx *ctx, const sqg_batch *hb, int64_t fi
     { const int rcj = cov_join(ctx); if (rcj) return rcj; }
     PHASE_BEGIN("h2d");
     const size_t n = (size_t)hb->n_rec, nb = (size_t)hb->n_blk;
-#define UP(buf, src, cnt)                                                                                       \
-    do {                                                                                                        \
-        CK(ctx->buf.ensure((cnt) ? (cnt) : 1));                                                                 \
-        if (cnt) CK(cudaMemcpyAsync(ctx->buf.p, hb->src, (cnt) * sizeof(*hb->src), cudaMemcpyHostToDevice, ctx->stream)); \
-    } while (0)
-    UP(o_ref_id, ref_id, n); UP(o_pos, pos, n); UP(o_mate_ref_id, mate_ref_id, n); UP(o_mate_pos, mate_pos, n); UP(o_end_pos, end_pos, n);
-    UP(o_flag, flag, n); UP(o_total_len, total_len, n); UP(o_lowphred_run, lowphred_run, n); UP(o_mapq, mapq, n); UP(o_aux, aux, n);
-    UP(o_blk_off, blk_off, n + 1);
-    UP(o_blk_ref_pos, blk_ref_pos, nb); UP(o_blk_match_ref, blk_match_ref, nb); UP(o_blk_read_pos, blk_read_pos, nb); UP(o_blk_match_read, blk_match_read, nb);
-#undef UP
+#define X(T, name, ext)                                                                                                  \
+    {                                                                                                                    \
+        const size_t cnt = batch_extent(ext, n, nb);                                                                     \
+        CK(ctx->o_##name.ensure(cnt ? cnt : 1));                                                                         \
+        if (cnt) CK(cudaMemcpyAsync(ctx->o_##name.p, hb->name, cnt * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));  \
+    }
+    SQ_BATCH_ARRAYS(X)
+#undef X
     point_batch_at_own_arrays(ctx, hb->n_rec, hb->n_blk);
     PHASE_END("h2d");
     reset_batch_state(ctx, true, first_record_index, false);
@@ -775,19 +787,18 @@ extern "C" int sqg_load_concordant_wire(sqg_ctx *ctx, const sqg_wire *w, int64_t
     if (!ctx->stream_up) CK(cudaStreamCreateWithFlags(&ctx->stream_up, cudaStreamNonBlocking));
     PHASE_BEGIN("h2d");
     const size_t n1 = n ? (size_t)n : 1, nb1 = nb ? (size_t)nb : 1, nt1 = (size_t)nt + 1, nwb1 = nwb ? (size_t)nwb : 1;
-    CK(ctx->o_ref_id.ensure(n1)); CK(ctx->o_pos.ensure(n1)); CK(ctx->o_mate_ref_id.ensure(n1)); CK(ctx->o_mate_pos.ensure(n1)); CK(ctx->o_end_pos.ensure(n1));
-    CK(ctx->o_flag.ensure(n1)); CK(ctx->o_total_len.ensure(n1)); CK(ctx->o_lowphred_run.ensure(n1)); CK(ctx->o_mapq.ensure(n1)); CK(ctx->o_aux.ensure(n1));
-    CK(ctx->o_blk_off.ensure(n1 + 1));
-    CK(ctx->o_blk_ref_pos.ensure(nb1)); CK(ctx->o_blk_match_ref.ensure(nb1)); CK(ctx->o_blk_read_pos.ensure(nb1)); CK(ctx->o_blk_match_read.ensure(nb1));
+#define X(T, name, ext) CK(ctx->o_##name.ensure(batch_extent(ext, n1, nb1)));
+    SQ_BATCH_ARRAYS(X)
+#undef X
     CK(ctx->w_dpos.ensure(n1)); CK(ctx->w_span.ensure(n1)); CK(ctx->w_dmate.ensure(n1)); CK(ctx->w_lp.ensure(n1)); CK(ctx->w_an.ensure(n1));
     CK(ctx->w_bdref.ensure(nwb1)); CK(ctx->w_bmref.ensure(nwb1)); CK(ctx->w_brpos.ensure(nwb1)); CK(ctx->w_bmread.ensure(nwb1)); CK(ctx->w_tile_wblk.ensure(nt1));
     CK(ctx->w_tile_ref.ensure(nt1)); CK(ctx->w_tile_pos.ensure(nt1)); CK(ctx->w_tile_blk.ensure(nt1)); CK(ctx->w_tile_rexc.ensure(nt1)); CK(ctx->w_tile_bexc.ensure(nt1));
     CK(ctx->w_rec_exc.ensure(w->n_rec_exc ? (size_t)w->n_rec_exc : 1)); CK(ctx->w_blk_exc.ensure(w->n_blk_exc ? (size_t)w->n_blk_exc : 1));
-    CK(ctx->d_counters.ensure(32)); CK(ctx->h_counters.ensure(32));
+    CK(ctx->cnt.ensure());
     cudaStream_t up = ctx->stream_up;
     // the copy stream starts after everything the main stream still has queued on the previous batch
     CK(cudaEventRecord(ctx->ev_fork, ctx->stream)); CK(cudaStreamWaitEvent(up, ctx->ev_fork, 0));
-    CK(cudaMemsetAsync(ctx->d_counters.p + 28, 0, sizeof(int64_t), ctx->stream));
+    CK(ctx->cnt.zero(ctx->stream, &ctx->cnt.d.p->wire_bad));
 #define UPW(dst, src, off, cnt) do { if ((cnt) > 0) CK(cudaMemcpyAsync((dst) + (off), (src) + (off), (size_t)(cnt) * sizeof(*(src)), cudaMemcpyHostToDevice, up)); } while (0)
     if (nt > 0) {
         UPW(ctx->w_tile_ref.p, w->tile_ref_id, 0, nt); UPW(ctx->w_tile_pos.p, w->tile_pos, 0, nt);
@@ -805,7 +816,7 @@ extern "C" int sqg_load_concordant_wire(sqg_ctx *ctx, const sqg_wire *w, int64_t
     wo.ref_id = ctx->o_ref_id.p; wo.pos = ctx->o_pos.p; wo.mate_ref_id = ctx->o_mate_ref_id.p; wo.mate_pos = ctx->o_mate_pos.p; wo.end_pos = ctx->o_end_pos.p;
     wo.lowphred_run = ctx->o_lowphred_run.p; wo.aux = ctx->o_aux.p; wo.blk_off = ctx->o_blk_off.p; wo.blk_ref_pos = ctx->o_blk_ref_pos.p; wo.blk_match_ref = ctx->o_blk_match_ref.p;
     wo.blk_read_pos = ctx->o_blk_read_pos.p; wo.blk_match_read = ctx->o_blk_match_read.p;
-    wo.bad = (int32_t *)(ctx->d_counters.p + 28);
+    wo.bad = &ctx->cnt.d.p->wire_bad;
     point_batch_at_own_arrays(ctx, n, nb);
     // The classification tile kernel needs nothing but the batch: it follows every chunk's widening kernel on the main stream, so
     // that it, too, runs while the later chunks are on the bus (run_classify then only finishes: scans, lists).  A tile looks at
@@ -901,14 +912,12 @@ extern "C" int sqg_download_concordant(sqg_ctx *ctx, sqg_batch *out) {
     if (out->n_rec != b.n_rec || out->n_blk != b.n_blk) FAIL(SQG_EINVAL, "sqg_download_concordant: n_rec / n_blk do not match the resident batch");
     CK(cudaSetDevice(ctx->device));
     const size_t n = (size_t)b.n_rec, nb = (size_t)b.n_blk;
-#define DN(field, cnt) do { if ((cnt) > 0) CK(cudaMemcpyAsync((void *)out->field, b.field, (cnt) * sizeof(*b.field), cudaMemcpyDeviceToHost, ctx->stream)); } while (0)
-    DN(ref_id, n); DN(pos, n); DN(mate_ref_id, n); DN(mate_pos, n); DN(end_pos, n); DN(flag, n); DN(total_len, n); DN(lowphred_run, n); DN(mapq, n); DN(aux, n);
-    DN(blk_off, n + 1); DN(blk_ref_pos, nb); DN(blk_match_ref, nb); DN(blk_read_pos, nb); DN(blk_match_read, nb);
-#undef DN
-    if (ctx->wire_loaded) CK(cudaMemcpyAsync(ctx->h_counters.p + 28, ctx->d_counters.p + 28, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+#define X(T, name, ext) if (const size_t cnt = batch_extent(ext, n, nb)) CK(cudaMemcpyAsync((void *)out->name, b.name, cnt * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
+    SQ_BATCH_ARRAYS(X)
+#undef X
+    if (ctx->wire_loaded) CK(ctx->cnt.to_host(ctx->stream, &ctx->cnt.d.p->wire_bad));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (ctx->wire_loaded && *(int32_t *)(ctx->h_counters.p + 28)) FAIL(SQG_EINVAL, "wire batch is inconsistent (escape without an exception entry, or block counts that contradict the tile table)");
-    return SQG_OK;
+    return wire_check(ctx);
 }
 
 extern "C" int sqg_attach_concordant_device(sqg_ctx *ctx, const sqg_batch *db, int64_t first_record_index) {
@@ -918,9 +927,9 @@ extern "C" int sqg_attach_concordant_device(sqg_ctx *ctx, const sqg_batch *db, i
     if (ctx->cov_pending) { CK(cudaStreamSynchronize(ctx->stream_cov)); ctx->cov_pending = false; }  // the previous batch's arrays belong to the caller again
     DevBatch &b = ctx->batch;
     b.n_rec = db->n_rec; b.n_blk = db->n_blk;
-    b.ref_id = db->ref_id; b.pos = db->pos; b.mate_ref_id = db->mate_ref_id; b.mate_pos = db->mate_pos; b.end_pos = db->end_pos;
-    b.flag = db->flag; b.total_len = db->total_len; b.lowphred_run = db->lowphred_run; b.mapq = db->mapq; b.aux = db->aux;
-    b.blk_off = db->blk_off; b.blk_ref_pos = db->blk_ref_pos; b.blk_match_ref = db->blk_match_ref; b.blk_read_pos = db->blk_read_pos; b.blk_match_read = db->blk_match_read;
+#define X(T, name, ext) b.name = db->name;
+    SQ_BATCH_ARRAYS(X)
+#undef X
     reset_batch_state(ctx, false, first_record_index, false);
     return SQG_OK;
 }
@@ -977,20 +986,16 @@ static int device_prepass(sqg_ctx *ctx, size_t nr) {
     c.first_low = ctx->dc_first_low.p; c.second_low = ctx->dc_second_low.p; c.multi = ctx->dc_multi.p;
     c.chr = ctx->dc_ref_id.p; c.pos = ctx->dc0_ref_pos.p; c.rpos = ctx->dc0_read_pos.p; c.mref = ctx->dc0_match_ref.p; c.mread = ctx->dc0_match_read.p; c.rev = ctx->dc_rev.p;
     PCK(ctx->d_pre_ndis.ensure(nr + 1)); PCK(ctx->d_pre_pusher.ensure(nr + 1)); PCK(ctx->d_pre_lastk.ensure(nr + 1)); PCK(ctx->d_pre_off.ensure(nr + 2));
-    PCK(ctx->d_pre_part.ensure(4 * nr + n_ref + 1)); PCK(ctx->d_pre_part2.ensure(4 * nr + n_ref + 1)); PCK(ctx->d_pre_cnt.ensure(8)); PCK(ctx->h_pre_cnt.ensure(8));
-    auto temp = [&](size_t bytes) { return ctx->d_temp3.ensure(bytes + 256); };
+    PCK(ctx->d_pre_part.ensure(4 * nr + n_ref + 1)); PCK(ctx->d_pre_part2.ensure(4 * nr + n_ref + 1)); PCK(ctx->pre_cnt.ensure());
+    PreCounters *dc = ctx->pre_cnt.d.p, *hc = ctx->pre_cnt.h.p;
     int64_t launches = 0;
     PCK(cudaMemsetAsync(ctx->d_pre_ndis.p + nr, 0, 4, st));
     k_pre_count<<<blocks_for((int64_t)nr), kThreads, 0, st>>>(c, ctx->d_pre_ndis.p, ctx->d_pre_pusher.p, ctx->d_pre_lastk.p);
-    size_t tb = 0, tb2 = 0;
-    PCK(cub::DeviceScan::ExclusiveSum(nullptr, tb, ctx->d_pre_ndis.p, ctx->d_pre_off.p, (int)(nr + 1), st));
-    PCK(cub::DeviceScan::ExclusiveScan(nullptr, tb2, ctx->d_pre_pusher.p, ctx->d_pre_pusher.p, MaxI32(), (int32_t)-1, (int)nr, st));
-    PCK(temp(std::max(tb, tb2)));
-    PCK(cub::DeviceScan::ExclusiveSum(ctx->d_temp3.p, tb, ctx->d_pre_ndis.p, ctx->d_pre_off.p, (int)(nr + 1), st));
-    PCK(cub::DeviceScan::ExclusiveScan(ctx->d_temp3.p, tb2, ctx->d_pre_pusher.p, ctx->d_pre_pusher.p, MaxI32(), (int32_t)-1, (int)nr, st));
-    PCK(cudaMemcpyAsync(ctx->h_pre_cnt.p, ctx->d_pre_off.p + nr, 8, cudaMemcpyDeviceToHost, st));
+    PCK(cub_call(ctx->d_temp3, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveSum(t, tb, ctx->d_pre_ndis.p, ctx->d_pre_off.p, (int)(nr + 1), st); }));
+    PCK(cub_call(ctx->d_temp3, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveScan(t, tb, ctx->d_pre_pusher.p, ctx->d_pre_pusher.p, MaxI32(), (int32_t)-1, (int)nr, st); }));
+    PCK(cudaMemcpyAsync(&hc->n_disc, ctx->d_pre_off.p + nr, 8, cudaMemcpyDeviceToHost, st));
     PCK(cudaStreamSynchronize(st));
-    const int64_t nD = ctx->h_pre_cnt.p[0];
+    const int64_t nD = hc->n_disc;
     if (nD >= 0x7fffff00ll) return (int)cudaErrorInvalidValue;
     PCK(ctx->d_gs_keys.ensure((size_t)nD + 1)); PCK(ctx->d_gs_idx.ensure((size_t)nD + 1)); PCK(ctx->d_gs_scratch.ensure(gsort::bytes_needed((size_t)nD)));
     PCK(ctx->d_disc.ensure((size_t)nD + 1)); PCK(ctx->d_pre_endkey.ensure((size_t)nD + 1)); PCK(ctx->d_pre_excl.ensure((size_t)nD + 1)); PCK(ctx->d_pre_incl.ensure((size_t)nD + 1));
@@ -998,10 +1003,9 @@ static int device_prepass(sqg_ctx *ctx, size_t nr) {
     // PartAlignPos is resize()d to n_ref entries (0, 0) and then appended to (:203-204)
     PCK(cudaMemsetAsync(ctx->d_pre_part.p, 0, (size_t)n_ref * 8, st));
     const unsigned long long np0 = (unsigned long long)n_ref;
-    PCK(cudaMemcpyAsync(ctx->d_pre_cnt.p, &np0, 8, cudaMemcpyHostToDevice, st));
-    k_pre_write<<<blocks_for((int64_t)nr), kThreads, 0, st>>>(c, ctx->d_pre_off.p, ctx->d_pre_pusher.p, ctx->d_pre_lastk.p, ctx->d_gs_keys.p, ctx->d_gs_idx.p, ctx->d_pre_part.p,
-                                                                 (unsigned long long *)ctx->d_pre_cnt.p);
-    PCK(cudaMemcpyAsync(ctx->h_pre_cnt.p + 1, ctx->d_pre_cnt.p, 8, cudaMemcpyDeviceToHost, st));
+    PCK(cudaMemcpyAsync(&dc->n_part, &np0, 8, cudaMemcpyHostToDevice, st));
+    k_pre_write<<<blocks_for((int64_t)nr), kThreads, 0, st>>>(c, ctx->d_pre_off.p, ctx->d_pre_pusher.p, ctx->d_pre_lastk.p, ctx->d_gs_keys.p, ctx->d_gs_idx.p, ctx->d_pre_part.p, &dc->n_part);
+    PCK(ctx->pre_cnt.to_host(st, &dc->n_part));
     launches += 6;
     // std::sort's permutation of bamdiscordant (:264): tie order is observable (SURVEY.md App. A-11)
     int rc = gsort::sort_like_std_device(ctx->d_gs_keys.p, ctx->d_gs_idx.p, (size_t)nD, ctx->d_gs_scratch.p, st, &launches);
@@ -1009,9 +1013,8 @@ static int device_prepass(sqg_ctx *ctx, size_t nr) {
     if (rc < 0) return -rc;
     if (rc != 0) {  // std::sort would have left the quicksort path (never seen on alignment data): the CPU twin, from a fresh copy of the keys
         const unsigned long long np1 = (unsigned long long)n_ref;
-        PCK(cudaMemcpyAsync(ctx->d_pre_cnt.p, &np1, 8, cudaMemcpyHostToDevice, st));
-        k_pre_write<<<blocks_for((int64_t)nr), kThreads, 0, st>>>(c, ctx->d_pre_off.p, ctx->d_pre_pusher.p, ctx->d_pre_lastk.p, ctx->d_gs_keys.p, ctx->d_gs_idx.p, ctx->d_pre_part.p,
-                                                                     (unsigned long long *)ctx->d_pre_cnt.p);
+        PCK(cudaMemcpyAsync(&dc->n_part, &np1, 8, cudaMemcpyHostToDevice, st));
+        k_pre_write<<<blocks_for((int64_t)nr), kThreads, 0, st>>>(c, ctx->d_pre_off.p, ctx->d_pre_pusher.p, ctx->d_pre_lastk.p, ctx->d_gs_keys.p, ctx->d_gs_idx.p, ctx->d_pre_part.p, &dc->n_part);
         std::vector<uint64_t> hk((size_t)nD); std::vector<uint32_t> hi((size_t)nD);
         PCK(cudaMemcpyAsync(hk.data(), ctx->d_gs_keys.p, (size_t)nD * 8, cudaMemcpyDeviceToHost, st));
         PCK(cudaMemcpyAsync(hi.data(), ctx->d_gs_idx.p, (size_t)nD * 4, cudaMemcpyDeviceToHost, st));
@@ -1024,37 +1027,29 @@ static int device_prepass(sqg_ctx *ctx, size_t nr) {
         PCK(cudaStreamSynchronize(st));
     }
     PCK(cudaStreamSynchronize(st));
-    const int64_t nP = ctx->h_pre_cnt.p[1];
+    const int64_t nP = (int64_t)hc->n_part;
     PCK(ctx->d_pchr.ensure((size_t)nP + 1)); PCK(ctx->d_ppos.ensure((size_t)nP + 1));
     {   // sort(PartAlignPos) by (chr, pos) (:262): a total order on the values, any stable or unstable sort agrees
         int key_bits = 33;
         while (key_bits < 64 && (1ll << (key_bits - 32)) < (long long)n_ref) key_bits++;
-        PCK(cub::DeviceRadixSort::SortKeys(nullptr, tb, ctx->d_pre_part.p, ctx->d_pre_part2.p, (int)nP, 0, key_bits, st));
-        PCK(temp(tb));
-        PCK(cub::DeviceRadixSort::SortKeys(ctx->d_temp3.p, tb, ctx->d_pre_part.p, ctx->d_pre_part2.p, (int)nP, 0, key_bits, st));
+        PCK(cub_call(ctx->d_temp3, [&](void *t, size_t &tb) { return cub::DeviceRadixSort::SortKeys(t, tb, ctx->d_pre_part.p, ctx->d_pre_part2.p, (int)nP, 0, key_bits, st); }));
         k_pre_split_part<<<blocks_for(nP), kThreads, 0, st>>>(ctx->d_pre_part2.p, nP, ctx->d_pchr.p, ctx->d_ppos.p);
         launches += 4;
     }
     k_pre_gather<<<blocks_for(nD + 1), kThreads, 0, st>>>(c, ctx->d_gs_idx.p, nD, ctx->d_disc.p, ctx->d_pre_endkey.p);
     int32_t nG = 0;
     if (nD > 0) {
-        PCK(cub::DeviceScan::ExclusiveScan(nullptr, tb, ctx->d_pre_endkey.p, ctx->d_pre_excl.p, MaxU64(), (uint64_t)0, (int)nD, st));
-        PCK(cub::DeviceScan::InclusiveScan(nullptr, tb2, ctx->d_pre_endkey.p, ctx->d_pre_incl.p, MaxU64(), (int)nD, st));
-        PCK(temp(std::max(tb, tb2)));
-        PCK(cub::DeviceScan::ExclusiveScan(ctx->d_temp3.p, tb, ctx->d_pre_endkey.p, ctx->d_pre_excl.p, MaxU64(), (uint64_t)0, (int)nD, st));
-        PCK(cub::DeviceScan::InclusiveScan(ctx->d_temp3.p, tb2, ctx->d_pre_endkey.p, ctx->d_pre_incl.p, MaxU64(), (int)nD, st));
+        PCK(cub_call(ctx->d_temp3, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveScan(t, tb, ctx->d_pre_endkey.p, ctx->d_pre_excl.p, MaxU64(), (uint64_t)0, (int)nD, st); }));
+        PCK(cub_call(ctx->d_temp3, [&](void *t, size_t &tb) { return cub::DeviceScan::InclusiveScan(t, tb, ctx->d_pre_endkey.p, ctx->d_pre_incl.p, MaxU64(), (int)nD, st); }));
         k_pre_opens<<<blocks_for(nD), kThreads, 0, st>>>(ctx->d_disc.p, ctx->d_pre_excl.p, nD, ctx->params.read_len, ctx->d_pre_opens.p);
         cub::CountingInputIterator<int32_t> cnt(0);
         PreOpenOp op{ctx->d_pre_opens.p};
-        int32_t *d_ng = (int32_t *)(ctx->d_pre_cnt.p + 2);
-        PCK(cub::DeviceSelect::If(nullptr, tb, cnt, ctx->d_pre_open.p, d_ng, (int)nD, op, st));
-        PCK(temp(tb));
-        PCK(cub::DeviceSelect::If(ctx->d_temp3.p, tb, cnt, ctx->d_pre_open.p, d_ng, (int)nD, op, st));
-        PCK(cudaMemcpyAsync(ctx->h_pre_cnt.p + 2, ctx->d_pre_cnt.p + 2, 8, cudaMemcpyDeviceToHost, st));
+        PCK(cub_call(ctx->d_temp3, [&](void *t, size_t &tb) { return cub::DeviceSelect::If(t, tb, cnt, ctx->d_pre_open.p, &dc->n_groups, (int)nD, op, st); }));
+        PCK(ctx->pre_cnt.to_host(st, &dc->n_groups));
         PCK(cudaStreamSynchronize(st));
-        nG = *(int32_t *)(ctx->h_pre_cnt.p + 2);
+        nG = hc->n_groups;
         PCK(ctx->d_groups.ensure((size_t)nG + 1));
-        k_pre_groups<<<blocks_for(nG), kThreads, 0, st>>>(ctx->d_disc.p, ctx->d_pre_open.p, d_ng, ctx->d_pre_excl.p, ctx->d_pre_incl.p, nD, ctx->d_groups.p);
+        k_pre_groups<<<blocks_for(nG), kThreads, 0, st>>>(ctx->d_disc.p, ctx->d_pre_open.p, &dc->n_groups, ctx->d_pre_excl.p, ctx->d_pre_incl.p, nD, ctx->d_groups.p);
         launches += 9;
     } else PCK(ctx->d_groups.ensure(1));
     PCK(cudaGetLastError());
@@ -1136,13 +1131,10 @@ static int finish_prepass(sqg_ctx *ctx) {
     ctx->prepass_uploaded = true;
     return SQG_OK;
 }
-static int ensure_temp(sqg_ctx *ctx, size_t bytes) { CK(ctx->d_temp.ensure(bytes + 256)); return SQG_OK; }
-#define ENSURE_TEMP(bytes) do { int rc_ = ensure_temp(ctx, bytes); if (rc_) return rc_; } while (0)
-
 static bool batch_bulk_ok(const DevBatch &b) {  // TMA bulk copies need 16-byte aligned sources
-    const void *ptrs[] = {b.ref_id, b.pos, b.mate_ref_id, b.mate_pos, b.end_pos, b.flag, b.total_len, b.lowphred_run, b.mapq, b.aux, b.blk_off,
-                          b.blk_ref_pos, b.blk_match_ref, b.blk_read_pos, b.blk_match_read};
-    for (const void *q : ptrs) if (((uintptr_t)q) & 15u) return false;
+#define X(T, name, ext) if (((uintptr_t)b.name) & 15u) return false;
+    SQ_BATCH_ARRAYS(X)
+#undef X
     return true;
 }
 static constexpr size_t kTileSmemBytes = sizeof(TileStage) + 128;
@@ -1153,20 +1145,16 @@ static int classify_setup(sqg_ctx *ctx, int64_t cand_cap, P1Out &o) {
     const DevBatch &b = ctx->batch;
     const int64_t n = b.n_rec, n_tiles = (n + kTile - 1) / kTile;
     CK(ctx->d_cls.ensure(n + 4)); CK(ctx->d_flen.ensure(n + 4)); CK(ctx->d_scratch32.ensure(n + 1));
-    CK(ctx->d_counters.ensure(32)); CK(ctx->h_counters.ensure(32));
     CK(ctx->d_qstage_key.ensure((size_t)n + 1)); CK(ctx->d_qstage_end.ensure((size_t)n + 1));
     CK(ctx->d_tileagg.ensure(n_tiles + 1)); CK(ctx->d_chain64.ensure(n_tiles + 8)); CK(ctx->d_ccmax.ensure(n_tiles + 1)); CK(ctx->d_cov_nq.ensure(n_tiles + 2)); CK(ctx->d_cov_qmax.ensure(n_tiles + 2));
     CK(ctx->d_cand_key.ensure(cand_cap));
     o.cls = ctx->d_cls.p; o.first_len = ctx->d_flen.p; o.agg = ctx->d_tileagg.p; o.ccmax = ctx->d_ccmax.p; o.cov_nq = ctx->d_cov_nq.p; o.cov_qmax = ctx->d_cov_qmax.p; o.qstage_key = ctx->d_qstage_key.p; o.qstage_end = ctx->d_qstage_end.p; o.gate_word = ctx->d_chain64.p; o.n_tiles = (int32_t)n_tiles;
     o.cand_rec = ctx->d_scratch32.p; o.cand_key = ctx->d_cand_key.p; o.cand_cap = (int32_t)cand_cap;
-    // counters: [0..1] totals n_gap, n_pc, n_dp (int32) | [2] first_kept | [3] lmax | [4] n_cand, ticket (int32) | [20] validation flags
-    CK(cudaMemsetAsync(ctx->d_counters.p, 0, 5 * sizeof(int64_t), ctx->stream));
-    CK(cudaMemsetAsync(ctx->d_counters.p + 20, 0, sizeof(int64_t), ctx->stream));
+    Counters *dc = ctx->cnt.d.p;
+    CK(ctx->cnt.zero(ctx->stream, &dc->totals, &dc->bad_flags));
     CK(cudaMemsetAsync(ctx->d_chain64.p, 0, n_tiles * sizeof(uint64_t), ctx->stream));
-    CK(cudaMemcpyAsync(ctx->d_counters.p + 2, &n, sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
-    o.first_kept = (long long *)(ctx->d_counters.p + 2); o.lmax = (int32_t *)(ctx->d_counters.p + 3);
-    o.n_cand = (int32_t *)(ctx->d_counters.p + 4); o.ticket = o.n_cand + 1;
-    o.bad_flags = (int32_t *)(ctx->d_counters.p + 20);
+    CK(cudaMemcpyAsync(&dc->first_kept, &n, sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    o.first_kept = &dc->first_kept; o.lmax = &dc->lmax; o.n_cand = &dc->n_cand; o.ticket = &dc->ticket; o.bad_flags = &dc->bad_flags;
     {
         BatchDesc hd; hd.b = b; hd.p = ctx->params;
         CK(ctx->d_desc.ensure(sizeof(BatchDesc)));
@@ -1192,7 +1180,9 @@ static int run_classify(sqg_ctx *ctx) {
     const DevBatch &b = ctx->batch;
     const int64_t n = b.n_rec;
     PHASE_BEGIN("classify");
-    CK(ctx->d_counters.ensure(32)); CK(ctx->h_counters.ensure(32));
+    CK(ctx->cnt.ensure());
+    Counters *dc = ctx->cnt.d.p;
+    const Counters &hc = *ctx->cnt.h.p;
     ctx->n_gap = 0; ctx->n_pc = 0; ctx->n_dp = 0; ctx->lmax = 0; ctx->first_kept = n; ctx->end_other = 0; ctx->classify_attempts = 0;
     if (n > 0) {
         const int64_t n_tiles = (n + kTile - 1) / kTile;
@@ -1200,7 +1190,6 @@ static int run_classify(sqg_ctx *ctx) {
         int32_t n_cand = 0;
         for (int attempt = 0; attempt < 2; attempt++) {
             cand_cap = std::min<int64_t>(cand_cap, n + 1);
-            int32_t *totals = (int32_t *)ctx->d_counters.p;
             if (attempt == 0 && ctx->classify_prelaunched) {
                 // the tile kernel already ran, chunk by chunk, behind the widening kernels of the wire upload
                 cand_cap = ctx->pre_cand_cap;
@@ -1212,42 +1201,35 @@ static int run_classify(sqg_ctx *ctx) {
                 { const int rc_ = classify_launch(ctx, o, n_tiles); if (rc_) return rc_; }
                 PHASE_END("k_classify");
             }
-            LAUNCH(k_tile_scan, 1, 1024, ctx->d_tileagg.p, (int32_t)n_tiles, totals, (uint64_t *)(ctx->d_counters.p + 21));
-            CK(cudaMemcpyAsync(ctx->h_counters.p, ctx->d_counters.p, 5 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-            CK(cudaMemcpyAsync(ctx->h_counters.p + 20, ctx->d_counters.p + 20, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-            if (ctx->wire_loaded) CK(cudaMemcpyAsync(ctx->h_counters.p + 28, ctx->d_counters.p + 28, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+            LAUNCH(k_tile_scan, 1, 1024, ctx->d_tileagg.p, (int32_t)n_tiles, dc->totals, &dc->end_other);
+            CK(ctx->cnt.to_host(ctx->stream, &dc->totals, &dc->end_other));
+            if (ctx->wire_loaded) CK(ctx->cnt.to_host(ctx->stream, &dc->wire_bad));
             CK(cudaStreamSynchronize(ctx->stream));
-            if (ctx->wire_loaded && *(int32_t *)(ctx->h_counters.p + 28)) FAIL(SQG_EINVAL, "wire batch is inconsistent (escape without an exception entry, or block counts that contradict the tile table)");
-            const int32_t flags = *(int32_t *)(ctx->h_counters.p + 20);
+            { const int rc_ = wire_check(ctx); if (rc_) return rc_; }
+            const int32_t flags = hc.bad_flags;
             if (flags & 1) FAIL(SQG_EINVAL, "record with ref_id outside [-1, n_ref)");
             if (flags & 2) FAIL(SQG_EUNSUPPORTED, "mapped record with ref_id -1");
             if (flags & 4) FAIL(SQG_EUNSUPPORTED, "record with more than 16 aligned blocks or a decreasing blk_off");
             if (flags & 8) FAIL(SQG_EINVAL, "batch is not sorted by (ref_id, pos)");
-            n_cand = *(int32_t *)(ctx->h_counters.p + 4);
+            n_cand = hc.n_cand;
             ctx->classify_attempts = attempt + 1;
             if (!(flags & 16)) break;
             if (attempt == 1) FAIL(SQG_ENOMEM, "coverage-gap candidate buffer overflow");
             cand_cap = n + 1;  // every record can be a candidate at worst
         }
-        const int32_t *sel = (const int32_t *)ctx->h_counters.p;
-        ctx->n_pc = sel[1]; ctx->n_dp = sel[2]; ctx->first_kept = ctx->h_counters.p[2];
-        ctx->lmax = *(const int32_t *)(ctx->h_counters.p + 3);
-        ctx->end_other = (uint64_t)ctx->h_counters.p[21];
+        ctx->n_pc = hc.totals[1]; ctx->n_dp = hc.totals[2]; ctx->first_kept = hc.first_kept; ctx->lmax = hc.lmax; ctx->end_other = hc.end_other;
         CK(ctx->d_gap.ensure((size_t)n_cand + 1)); CK(ctx->d_other.ensure((size_t)n_cand + 1));
         CK(ctx->d_pc.ensure((size_t)ctx->n_pc + 1)); CK(ctx->d_dp.ensure((size_t)ctx->n_dp + 1));
         if (n_cand > 0) {
-            LAUNCH(k_finish_gaps, blocks_for(n_cand), kThreads, b, ctx->d_tileagg.p, ctx->d_scratch32.p, ctx->d_cand_key.p, n_cand, ctx->params.read_len, (int32_t *)ctx->d_counters.p);
-            size_t tb = 0;
-            CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, ctx->d_scratch32.p, ctx->d_gap.p, ctx->d_cand_key.p, ctx->d_other.p, n_cand, 0, 32, ctx->stream));
-            ENSURE_TEMP(tb);
-            CK(cub::DeviceRadixSort::SortPairs(ctx->d_temp.p, tb, ctx->d_scratch32.p, ctx->d_gap.p, ctx->d_cand_key.p, ctx->d_other.p, n_cand, 0, 32, ctx->stream));
+            LAUNCH(k_finish_gaps, blocks_for(n_cand), kThreads, b, ctx->d_tileagg.p, ctx->d_scratch32.p, ctx->d_cand_key.p, n_cand, ctx->params.read_len, dc->totals);
+            CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceRadixSort::SortPairs(t, tb, ctx->d_scratch32.p, ctx->d_gap.p, ctx->d_cand_key.p, ctx->d_other.p, n_cand, 0, 32, ctx->stream); }));
             ctx->launches += 3;
         }
         if (ctx->n_pc + ctx->n_dp > 0) LAUNCH(k_compact_lists, (unsigned)n_tiles, kTileThreads, ctx->d_cls.p, n, ctx->d_tileagg.p, ctx->d_pc.p, ctx->d_dp.p);
-        CK(cudaMemcpyAsync(ctx->h_counters.p, ctx->d_counters.p, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(ctx->cnt.to_host(ctx->stream, &dc->totals));
         PHASE_END("classify");
         CK(cudaStreamSynchronize(ctx->stream));
-        ctx->n_gap = sel[0];
+        ctx->n_gap = hc.totals[0];
     } else {
         PHASE_END("classify");
         CK(ctx->d_gap.ensure(1)); CK(ctx->d_other.ensure(1)); CK(ctx->d_pc.ensure(1)); CK(ctx->d_dp.ensure(1));
@@ -1399,8 +1381,8 @@ static int tile_genome(sqg_ctx *ctx, std::vector<SeedNode> &seedv) {
 }
 
 // Phase 3, first pass (sq_phase3.cuh: k_cov_compact): enqueued as soon as the class bytes exist -- it does not depend on the
-// segment table, so sqg_build_nodes runs it while the host still waits for the chimeric pre-pass.  The count lands in
-// h_counters[15] once the stream has been synchronised.
+// segment table, so sqg_build_nodes runs it while the host still waits for the chimeric pre-pass.  The count lands in the
+// mirror's cov_nq once the stream has been synchronised.
 static int run_cov_compact(sqg_ctx *ctx) {
     if (ctx->cov_compacted) return SQG_OK;
     const DevBatch &b = ctx->batch;
@@ -1415,13 +1397,9 @@ static int run_cov_compact(sqg_ctx *ctx) {
         // rank offsets and running maxima of the classification tiles: scans of the per-tile counts phase 1 left (no look-back chain)
         const int64_t n_ct = (n + kTile - 1) / kTile;
         CK(ctx->d_cov_rank0.ensure(n_ct + 2)); CK(ctx->d_cov_incmax.ensure(n_ct + 2));
-        size_t tb1 = 0, tb2 = 0;
-        CK(cub::DeviceScan::ExclusiveSum(nullptr, tb1, ctx->d_cov_nq.p, ctx->d_cov_rank0.p, (int)(n_ct + 1), st));
-        CK(cub::DeviceScan::InclusiveScan(nullptr, tb2, ctx->d_cov_qmax.p, ctx->d_cov_incmax.p, MaxU64(), (int)n_ct, st));
-        CK(ctx->d_temp_cov.ensure(std::max(tb1, tb2) + 256));
         CK(cudaMemsetAsync(ctx->d_cov_nq.p + n_ct, 0, 4, st));
-        CK(cub::DeviceScan::ExclusiveSum(ctx->d_temp_cov.p, tb1, ctx->d_cov_nq.p, ctx->d_cov_rank0.p, (int)(n_ct + 1), st));
-        CK(cub::DeviceScan::InclusiveScan(ctx->d_temp_cov.p, tb2, ctx->d_cov_qmax.p, ctx->d_cov_incmax.p, MaxU64(), (int)n_ct, st));
+        CK(cub_call(ctx->d_temp_cov, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveSum(t, tb, ctx->d_cov_nq.p, ctx->d_cov_rank0.p, (int)(n_ct + 1), st); }));
+        CK(cub_call(ctx->d_temp_cov, [&](void *t, size_t &tb) { return cub::DeviceScan::InclusiveScan(t, tb, ctx->d_cov_qmax.p, ctx->d_cov_incmax.p, MaxU64(), (int)n_ct, st); }));
         ctx->launches += 4;
         int rc = phase_begin(ctx, "k_cov_compact", st);
         if (rc) return rc;
@@ -1431,8 +1409,8 @@ static int run_cov_compact(sqg_ctx *ctx) {
         CK(cudaGetLastError());
         rc = phase_end(ctx, "k_cov_compact", st);
         if (rc) return rc;
-        CK(cudaMemcpyAsync(ctx->d_counters.p + 15, ctx->d_cov_rank0.p + n_ct, sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 15, ctx->d_counters.p + 15, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(&ctx->cnt.d.p->cov_nq, ctx->d_cov_rank0.p + n_ct, sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+        CK(ctx->cnt.to_host(st, &ctx->cnt.d.p->cov_nq));
         CK(cudaEventRecord(ctx->ev_cov_done, st));
         ctx->cov_pending = true;
     } else { CK(ctx->d_qkey.ensure(1)); CK(ctx->d_qend.ensure(1)); CK(ctx->d_covtile.ensure(1)); }
@@ -1464,10 +1442,7 @@ static int count_short_other(sqg_ctx *ctx, int64_t n_short, int64_t n_unstable) 
     cub::CountingInputIterator<int64_t> cnt(0);
     cub::TransformInputIterator<int32_t, OtherCountOp, cub::CountingInputIterator<int64_t>> it(cnt, op);
     CK(ctx->d_other_off.ensure((size_t)n + 2));
-    size_t tb = 0;
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, it, ctx->d_other_off.p, (int)(n + 1), ctx->stream));
-    ENSURE_TEMP(tb);
-    CK(cub::DeviceScan::ExclusiveSum(ctx->d_temp.p, tb, it, ctx->d_other_off.p, (int)(n + 1), ctx->stream));
+    CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveSum(t, tb, it, ctx->d_other_off.p, (int)(n + 1), ctx->stream); }));
     ctx->launches += 2;
     int32_t m32 = 0;
     CK(cudaMemcpyAsync(&m32, ctx->d_other_off.p + n, 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1495,9 +1470,7 @@ static int count_short_other(sqg_ctx *ctx, int64_t n_short, int64_t n_unstable) 
         CK(cudaStreamSynchronize(ctx->stream));
     }
     LAUNCH(k_other_own, blocks_for(M), kThreads, ctx->nt, ctx->d_other_key.p, ctx->d_other_idx.p, ctx->d_other_len.p, M, ctx->d_other_own.p);
-    CK(cub::DeviceScan::InclusiveScan(nullptr, tb, ctx->d_other_own.p, ctx->d_other_own.p, MaxI32(), (int)M, ctx->stream));
-    ENSURE_TEMP(tb);
-    CK(cub::DeviceScan::InclusiveScan(ctx->d_temp.p, tb, ctx->d_other_own.p, ctx->d_other_own.p, MaxI32(), (int)M, ctx->stream));
+    CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::InclusiveScan(t, tb, ctx->d_other_own.p, ctx->d_other_own.p, MaxI32(), (int)M, ctx->stream); }));
     ctx->launches += 2;
     LAUNCH(k_other_apply, blocks_for(M), kThreads, ctx->nt, ctx->d_other_key.p, ctx->d_other_idx.p, ctx->d_other_len.p, ctx->d_other_own.p, M, cnt_other, sum_other);
     return SQG_OK;
@@ -1522,6 +1495,8 @@ static int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges) {
     int64_t slow_cap = std::max<int64_t>({(int64_t)ctx->d_slow.cap, n / 8 + 4096});
     int64_t short_cap = std::max<int64_t>({(int64_t)ctx->d_shorts.cap, n / 256 + 4096});
     CK(ctx->dc_res0.ensure(ctx->c_n_reads + 1)); CK(ctx->d_scratch32.ensure(n + 1));
+    Counters *dc = ctx->cnt.d.p;
+    const Counters &hc = *ctx->cnt.h.p;
     int64_t n_raw = 0;
     int64_t n_short = 0, n_unstable = 0;
     if (ctx->chim_upload_pending) {  // the chimeric arrays: uploaded by the pre-pass thread behind its own work
@@ -1543,17 +1518,15 @@ static int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges) {
         if (do_edges) { CK(ctx->d_ekeys.ensure(cap)); CK(ctx->d_ew.ensure(cap)); CK(ctx->d_sens.ensure(sens_cap)); CK(ctx->d_head.ensure(sens_cap)); }
         cap = do_edges ? (int64_t)std::min(ctx->d_ekeys.cap, ctx->d_ew.cap) : 0;
         sens_cap = do_edges ? (int64_t)std::min(ctx->d_sens.cap, ctx->d_head.cap) : 0;
-        // counters: [9] raw pairs | [10] sensitive concordant reads, sensitive chimeric reads (int32 each)
-        CK(cudaMemsetAsync(ctx->d_counters.p + 9, 0, 2 * sizeof(int64_t), ctx->stream));
-        unsigned long long *d_cnt = (unsigned long long *)(ctx->d_counters.p + 9);
-        int32_t *d_nsens = (int32_t *)(ctx->d_counters.p + 10);
-        PairSink sink{ctx->d_ekeys.p, ctx->d_ew.p, cap, d_cnt};
+        CK(ctx->cnt.zero(ctx->stream, &dc->n_raw, &dc->n_sens));
+        int32_t *d_nsens = dc->n_sens;
+        PairSink sink{ctx->d_ekeys.p, ctx->d_ew.p, cap, &dc->n_raw};
         if (do_depth) {
             CK(cudaMemsetAsync(ctx->d_cnt3.p, 0, (3 * (size_t)N + 4) * 4, ctx->stream));
             CK(cudaMemsetAsync(ctx->d_sum3.p, 0, (3 * (size_t)N + 4) * 4, ctx->stream));
             if (nD > 0 && ctx->shard_index == 0) LAUNCH(k_depth_disc, blocks_for(nD), kThreads, ctx->nt, ctx->d_disc.p, nD, ctx->d_cnt3.p, ctx->d_sum3.p);
         }
-        CK(cudaMemsetAsync(ctx->d_counters.p + 22, 0, 2 * sizeof(int64_t), ctx->stream));  // [22] used_init flag | [23] out hint
+        CK(ctx->cnt.zero(ctx->stream, &dc->used_init, &dc->out_hint));
         if (do_edges && ctx->c_n_blk > 0) {  // every pass trims the ORIGINAL blocks (a trimmed block can fit another segment)
             const size_t nbb = (size_t)ctx->c_n_blk * 4;
             CK(cudaMemcpyAsync(ctx->dc_ref_pos.p, ctx->dc0_ref_pos.p, nbb, cudaMemcpyDeviceToDevice, ctx->stream));
@@ -1577,14 +1550,12 @@ static int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges) {
             a.other_nonempty = do_depth ? ctx->d_cnt3.p + 3 * (size_t)N : nullptr;
             a.dtile = ctx->d_dtile.p; a.res0 = ctx->d_scratch32.p; a.sink = sink;
             a.sens = ctx->d_sens.p; a.n_sens = d_nsens; a.sens_cap = conc_sens_cap;
-            a.path_counts = (unsigned long long *)(ctx->d_counters.p + 16);
-            CK(cudaMemsetAsync(ctx->d_counters.p + 16, 0, 3 * sizeof(int64_t), ctx->stream));
+            CK(ctx->cnt.zero(ctx->stream, &dc->path_counts, &dc->n_short));
             CK(ctx->d_slow.ensure(slow_cap));
-            a.slow_list = ctx->d_slow.p; a.n_slow = (int32_t *)(ctx->d_counters.p + 18); a.slow_cap = (int32_t)std::min<int64_t>(ctx->d_slow.cap, 0x7fffffff);
-            // ReadsOther blocks of <= 3 bp: counters [27] = #short blocks, #order-dependent ones (int32 each)
+            a.path_counts = dc->path_counts;
+            a.slow_list = ctx->d_slow.p; a.n_slow = &dc->n_slow; a.slow_cap = (int32_t)std::min<int64_t>(ctx->d_slow.cap, 0x7fffffff);
             CK(ctx->d_omask.ensure((size_t)N + 2)); CK(ctx->d_shorts.ensure((size_t)short_cap));
-            a.omask = ctx->d_omask.p; a.shorts = ctx->d_shorts.p; a.n_short = (int32_t *)(ctx->d_counters.p + 27); a.short_cap = (int32_t)std::min<int64_t>(short_cap, 0x7fffffff);
-            CK(cudaMemsetAsync(ctx->d_counters.p + 27, 0, sizeof(int64_t), ctx->stream));
+            a.omask = ctx->d_omask.p; a.shorts = ctx->d_shorts.p; a.n_short = dc->n_short; a.short_cap = (int32_t)std::min<int64_t>(short_cap, 0x7fffffff);
             if (do_depth) CK(cudaMemsetAsync(ctx->d_omask.p, 0, ((size_t)N + 2) * 4, ctx->stream));
             {
                 struct { BatchDesc d; NodeTable nt; } hd;
@@ -1627,25 +1598,22 @@ static int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges) {
                 // pairs: 7 blocks (72 registers) 6.7 ms, 8 blocks 5.4 ms, 10 and 12 blocks (48 / 40 registers) 5.5 ms
                 LAUNCH(k_edges_generic<8>, 148 * 16, 128, a);
                 PHASE_END("k_edges_generic");
-                LAUNCH(k_fix_heads, 256, 128, ctx->d_scratch32.p, ctx->d_sens.p, d_nsens, conc_sens_cap, ctx->d_head.p, ctx->shard_init_hint, (int32_t *)(ctx->d_counters.p + 22));
+                LAUNCH(k_fix_heads, 256, 128, ctx->d_scratch32.p, ctx->d_sens.p, d_nsens, conc_sens_cap, ctx->d_head.p, ctx->shard_init_hint, &dc->used_init);
                 LAUNCH(k_fix_chains<false>, 256, 128, b, cd, ctx->params, ctx->nt, ctx->d_scratch32.p, n, ctx->d_sens.p, d_nsens, conc_sens_cap, ctx->d_head.p, sink);
-                if (ctx->shard_count > 1) LAUNCH(k_last_located, 1, 1, ctx->d_scratch32.p, n, (int32_t *)(ctx->d_counters.p + 23));
+                if (ctx->shard_count > 1) LAUNCH(k_last_located, 1, 1, ctx->d_scratch32.p, n, &dc->out_hint);
             }
             PHASE_END("k_assign");
         }
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 9, ctx->d_counters.p + 9, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 16, ctx->d_counters.p + 16, 3 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 22, ctx->d_counters.p + 22, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 27, ctx->d_counters.p + 27, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(ctx->cnt.to_host(ctx->stream, &dc->n_raw, &dc->out_hint));
         CK(cudaStreamSynchronize(ctx->stream));
-        n_short = do_depth && n > 0 ? ((int32_t *)(ctx->h_counters.p + 27))[0] : 0;
-        n_unstable = do_depth && n > 0 ? ((int32_t *)(ctx->h_counters.p + 27))[1] : 0;
-        ctx->shard_lead_sensitive = *(int32_t *)(ctx->h_counters.p + 22) != 0;
-        ctx->shard_out_hint = (ctx->shard_count > 1 && do_edges && n > 0) ? *(int32_t *)(ctx->h_counters.p + 23) : -1;
-        n_raw = ctx->h_counters.p[9];
-        const int32_t ns_conc = ((int32_t *)(ctx->h_counters.p + 10))[0], ns_chim = ((int32_t *)(ctx->h_counters.p + 10))[1];
+        n_short = do_depth && n > 0 ? hc.n_short[0] : 0;
+        n_unstable = do_depth && n > 0 ? hc.n_short[1] : 0;
+        ctx->shard_lead_sensitive = hc.used_init != 0;
+        ctx->shard_out_hint = (ctx->shard_count > 1 && do_edges && n > 0) ? hc.out_hint : -1;
+        n_raw = (int64_t)hc.n_raw;
+        const int32_t ns_conc = hc.n_sens[0], ns_chim = hc.n_sens[1];
         ctx->n_sensitive = (int64_t)ns_conc + ns_chim;
-        const int64_t n_slow = *(int32_t *)(ctx->h_counters.p + 18);
+        const int64_t n_slow = hc.n_slow;
         if (n_short <= short_cap && (!do_edges || (n_raw <= cap && ns_conc <= conc_sens_cap && n_slow <= slow_cap))) break;
         slow_cap = std::max(slow_cap, n_slow + 4096);
         short_cap = std::max(short_cap, n_short + 4096);
@@ -1685,6 +1653,8 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
     if (nD <= 0) FAIL(SQG_EUNSUPPORTED, "no discordant block in the chimeric reads: BuildNode_STAR is undefined there (SegmentGraph.cpp:757 on an empty vector)");
 
     PHASE_BEGIN("seed");
+    Counters *dc = ctx->cnt.d.p;
+    const Counters &hc = *ctx->cnt.h.p;
     CK(ctx->d_trigger.ensure(nG + 1));
     LAUNCH(k_triggers, blocks_for(nG), kThreads, b, ctx->d_cls.p, ctx->d_groups.p, nG, ctx->d_trigger.p);
     // ConcordRest candidates, sorted by (chr,pos)
@@ -1705,23 +1675,20 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
     int64_t n_rest = 0;
     for (int attempt = 0; attempt < 2; attempt++) {
         CK(ctx->d_rest.ensure(rest_cap)); CK(ctx->d_rest2.ensure(rest_cap)); CK(ctx->d_restkey.ensure(rest_cap)); CK(ctx->d_restkey2.ensure(rest_cap));
-        CK(cudaMemsetAsync(ctx->d_counters.p + 4, 0, sizeof(int64_t), ctx->stream));
+        CK(ctx->cnt.zero(ctx->stream, &dc->n_rest));
         if (n > 0) LAUNCH(k_rest_collect, blocks_for((n + 3) / 4), kThreads, b, ctx->d_cls.p, ctx->d_groups.p, ctx->d_disc.p, nG, ctx->params.read_len, rbins, ctx->d_reflen.p,
-                          ctx->d_rest.p, ctx->d_restkey.p, rest_cap, ctx->d_counters.p + 4);
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 4, ctx->d_counters.p + 4, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+                          ctx->d_rest.p, ctx->d_restkey.p, rest_cap, &dc->n_rest);
+        CK(ctx->cnt.to_host(ctx->stream, &dc->n_rest));
         CK(cudaStreamSynchronize(ctx->stream));
-        n_rest = ctx->h_counters.p[4];
+        n_rest = hc.n_rest;
         lap("  seed: triggers + rest collect");
         if (n_rest <= rest_cap) break;
         rest_cap = n_rest + 1024;
     }
     if (n_rest > 0) {
-        size_t tb = 0;
         int key_bits = 1;  // the owning group: the table is binned by group, not ordered inside a group
         while (key_bits < 32 && (1ll << key_bits) < (long long)nG) key_bits++;
-        CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, ctx->d_restkey.p, ctx->d_restkey2.p, ctx->d_rest.p, ctx->d_rest2.p, (int)n_rest, 0, key_bits, ctx->stream));
-        ENSURE_TEMP(tb);
-        CK(cub::DeviceRadixSort::SortPairs(ctx->d_temp.p, tb, ctx->d_restkey.p, ctx->d_restkey2.p, ctx->d_rest.p, ctx->d_rest2.p, (int)n_rest, 0, key_bits, ctx->stream));
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceRadixSort::SortPairs(t, tb, ctx->d_restkey.p, ctx->d_restkey2.p, ctx->d_rest.p, ctx->d_rest2.p, (int)n_rest, 0, key_bits, ctx->stream); }));
         ctx->launches += 4;
     }
     // the state machine, island-parallel
@@ -1767,19 +1734,16 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
     in.dense_max_r = kSeedDenseRange;
     CK(ctx->d_cutflag.ensure(nG + 1)); CK(ctx->d_isl.ensure(nG + 2));
     LAUNCH(k_island_cuts, blocks_for(nG, 64), 64, in, ctx->d_cutflag.p);
-    CK(cudaMemsetAsync(ctx->d_counters.p + 5, 0, sizeof(int64_t), ctx->stream));
+    CK(ctx->cnt.zero(ctx->stream, &dc->n_isl));
     if (g_hi - g_lo > 0) {
         cub::CountingInputIterator<int32_t> cnt(g_lo);
         IsCutOp op{ctx->d_cutflag.p};
-        size_t tb = 0;
-        CK(cub::DeviceSelect::If(nullptr, tb, cnt, ctx->d_isl.p, (int32_t *)(ctx->d_counters.p + 5), g_hi - g_lo, op, ctx->stream));
-        ENSURE_TEMP(tb);
-        CK(cub::DeviceSelect::If(ctx->d_temp.p, tb, cnt, ctx->d_isl.p, (int32_t *)(ctx->d_counters.p + 5), g_hi - g_lo, op, ctx->stream));
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceSelect::If(t, tb, cnt, ctx->d_isl.p, &dc->n_isl, g_hi - g_lo, op, ctx->stream); }));
         ctx->launches += 2;
     }
-    CK(cudaMemcpyAsync(ctx->h_counters.p + 5, ctx->d_counters.p + 5, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx->cnt.to_host(ctx->stream, &dc->n_isl));
     CK(cudaStreamSynchronize(ctx->stream));
-    const int32_t n_isl = *(int32_t *)(ctx->h_counters.p + 5);
+    const int32_t n_isl = hc.n_isl;
     lap("  seed: island cuts");
     CK(ctx->d_cap_ops.ensure(2 * (size_t)n_isl + 4)); CK(ctx->d_cap_mar.ensure(n_isl + 2)); CK(ctx->d_off_ops.ensure(n_isl + 2)); CK(ctx->d_off_mar.ensure(n_isl + 2));
     CK(ctx->d_isl_nout.ensure(n_isl + 1)); CK(ctx->d_isl_gdone.ensure(n_isl + 1));
@@ -1787,53 +1751,41 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
     CK(cudaMemsetAsync(ctx->d_isl_nout.p, 0, (n_isl + 1) * 4, ctx->stream));
     CK(ctx->d_span.ensure(n_isl + 2)); CK(ctx->d_heavy.ensure(n_isl + 2)); CK(ctx->d_light.ensure(n_isl + 2));
     LAUNCH(k_island_caps, blocks_for(n_isl, 64), 64, in, ctx->d_isl.p, n_isl, ctx->d_cap_ops.p, ctx->d_cap_mar.p, ctx->d_span.p);
-    {
-        size_t tb = 0;
-        CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, ctx->d_cap_ops.p, ctx->d_off_ops.p, n_isl + 1, ctx->stream));
-        ENSURE_TEMP(tb);
-        CK(cub::DeviceScan::ExclusiveSum(ctx->d_temp.p, tb, ctx->d_cap_ops.p, ctx->d_off_ops.p, n_isl + 1, ctx->stream));
-        CK(cub::DeviceScan::ExclusiveSum(ctx->d_temp.p, tb, ctx->d_cap_mar.p, ctx->d_off_mar.p, n_isl + 1, ctx->stream));
-        ctx->launches += 4;
-    }
+    CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveSum(t, tb, ctx->d_cap_ops.p, ctx->d_off_ops.p, n_isl + 1, ctx->stream); }));
+    CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveSum(t, tb, ctx->d_cap_mar.p, ctx->d_off_mar.p, n_isl + 1, ctx->stream); }));
+    ctx->launches += 4;
     int64_t tot[2];
     CK(cudaMemcpyAsync(&tot[0], ctx->d_off_ops.p + n_isl, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(&tot[1], ctx->d_off_mar.p + n_isl, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     lap("  seed: island caps + offsets");
     CK(ctx->d_ops.ensure(tot[0] + 1)); CK(ctx->d_margin.ensure(tot[1] + 1));
-    int32_t *d_err = (int32_t *)(ctx->d_counters.p + 7), *d_nprefix = (int32_t *)(ctx->d_counters.p + 6);
-    CK(cudaMemsetAsync(ctx->d_counters.p + 6, 0, 2 * sizeof(int64_t), ctx->stream));
-    CK(cudaMemsetAsync(ctx->d_counters.p + 29, 0, sizeof(int64_t), ctx->stream));
-    in.win_count = (unsigned long long *)(ctx->d_counters.p + 29);
+    int32_t *d_err = &dc->seed_err, *d_nprefix = &dc->n_prefix;
+    CK(ctx->cnt.zero(ctx->stream, &dc->n_prefix, &dc->win_count));
+    in.win_count = &dc->win_count;
     // (a shard that follows one with an emitted segment starts with an inherited last segment: no sequential prefix)
     if (!(ctx->shard_index > 0 && ctx->shard_prior_emission) && n_isl > 0)
         LAUNCH(k_seed_prefix, 1, kSeedBlock, in, ctx->d_isl.p, n_isl, ctx->d_off_ops.p, ctx->d_off_mar.p, ctx->d_ops.p, ctx->d_margin.p,
                ctx->d_isl_nout.p, ctx->d_isl_gdone.p, d_err, d_nprefix);
-    CK(cudaMemsetAsync(ctx->d_counters.p + 13, 0, sizeof(int64_t), ctx->stream));
+    CK(ctx->cnt.zero(ctx->stream, &dc->n_heavy_light));
     if (n_isl > 0) {
         cub::CountingInputIterator<int32_t> cnt(0);
-        size_t tb = 0;
         IsHeavyOp oh{ctx->d_span.p, d_nprefix, true}, ol{ctx->d_span.p, d_nprefix, false};
-        int32_t *d_nh = (int32_t *)(ctx->d_counters.p + 13);
-        CK(cub::DeviceSelect::If(nullptr, tb, cnt, ctx->d_heavy.p, d_nh, n_isl, oh, ctx->stream));
-        ENSURE_TEMP(tb);
-        CK(cub::DeviceSelect::If(ctx->d_temp.p, tb, cnt, ctx->d_heavy.p, d_nh, n_isl, oh, ctx->stream));
-        CK(cub::DeviceSelect::If(ctx->d_temp.p, tb, cnt, ctx->d_light.p, d_nh + 1, n_isl, ol, ctx->stream));
+        int32_t *d_nh = dc->n_heavy_light;
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceSelect::If(t, tb, cnt, ctx->d_heavy.p, d_nh, n_isl, oh, ctx->stream); }));
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceSelect::If(t, tb, cnt, ctx->d_light.p, d_nh + 1, n_isl, ol, ctx->stream); }));
         ctx->launches += 3;
     }
-    CK(cudaMemcpyAsync(ctx->h_counters.p + 13, ctx->d_counters.p + 13, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx->cnt.to_host(ctx->stream, &dc->n_heavy_light));
     CK(cudaStreamSynchronize(ctx->stream));
-    const int32_t n_heavy = ((int32_t *)(ctx->h_counters.p + 13))[0], n_light = ((int32_t *)(ctx->h_counters.p + 13))[1];
+    const int32_t n_heavy = hc.n_heavy_light[0], n_light = hc.n_heavy_light[1];
     ctx->n_heavy = n_heavy;
     lap("  seed: prefix + heavy/light split");
     if (n_heavy > 1) {  // longest islands first: the kernel's critical path is its largest island
         // d_cap_ops is free again after the offset scans: sort scratch [keys | keys2]
         int32_t *k1 = ctx->d_cap_ops.p, *k2 = ctx->d_cap_ops.p + n_heavy;
         LAUNCH(k_gather_i32, blocks_for(n_heavy), kThreads, ctx->d_span.p, ctx->d_heavy.p, n_heavy, k1);
-        size_t tb = 0;
-        CK(cub::DeviceRadixSort::SortPairsDescending(nullptr, tb, k1, k2, ctx->d_heavy.p, ctx->d_light.p + n_light, n_heavy, 0, 32, ctx->stream));
-        ENSURE_TEMP(tb);
-        CK(cub::DeviceRadixSort::SortPairsDescending(ctx->d_temp.p, tb, k1, k2, ctx->d_heavy.p, ctx->d_light.p + n_light, n_heavy, 0, 32, ctx->stream));
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceRadixSort::SortPairsDescending(t, tb, k1, k2, ctx->d_heavy.p, ctx->d_light.p + n_light, n_heavy, 0, 32, ctx->stream); }));
         CK(cudaMemcpyAsync(ctx->d_heavy.p, ctx->d_light.p + n_light, n_heavy * 4, cudaMemcpyDeviceToDevice, ctx->stream));
         ctx->launches += 2;
     }
@@ -1859,17 +1811,15 @@ static int seed_stage(sqg_ctx *ctx, HostLap &lap) {
     // this batch's op lists in island order: compacted on the device (the islands' scratch is sized for the worst case, two ops
     // per margin -- copying that capacity cost more than the whole tiling stage), then one small copy
     CK(ctx->d_ops_dense.ensure((size_t)(tot[0] > 0 ? tot[0] : 1)));
-    LAUNCH(k_ops_dense, 1, 1024, ctx->d_isl.p, n_isl, g_hi, ctx->d_isl_nout.p, ctx->d_isl_gdone.p, ctx->d_off_ops.p, ctx->d_ops.p, ctx->d_ops_dense.p, ctx->d_counters.p + 24);
-    CK(cudaMemcpyAsync(ctx->h_counters.p + 24, ctx->d_counters.p + 24, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->h_counters.p + 6, ctx->d_counters.p + 6, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->h_counters.p + 29, ctx->d_counters.p + 29, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    LAUNCH(k_ops_dense, 1, 1024, ctx->d_isl.p, n_isl, g_hi, ctx->d_isl_nout.p, ctx->d_isl_gdone.p, ctx->d_off_ops.p, ctx->d_ops.p, ctx->d_ops_dense.p, dc->ops_dense);
+    CK(ctx->cnt.to_host(ctx->stream, &dc->ops_dense, &dc->win_count));
     std::vector<int64_t> trig_last(1, n);
     if (nG > 0) CK(cudaMemcpyAsync(trig_last.data(), ctx->d_trigger.p + (nG - 1), sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    const int32_t serr = *(int32_t *)(ctx->h_counters.p + 7);
+    const int32_t serr = hc.seed_err;
     if (serr) FAIL(SQG_ENOMEM, serr == 1 ? "seed machine: margin scratch overflow" : "seed machine: output overflow");
-    const int64_t n_ops_dense = ctx->h_counters.p[24];
-    const int32_t g_done = (int32_t)ctx->h_counters.p[25];  // (== nG exactly when every group was triggered by this batch)
+    const int64_t n_ops_dense = hc.ops_dense[0];
+    const int32_t g_done = (int32_t)hc.ops_dense[1];  // (== nG exactly when every group was triggered by this batch)
     CK(ctx->h_ops.ensure((size_t)n_ops_dense + 1));
     if (n_ops_dense > 0) {
         CK(cudaMemcpyAsync(ctx->h_ops.p, ctx->d_ops_dense.p, (size_t)n_ops_dense * sizeof(SeedOp), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2004,22 +1954,17 @@ static int plan_resident(sqg_ctx *ctx, int32_t n_shards, int64_t *cuts, int32_t 
         CK(ctx->d_plan_reach.ensure((size_t)n)); CK(ctx->d_plan_keep.ensure((size_t)n)); CK(ctx->d_plan_upd.ensure((size_t)n));
         CK(ctx->d_plan_cand.ensure((size_t)n)); CK(ctx->d_plan_sel.ensure((size_t)n));
         LAUNCH(k_plan_prep, blocks_for(n), kThreads, b, ctx->d_cls.p, ctx->d_plan_reach.p, ctx->d_plan_keep.p, ctx->d_plan_upd.p);
-        size_t tb1 = 0, tb2 = 0, tb3 = 0;
-        int32_t *d_nsel = (int32_t *)(ctx->d_counters.p + 5);
-        CK(cub::DeviceScan::ExclusiveScan(nullptr, tb1, ctx->d_plan_reach.p, ctx->d_plan_reach.p, MaxU64(), (uint64_t)0, (int)n, ctx->stream));
-        CK(cub::DeviceScan::ExclusiveScan(nullptr, tb2, ctx->d_plan_keep.p, ctx->d_plan_keep.p, MaxI32(), (int32_t)-1, (int)n, ctx->stream));
-        CK(cub::DeviceSelect::If(nullptr, tb3, ctx->d_plan_cand.p, ctx->d_plan_sel.p, d_nsel, (int)n, PlanIsCand(), ctx->stream));
-        ENSURE_TEMP(std::max({tb1, tb2, tb3}));
-        CK(cub::DeviceScan::ExclusiveScan(ctx->d_temp.p, tb1, ctx->d_plan_reach.p, ctx->d_plan_reach.p, MaxU64(), (uint64_t)0, (int)n, ctx->stream));
-        CK(cub::DeviceScan::ExclusiveScan(ctx->d_temp.p, tb2, ctx->d_plan_keep.p, ctx->d_plan_keep.p, MaxI32(), (int32_t)-1, (int)n, ctx->stream));
-        CK(cub::DeviceScan::ExclusiveScan(ctx->d_temp.p, tb2, ctx->d_plan_upd.p, ctx->d_plan_upd.p, MaxI32(), (int32_t)-1, (int)n, ctx->stream));
+        int32_t *d_nsel = &ctx->cnt.d.p->n_plan_cand;
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveScan(t, tb, ctx->d_plan_reach.p, ctx->d_plan_reach.p, MaxU64(), (uint64_t)0, (int)n, ctx->stream); }));
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveScan(t, tb, ctx->d_plan_keep.p, ctx->d_plan_keep.p, MaxI32(), (int32_t)-1, (int)n, ctx->stream); }));
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveScan(t, tb, ctx->d_plan_upd.p, ctx->d_plan_upd.p, MaxI32(), (int32_t)-1, (int)n, ctx->stream); }));
         LAUNCH(k_plan_cands, blocks_for(n), kThreads, b, ctx->params, ctx->d_cls.p, ctx->d_plan_reach.p, ctx->d_plan_keep.p, ctx->d_plan_upd.p,
                ctx->d_groups.p, ctx->d_disc.p, ctx->pre_nG, ctx->d_plan_cand.p);
-        CK(cub::DeviceSelect::If(ctx->d_temp.p, tb3, ctx->d_plan_cand.p, ctx->d_plan_sel.p, d_nsel, (int)n, PlanIsCand(), ctx->stream));
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceSelect::If(t, tb, ctx->d_plan_cand.p, ctx->d_plan_sel.p, d_nsel, (int)n, PlanIsCand(), ctx->stream); }));
         ctx->launches += 4;
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 5, ctx->d_counters.p + 5, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(ctx->cnt.to_host(ctx->stream, d_nsel));
         CK(cudaStreamSynchronize(ctx->stream));
-        n_cand = *(const int32_t *)(ctx->h_counters.p + 5);
+        n_cand = ctx->cnt.h.p->n_plan_cand;
         CK(ctx->h_plan_sel.ensure((size_t)n_cand + 1));
         if (n_cand > 0) CK(cudaMemcpyAsync(ctx->h_plan_sel.p, ctx->d_plan_sel.p, (size_t)n_cand * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
     }
@@ -2034,7 +1979,6 @@ extern "C" int sqg_plan_shards_resident(sqg_ctx *ctx, int32_t n_shards, int64_t 
     if (!ctx->have_batch || !ctx->have_chim) FAIL(SQG_ESTATE, "load the concordant batch and the chimeric reads first");
     if (ctx->batch_restricted) FAIL(SQG_ESTATE, "sqg_plan_shards_resident: the batch is one shard's range already (sqg_keep_records); plan on the whole stream");
     CK(cudaSetDevice(ctx->device));
-    CK(ctx->d_counters.ensure(32)); CK(ctx->h_counters.ensure(32));
     const int rc = plan_resident(ctx, n_shards, cuts, n_planned);
     // the scratch is as large as the batch and only needed once per load
     ctx->d_plan_reach.release(); ctx->d_plan_keep.release(); ctx->d_plan_upd.release(); ctx->d_plan_cand.release(); ctx->d_plan_sel.release();
@@ -2068,10 +2012,9 @@ extern "C" int sqg_keep_records(sqg_ctx *ctx, int64_t lo, int64_t hi) {
         e = cudaMemcpyAsync(tmp.p, p + (size_t)first * elem, bytes, cudaMemcpyDeviceToDevice, st);
         if (e == cudaSuccess) e = cudaMemcpyAsync(p, tmp.p, bytes, cudaMemcpyDeviceToDevice, st);
     };
-    move(ctx->o_ref_id.p, 4, lo, nr); move(ctx->o_pos.p, 4, lo, nr); move(ctx->o_mate_ref_id.p, 4, lo, nr); move(ctx->o_mate_pos.p, 4, lo, nr);
-    move(ctx->o_end_pos.p, 4, lo, nr); move(ctx->o_flag.p, 2, lo, nr); move(ctx->o_total_len.p, 2, lo, nr); move(ctx->o_lowphred_run.p, 2, lo, nr);
-    move(ctx->o_mapq.p, 1, lo, nr); move(ctx->o_aux.p, 1, lo, nr);
-    move(ctx->o_blk_ref_pos.p, 4, b0, nb); move(ctx->o_blk_match_ref.p, 4, b0, nb); move(ctx->o_blk_read_pos.p, 2, b0, nb); move(ctx->o_blk_match_read.p, 2, b0, nb);
+#define X(T, name, ext) if (ext != BX_OFF) move(ctx->o_##name.p, sizeof(T), ext == BX_REC ? lo : b0, ext == BX_REC ? nr : nb);
+    SQ_BATCH_ARRAYS(X)  // (blk_off is rebased below)
+#undef X
     CK(e);
     CK(cudaMemcpyAsync(tmp.p, ctx->o_blk_off.p + lo, (size_t)(nr + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
     LAUNCH(k_keep_offsets, blocks_for(nr + 1), kThreads, ctx->o_blk_off.p, (const uint32_t *)tmp.p, nr + 1, (uint32_t)b0);
@@ -2087,27 +2030,19 @@ static int reduce_edges(sqg_ctx *ctx, int64_t n_raw, const int32_t *d_weights_in
     ctx->n_unique_edges = 0;
     CK(ctx->d_ekeys2.ensure(n_raw + 1)); CK(ctx->d_ukeys.ensure(n_raw + 1)); CK(ctx->d_ecount.ensure(n_raw + 1));
     if (n_raw > 0) {
-        size_t tb = 0;
+        int32_t *d_nu = &ctx->cnt.d.p->n_unique;
         if (!d_weights_in) {
-            CK(cub::DeviceRadixSort::SortKeys(nullptr, tb, ctx->d_ekeys.p, ctx->d_ekeys2.p, (int)n_raw, 0, 64, ctx->stream));
-            ENSURE_TEMP(tb);
-            CK(cub::DeviceRadixSort::SortKeys(ctx->d_temp.p, tb, ctx->d_ekeys.p, ctx->d_ekeys2.p, (int)n_raw, 0, 64, ctx->stream));
-            CK(cub::DeviceRunLengthEncode::Encode(nullptr, tb, ctx->d_ekeys2.p, ctx->d_ukeys.p, ctx->d_ecount.p, (int32_t *)(ctx->d_counters.p + 8), (int)n_raw, ctx->stream));
-            ENSURE_TEMP(tb);
-            CK(cub::DeviceRunLengthEncode::Encode(ctx->d_temp.p, tb, ctx->d_ekeys2.p, ctx->d_ukeys.p, ctx->d_ecount.p, (int32_t *)(ctx->d_counters.p + 8), (int)n_raw, ctx->stream));
+            CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceRadixSort::SortKeys(t, tb, ctx->d_ekeys.p, ctx->d_ekeys2.p, (int)n_raw, 0, 64, ctx->stream); }));
+            CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceRunLengthEncode::Encode(t, tb, ctx->d_ekeys2.p, ctx->d_ukeys.p, ctx->d_ecount.p, d_nu, (int)n_raw, ctx->stream); }));
         } else {
             CK(ctx->d_sens.ensure(n_raw + 1));
-            CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, ctx->d_ekeys.p, ctx->d_ekeys2.p, d_weights_in, ctx->d_sens.p, (int)n_raw, 0, 64, ctx->stream));
-            ENSURE_TEMP(tb);
-            CK(cub::DeviceRadixSort::SortPairs(ctx->d_temp.p, tb, ctx->d_ekeys.p, ctx->d_ekeys2.p, d_weights_in, ctx->d_sens.p, (int)n_raw, 0, 64, ctx->stream));
-            CK(cub::DeviceReduce::ReduceByKey(nullptr, tb, ctx->d_ekeys2.p, ctx->d_ukeys.p, ctx->d_sens.p, ctx->d_ecount.p, (int32_t *)(ctx->d_counters.p + 8), cub::Sum(), (int)n_raw, ctx->stream));
-            ENSURE_TEMP(tb);
-            CK(cub::DeviceReduce::ReduceByKey(ctx->d_temp.p, tb, ctx->d_ekeys2.p, ctx->d_ukeys.p, ctx->d_sens.p, ctx->d_ecount.p, (int32_t *)(ctx->d_counters.p + 8), cub::Sum(), (int)n_raw, ctx->stream));
+            CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceRadixSort::SortPairs(t, tb, ctx->d_ekeys.p, ctx->d_ekeys2.p, d_weights_in, ctx->d_sens.p, (int)n_raw, 0, 64, ctx->stream); }));
+            CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceReduce::ReduceByKey(t, tb, ctx->d_ekeys2.p, ctx->d_ukeys.p, ctx->d_sens.p, ctx->d_ecount.p, d_nu, cub::Sum(), (int)n_raw, ctx->stream); }));
         }
         ctx->launches += 5;
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 8, ctx->d_counters.p + 8, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(ctx->cnt.to_host(ctx->stream, d_nu));
         CK(cudaStreamSynchronize(ctx->stream));
-        ctx->n_unique_edges = *(int32_t *)(ctx->h_counters.p + 8);
+        ctx->n_unique_edges = ctx->cnt.h.p->n_unique;
     }
     ctx->have_edge_table = true;
     return SQG_OK;
@@ -2153,12 +2088,13 @@ extern "C" int sqg_build_edges(sqg_ctx *ctx, int32_t **ind1, int32_t **ind2, uin
         int64_t cap = std::max<int64_t>((int64_t)ctx->d_chimdiff.cap / 5, 4096);
         for (int attempt = 0; attempt < 2; attempt++) {
             CK(ctx->d_chimdiff.ensure((size_t)cap * 5));
-            CK(cudaMemsetAsync(ctx->d_counters.p + 26, 0, sizeof(int64_t), ctx->stream));
+            int32_t *d_nd = &ctx->cnt.d.p->n_chim_diff;
+            CK(ctx->cnt.zero(ctx->stream, d_nd));
             LAUNCH(k_chim_diff, blocks_for(nb), kThreads, ctx->dc0_ref_pos.p, ctx->dc0_read_pos.p, ctx->dc0_match_ref.p, ctx->dc0_match_read.p,
-                   ctx->dc_ref_pos.p, ctx->dc_read_pos.p, ctx->dc_match_ref.p, ctx->dc_match_read.p, nb, ctx->d_chimdiff.p, (int32_t)std::min<int64_t>(cap, 0x7fffffff), (int32_t *)(ctx->d_counters.p + 26));
-            CK(cudaMemcpyAsync(ctx->h_counters.p + 26, ctx->d_counters.p + 26, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+                   ctx->dc_ref_pos.p, ctx->dc_read_pos.p, ctx->dc_match_ref.p, ctx->dc_match_read.p, nb, ctx->d_chimdiff.p, (int32_t)std::min<int64_t>(cap, 0x7fffffff), d_nd);
+            CK(ctx->cnt.to_host(ctx->stream, d_nd));
             CK(cudaStreamSynchronize(ctx->stream));
-            const int64_t nd = *(int32_t *)(ctx->h_counters.p + 26);
+            const int64_t nd = ctx->cnt.h.p->n_chim_diff;
             if (nd <= cap) {
                 CK(ctx->h_chimdiff.ensure((size_t)nd * 5 + 1));
                 if (nd > 0) {
@@ -2220,7 +2156,7 @@ static int cov_prepare(sqg_ctx *ctx, const int32_t *bp_chr, const int32_t *bp_po
     CK(cudaStreamSynchronize(ctx->stream_cov));
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->cov_K = K;
-    ctx->cov_nq = n > 0 ? ctx->h_counters.p[15] : 0;
+    ctx->cov_nq = n > 0 ? ctx->cnt.h.p->cov_nq : 0;
     return SQG_OK;
 }
 
@@ -2236,28 +2172,25 @@ static int cov_chain(sqg_ctx *ctx, int64_t k_begin, int64_t k_end) {  // resolve
     LAUNCH(k_cov_r0_tiles, blocks_for(K), kThreads, ctx->d_qkey.p, ctx->d_covtile.p, (int32_t)(n > 0 ? n_tiles : 0), nq, bpchr, bppos, K, ctx->params.concord_dist_pos, bpkey, r0, t);
     {   // t[k] = max(r0[k], t[k-1]+1) whenever the qualifying record right after t[k-1] passes breakpoint k (the common case):
         // a max-plus prefix scan, verified in parallel; the literal one-step-per-record chain runs only if a candidate fails
-        size_t tb = 0;
-        CK(cub::DeviceScan::InclusiveScan(nullptr, tb, t, t, MaxI64(), (int)K, ctx->stream));
-        ENSURE_TEMP(tb);
-        CK(cub::DeviceScan::InclusiveScan(ctx->d_temp.p, tb, t, t, MaxI64(), (int)K, ctx->stream));
+        Counters *dc = ctx->cnt.d.p;
+        const Counters &hc = *ctx->cnt.h.p;
+        CK(cub_call(ctx->d_temp, [&](void *tmp, size_t &tb) { return cub::DeviceScan::InclusiveScan(tmp, tb, t, t, MaxI64(), (int)K, ctx->stream); }));
         ctx->launches += 2;
-        CK(cudaMemsetAsync(ctx->d_counters.p + 12, 0, sizeof(int64_t), ctx->stream));
-        LAUNCH(k_cov_verify, blocks_for(K), kThreads, ctx->d_qkey.p, nq, bpchr, bppos, K, ctx->params.concord_dist_pos, r0, t, (int32_t *)(ctx->d_counters.p + 12));
-        CK(cudaMemcpyAsync(ctx->h_counters.p + 12, ctx->d_counters.p + 12, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(ctx->cnt.zero(ctx->stream, &dc->cov_fail));
+        LAUNCH(k_cov_verify, blocks_for(K), kThreads, ctx->d_qkey.p, nq, bpchr, bppos, K, ctx->params.concord_dist_pos, r0, t, &dc->cov_fail);
+        CK(ctx->cnt.to_host(ctx->stream, &dc->cov_fail));
         CK(cudaStreamSynchronize(ctx->stream));
-        ctx->cov_chain_fallback = *(int32_t *)(ctx->h_counters.p + 12) != 0;
+        ctx->cov_chain_fallback = hc.cov_fail != 0;
         if (ctx->cov_chain_fallback) {
             // literal chain, chunked at large jumps of r0 (one warp per chunk), validated; whole-list replay as a last resort
             cub::CountingInputIterator<int32_t> cnt(0);
             IsChainCutOp cop{r0, t};
             CK(ctx->d_chunks.ensure(K + 1));
             int32_t *chunks = ctx->d_chunks.p;
-            CK(cub::DeviceSelect::If(nullptr, tb, cnt, chunks, (int32_t *)(ctx->d_counters.p + 14), (int)K, cop, ctx->stream));
-            ENSURE_TEMP(tb);
-            CK(cub::DeviceSelect::If(ctx->d_temp.p, tb, cnt, chunks, (int32_t *)(ctx->d_counters.p + 14), (int)K, cop, ctx->stream));
-            CK(cudaMemcpyAsync(ctx->h_counters.p + 14, ctx->d_counters.p + 14, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cub_call(ctx->d_temp, [&](void *tmp, size_t &tb) { return cub::DeviceSelect::If(tmp, tb, cnt, chunks, &dc->n_chunks, (int)K, cop, ctx->stream); }));
+            CK(ctx->cnt.to_host(ctx->stream, &dc->n_chunks));
             CK(cudaStreamSynchronize(ctx->stream));
-            const int32_t n_chunks = *(int32_t *)(ctx->h_counters.p + 14);
+            const int32_t n_chunks = hc.n_chunks;
             ctx->launches += 2;
             CK(ctx->d_chain_used.ensure(2 * (size_t)n_chunks + 2));
             int64_t *used = ctx->d_chain_used.p, *need = ctx->d_chain_used.p + n_chunks + 1;
@@ -2267,11 +2200,11 @@ static int cov_chain(sqg_ctx *ctx, int64_t k_begin, int64_t k_end) {  // resolve
             ctx->cov_chain_chunks = n_chunks;
             bool settled = false;
             for (int round = 0; round < 16 && !settled; round++) {
-                CK(cudaMemsetAsync(ctx->d_counters.p + 12, 0, sizeof(int64_t), ctx->stream));
-                LAUNCH(k_cov_chain_check, blocks_for(n_chunks), kThreads, chunks, n_chunks, r0, t, used, need, (int32_t *)(ctx->d_counters.p + 12));
-                CK(cudaMemcpyAsync(ctx->h_counters.p + 12, ctx->d_counters.p + 12, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+                CK(ctx->cnt.zero(ctx->stream, &dc->cov_redo));
+                LAUNCH(k_cov_chain_check, blocks_for(n_chunks), kThreads, chunks, n_chunks, r0, t, used, need, &dc->cov_redo);
+                CK(ctx->cnt.to_host(ctx->stream, &dc->cov_redo));
                 CK(cudaStreamSynchronize(ctx->stream));
-                if (*(int32_t *)(ctx->h_counters.p + 12) == 0) { settled = true; break; }
+                if (hc.cov_redo == 0) { settled = true; break; }
                 LAUNCH(k_cov_chain, blocks_for((int64_t)n_chunks * 32, 128), 128, ctx->d_qkey.p, nq, bpchr, bppos, K, ctx->params.concord_dist_pos, r0, t, chunks, n_chunks,
                        used, (const int64_t *)need);
             }
@@ -2560,9 +2493,7 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
     // with no qualities anywhere in the file the host decoder synthesises them ('I' everywhere, decode_alignment), which only
     // matters when the threshold lies above 'I': then the run is the read length of the CIGAR
     const bool keep_lseq = thr > 'I';
-    CK(ctx->bam_small.ensure(BS_N)); CK(ctx->bam_hsmall.ensure(BS_N));
-    CK(ctx->d_counters.ensure(32)); CK(ctx->h_counters.ensure(32));  // sqg_download_concordant reads the wire-consistency slot
-    CK(cudaMemsetAsync(ctx->d_counters.p + 28, 0, sizeof(int64_t), st));
+    CK(ctx->bam_small.ensure(BS_N)); CK(ctx->bam_hsmall.ensure(BS_N)); CK(ctx->cnt.ensure());  // (sqg_stat: as after a wire load)
     for (int i = 0; i < 2; i++) CK(ctx->bam_stage[i].ensure(kBamStage));
     for (const char *nm : {"bam_h2d", "bam_inflate", "bam_records", "bam_decode"}) { ctx->acc_ms[nm] = 0.f; PhaseTimer &t = ctx->timers[nm]; if (!t.a) { CK(cudaEventCreate(&t.a)); CK(cudaEventCreate(&t.b)); } t.done = false; }
     const int64_t zero_small[BS_N] = {0, 0, 0, -1, 0, 0};  // BS_ERRKEY: ~0 as unsigned, the neutral element of atomicMin
@@ -2641,10 +2572,7 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
             LAUNCH_ON(st, k_bam_rewalk, blocks_for(S, 128), 128, bw, ctx->bam_start.p, ctx->bam_exit.p, ctx->bam_cnt.p, ctx->bam_bad.p, ctx->bam_newstart.p, ctx->bam_redo.p);
         }
         CK(cudaMemsetAsync(ctx->bam_cnt.p + S, 0, 4, st));
-        size_t tb = 0;
-        CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, ctx->bam_cnt.p, ctx->bam_base.p, (int)(S + 1), st));
-        { const int rc_ = ensure_temp(ctx, tb); if (rc_) return rc_; }
-        CK(cub::DeviceScan::ExclusiveSum(ctx->d_temp.p, tb, ctx->bam_cnt.p, ctx->bam_base.p, (int)(S + 1), st));
+        CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::ExclusiveSum(t, tb, ctx->bam_cnt.p, ctx->bam_base.p, (int)(S + 1), st); }));
         int64_t nrec_w = 0, tail = 0;
         uint32_t nrec32 = 0;
         CK(cudaMemcpyAsync(&nrec32, ctx->bam_base.p + S, 4, cudaMemcpyDeviceToHost, st));
@@ -2662,9 +2590,9 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
         // -- decode into the resident batch (capacity grows geometrically and keeps what earlier windows wrote)
         CK(cudaEventRecord(ctx->timers["bam_decode"].a, st));
         const size_t need = (size_t)(R + nrec_w) + 1, used = (size_t)R;
-        CK(ctx->o_ref_id.grow(need, used, st)); CK(ctx->o_pos.grow(need, used, st)); CK(ctx->o_mate_ref_id.grow(need, used, st)); CK(ctx->o_mate_pos.grow(need, used, st));
-        CK(ctx->o_end_pos.grow(need, used, st)); CK(ctx->o_flag.grow(need, used, st)); CK(ctx->o_total_len.grow(need, used, st)); CK(ctx->o_lowphred_run.grow(need, used, st));
-        CK(ctx->o_mapq.grow(need, used, st)); CK(ctx->o_aux.grow(need, used, st)); CK(ctx->o_blk_off.grow(need + 1, used + 1, st));
+#define X(T, name, ext) if (ext != BX_BLK) CK(ctx->o_##name.grow(need + (ext == BX_OFF), used + (ext == BX_OFF), st));
+        SQ_BATCH_ARRAYS(X)
+#undef X
         if (keep_lseq) CK(ctx->bam_lseq.grow(need, used, st));
         if (R == 0) CK(cudaMemsetAsync(ctx->o_blk_off.p, 0, 4, st));
         CK(ctx->bam_nblk.ensure((size_t)nrec_w + 1)); CK(ctx->bam_incl.ensure((size_t)nrec_w + 1));
@@ -2673,18 +2601,16 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
         uint64_t nblk_w = 0;
         if (nrec_w > 0) {
             LAUNCH_ON(st, k_bam_decode, blocks_for(nrec_w), kThreads, dwin, ctx->bam_recoff.p, nrec_w, R, prm, ns, bo, ctx->bam_nblk.p, ctx->bam_small.p);
-            tb = 0;
-            CK(cub::DeviceScan::InclusiveSum(nullptr, tb, ctx->bam_nblk.p, ctx->bam_incl.p, (int)nrec_w, st));
-            { const int rc_ = ensure_temp(ctx, tb); if (rc_) return rc_; }
-            CK(cub::DeviceScan::InclusiveSum(ctx->d_temp.p, tb, ctx->bam_nblk.p, ctx->bam_incl.p, (int)nrec_w, st));
+            CK(cub_call(ctx->d_temp, [&](void *t, size_t &tb) { return cub::DeviceScan::InclusiveSum(t, tb, ctx->bam_nblk.p, ctx->bam_incl.p, (int)nrec_w, st); }));
             CK(cudaMemcpyAsync(&nblk_w, ctx->bam_incl.p + (nrec_w - 1), 8, cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
         }
         if (B + nblk_w > 0xFFFFFFFFull) { fatal = SQG_EUNSUPPORTED; fatal_msg = "more than 2^32 - 1 aligned blocks in one batch: shard the stream"; }
         else if (nrec_w > 0) {
             const size_t bneed = (size_t)(B + nblk_w) + 1;
-            CK(ctx->o_blk_ref_pos.grow(bneed, (size_t)B, st)); CK(ctx->o_blk_match_ref.grow(bneed, (size_t)B, st));
-            CK(ctx->o_blk_read_pos.grow(bneed, (size_t)B, st)); CK(ctx->o_blk_match_read.grow(bneed, (size_t)B, st));
+#define X(T, name, ext) if (ext == BX_BLK) CK(ctx->o_##name.grow(bneed, (size_t)B, st));
+            SQ_BATCH_ARRAYS(X)
+#undef X
             bo.blk_ref_pos = ctx->o_blk_ref_pos.p; bo.blk_match_ref = ctx->o_blk_match_ref.p; bo.blk_read_pos = ctx->o_blk_read_pos.p; bo.blk_match_read = ctx->o_blk_match_read.p;
             LAUNCH_ON(st, k_bam_blocks, blocks_for(nrec_w), kThreads, dwin, ctx->bam_recoff.p, nrec_w, R, B, ctx->bam_incl.p, ctx->bam_nblk.p, bo);
         }
@@ -2710,14 +2636,11 @@ static int bam_load(sqg_ctx *ctx, const char *path, const sqg_bam_decode *opt, i
         FAIL(SQG_EUNSUPPORTED, sqh::packer_refusal(key >> 33, (int)(key >> 32 & 1) + 1, (uint32_t)key));
     }
     if (fatal) FAIL(fatal, fatal_msg);
-    if (R == 0) {  // an empty batch still has its blk_off[0]
-        CK(ctx->o_blk_off.grow(1, 0, st));
-        CK(cudaMemsetAsync(ctx->o_blk_off.p, 0, 4, st));
-    }
     if (keep_lseq && R > 0 && ctx->bam_hsmall.p[BS_SEQ] == 0) LAUNCH_ON(st, k_bam_null_qual, blocks_for(R), kThreads, ctx->o_lowphred_run.p, ctx->bam_lseq.p, R);
-    for (auto *b : {&ctx->o_ref_id, &ctx->o_pos, &ctx->o_mate_ref_id, &ctx->o_mate_pos, &ctx->o_end_pos, &ctx->o_blk_ref_pos, &ctx->o_blk_match_ref}) CK(b->grow(1, 0, st));
-    for (auto *b : {&ctx->o_flag, &ctx->o_total_len, &ctx->o_lowphred_run, &ctx->o_blk_read_pos, &ctx->o_blk_match_read}) CK(b->grow(1, 0, st));
-    CK(ctx->o_mapq.grow(1, 0, st)); CK(ctx->o_aux.grow(1, 0, st));
+#define X(T, name, ext) CK(ctx->o_##name.grow(1, 0, st));
+    SQ_BATCH_ARRAYS(X)  // (every array exists, also for an empty batch)
+#undef X
+    if (R == 0) CK(cudaMemsetAsync(ctx->o_blk_off.p, 0, 4, st));  // an empty batch still has its blk_off[0]
     point_batch_at_own_arrays(ctx, R, (int64_t)B);
     reset_batch_state(ctx, true, first_record_index, false);
     return SQG_OK;

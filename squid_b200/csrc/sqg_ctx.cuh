@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include <condition_variable>
+#include <cstddef>
 #include <functional>
 #include <map>
 #include <mutex>
@@ -118,6 +119,67 @@ struct PhaseTimer {
     bool done = false;
 };
 
+// The arrays of a concordant batch, in the order of DevBatch and sqg_batch, whose member names they share with the context's
+// own o_* buffers: X(element type, name, extent).
+enum BatchExtent { BX_REC, BX_OFF, BX_BLK };  // one per record, n_rec + 1 (blk_off), one per aligned block
+#define SQ_BATCH_ARRAYS(X)                                                                                                   \
+    X(int32_t, ref_id, BX_REC) X(int32_t, pos, BX_REC) X(int32_t, mate_ref_id, BX_REC) X(int32_t, mate_pos, BX_REC)          \
+    X(int32_t, end_pos, BX_REC) X(uint16_t, flag, BX_REC) X(uint16_t, total_len, BX_REC) X(uint16_t, lowphred_run, BX_REC)   \
+    X(uint8_t, mapq, BX_REC) X(uint8_t, aux, BX_REC) X(uint32_t, blk_off, BX_OFF) X(int32_t, blk_ref_pos, BX_BLK)            \
+    X(int32_t, blk_match_ref, BX_BLK) X(uint16_t, blk_read_pos, BX_BLK) X(uint16_t, blk_match_read, BX_BLK)
+inline size_t batch_extent(BatchExtent x, size_t n_rec, size_t n_blk) { return x == BX_REC ? n_rec : x == BX_OFF ? n_rec + 1 : n_blk; }
+
+// What the stages of a context exchange with the device in small counts and flags.  Kernels receive pointers to these fields,
+// so the adjacent pairs stay adjacent: a kernel that takes one pointer writes p[0] and p[1].
+struct Counters {
+    // classification (k_classify_tiles, k_tile_scan, k_finish_gaps)
+    int32_t totals[3], lmax;           // gap, partial and displaced records; longest first block of a concordant record
+    long long first_kept;              // initialised to n_rec
+    int32_t n_cand, ticket;            // coverage-gap candidates; next tile to classify
+    int32_t bad_flags;                 // P1Out::bad_flags
+    uint64_t end_other;                // otherChr/otherrightmost after the last record
+    int32_t wire_bad;                  // the wire decode found the batch contradicting itself (WireOut::bad)
+    // seed stage
+    int64_t n_rest;                    // ConcordRest candidates
+    int32_t n_isl, n_heavy_light[2];   // islands; those run by a whole block, by one warp
+    int64_t ops_dense[2];              // k_ops_dense: ops of the processed islands, first group not processed
+    int32_t n_prefix, seed_err;        // islands of the sequential prefix; overflow of the seed machine (1 margins, 2 output)
+    unsigned long long win_count;      // window records the groups looked at (SeedInputs::win_count)
+    // shard planner
+    int32_t n_plan_cand;
+    // phase 2 and the edge table
+    unsigned long long n_raw;          // raw (edge key, weight) pairs
+    int32_t n_sens[2];                 // sensitive concordant reads, sensitive chimeric reads
+    unsigned long long path_counts[2]; // P2Args::path_counts
+    int32_t n_slow, n_short[2];        // records left to k_edges_generic; ReadsOther blocks of <= 3 bp, those of them order-dependent
+    int32_t used_init, out_hint;       // range shards: the initial hint was used; last located segment
+    int32_t n_unique, n_chim_diff;     // rows of the edge table; chimeric blocks that LocateRead trimmed
+    // coverage
+    int32_t cov_fail, cov_redo;        // k_cov_verify: some max-plus candidate is wrong; k_cov_chain_check: chunks to replay
+    int32_t n_chunks;
+    int64_t cov_nq;                    // qualifying records.  Written on stream_cov beside the other stages, so it lies outside
+                                       // every run of fields that the main stream copies to the mirror.
+};
+// The chimeric pre-pass's counts, on its own thread and stream3: discordant blocks, PartAlignPos entries, groups
+struct PreCounters { int64_t n_disc; unsigned long long n_part; int32_t n_groups; };
+static_assert(offsetof(Counters, first_kept) % 8 == 0 && offsetof(Counters, end_other) % 8 == 0 && offsetof(Counters, n_rest) % 8 == 0 &&
+              offsetof(Counters, ops_dense) % 8 == 0 && offsetof(Counters, win_count) % 8 == 0 && offsetof(Counters, n_raw) % 8 == 0 &&
+              offsetof(Counters, path_counts) % 8 == 0 && offsetof(PreCounters, n_part) % 8 == 0, "fields that kernels write through 64-bit pointers");
+
+// A counter block: one device allocation and its pinned host mirror, allocated on first use.  zero() and to_host() take the
+// device fields *first through *last, a run in declaration order (or *first alone).  Both only enqueue: a stage reads the
+// mirror `h` after the synchronise it has anyway.
+template <class C> struct CounterBlock {
+    DBuf<C> d;
+    HBuf<C> h;
+    cudaError_t ensure() { const cudaError_t e = d.ensure(1); return e != cudaSuccess ? e : h.ensure(1); }
+    template <class A, class B> static size_t span(const A *first, const B *last) { return (const char *)(last ? (const void *)(last + 1) : (const void *)(first + 1)) - (const char *)first; }
+    template <class A, class B = A> cudaError_t zero(cudaStream_t st, A *first, B *last = nullptr) { return cudaMemsetAsync(first, 0, span(first, last), st); }
+    template <class A, class B = A> cudaError_t to_host(cudaStream_t st, const A *first, const B *last = nullptr) {
+        return cudaMemcpyAsync((char *)h.p + ((const char *)first - (const char *)d.p), first, span(first, last), cudaMemcpyDeviceToHost, st);
+    }
+};
+
 }  // namespace sq
 
 struct sqg_ctx {
@@ -139,10 +201,9 @@ struct sqg_ctx {
     bool batch_restricted = false;   // sqg_keep_records has cut the batch down to one shard's range
     int64_t first_record_index = 0;
     sq::DevBatch batch;
-    sq::DBuf<int32_t> o_ref_id, o_pos, o_mate_ref_id, o_mate_pos, o_end_pos, o_blk_ref_pos, o_blk_match_ref;
-    sq::DBuf<uint16_t> o_flag, o_total_len, o_lowphred_run, o_blk_read_pos, o_blk_match_read;
-    sq::DBuf<uint8_t> o_mapq, o_aux;
-    sq::DBuf<uint32_t> o_blk_off;
+#define X(T, name, ext) sq::DBuf<T> o_##name;
+    SQ_BATCH_ARRAYS(X)
+#undef X
     // wire-form upload (sqg_load_concordant_wire): staging of the delta-coded arrays, the copy stream and one event per chunk
     sq::DBuf<uint16_t> w_dpos, w_span, w_bdref, w_bmref, w_brpos, w_bmread;
     sq::DBuf<int16_t> w_dmate;
@@ -192,8 +253,7 @@ struct sqg_ctx {
     int64_t first_kept = 0;
     uint64_t end_other = 0;      // otherChr/otherrightmost after the last record of the batch
     sq::DBuf<unsigned char> d_temp;  // CUB temp storage
-    sq::DBuf<int64_t> d_counters;    // small device counters
-    sq::HBuf<int64_t> h_counters;
+    sq::CounterBlock<sq::Counters> cnt;
 
     // chimeric side
     bool have_chim = false, prepass_uploaded = false;
@@ -238,7 +298,7 @@ struct sqg_ctx {
     int64_t n_short_other = 0, n_unstable_other = 0; int other_sort_status = -1;
     // the chimeric pre-pass on the device (sq_prepass.cuh)
     sq::DBuf<int32_t> d_pre_ndis, d_pre_pusher, d_pre_lastk, d_pre_open; sq::DBuf<int64_t> d_pre_off; sq::DBuf<uint64_t> d_pre_part, d_pre_part2, d_pre_endkey, d_pre_excl, d_pre_incl;
-    sq::DBuf<uint8_t> d_pre_opens, dc_first_low, dc_second_low, dc_multi, d_temp3; sq::DBuf<int64_t> d_pre_cnt; sq::HBuf<int64_t> h_pre_cnt;
+    sq::DBuf<uint8_t> d_pre_opens, dc_first_low, dc_second_low, dc_multi, d_temp3; sq::CounterBlock<sq::PreCounters> pre_cnt;
     sq::PhaseTimer *prepass_timer = nullptr;
     int32_t pre_nD = 0, pre_nG = 0, pre_nP = 0;   // sizes of the pre-pass products
     sq::DBuf<sq::SeedOp> d_ops;
