@@ -13,7 +13,7 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "squid_b200", "csrc")
 OUT = os.path.join(ROOT, "squid_b200", "libsquid_b200.so")
-CU = ["sqg_api.cu"]
+CU = ["sqg_api.cu", "sqg_load.cu", "sqg_bam.cu", "sqg_prepass.cu", "sqg_classify.cu", "sqg_nodes.cu", "sqg_edges.cu", "sqg_cov.cu"]
 CPP = ["host/readrec.cpp", "host/chimeric.cpp", "host/prepass.cpp", "host/host_api.cpp", "host/plan.cpp", "host/bam.cpp", "host/exactbp.cpp", "host/writeio.cpp", "host/wire.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC,-fopenmp,-Wno-deprecated-declarations",
               "-Wno-deprecated-declarations", "-I", os.path.join(ROOT, "include"), "-I", CSRC]

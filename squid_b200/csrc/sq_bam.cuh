@@ -1,5 +1,5 @@
 // The BAM record rules, as `SQ_HD` code: the one definition the host BAM front end (host/bam.cpp), the device decoder
-// (sqg_load_concordant_bam in sqg_api.cu) and its CPU stepping (tests/emul/emul_bam.cpp) all run.
+// (sqg_load_concordant_bam in sqg_bam.cu) and its CPU stepping (tests/emul/emul_bam.cpp) all run.
 //   * Record well-formedness (bam_rec_check), aux value sizes and the XA / IH scan with BamTools' GetTag<int> semantics.
 //   * Record boundaries, whatever the writer.  A window is cut into segments at its BGZF member starts.  Per segment a
 //     speculative first record start is searched (the first offset from which a chain of plausible records reaches the

@@ -8,7 +8,7 @@
 
 #if defined(__CUDACC__)
 #define SQ_HD __host__ __device__ __forceinline__
-#define SQ_HD_NOINLINE __host__ __device__ __noinline__
+#define SQ_HD_NOINLINE __host__ __device__ __noinline__ inline  // (inline: several translation units include it)
 #else
 #define SQ_HD inline
 #define SQ_HD_NOINLINE inline

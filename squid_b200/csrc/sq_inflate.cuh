@@ -1,5 +1,5 @@
 // RFC 1951 inflate of one BGZF member and its CRC32, as `SQ_HD` rules: the device runs them one member per warp
-// (k_bam_inflate in sqg_api.cu: lane 0 decodes, the warp copies long matches), tests/emul/emul_bam.cpp steps them on the CPU
+// (k_bam_inflate in sqg_bam.cu: lane 0 decodes, the warp copies long matches), tests/emul/emul_bam.cpp steps them on the CPU
 // against zlib.  What counts as a corrupt stream is what zlib's raw inflate refuses (inflate.c / inftrees.c), because the host
 // front end (host/bam.cpp) is the yardstick: over-subscribed codes, incomplete codes except a lone 1-bit code for literals or
 // distances, a missing end-of-block code, HLIT > 286 or HDIST > 30, a repeat with no previous length or past the end, literal /

@@ -13,7 +13,6 @@
 #define SQ_PHASE2_CUH
 #include "sq_depth_cover.cuh"
 #include "sq_locate.cuh"
-#include "sq_phase1.cuh"
 #include "sq_stream.cuh"
 
 namespace sq {
@@ -295,7 +294,7 @@ __global__ void __launch_bounds__(kTileThreads, 7) k_assign_tiles(DevBatch b, P2
     }
     // ---- the multi-block records that left the tile's segment ----------------------------------------------------------------
     // They go to k_edges_generic's list.  (Measured and dropped: processing them right here with the generic rules, from the
-    // staged tile -- slower, see sqg_api.cu.  Also measured and dropped: a register-only rule set for the plain ones among them --
+    // staged tile -- slower, see sqg_edges.cu.  Also measured and dropped: a register-only rule set for the plain ones among them --
     // every block well inside one segment, nine in ten -- run here as a "pass B2": 43 M of the 53 M records of the benchmark leave
     // the list, k_edges_generic 5.4 -> 1.5 ms, this kernel 5.5 -> 9.3 ms: the same cost per record either way.)
     if (DO_EDGES) {

@@ -21,6 +21,32 @@ constexpr int kWarpsPerTile = kTileThreads / 32;
 constexpr int kTileChunks = kTile / 32;  // 32-record chunks: chunk c = records [32c, 32c+32) of the tile
 constexpr int kTileBlkCap = 1152;    // staged blocks per tile (K <= 2.2 with the 8-element alignment slack: all but ~0.1 % of the tiles at the App. C block mix, whose K varies from gene to gene); denser tiles read HBM directly
 
+// ---- what the host hands the stream kernels: the batch descriptor and the classification pass's outputs (sq_phase1.cuh),
+// which the wire upload sets up as well as the classification stage --------------------------------------------------------
+// (`desc` = device copy of the batch descriptor: taking the address of the kernel parameter would force a per-thread copy)
+struct BatchDesc { DevBatch b; Params p; };
+struct TileAgg {   // per tile: aggregate, then (after k_tile_scan) exclusive prefix
+    uint64_t okmax;
+    uint32_t n_pc, n_dp;
+};
+struct P1Out {
+    uint8_t *cls;
+    uint16_t *first_len;      // per record: length of the first kept block of a CLS_CONC record (65535 = too long for 16 bits), else 0
+    TileAgg *agg;             // n_tiles
+    uint32_t *cov_nq; uint64_t *cov_qmax;  // n_tiles: records of the tile that qualify for phase 3 (sq_phase3.cuh), their maximum start key
+    uint64_t *qstage_key; int32_t *qstage_end;  // n_rec: the (start key, fragment end) pairs of those records, compacted inside each tile:
+                                                // tile t owns [t * kTile, t * kTile + cov_nq[t]) (k_cov_gather closes the gaps)
+    int32_t *ccmax;           // n_tiles: maximum end of the ConcordantCluster entries of the tile (kNoCcEnd: none; kCcWalkTile: several chromosomes)
+    uint64_t *gate_word;      // n_tiles, zeroed: one-word chain of "1 + index of the last gate-passing record"
+    int32_t *cand_rec; uint64_t *cand_key; int32_t *n_cand; int32_t cand_cap;
+    int32_t *lmax;
+    long long *first_kept;    // initialised to n_rec
+    int32_t *bad_flags;       // 1 ref_id range, 2 mapped with ref_id -1, 4 blk_off, 8 unsorted, 16 candidate overflow
+    int32_t *ticket;
+    int32_t n_tiles;
+    const struct BatchDesc *desc;  // device copy of (batch, params) for the out-of-line HBM path
+};
+
 // ---- mbarrier + bulk copy ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {

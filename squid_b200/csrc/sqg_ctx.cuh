@@ -4,8 +4,12 @@
 #define SQG_CTX_CUH
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <chrono>
 #include <condition_variable>
 #include <cstddef>
+#include <cstdio>
+#include <cstdlib>
 #include <functional>
 #include <map>
 #include <mutex>
@@ -13,16 +17,18 @@
 #include <string>
 #include <vector>
 
+// No header reached from here defines a kernel: each stage's .cu includes the headers of its own kernels, and a kernel compiled
+// in two translation units would fail the link.
 #include "sq_bam.cuh"
 #include "sq_common.cuh"
 #include "sq_seed.cuh"
-#include "sq_phase1.cuh"
-#include "sq_phase2.cuh"
-#include "sq_phase3.cuh"
-#include "sq_plan.cuh"
+#include "sq_stream.cuh"
 #include "squid_b200.h"
 
 namespace sq {
+
+struct DepthTile;  // sq_phase2.cuh
+struct CovTile;    // sq_phase3.cuh
 
 // Device / pinned host buffers own their storage: freed by the destructor, or earlier by release().  Moves hand it over.
 template <class T> struct DBuf {
@@ -228,7 +234,7 @@ struct sqg_ctx {
     sq::DBuf<uint64_t> bam_incl, bam_nhash;
     sq::DBuf<int32_t> bam_nlen;
     sq::DBuf<uint8_t> bam_bad, bam_redo;
-    sq::DBuf<uint16_t> bam_lseq;           // read length from the CIGAR, kept only for the synthesised-quality rule (see sqg_api.cu)
+    sq::DBuf<uint16_t> bam_lseq;           // read length from the CIGAR, kept only for the synthesised-quality rule (see sqg_bam.cu)
     sq::HBuf<uint8_t> bam_stage[2];
     sq::HBuf<int64_t> bam_hsmall;
     std::vector<cudaEvent_t> bam_ev;       // [0..1]: staging buffer free again
@@ -367,4 +373,98 @@ struct sqg_ctx {
     sq::HBuf<int32_t> h_chr, h_pos, h_len, h_cnt3, h_sum3, h_ind1, h_ind2, h_w;
     sq::HBuf<uint8_t> h_heads;
 };
+
+// ---- host mechanics of every stage ----------------------------------------------------------------------------------------
+#define CK(call)                                                                                   \
+    do {                                                                                           \
+        cudaError_t e_ = (call);                                                                   \
+        if (e_ != cudaSuccess) {                                                                   \
+            ctx->err = std::string(#call) + ": " + cudaGetErrorString(e_);                         \
+            return SQG_ECUDA;                                                                      \
+        }                                                                                          \
+    } while (0)
+#define FAIL(code, msg) do { ctx->err = (msg); return (code); } while (0)
+#define LAUNCH_ON(st, kernel, grid, block, ...)                                                    \
+    do {                                                                                           \
+        kernel<<<(grid), (block), 0, (st)>>>(__VA_ARGS__);                                         \
+        ctx->launches++;                                                                           \
+        CK(cudaGetLastError());                                                                    \
+    } while (0)
+#define LAUNCH(kernel, grid, block, ...) LAUNCH_ON(ctx->stream, kernel, grid, block, __VA_ARGS__)
+
+struct HostLap {  // SQG_TIMING=1: wall-clock laps of the host side of a call, to stderr
+    bool on; std::chrono::steady_clock::time_point t0;
+    HostLap() : on(getenv("SQG_TIMING") != nullptr), t0(std::chrono::steady_clock::now()) {}
+    void operator()(const char *what) {
+        if (!on) return;
+        const auto t = std::chrono::steady_clock::now();
+        fprintf(stderr, "[sqg] %-28s %8.3f ms\n", what, 1e3 * std::chrono::duration<double>(t - t0).count());
+        t0 = t;
+    }
+};
+static constexpr int kThreads = 256;
+inline unsigned blocks_for(int64_t n, int threads = kThreads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
+
+inline int phase_begin(sqg_ctx *ctx, const char *name, cudaStream_t st = nullptr) {
+    sq::PhaseTimer &t = ctx->timers[name];
+    if (!t.a) { CK(cudaEventCreate(&t.a)); CK(cudaEventCreate(&t.b)); }
+    t.done = false;
+    CK(cudaEventRecord(t.a, st ? st : ctx->stream));
+    return SQG_OK;
+}
+inline int phase_end(sqg_ctx *ctx, const char *name, cudaStream_t st = nullptr) {
+    sq::PhaseTimer &t = ctx->timers[name];
+    CK(cudaEventRecord(t.b, st ? st : ctx->stream));
+    t.done = true;
+    return SQG_OK;
+}
+// everything that rewrites what the coverage compaction reads (batch, class bytes, chain scratch) first waits for it
+inline int cov_join(sqg_ctx *ctx) {
+    if (ctx->cov_pending) { CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_cov_done, 0)); ctx->cov_pending = false; }
+    return SQG_OK;
+}
+#define PHASE_BEGIN(name) do { int rc_ = phase_begin(ctx, name); if (rc_) return rc_; } while (0)
+#define PHASE_END(name) do { int rc_ = phase_end(ctx, name); if (rc_) return rc_; } while (0)
+// One CUB device-wide call: `call(temp, bytes)` with temp == nullptr for the size query, the scratch grown to fit, the call.
+// The scratch belongs to the stream of the call: d_temp (ctx->stream), d_temp3 (the pre-pass, stream3) and d_temp_cov
+// (stream_cov) are in use at the same time.
+template <class F> inline cudaError_t cub_call(sq::DBuf<unsigned char> &temp, F &&call) {
+    size_t bytes = 0;
+    cudaError_t e = call(nullptr, bytes);
+    if (e == cudaSuccess) e = temp.ensure(bytes + 256);
+    return e == cudaSuccess ? call(temp.p, bytes) : e;
+}
+
+struct MaxI32 { __device__ int32_t operator()(int32_t a, int32_t b) const { return a > b ? a : b; } };
+struct MaxU64 { __device__ uint64_t operator()(uint64_t a, uint64_t b) const { return a > b ? a : b; } };
+struct MaxI64 { __device__ int64_t operator()(int64_t a, int64_t b) const { return a > b ? a : b; } };
+
+inline bool batch_bulk_ok(const sq::DevBatch &b) {  // TMA bulk copies need 16-byte aligned sources
+#define X(T, name, ext) if (((uintptr_t)b.name) & 15u) return false;
+    SQ_BATCH_ARRAYS(X)
+#undef X
+    return true;
+}
+static constexpr size_t kTileSmemBytes = sizeof(sq::TileStage) + 128;
+
+// ---- what one stage calls in another --------------------------------------------------------------------------------------
+// sqg_load.cu
+void point_batch_at_own_arrays(sqg_ctx *ctx, int64_t n_rec, int64_t n_blk);
+void reset_batch_state(sqg_ctx *ctx, bool owned, int64_t first_record_index, bool wire);
+int wire_check(sqg_ctx *ctx);
+// sqg_prepass.cu
+int finish_prepass(sqg_ctx *ctx);
+// std::sort's permutation of (keys, idx)[0, n) on `st`: the device sort (sq_gpusort.cuh, its scratch grown to fit, its kernels
+// added to *launches), or, when it declines, the CPU twin on `cpu_threads` threads from the keys and payload `refill` writes
+// again, both uploaded.  *status: the device sort's verdict (0 sorted, 2 / 3 declined, < 0 CUDA error of the sort or its scratch).
+cudaError_t replay_std_sort(uint64_t *keys, uint32_t *idx, size_t n, sq::DBuf<unsigned char> &scratch, cudaStream_t st, int64_t *launches, int cpu_threads,
+                            const std::function<cudaError_t()> &refill, int *status);
+// sqg_classify.cu
+int classify_setup(sqg_ctx *ctx, int64_t cand_cap, sq::P1Out &o);
+int classify_launch(sqg_ctx *ctx, const sq::P1Out &o, int64_t tiles);
+int run_classify(sqg_ctx *ctx);
+// sqg_edges.cu
+int run_assign(sqg_ctx *ctx, bool do_depth, bool do_edges);
+// sqg_cov.cu
+int run_cov_compact(sqg_ctx *ctx);
 #endif

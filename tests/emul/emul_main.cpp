@@ -245,7 +245,7 @@ int main(int argc, char **argv) {
     for (int32_t c = n_ref - 1; c >= 0; c--) if (chr_first[c] == N && c + 1 <= n_ref) chr_first[c] = chr_first[c + 1];
     NodeTable nt;
     nt.n = N; nt.n_ref = n_ref; nt.chr = nchr.data(); nt.pos = npos.data(); nt.end = nend.data(); nt.chr_first = chr_first.data();
-    // coarse position index, as sqg_api.cu builds it (a small shift makes every branch of seg_at run on the test cases)
+    // coarse position index, as sqg_nodes.cu builds it (a small shift makes every branch of seg_at run on the test cases)
     std::vector<int32_t> bin_off(n_ref + 1, 0), bin_seg;
     nt.bin_shift = getenv("SQ_EMUL_BIN_SHIFT") ? atoi(getenv("SQ_EMUL_BIN_SHIFT")) : 12;
     if (nt.bin_shift > 0) {

@@ -3,7 +3,7 @@
 //   seg_index_check TABLE BIN_SHIFT FORM
 //
 // TABLE: int32 n_ref, ref_len[n_ref], then rows (chr, pos, len) sorted by chromosome that tile each chromosome.  The index is
-// built in FORM "packed" (headers and bin entries, as sqg_api.cu builds it for the device) or "plain" (chr_first, bin_off,
+// built in FORM "packed" (headers and bin entries, as sqg_nodes.cu builds it for the device) or "plain" (chr_first, bin_off,
 // bin_seg, as the CPU stepping harness builds it); BIN_SHIFT 0: no bins, the binary-search fallback.  For every position of every
 // chromosome and a few positions past both ends, every lookup is compared with its definition over the plain arrays
 // (std::upper_bound / std::lower_bound).  Prints the number of positions checked and exits 1 on the first mismatch.
